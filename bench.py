@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port) on the host cores
+  python bench.py --steps K --warmup W --dump-outputs DIR  # ... and write what the last timed step returned as DIR/*.npy
 
 Headline (`value`, every N): BASELINE.json configs[1] -- synthetic 4-bodypart reaching video, 747x832, estimate_pose
 inference.  A "step" is one pass of the hot path over one batch of frames: ResNet-50 OS16 scoremap net + part_pred deconv
@@ -30,6 +31,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (no __pycache__ of the modules it imports)
 
 H, W, NJ = 747, 832, 4
 METRIC = "frames/sec (ResNet-50 scoremap + DGP soft-argmax/potentials)"
@@ -296,7 +298,7 @@ def measure_device(wl, steps, warmup, world, local_rank, profile=True):
     torch.cuda.synchronize()
     e0.record()
     for i in range(steps):
-        wl.step(i, world)
+        outputs = wl.step(i, world)
     e1.record()
     torch.cuda.synchronize()
     barrier(world)
@@ -310,7 +312,7 @@ def measure_device(wl, steps, warmup, world, local_rank, profile=True):
         prof = wl.eng.get_profile()
         ms_prof = ms_local
     return {"ms": ms, "launches": launches, "clocks": clocks, "prof": prof, "ms_prof": ms_prof,
-            "value": world * wl.B * steps / (ms / 1e3)}
+            "value": world * wl.B * steps / (ms / 1e3), "outputs": outputs}
 
 
 def measure_e2e(wl, frames_per_gpu, world):
@@ -365,55 +367,19 @@ def check_sharded_equals_single(wl, res, world, rank, k=8):
             "what": "mu, integer peaks, likelihoods, skeleton distances, temporal potentials across the shard edge; bit for bit"}
 
 
-def traffic_child(args):
-    """Body of the ncu child process (bench.py --traffic-child): two plain steps of the headline workload, nothing timed."""
-    wl = Workload(args.config, 0, 0, args.precision, args.batch)
-    for i in range(2):
-        wl.step(i, 1)
-    torch.cuda.synchronize()
-    wl.close()
+def dump_outputs(outputs, out_dir):
+    """Write the arrays one step returned (soft-argmax read-out and potentials) as out_dir/<name>.npy: float32 arrays as
+    they are, integer ones (the peaks) as float64, which holds them exactly."""
+    out, pot = outputs
+    arrays = dict(out)
+    arrays.update({k: v for k, v in pot.items() if not k.startswith("_") and v is not None})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in sorted(arrays.items()):
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
-def measure_traffic_ncu(args, B, gemm_per_step, timeout_s=240):
-    """DRAM bytes per conv_gemm launch measured IN this run: rank 0 re-runs two steps of the workload in a child process under
-    `ncu --metrics dram__bytes_read.sum,dram__bytes_write.sum -k regex:conv_gemm_kernel` (after the timed regions; nothing
-    timed runs under the profiler) and averages the launches of the second step.  Returns (bytes per launch | None, note)."""
-    import csv
-    import shutil
-    import subprocess
-    import tempfile
-    ncu = shutil.which("ncu") or "/usr/local/cuda/bin/ncu"
-    if not os.path.exists(ncu):
-        return None, "ncu not found on this box"
-    with tempfile.TemporaryDirectory() as td:
-        log = os.path.join(td, "dram.csv")
-        cmd = [ncu, "--metrics", "dram__bytes_read.sum,dram__bytes_write.sum", "--clock-control", "none", "-k",
-               "regex:conv_gemm_kernel", "--csv", "--log-file", log, sys.executable, os.path.abspath(__file__), "--traffic-child",
-               "--config", args.config, "--precision", args.precision, "--batch", str(B)]
-        env = {k: v for k, v in os.environ.items() if k not in ("RANK", "LOCAL_RANK", "WORLD_SIZE", "MASTER_ADDR", "MASTER_PORT")}
-        try:
-            r = subprocess.run(cmd, stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, timeout=timeout_s, env=env)
-        except subprocess.TimeoutExpired:
-            return None, "ncu child exceeded %d s" % timeout_s
-        if r.returncode != 0 or not os.path.exists(log):
-            return None, "ncu child failed (rc %d): %s" % (r.returncode, r.stderr.decode(errors="replace")[-200:].replace("\n", " "))
-        scale = {"byte": 1.0, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9}
-        per_launch = {}
-        with open(log) as f:
-            for row in csv.DictReader(l for l in f if not l.startswith("==")):
-                if row.get("Metric Name") in ("dram__bytes_read.sum", "dram__bytes_write.sum"):
-                    v = float(row["Metric Value"].replace(",", "")) * scale.get(row.get("Metric Unit", "byte"), 1.0)
-                    per_launch[int(row["ID"])] = per_launch.get(int(row["ID"]), 0.0) + v
-    ids = sorted(per_launch)
-    if len(ids) < 2 * gemm_per_step:
-        return None, "ncu child reported %d conv_gemm launches, expected %d" % (len(ids), 2 * gemm_per_step)
-    last = ids[-gemm_per_step:]
-    return sum(per_launch[i] for i in last) / gemm_per_step, (
-        "dram__bytes_read.sum + dram__bytes_write.sum per conv_gemm launch, measured in this run: the %d GEMM launches of one "
-        "step (B=%d) re-run in a child process under ncu (--clock-control none) after the timed regions" % (gemm_per_step, B))
-
-
-def roofline_of(wl, m, steps, peaks, peak_src, args=None):
+def roofline_of(wl, m, steps, peaks, peak_src):
     prof = m["prof"]
     gemm_ms, gemm_n = prof["conv_gemm"]
     frames_timed = wl.B * steps
@@ -421,16 +387,7 @@ def roofline_of(wl, m, steps, peaks, peak_src, args=None):
     peak_tf = peaks.get("bf16_tflops_sustained", peaks.get("bf16_tflops"))
     traffic, traffic_note = None, "no ncu --set full capture of the current kernel sources under profiles/"
     tpath = os.path.join(ROOT, "profiles", "r02_traffic.json")
-    min_bytes = None
-    if os.path.exists(tpath):
-        with open(tpath) as f:
-            min_bytes = json.load(f).get("minimum_bytes_per_frame_16bit")
-    if args is not None and not args.no_ncu_traffic and gemm_n > 0:
-        traffic, traffic_note = measure_traffic_ncu(args, wl.B, gemm_n // steps)
-        if traffic is not None and min_bytes and wl.key == "b":
-            traffic_note += "; algorithmic minimum %.0f MB/launch" % (min_bytes * wl.B / (gemm_n // steps) / 1e6)
-    if traffic is None and os.path.exists(tpath) and wl.key == "b":
-        live_note = traffic_note
+    if os.path.exists(tpath) and wl.key == "b":
         with open(tpath) as f:
             tj = json.load(f)
         if tj.get("csrc_sha") == csrc_sha():
@@ -441,8 +398,6 @@ def roofline_of(wl, m, steps, peaks, peak_src, args=None):
                                tj["minimum_bytes_per_frame_16bit"] * wl.B / tj["gemm_launches_per_step"] / 1e6))
         else:
             traffic_note = "profiles/r02_traffic.json describes other kernel sources (csrc sha %s != %s): not quoted" % (tj.get("csrc_sha"), csrc_sha())
-        if args is not None and not args.no_ncu_traffic:
-            traffic_note = "in-run ncu measurement unavailable (%s); %s" % (live_note, traffic_note)
     return {"bound": "tensor", "kernel": "conv_gemm_kernel (tcgen05 implicit GEMM, %d launches)" % gemm_n,
             "achieved": achieved_tf, "peak": peak_tf, "unit": "TFLOP/s",
             "frac": (achieved_tf / peak_tf) if achieved_tf else None, "traffic": traffic, "traffic_note": traffic_note,
@@ -501,10 +456,12 @@ def main():
     ap.add_argument("--precision", default=PRECISION, choices=["fp16", "bf16"])
     ap.add_argument("--e2e-frames", type=int, default=10000, help="frames per GPU of the end-to-end video (configs[1]: 10 k)")
     ap.add_argument("--cpu-frames", type=int, default=64, help="frames of the workload the CPU baseline times (about 10 s on 16 cores)")
-    ap.add_argument("--no-ncu-traffic", action="store_true",
-                    help="do not measure roofline.traffic with an ncu child process (falls back to profiles/r02_traffic.json)")
-    ap.add_argument("--traffic-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline returned as DIR/<name>.npy (rank 0's frames); "
+                         "the same arguments give the same inputs, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     global H, W, NJ, WORKLOAD
@@ -517,10 +474,6 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         run_reference(args, rank)
-        return
-    if args.traffic_child:
-        torch.cuda.set_device(0)
-        traffic_child(args)
         return
 
     import torch.distributed as dist
@@ -537,10 +490,11 @@ def main():
     sa_fill = softargmax_roofline(local_rank, peaks) if (rank == 0 and not args.no_aux) else None
     wl = Workload(args.config, local_rank, rank, args.precision, args.batch)
     m = measure_device(wl, args.steps, args.warmup, world, local_rank)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(m["outputs"], args.dump_outputs)
     res, e2e = measure_e2e(wl, args.e2e_frames, world)
     finite = bool(np.isfinite(res["x"]).all())
-    # roofline.traffic is measured in the run by an ncu child process at N = 1 (at N > 1 the other ranks would wait on it)
-    roof = roofline_of(wl, m, args.steps, peaks, peak_src, args if world == 1 else None) if rank == 0 else None
+    roof = roofline_of(wl, m, args.steps, peaks, peak_src) if rank == 0 else None
     sa_ms, sa_n = m["prof"]["softargmax"]
     fam = {k: v[0] for k, v in m["prof"].items()}
     B = wl.B

@@ -5,7 +5,7 @@ set -u
 R=${1:-r02}
 O=gpurun_out
 mkdir -p $O
-B="python bench.py --steps 1 --warmup 3 --no-aux --no-train --no-cpu-baseline --no-ncu-traffic --e2e-frames 62"
+B="python bench.py --steps 1 --warmup 3 --no-aux --no-train --no-cpu-baseline --e2e-frames 62"
 # 1. bench line (not under a profiler)
 timeout 900 python bench.py 2>$O/bench_${R}.err | tail -1 > $O/${R}_bench_1gpu.json
 # 2. in-step per-layer table (events between launches) at the clocks / power state of the real step
