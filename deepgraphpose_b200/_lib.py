@@ -66,6 +66,7 @@ SIGNATURES = {
     "dgp_last_error": (C.c_char_p, [_vp]),
     "dgp_load_weights": (_i, [_vp, C.c_char_p, _vp, _i64p, _i, _i]),
     "dgp_finalize_weights": (_i, [_vp]),
+    "dgp_net_depth": (_i, [_vp, C.POINTER(_i)]),
     "dgp_output_dims": (_i, [_i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
     "dgp_forward": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "dgp_extract_features": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),

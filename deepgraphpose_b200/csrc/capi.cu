@@ -158,7 +158,7 @@ int build_conv_layer(dgp_handle* h, const std::string& scope, int R, int S, int 
 // conv1: 7x7 stride 2 on 3 channels == 4x4 stride-1 conv on the 2x2 space-to-depth image (12 -> 16 channels);
 // one TMA "pixel" is a window of 4 horizontally adjacent s2d pixels (64 channels), the 4 window rows are the taps.
 int build_conv1_layer(dgp_handle* h) {
-  const std::string scope = "resnet_v1_50/conv1";
+  const std::string scope = h->net_scope + "/conv1";
   const HostVar* w = find_var(h, scope + "/weights");
   if (!w) return fail(h, DGP_ERR_STATE, "missing variable %s/weights", scope.c_str());
   if (w->shape.size() != 4 || w->shape[0] != 7 || w->shape[1] != 7 || w->shape[2] != 3 || w->shape[3] != 64)
@@ -602,7 +602,7 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
     st.kind = STEP_GEMM;
     if (unfused) {
       st.out_ptr = c1;
-      st.end_point = "resnet_v1_50/conv1";
+      st.end_point = h->net_scope + "/conv1";
       st.oN = B; st.oH = pl->H1; st.oW = pl->W1; st.oC = 64;
     } else {
       st.out_ptr = xa;
@@ -614,7 +614,7 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
     Step st; st.kind = STEP_POOL;
     st.pin = (const __nv_bfloat16*)c1; st.pN = B; st.pH = pl->H1; st.pW = pl->W1; st.pC = 64; st.pad_t = pad_t; st.pad_l = pad_l;
     st.out_ptr = xa;
-    st.end_point = "resnet_v1_50/pool1";
+    st.end_point = h->net_scope + "/pool1";
     st.oN = B; st.oH = Hc; st.oW = Wc; st.oC = 64;
     pl->steps.push_back(st);
   }
@@ -879,19 +879,41 @@ int dgp_finalize_weights(dgp_handle* h) {
   if (!h) return DGP_ERR_INVALID;
   if (h->finalized) return fail(h, DGP_ERR_STATE, "weights already finalized");
   CU_OK(h, cudaSetDevice(h->device));
+  // The backbone is the one the variable names describe (as Saver.restore works off names): slim's resnet_v1_50 / _101 /
+  // _152 differ only in the number of units of blocks 2 and 3; every layer of the deeper nets has a ResNet-50 shape.
+  static const struct { const char* scope; int depth, units[4]; } nets[3] = {
+      {"resnet_v1_50", 50, {3, 4, 6, 3}}, {"resnet_v1_101", 101, {3, 4, 23, 3}}, {"resnet_v1_152", 152, {3, 8, 36, 3}}};
+  std::string scope;
+  for (const auto& kv : h->host_vars) {
+    if (kv.first.compare(0, 10, "resnet_v1_") != 0) continue;
+    const std::string p = kv.first.substr(0, kv.first.find('/'));
+    if (scope.empty()) scope = p;
+    else if (p != scope)
+      return fail(h, DGP_ERR_INVALID, "the weights mix the backbone scopes %s and %s", scope.c_str(), p.c_str());
+  }
+  const int* units = nullptr;
+  for (const auto& n : nets)
+    if (scope == n.scope) { h->depth = n.depth; units = n.units; }
+  if (!units) {
+    if (scope.empty())
+      return fail(h, DGP_ERR_INVALID, "no backbone variables: expected names under resnet_v1_50/, resnet_v1_101/ or resnet_v1_152/");
+    return fail(h, DGP_ERR_INVALID, "unsupported backbone scope %s (resnet_v1_50, resnet_v1_101 or resnet_v1_152)", scope.c_str());
+  }
+  h->net_scope = scope;
   int rc = build_conv1_layer(h);
   if (rc) return rc;
-  // slim resnet_v1_50 + stack_blocks_dense(output_stride=16): see oracle/resnet_v1.py::unit_plan
-  static const struct { const char* name; int base, units, stride; } blocks[4] = {
-      {"block1", 64, 3, 2}, {"block2", 128, 4, 2}, {"block3", 256, 6, 2}, {"block4", 512, 3, 1}};
+  // slim resnet_v1_<depth> + stack_blocks_dense(output_stride=16): see oracle/resnet_v1.py::unit_plan
+  static const struct { const char* name; int base, stride; } blocks[4] = {
+      {"block1", 64, 2}, {"block2", 128, 2}, {"block3", 256, 2}, {"block4", 512, 1}};
   int cin = 64, current_stride = 1, rate = 1;
   const int target = 4;
-  for (const auto& b : blocks)
-    for (int u = 0; u < b.units; ++u) {
-      const int ustride = (u == b.units - 1) ? b.stride : 1;
+  for (int bi = 0; bi < 4; ++bi) {
+    const auto& b = blocks[bi];
+    for (int u = 0; u < units[bi]; ++u) {
+      const int ustride = (u == units[bi] - 1) ? b.stride : 1;
       UnitDesc ud;
       char sc[128];
-      snprintf(sc, sizeof(sc), "resnet_v1_50/%s/unit_%d/bottleneck_v1", b.name, u + 1);
+      snprintf(sc, sizeof(sc), "%s/%s/unit_%d/bottleneck_v1", scope.c_str(), b.name, u + 1);
       ud.scope = sc; ud.depth = b.base * 4; ud.base = b.base;
       if (current_stride == target) { ud.stride = 1; ud.rate = rate; rate *= ustride; }
       else { ud.stride = ustride; ud.rate = 1; current_stride *= ustride; }
@@ -905,10 +927,18 @@ int dgp_finalize_weights(dgp_handle* h) {
       cin = ud.depth;
       h->units.push_back(ud);
     }
+  }
   if ((rc = build_head_layer(h))) return rc;
   if ((rc = upload_arena(h))) return rc;
   h->host_vars.clear();
   h->finalized = true;
+  return DGP_OK;
+}
+
+int dgp_net_depth(const dgp_handle* h, int* depth) {
+  if (!h || !depth) return DGP_ERR_INVALID;
+  if (!h->finalized) return fail(const_cast<dgp_handle*>(h), DGP_ERR_STATE, "dgp_net_depth before dgp_finalize_weights");
+  *depth = h->depth;
   return DGP_OK;
 }
 

@@ -80,6 +80,7 @@ struct DgradWJob {
   int Cout, taps, Cin;
   int tile_start;
 };
+constexpr int kDgradWMaxJobs = 256;  // build_dgrad_w_kernel looks a block's job up with one thread per job (256 threads)
 cudaError_t launch_build_dgrad_w(const DgradWJob* jobs_dev, int njobs, int total_tiles, const float* master,
                                  const float* scale_arena, int fp16, cudaStream_t s);
 cudaError_t launch_build_head_dgrad_w(const float* wh, int rows, int C, void* whT, int Kd, int fp16, cudaStream_t s);

@@ -38,9 +38,9 @@ __global__ void __launch_bounds__(256) build_dgrad_w_kernel(const DgradWJob* __r
                                                             const float* __restrict__ master,
                                                             const float* __restrict__ scale_arena, int fp16) {
   __shared__ float tile[32][33];
-  // all layers in ONE launch: a block finds its layer from the prefix of 32x32-tile counts (<= 52 entries, ascending, first
-  // one 0).  Thread t tests entry t and the block counts the hits -- one load latency instead of a serial walk of up to 52
-  // dependent loads per block (that walk was most of this kernel's 90 us).
+  // all layers in ONE launch: a block finds its layer from the prefix of 32x32-tile counts (<= kDgradWMaxJobs entries,
+  // ascending, first one 0; 52 at ResNet-50, 154 at ResNet-152).  Thread t tests entry t and the block counts the hits -- one
+  // load latency instead of a serial walk of up to njobs dependent loads per block (that walk was most of this kernel's 90 us).
   const int hit = (int)threadIdx.x < njobs && (int)blockIdx.x >= jobs[threadIdx.x].tile_start;
   const int job = __syncthreads_count(hit) - 1;
   const DgradWJob jb = jobs[job];
@@ -156,7 +156,7 @@ cudaError_t launch_refresh_bn(const float* gamma, const float* beta, const float
 cudaError_t launch_build_dgrad_w(const DgradWJob* jobs_dev, int njobs, int total_tiles, const float* master,
                                  const float* scale_arena, int fp16, cudaStream_t s) {
   if (njobs < 1 || total_tiles < 1) return cudaSuccess;
-  if (njobs > 256) return cudaErrorInvalidValue;   // the kernel's job lookup is one thread per job
+  if (njobs > kDgradWMaxJobs) return cudaErrorInvalidValue;   // the kernel's job lookup is one thread per job
   build_dgrad_w_kernel<<<total_tiles, 256, 0, s>>>(jobs_dev, njobs, master, scale_arena, fp16);
   return cudaGetLastError();
 }

@@ -1,4 +1,5 @@
-// Training step of fit_dgp on the GPU: network backward (dgrad / wgrad of the 53 convs + deconv heads), frozen-BN
+// Training step of fit_dgp on the GPU: network backward (dgrad / wgrad of the 53 / 104 / 155 convs of
+// ResNet-50 / 101 / 152 + deconv heads), frozen-BN
 // parameter gradients, global-norm clipping and the Momentum update.
 // Reference: src/deepgraphpose/models/fitdgp.py:706-713
 //   optimizer = MomentumOptimizer(lr, 0.9); grads = compute_gradients(total_loss, TF.trainable_variables());
@@ -49,7 +50,7 @@ struct Backward {
   float *g_logits = nullptr, *g_locref = nullptr;
   // Deferred frozen-BN gradients: every mask site leaves its per-row-block sums of dy in its own region of `bn_part`, every
   // wgrad its <W, dW_raw> products in its slice of `rowdot`; ONE kernel at the end of the backward turns both into dbeta / dgamma
-  // for all 26 k channels (instead of ~100 latency-bound launches of 3-7 us each inside the pass).
+  // for every channel (26 560 at ResNet-50, 75 712 at ResNet-152; instead of ~100 latency-bound launches of 3-7 us each inside the pass).
   float* bn_part = nullptr;
   float* rowdot = nullptr;
   BnGroup* bn_table = nullptr;
@@ -603,6 +604,9 @@ int dgp_train_enable(dgp_handle* h) {
     ts->wd_tiles += (L.Cin / 32) * (L.Cout / 32) * L.R * L.S;
     jobs.push_back(jb);
   }
+  if (jobs.size() > (size_t)kDgradWMaxJobs)
+    return fail(h, DGP_ERR_UNSUPPORTED, "%zu conv layers exceed the %d of the one-launch dgrad operand rebuild", jobs.size(),
+                kDgradWMaxJobs);
   ts->n_wd_jobs = (int)jobs.size();
   CU_OK(h, cudaMalloc(&ts->wd_jobs, jobs.size() * sizeof(DgradWJob)));
   CU_OK(h, cudaMemcpy(ts->wd_jobs, jobs.data(), jobs.size() * sizeof(DgradWJob), cudaMemcpyHostToDevice));

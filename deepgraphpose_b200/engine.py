@@ -24,12 +24,13 @@ def output_dims(H, W):
     return (a.value, b.value), (c.value, d.value)
 
 
-def suggest_batch(H, W, lo=24, hi=48, num_sms=148):
+def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3)):
     """Frames per batch that minimise wave quantisation of the persistent conv-GEMM grid (one CTA per SM).
 
     Every GEMM layer runs ceil(B*pixels/tile_rows) * n_blocks tiles on `num_sms` CTAs; a batch size for which the
     dominant layers' tile counts are (just under) a multiple of the SM count avoids a nearly empty last wave.  Layers are
-    weighted by their roofline bound (max of bf16 tensor time and HBM time), tile shapes follow csrc/capi.cu."""
+    weighted by their roofline bound (max of bf16 tensor time and HBM time), tile shapes follow csrc/capi.cu.  ``units``: the
+    bottleneck units per block of the backbone (ResNet-50 by default; synthetic.BLOCK_UNITS for the others)."""
     c2 = lambda v: -(-v // 2)
     layers = []  # (pixels per frame, tile rows, n_blocks, weight)
     hh, ww = c2(H), c2(W)
@@ -41,9 +42,9 @@ def suggest_batch(H, W, lo=24, hi=48, num_sms=148):
     add(hh * ww, 256, 64, 32 + 128)
     hh, ww = c2(hh), c2(ww)
     cin = 64
-    for base, units, bstride in ((64, 3, 2), (128, 4, 2), (256, 6, 1), (512, 3, 1)):
-        for u in range(units):
-            s_ = bstride if u == units - 1 else 1
+    for base, n_units, bstride in zip((64, 128, 256, 512), units, (2, 2, 1, 1)):
+        for u in range(n_units):
+            s_ = bstride if u == n_units - 1 else 1
             depth = 4 * base
             ho, wo = (c2(hh), c2(ww)) if s_ == 2 else (hh, ww)
             if cin != depth:
@@ -115,6 +116,7 @@ class Engine:
         check(self.lib.dgp_create(C.byref(cfg), C.byref(h)))
         self.h = h
         self.weights_loaded = False
+        self.net_type = None  # "resnet_50" / "resnet_101" / "resnet_152": the backbone the loaded weights name
 
     def close(self):
         if getattr(self, "h", None):
@@ -139,6 +141,9 @@ class Engine:
             self._check(self.lib.dgp_load_weights(self.h, name.encode(), a.ctypes.data_as(C.c_void_p), shape, a.ndim, 0))
         self._check(self.lib.dgp_finalize_weights(self.h))
         self.weights_loaded = True
+        depth = C.c_int()
+        self._check(self.lib.dgp_net_depth(self.h, C.byref(depth)))
+        self.net_type = "resnet_%d" % depth.value
         # the frozen moving statistics are not trainable state of the handle; keep them for checkpoint export
         self._frozen = {k: np.array(v, dtype=np.float32) for k, v in variables.items()
                         if k.endswith("/moving_mean") or k.endswith("/moving_variance")}
@@ -456,10 +461,10 @@ class Engine:
         self._check(self.lib.dgp_set_variable(self.h, name.encode(), code, a.ctypes.data_as(C.c_void_p), a.size))
 
     def variable_names(self):
-        """TF names of every trainable variable of the graph (slim resnet_v1_50 + the deconv heads)."""
-        from .synthetic import resnet50_conv_specs
+        """TF names of every trainable variable of the graph (slim resnet_v1_<depth> of the loaded weights + the deconv heads)."""
+        from .synthetic import conv_specs
         names = []
-        for scope, *_ in resnet50_conv_specs():
+        for scope, *_ in conv_specs(self.net_type):
             names += [scope + "/weights", scope + "/BatchNorm/gamma", scope + "/BatchNorm/beta"]
         for head in ["part_pred"] + (["locref_pred"] if self.location_refinement else []):
             names += ["pose/%s/block4/weights" % head, "pose/%s/block4/biases" % head]

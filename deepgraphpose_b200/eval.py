@@ -21,40 +21,56 @@ def _cfg_get(cfg, key, default=None):
     return getattr(cfg, key, default)
 
 
-def load_variables(dgp_model_file, num_joints, location_refinement):
+def load_variables(dgp_model_file, num_joints, location_refinement, net_type="resnet_50"):
     """Weights for the graph.  Accepts a ``{tf_var_name: ndarray}`` dict, a ``.npz`` of such arrays, or
-    ``"synthetic"`` / ``"synthetic:<seed>"`` (random-init weights, BASELINE.json configs), or the prefix of a TensorFlow
-    checkpoint bundle (``snapshot-step2-final--0`` -> ``.index`` + ``.data-0000N-of-0000M``, read by tf_checkpoint.py)."""
+    ``"synthetic"`` / ``"synthetic:<seed>"`` (random-init weights of ``net_type``, BASELINE.json configs), or the prefix of a
+    TensorFlow checkpoint bundle (``snapshot-step2-final--0`` -> ``.index`` + ``.data-0000N-of-0000M``, read by
+    tf_checkpoint.py)."""
     if isinstance(dgp_model_file, dict):
         return dgp_model_file
     name = str(dgp_model_file)
     if name.startswith("synthetic"):
         seed = int(name.split(":")[1]) if ":" in name else 0
-        return synthetic.make_weights(num_joints, seed=seed, location_refinement=location_refinement)
+        return synthetic.make_weights(num_joints, seed=seed, location_refinement=location_refinement, net_type=net_type)
     if name.endswith(".npz") and os.path.exists(name):
         with np.load(name) as z:
             return {k: z[k] for k in z.files}
     prefix = name[:-6] if name.endswith(".index") else name
     if os.path.exists(prefix + ".index"):
-        # a TensorFlow checkpoint bundle (DLC / DGP snapshot, resnet_v1_50.ckpt): restorer.restore without TensorFlow
+        # a TensorFlow checkpoint bundle (DLC / DGP snapshot, resnet_v1_{50,101,152}.ckpt): restorer.restore without TensorFlow
         from . import tf_checkpoint
         return tf_checkpoint.model_variables(tf_checkpoint.read_checkpoint(prefix))
     raise FileNotFoundError("no weights at %r: pass a {tf_var_name: ndarray} dict, an .npz of it, 'synthetic[:seed]', or the "
                             "prefix of a TensorFlow checkpoint (<prefix>.index + <prefix>.data-*)" % (name,))
 
 
+def check_net_type(net_type, variables):
+    """The backbone of ``variables`` (from their slim scope); ValueError if ``net_type`` (a dlc_cfg's, None = follow the
+    weights) names another one or is not resnet_50 / resnet_101 / resnet_152."""
+    if net_type is not None:
+        synthetic.net_scope(net_type)
+    found = synthetic.net_type_of(variables)
+    if net_type is not None and found != net_type:
+        raise ValueError("dlc_cfg net_type is %r but the weights hold %r (%s/...)" % (net_type, found, synthetic.net_scope(found)))
+    return found
+
+
 def setup_dgp_eval_graph(dlc_cfg, dgp_model_file, loc_ref=False, gauss_len=1, gamma=1, device=None):
-    """eval.py:147-214.  Returns (sess, mu_n, softmax_tensor, scmap, locref, inputs)."""
+    """eval.py:147-214.  Returns (sess, mu_n, softmax_tensor, scmap, locref, inputs).  ``dlc_cfg.net_type`` (resnet_50,
+    resnet_101 or resnet_152) must match the backbone the weights name; without it the weights decide."""
+    return _setup_eval_graph(dlc_cfg, dgp_model_file, _cfg_get(dlc_cfg, "net_type"), loc_ref, gauss_len, gamma, device)
+
+
+def _setup_eval_graph(dlc_cfg, dgp_model_file, net_type, loc_ref=False, gauss_len=1, gamma=1, device=None):
     nj = int(_cfg_get(dlc_cfg, "num_joints"))
-    net_type = _cfg_get(dlc_cfg, "net_type", "resnet_50")
-    if net_type != "resnet_50":
-        raise ValueError("only net_type='resnet_50' is on the B200 path (got %r)" % (net_type,))
+    variables = load_variables(dgp_model_file, nj, bool(loc_ref), net_type or "resnet_50")
+    check_net_type(net_type, variables)
     eng = Engine(nj, location_refinement=bool(loc_ref), device=device,
                  stride=float(_cfg_get(dlc_cfg, "stride", 8.0)),
                  locref_stdev=float(_cfg_get(dlc_cfg, "locref_stdev", 7.2801)),
                  mean_pixel=tuple(_cfg_get(dlc_cfg, "mean_pixel", (123.68, 116.779, 103.939))),
                  precision=_cfg_get(dlc_cfg, "precision", "fp16"))
-    eng.load_weights(load_variables(dgp_model_file, nj, bool(loc_ref)))
+    eng.load_weights(variables)
     handles = {
         "inputs": Handle("Placeholder:0", "inputs"),
         "mu_n": Handle("Sum:0", "mu_n"),
@@ -222,7 +238,9 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
     """eval.py:217-372.  ``proj_cfg_file`` may be a dict-like dlc_cfg (num_joints, stride, ...) or a DLC project yaml with
     ``bodyparts``; ``video_file`` a path or a uint8 array (T,H,W,3).  Returns {'x','y','likelihoods'} (T,nj) each.
     A video file is STREAMED: decoded frame by frame (as the reference's ``clip.iter_frames()``, eval.py:306) into a pinned
-    ring that the GPU drains batch by batch, so a 100 k-frame clip needs no more host memory than a 100-frame one."""
+    ring that the GPU drains batch by batch, so a 100 k-frame clip needs no more host memory than a 100-frame one.
+    The backbone (ResNet-50, -101 or -152) is the one the weights' names describe, as the reference's estimate_pose tries
+    each snapshot scope (eval.py:271-276)."""
     if isinstance(proj_cfg_file, (dict,)) or hasattr(proj_cfg_file, "num_joints"):
         dlc_cfg = proj_cfg_file
     else:
@@ -239,7 +257,7 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
             print("labels already exist! video at %s will not be processed" % video_file)
             return save_file + ".csv"
         source, H, W, n_frames, scale_x, scale_y = _video_source(video_file, new_size, crop_size)
-        sess, mu_n, _, scmap, _, inputs = setup_dgp_eval_graph(dlc_cfg, dgp_model_file)
+        sess, mu_n, _, scmap, _, inputs = _setup_eval_graph(dlc_cfg, dgp_model_file, None)
         # the container's frame count is a hint only (it can be off by a few frames): read until the decoder runs dry
         res = estimate_pose_stream(sess.engine, source, H, W, None, batch=batch)
     else:
@@ -257,7 +275,7 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
                     im = im.crop(crop_size)
                 out.append(np.asarray(im))
             frames = np.stack(out)
-        sess, mu_n, _, scmap, _, inputs = setup_dgp_eval_graph(dlc_cfg, dgp_model_file)
+        sess, mu_n, _, scmap, _, inputs = _setup_eval_graph(dlc_cfg, dgp_model_file, None)
         res = estimate_pose_frames(sess.engine, frames, batch=batch)
     sess.close()
     labels = {"x": res["x"] * scale_x, "y": res["y"] * scale_y, "likelihoods": res["likelihoods"]}

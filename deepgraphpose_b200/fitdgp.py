@@ -208,7 +208,7 @@ def dgp_loss(data_batcher, dgp_cfg, variables=None, device=None):
                  locref_stdev=float(_get(dgp_cfg, "locref_stdev", 7.2801)),
                  mean_pixel=tuple(_get(dgp_cfg, "mean_pixel", (123.68, 116.779, 103.939))),
                  precision=_get(dgp_cfg, "precision", "fp16"))
-    eng.load_weights(load_variables(variables, nj, True))
+    eng.load_weights(load_variables(variables, nj, True, _get(dgp_cfg, "net_type", "resnet_50")))
     graph = SimpleNamespace(engine=eng, cfg=dgp_cfg, edges=skeleton_edges(S0) if S0.shape[0] else [], ws=ws, ws_max=ws_max,
                             n_frames_total=float(data_batcher.n_frames_total),
                             n_visible_frames_total=float(data_batcher.n_visible_frames_total))

@@ -12,7 +12,9 @@ import ctypes as C
 import numpy as np
 import torch
 
+from . import synthetic
 from .engine import Engine, LOCREF_STDEV, MEAN_PIXEL, STRIDE, _ptr, _stream
+from .eval import check_net_type
 
 
 def _get(cfg, key, default=None):
@@ -56,8 +58,8 @@ class PoseNet:
         self.cfg = cfg
         if _get(cfg, "output_stride", 16) != 16 or _get(cfg, "deconvolutionstride", 2) != 2:
             raise ValueError("the B200 path implements output_stride=16, deconvolutionstride=2 (pose_net.py:31-34)")
-        if _get(cfg, "net_type", "resnet_50") != "resnet_50":
-            raise ValueError("only resnet_50 is on the B200 path")
+        self.net_type = _get(cfg, "net_type", "resnet_50")
+        synthetic.net_scope(self.net_type)   # resnet_50, resnet_101 or resnet_152 (pose_net.py:14-16)
         if _get(cfg, "intermediate_supervision", False):
             raise ValueError("intermediate_supervision is not on the B200 path (DGP never enables it)")
         self.num_joints = int(_get(cfg, "num_joints"))
@@ -69,7 +71,9 @@ class PoseNet:
             self.restore(variables)
 
     def restore(self, variables):
-        """Replaces Saver.restore: {tf_var_name: ndarray} with slim names (resnet_v1_50/..., pose/...)."""
+        """Replaces Saver.restore: {tf_var_name: ndarray} with slim names (resnet_v1_<depth>/..., pose/...); the backbone they
+        name must be the cfg's net_type (ValueError otherwise)."""
+        check_net_type(self.net_type, variables)
         self.engine.load_weights(variables)
 
     def _frames(self, inputs):
@@ -83,10 +87,10 @@ class PoseNet:
 
     def extract_features(self, inputs):
         """pose_net.py:36-54 -> (net (N,hf,wf,2048) float32, end_points).  ``end_points`` holds the block outputs the
-        reference's callers could read: only ``resnet_v1_50/block4`` (= net) is materialised on this path."""
+        reference's callers could read: only ``resnet_v1_<depth>/block4`` (= net) is materialised on this path."""
         net = self.engine.extract_features(self._frames(inputs)).as_subclass(Features)
         net.engine = self.engine
-        return net, {"resnet_v1_50/block4": net}
+        return net, {synthetic.net_scope(self.net_type) + "/block4": net}
 
     def prediction_layers(self, features, end_points=None, reuse=None):
         """pose_net.py:56-78 -> {'part_pred': (N,2h,2w,nj)[, 'locref': (N,2h,2w,2nj)]}."""

@@ -9,15 +9,48 @@ import numpy as np
 
 # (scope, base_depth, num_units, stride) -- slim resnet_v1_50
 RESNET50_BLOCKS = (("block1", 64, 3, 2), ("block2", 128, 4, 2), ("block3", 256, 6, 2), ("block4", 512, 3, 1))
+# units per block of slim resnet_v1_50 / _101 / _152 (DLC's net_type); channels, strides and dilation are the same
+BLOCK_UNITS = {"resnet_50": (3, 4, 6, 3), "resnet_101": (3, 4, 23, 3), "resnet_152": (3, 8, 36, 3)}
+NET_TYPES = tuple(BLOCK_UNITS)
+# Scale of the last BN gamma of every bottleneck (see make_weights).  Chosen with the fp32 oracle so that the deeper nets'
+# part_pred logits have the spread of the ResNet-50 set: std of the logits of seed 0, nj 4, on a 235x301 synthetic frame is
+# 4.10 at depth 50 (0.25), 4.07 at depth 101 (0.145) and 4.13 at depth 152 (0.14); at 0.25 the deeper nets reach 17 / 37
+# and saturate the sigmoid on 82 / 92 % of the map.
+CONV3_GAMMA_SCALE = {"resnet_50": 0.25, "resnet_101": 0.145, "resnet_152": 0.14}
 
 
-def resnet50_conv_specs():
-    """Yield (scope, kh, kw, cin, cout) for the 53 convs of slim resnet_v1_50 in execution order."""
-    specs = [("resnet_v1_50/conv1", 7, 7, 3, 64)]
+def net_scope(net_type):
+    """slim scope of the backbone variables: 'resnet_50' -> 'resnet_v1_50'."""
+    if net_type not in BLOCK_UNITS:
+        raise ValueError("net_type must be one of %s (got %r)" % (", ".join(NET_TYPES), net_type))
+    return "resnet_v1_" + net_type.split("_")[1]
+
+
+def net_blocks(net_type="resnet_50"):
+    """(scope, base_depth, num_units, stride) of the four blocks of slim resnet_v1_<depth>."""
+    net_scope(net_type)
+    return tuple((name, base, n, stride) for (name, base, _, stride), n in zip(RESNET50_BLOCKS, BLOCK_UNITS[net_type]))
+
+
+def net_type_of(variables):
+    """net_type ('resnet_50' / 'resnet_101' / 'resnet_152') of a {tf_var_name: array} dict, from its backbone scope."""
+    scopes = sorted({k.split("/", 1)[0] for k in variables if k.startswith("resnet_v1_")})
+    if len(scopes) != 1:
+        raise ValueError("the weights must hold exactly one backbone scope out of resnet_v1_50, resnet_v1_101, resnet_v1_152 "
+                         "(found %s)" % (", ".join(scopes) if scopes else "none"))
+    net_type = "resnet_" + scopes[0][len("resnet_v1_"):]
+    net_scope(net_type)
+    return net_type
+
+
+def conv_specs(net_type="resnet_50"):
+    """(scope, kh, kw, cin, cout) of every conv of slim resnet_v1_<depth> in execution order (53 / 104 / 155 convs)."""
+    prefix = net_scope(net_type)
+    specs = [(prefix + "/conv1", 7, 7, 3, 64)]
     cin = 64
-    for name, base, units, _ in RESNET50_BLOCKS:
+    for name, base, units, _ in net_blocks(net_type):
         for u in range(units):
-            scope = "resnet_v1_50/%s/unit_%d/bottleneck_v1" % (name, u + 1)
+            scope = "%s/%s/unit_%d/bottleneck_v1" % (prefix, name, u + 1)
             depth = base * 4
             if cin != depth:
                 specs.append((scope + "/shortcut", 1, 1, cin, depth))
@@ -28,14 +61,21 @@ def resnet50_conv_specs():
     return specs
 
 
-def make_weights(nj, seed=0, location_refinement=True, bn_random=True, head_gain=1.0, trained_like=False):
-    """Random-init weights of the DLC ResNet-50 pose net, TF names -> float32 ndarrays.
+def resnet50_conv_specs():
+    """Yield (scope, kh, kw, cin, cout) for the 53 convs of slim resnet_v1_50 in execution order."""
+    return conv_specs("resnet_50")
+
+
+def make_weights(nj, seed=0, location_refinement=True, bn_random=True, head_gain=1.0, trained_like=False, net_type="resnet_50"):
+    """Random-init weights of the DLC pose net on slim resnet_v1_<depth> (``net_type`` resnet_50 / resnet_101 /
+    resnet_152), TF names -> float32 ndarrays.
 
     conv: He-normal (fan-in) HWIO; BN: gamma~U(.5,1.5), beta~N(0,.1), mean~N(0,.1), var~U(.5,1.5)
     (``bn_random=False`` gives the TF initial values gamma=1, beta=0, mean=0, var=1 of config (a)).
-    The last BN of every bottleneck gets gamma scaled by 0.25 so the residual stream of the
-    16 units stays O(1) (otherwise logits saturate the sigmoid and every parity test degenerates
-    to ties).  Heads: xavier-uniform ``[3,3,cout,2048]`` scaled so logits have std ~3, zero bias.
+    The last BN of every bottleneck gets gamma scaled by CONV3_GAMMA_SCALE[net_type] (0.25 for the 16 units of ResNet-50,
+    less for the 33 / 50 units of the deeper nets) so the residual stream stays O(1) (otherwise logits saturate the sigmoid
+    and every parity test degenerates to ties).  ResNet-50 draws the same random stream whatever the other nets draw.
+    Heads: xavier-uniform ``[3,3,cout,2048]`` scaled so logits have std ~3, zero bias.
 
     ``trained_like=True`` gives the second weight set of the parity tests, shaped like a fine-tuned DLC snapshot rather than
     a fresh initialisation: (i) an ImageNet-style BatchNorm spectrum -- in every bottleneck's last BN 15 % of the channels
@@ -45,7 +85,8 @@ def make_weights(nj, seed=0, location_refinement=True, bn_random=True, head_gain
     """
     rng = np.random.default_rng(seed)
     W = {}
-    for scope, kh, kw, cin, cout in resnet50_conv_specs():
+    gamma_scale = CONV3_GAMMA_SCALE[net_type]
+    for scope, kh, kw, cin, cout in conv_specs(net_type):
         fan_in = kh * kw * cin
         gain = np.sqrt(2.0 / fan_in)
         if scope.endswith("/conv1") and cin == 3:
@@ -59,7 +100,7 @@ def make_weights(nj, seed=0, location_refinement=True, bn_random=True, head_gain
         else:
             g, b, m, v = np.ones(cout), np.zeros(cout), np.zeros(cout), np.ones(cout)
         if scope.endswith("/conv3"):
-            g = g * 0.25
+            g = g * gamma_scale
             if trained_like:
                 u = rng.uniform(size=cout)
                 tiny = 10.0 ** rng.uniform(-5.0, -2.0, cout)

@@ -65,14 +65,19 @@ const char* dgp_last_error(const dgp_handle* h);
  * dtype: 0 = float32.  The data is copied; call dgp_finalize_weights once all variables are loaded. */
 int dgp_load_weights(dgp_handle* h, const char* tf_var_name, const void* host_ptr, const int64_t* shape, int ndim,
                      int dtype);
-/* Converts to kernel layouts (bf16 [cout][kh*kw*cin] K-major, fp32 BN scale/shift) and uploads. */
+/* Converts to kernel layouts (bf16 [cout][kh*kw*cin] K-major, fp32 BN scale/shift) and uploads.  The backbone is the one
+ * the loaded names describe: every backbone variable must sit under exactly one of the slim scopes resnet_v1_50,
+ * resnet_v1_101 or resnet_v1_152 (units per block (3,4,6,3), (3,4,23,3), (3,8,36,3)); mixed scopes or none at all are
+ * DGP_ERR_INVALID. */
 int dgp_finalize_weights(dgp_handle* h);
+/* Depth of the backbone built by dgp_finalize_weights: 50, 101 or 152. */
+int dgp_net_depth(const dgp_handle* h, int* depth);
 
 /* Closed form of Dataset._compute_pred_dims (src/deepgraphpose/dataset.py:348-371). */
 int dgp_output_dims(int H, int W, int* h_feat, int* w_feat, int* h_out, int* w_out);
 
 /* Replaces sess.run([scmap(, locref)], {inputs: frames}) (eval.py:328, 746): PoseNet.extract_features
- * (pose_net.py:36-54: mean subtraction + slim resnet_v1_50 OS16, frozen BN) and the 3x3 stride-2 deconv heads
+ * (pose_net.py:36-54: mean subtraction + slim resnet_v1_<depth> OS16, frozen BN) and the 3x3 stride-2 deconv heads
  * (pose_net.py:18-26).  frames_dev: uint8 (B,H,W,3) RGB.  logits_dev: float32 (B,2h,2w,nj) part_pred logits.
  * locref_dev: float32 (B,2h,2w,2nj) or NULL. */
 int dgp_forward(dgp_handle* h, const uint8_t* frames_dev, int B, int H, int W, float* logits_dev, float* locref_dev,

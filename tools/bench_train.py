@@ -51,8 +51,10 @@ def cpu_train_step_seconds(nt, H, W, NJ):
     return time.perf_counter() - t0, os.cpu_count()
 
 
-def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=True, precision="fp16", wt=1.0):
-    """One data-parallel training benchmark on the already-initialised process group; returns the JSON dict (rank 0) or None."""
+def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=True, precision="fp16", wt=1.0,
+            net_type="resnet_50"):
+    """One data-parallel training benchmark on the already-initialised process group; returns the JSON dict (rank 0) or None.
+    ``net_type`` picks the backbone of the synthetic weights (the FLOP figures of the line are ResNet-50's)."""
     import argparse as _a
     args = _a.Namespace(steps=steps, warmup=warmup, nt=nt, height=height, width=width)
     import torch.distributed as dist
@@ -75,7 +77,7 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
                locref_loss_weight=0.05, stride=8.0)
     ws, ws_max = fitdgp.spatial_clique_params([labels], S0, 8.0, 1000.0, 1.2)
     eng = Engine(NJ, location_refinement=True, device=local_rank, precision=precision)
-    eng.load_weights(synthetic.make_weights(NJ, seed=0))
+    eng.load_weights(synthetic.make_weights(NJ, seed=0, net_type=net_type))
     eng.use_graphs(os.environ.get("DGP_TRAIN_GRAPHS", "1") != "0")
     c_comm = world > 1 and os.environ.get("DGP_DP_TORCH", "0") != "1"
     if c_comm:
