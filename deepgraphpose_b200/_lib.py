@@ -91,7 +91,11 @@ SIGNATURES = {
     "dgp_conv2d_wgrad": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "dgp_train_enable": (_i, [_vp]),
     "dgp_train_forward_backward": (_i, [_vp, _vp, _i, _i, _i, C.POINTER(DgpLossCfg), C.POINTER(DgpLossBatch), _i, _vp, _vp]),
+    "dgp_train_forward": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, C.POINTER(C.c_uint64), _vp]),
+    "dgp_train_backward": (_i, [_vp, C.c_uint64, _vp, _vp, _i, _vp]),
     "dgp_optimizer_step": (_i, [_vp, _f, _f, _f, _f, _vp]),
+    "dgp_get_param_buffer": (_i, [_vp, C.POINTER(_vp), C.POINTER(_sz)]),
+    "dgp_params_changed": (_i, [_vp, _vp]),
     "dgp_get_grad_buffer": (_i, [_vp, C.POINTER(_vp), C.POINTER(_sz)]),
     "dgp_train_early_bucket": (_i, [_vp, C.POINTER(_sz), C.POINTER(_sz)]),
     "dgp_train_wait_early_bucket": (_i, [_vp, _vp]),

@@ -102,7 +102,8 @@ __global__ void __launch_bounds__(1024) bn_grad_finalize_kernel(const float* __r
 __global__ void __launch_bounds__(1024) bn_finalize_all_kernel(const BnGroup* __restrict__ table, const float* __restrict__ part,
                                                                const float* __restrict__ rowdot, const float* __restrict__ mean,
                                                                const float* __restrict__ var, float eps,
-                                                               float* __restrict__ dgamma, float* __restrict__ dbeta) {
+                                                               float* __restrict__ dgamma, float* __restrict__ dbeta,
+                                                               const GradMode* __restrict__ mode) {
   const BnGroup g = table[blockIdx.x];
   const int cl = threadIdx.x & 7, rg = threadIdx.x >> 3;
   const float* pp = part + g.part_off + g.col + cl;
@@ -126,8 +127,8 @@ __global__ void __launch_bounds__(1024) bn_finalize_all_kernel(const BnGroup* __
   if (rg == 0) {
     const int c = blockIdx.x * 8 + cl;
     const float db = sm0[0][cl];
-    dbeta[c] = db;
-    dgamma[c] = (sm1[0][cl] - mean[c] * db) * rsqrtf(var[c] + eps);
+    store_grad(dbeta + c, db, mode);
+    store_grad(dgamma + c, (sm1[0][cl] - mean[c] * db) * rsqrtf(var[c] + eps), mode);
   }
 }
 
@@ -433,12 +434,13 @@ __global__ void __launch_bounds__(256) head_bias_partial_kernel(const float* __r
     partial[(size_t)blockIdx.x * C + threadIdx.x] = s;
   }
 }
-__global__ void head_bias_final_kernel(const float* __restrict__ partial, int nblocks, int C, float* __restrict__ dbias) {
+__global__ void head_bias_final_kernel(const float* __restrict__ partial, int nblocks, int C, float* __restrict__ dbias,
+                                       const GradMode* __restrict__ mode) {
   const int c = threadIdx.x;
   if (c >= C) return;
   float s = 0.0f;
   for (int b = 0; b < nblocks; ++b) s += partial[(size_t)b * C + c];
-  dbias[c] = s;
+  store_grad(dbias + c, s, mode);
 }
 
 __global__ void scale_inplace_kernel(float* __restrict__ x, size_t n, float s) {
@@ -472,8 +474,8 @@ cudaError_t launch_relu_bn_bwd(void* g, const void* act, int M, int C, float* pa
 }
 
 cudaError_t launch_bn_finalize_all(const BnGroup* table, int ngroups, const float* part, const float* rowdot, const float* mean,
-                                   const float* var, float eps, float* dgamma, float* dbeta, cudaStream_t s) {
-  bn_finalize_all_kernel<<<ngroups, 1024, 0, s>>>(table, part, rowdot, mean, var, eps, dgamma, dbeta);
+                                   const float* var, float eps, float* dgamma, float* dbeta, const GradMode* mode, cudaStream_t s) {
+  bn_finalize_all_kernel<<<ngroups, 1024, 0, s>>>(table, part, rowdot, mean, var, eps, dgamma, dbeta, mode);
   return cudaGetLastError();
 }
 
@@ -543,11 +545,12 @@ cudaError_t launch_col2im_bwd(const float* g_logits, const float* g_locref, int 
 int head_bias_blocks() { return 148; }
 
 // g: (npix, C) fp32; partial: [head_bias_blocks()][C] workspace
-cudaError_t launch_head_bias_grad(const float* g, size_t npix, int C, float* partial, float* dbias, cudaStream_t s) {
+cudaError_t launch_head_bias_grad(const float* g, size_t npix, int C, float* partial, float* dbias, const GradMode* mode,
+                                  cudaStream_t s) {
   if (C > 256) return cudaErrorInvalidValue;
   const int nthreads = (148 * 256 / C) * C;
   head_bias_partial_kernel<<<148, 256, 0, s>>>(g, npix * (size_t)C, C, nthreads, partial);
-  head_bias_final_kernel<<<1, 256, 0, s>>>(partial, 148, C, dbias);
+  head_bias_final_kernel<<<1, 256, 0, s>>>(partial, 148, C, dbias, mode);
   return cudaGetLastError();
 }
 

@@ -1335,7 +1335,7 @@ int dgp_conv2d_wgrad(dgp_handle* h, const void* x_dev, int N, int H, int W, int 
   CU_OK(h, cudaMalloc(&ws, wgrad_workspace_bytes(wp)));
   wp.partials = (float*)ws;
   cudaError_t e = launch_wgrad_gemm(wp, h->num_sms, (cudaStream_t)stream);
-  if (e == cudaSuccess) e = launch_wgrad_reduce(wp, nullptr, nullptr, dw_dev, 0, (cudaStream_t)stream);
+  if (e == cudaSuccess) e = launch_wgrad_reduce(wp, nullptr, nullptr, dw_dev, nullptr, (cudaStream_t)stream);
   h->launches += 2;
   if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);
   cudaFree(ws);

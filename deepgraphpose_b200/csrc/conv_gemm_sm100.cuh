@@ -17,6 +17,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "kernels.cuh"
+
 namespace dgp {
 
 constexpr int kBlockM = 128;
@@ -96,10 +98,11 @@ struct WgradParams {
 void wgrad_plan(WgradParams* p, int num_sms);
 size_t wgrad_workspace_bytes(const WgradParams& p);
 cudaError_t launch_wgrad_gemm(const WgradParams& p, int num_sms, cudaStream_t stream);
-// grad[co][kk] (=|+=) rowscale[co] * mask[co][kk] * sum over splits (fixed order); rowscale / mask may be null.
+// grad[co][kk] = rowscale[co] * mask[co][kk] * sum over splits (fixed order), stored through `mode` (nullptr: overwrite);
+// rowscale / mask may be null.
 // wmaster / rowdot_part (optional): also write <W[co, 4 kk], dW_raw[co, 4 kk]> per float4 of the row (Cout * Kw / 4 floats)
 cudaError_t launch_wgrad_reduce(const WgradParams& p, const float* rowscale, const float* mask, float* grad,
-                                int accumulate, cudaStream_t stream, const float* wmaster = nullptr,
+                                const GradMode* mode, cudaStream_t stream, const float* wmaster = nullptr,
                                 float* rowdot_part = nullptr);
 // dgamma = (row sums of rowdot_part - mean * dbeta) / sqrt(var + eps)  (frozen BN; exact, no division by gamma)
 cudaError_t launch_bn_gamma_grad(const float* rowdot_part, int Cout, int Kw, const float* mean, const float* var, float eps,

@@ -88,6 +88,7 @@ struct Plan {
   int Hp = 0, Wp = 0, pool_pad_t = 0, pool_pad_l = 0;
   float *logits = nullptr, *locref = nullptr;
   std::shared_ptr<void> bwd;  // train.cu: backward step list
+  uint64_t fwd_token = 0;     // train.cu: token of the dgp_train_forward whose activations the plan holds (0 = none)
 };
 
 }  // namespace dgp

@@ -92,6 +92,24 @@ cudaError_t launch_momentum_step(float* w, float* accum, const float* g, size_t 
                                  float grad_scale, const float* norm_clip, cudaStream_t s);
 
 // ---- network backward, bandwidth-class parts (bwd_kernels.cu)
+// How the kernels that finish a gradient write it into the gradient arena (wgrad_reduce_kernel, bn_finalize_all_kernel,
+// head_bias_final_kernel): arena = (accumulate ? arena : 0) + out_scale * finished value, the add after the fixed-order sum.
+// A device word read at run time, so that one captured backward graph serves both training entries; nullptr = overwrite
+// with out_scale 1.
+struct GradMode {
+  int accumulate;
+  float out_scale;
+};
+#ifdef __CUDACC__
+__device__ __forceinline__ void store_grad(float* dst, float v, const GradMode* mode) {
+  if (mode != nullptr) {
+    const GradMode m = *mode;
+    v *= m.out_scale;
+    if (m.accumulate) v = *dst + v;
+  }
+  *dst = v;
+}
+#endif
 // One entry per 8 consecutive BatchNorm channels (always one layer): where their dy sums ([rows][C] floats, this group at column
 // `col`) and their <W, dW_raw> products ([8][K4] floats) were left by the backward pass.
 struct BnGroup {
@@ -100,7 +118,7 @@ struct BnGroup {
 };
 // dbeta[c] = sum of the dy sums, dgamma[c] = (sum of the row-dot products - mean * dbeta) / sqrt(var + eps), all channels at once
 cudaError_t launch_bn_finalize_all(const BnGroup* table, int ngroups, const float* part, const float* rowdot, const float* mean,
-                                   const float* var, float eps, float* dgamma, float* dbeta, cudaStream_t s);
+                                   const float* var, float eps, float* dgamma, float* dbeta, const GradMode* mode, cudaStream_t s);
 int relu_bn_bwd_blocks(int M, int C);  // rows of `partial` ([blocks][C])
 // scatter_d != nullptr: g (N,H,W,C) += zero-inserted scatter_d (N,P,Q,C) first (gradient of the stride-2 identity shortcut)
 cudaError_t launch_relu_bn_bwd(void* g, const void* act, int M, int C, float* partial, int fp16, cudaStream_t s,
@@ -120,7 +138,8 @@ cudaError_t launch_col2im_bwd(const float* g_logits, const float* g_locref, int 
                               void* dG, int Kd, int fp16, cudaStream_t s);
 int head_bias_blocks();
 // g (npix, C) fp32 -> dbias[C]; partial: [head_bias_blocks()][C] floats of workspace
-cudaError_t launch_head_bias_grad(const float* g, size_t npix, int C, float* partial, float* dbias, cudaStream_t s);
+cudaError_t launch_head_bias_grad(const float* g, size_t npix, int C, float* partial, float* dbias, const GradMode* mode,
+                                  cudaStream_t s);
 
 cudaError_t launch_scale_inplace(float* x, size_t n, float scale, cudaStream_t s);
 

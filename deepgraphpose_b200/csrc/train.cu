@@ -82,6 +82,14 @@ struct TrainState {
   uint64_t ws_gen = 1;           // bumped whenever a shared workspace is reallocated (captured graphs hold its address)
   bool use_graphs = true;
   float loss_scale = 1.0f;       // head gradients are multiplied by this before the network backward (fp16 storage)
+  // What the gradient arena holds: arena_scale x the true gradient (loss_scale after dgp_train_forward_backward, 1 after
+  // dgp_train_backward); every reader divides by it.  grad_mode is the device word the arena-writing kernels read
+  // (GradMode), grad_mode_host the value last stored there.
+  float arena_scale = 1.0f;
+  bool arena_fused = false;      // the last backward was dgp_train_forward_backward's (no accumulation onto it)
+  GradMode* grad_mode = nullptr;
+  GradMode grad_mode_host = {0, 1.0f};
+  uint64_t fwd_seq = 0;          // tokens handed out by dgp_train_forward
   DgradWJob* wd_jobs = nullptr;  // device table for the one-launch rebuild of every dgrad operand
   int n_wd_jobs = 0, wd_tiles = 0;
   // Early all-reduce bucket: the weight gradients of block4 and the heads (two thirds of the arena, contiguous at the end of
@@ -121,6 +129,7 @@ void train_destroy(dgp_handle* h) {
   for (W16* p : ts->wd) cudaFree(p);
   cudaFree(ts->head_wd);
   cudaFree(ts->wd_jobs);
+  cudaFree(ts->grad_mode);
   if (ts->ev_early) cudaEventDestroy(ts->ev_early);
   for (cudaEvent_t e : ts->ev_bucket) if (e) cudaEventDestroy(e);
   if (ts->ev_bwd_done) cudaEventDestroy(ts->ev_bwd_done);
@@ -269,7 +278,8 @@ int add_wgrad_params(dgp_handle* h, Backward* bw, const WgradParams& wp0, const 
                          wp.partials = (float*)ts->wgrad_ws.p;
                          cudaError_t e = launch_wgrad_gemm(wp, sms, s);
                          if (e != cudaSuccess) return e;
-                         return launch_wgrad_reduce(wp, rowscale, mask, grad, 0, s, wmaster, wmaster ? bw->rowdot + rd_off : nullptr);
+                         return launch_wgrad_reduce(wp, rowscale, mask, grad, ts->grad_mode, s, wmaster,
+                                                    wmaster ? bw->rowdot + rd_off : nullptr);
                        }});
   bw->steps.back().rd = dy_buf;
   return DGP_OK;
@@ -367,8 +377,9 @@ int build_backward(dgp_handle* h, Plan* pl) {
     bn_need = std::max(bn_need, (size_t)head_bias_blocks() * 256 * sizeof(float));
     bw->steps.push_back({7, g_locref ? 4 : 2, [=](cudaStream_t s) {
                            float* partial = (float*)ts->bn_partial.p;
-                           cudaError_t e = launch_head_bias_grad(g_logits, npix, nj, partial, dbias, s);
-                           if (e == cudaSuccess && g_locref) e = launch_head_bias_grad(g_locref, npix, 2 * nj, partial, dbias + nj, s);
+                           cudaError_t e = launch_head_bias_grad(g_logits, npix, nj, partial, dbias, ts->grad_mode, s);
+                           if (e == cudaSuccess && g_locref)
+                             e = launch_head_bias_grad(g_locref, npix, 2 * nj, partial, dbias + nj, ts->grad_mode, s);
                            return e;
                          }});
   }
@@ -526,8 +537,10 @@ int build_backward(dgp_handle* h, Plan* pl) {
     const float eps = h->cfg.bn_epsilon;
     float* dgam = ts->grads + h->n_w;
     float* dbet = ts->grads + h->n_w + h->n_ch;
+    const GradMode* mode = ts->grad_mode;
     bw->steps.push_back({7, 1, [=](cudaStream_t s) {
-                           return launch_bn_finalize_all(bwp->bn_table, ngroups, bwp->bn_part, bwp->rowdot, mean, var, eps, dgam, dbet, s);
+                           return launch_bn_finalize_all(bwp->bn_table, ngroups, bwp->bn_part, bwp->rowdot, mean, var, eps, dgam, dbet,
+                                                         mode, s);
                          }});
     bw->steps.back().join = true;
   }
@@ -572,98 +585,35 @@ bool find_variable(dgp_handle* h, const std::string& name, VarRef* r) {
   return false;
 }
 
-}  // namespace
-}  // namespace dgp
-
-extern "C" {
-
-int dgp_train_enable(dgp_handle* h) {
-  if (!h) return DGP_ERR_INVALID;
-  if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_train_enable before dgp_finalize_weights");
-  if (h->train) return DGP_OK;
-  CU_OK(h, cudaSetDevice(h->device));
-  TrainState* ts = new TrainState();
-  h->train = ts;
-  CU_OK(h, cudaMalloc(&ts->grads, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->accum, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMemset(ts->grads, 0, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMemset(ts->accum, 0, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->norm_partial, sqnorm_partials() * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->norm_clip, 2 * sizeof(float)));
-  CU_OK(h, cudaMemset(ts->norm_clip, 0, 2 * sizeof(float)));
-  ts->wd.assign(h->layers.size(), nullptr);
-  std::vector<DgradWJob> jobs;
-  for (size_t i = 0; i < h->layers.size(); ++i) {
-    if ((int)i == h->conv1_layer || (int)i == h->head_layer) continue;
-    const ConvLayer& L = h->layers[i];
-    if (L.Cin % 32 || L.Cout % 32 || L.ch_off < 0) return fail(h, DGP_ERR_UNSUPPORTED, "%s: dgrad operand needs 32-aligned channels", L.scope.c_str());
-    CU_OK(h, cudaMalloc(&ts->wd[i], (size_t)L.Cin * L.R * L.S * L.Cout * sizeof(W16)));
-    DgradWJob jb;
-    jb.w_off = L.w_off; jb.wd = reinterpret_cast<uint16_t*>(ts->wd[i]); jb.ch_off = L.ch_off;
-    jb.Cout = L.Cout; jb.taps = L.R * L.S; jb.Cin = L.Cin; jb.tile_start = ts->wd_tiles;
-    ts->wd_tiles += (L.Cin / 32) * (L.Cout / 32) * L.R * L.S;
-    jobs.push_back(jb);
-  }
-  if (jobs.size() > (size_t)kDgradWMaxJobs)
-    return fail(h, DGP_ERR_UNSUPPORTED, "%zu conv layers exceed the %d of the one-launch dgrad operand rebuild", jobs.size(),
-                kDgradWMaxJobs);
-  ts->n_wd_jobs = (int)jobs.size();
-  CU_OK(h, cudaMalloc(&ts->wd_jobs, jobs.size() * sizeof(DgradWJob)));
-  CU_OK(h, cudaMemcpy(ts->wd_jobs, jobs.data(), jobs.size() * sizeof(DgradWJob), cudaMemcpyHostToDevice));
-  CU_OK(h, cudaEventCreateWithFlags(&ts->ev_early, cudaEventDisableTiming));
-  for (const UnitDesc& u : h->units)
-    if (u.scope.find("/block4/") != std::string::npos && u.shortcut >= 0) {
-      ts->early_off = h->layers[u.shortcut].w_off;
-      ts->early_cnt = h->n_w - ts->early_off;
-      break;
-    }
-  {
-    // bucket k = the weight gradients of one block (k = 0: block4 + heads ... k = 3: conv1 + block1 + the BN / bias tail)
-    const char* first[3] = {"/block4/unit_1/", "/block3/unit_1/", "/block2/unit_1/"};
-    ts->bucket_off[0] = h->n_w;
-    for (int k = 0; k < 3; ++k)
-      for (const UnitDesc& u : h->units)
-        if (u.scope.find(first[k]) != std::string::npos && u.shortcut >= 0) ts->bucket_off[k + 1] = h->layers[u.shortcut].w_off;
-    ts->bucket_off[4] = 0;
-    for (int k = 0; k < 3; ++k) CU_OK(h, cudaEventCreateWithFlags(&ts->ev_bucket[k], cudaEventDisableTiming));
-    CU_OK(h, cudaEventCreate(&ts->ev_bwd_done));
-    CU_OK(h, cudaEventCreate(&ts->ev_comm_done));
-    CU_OK(h, cudaStreamCreateWithFlags(&ts->comm_stream, cudaStreamNonBlocking));
-  }
-  ts->head_Kd = ceil_div(std::max(9 * h->ctot, h->layers[h->head_layer].Npad), 64) * 64;
-  CU_OK(h, cudaMalloc(&ts->head_wd, (size_t)2048 * ts->head_Kd * sizeof(W16)));
+// Stores the arena write mode the backward kernels read (GradMode) on `s`, when it differs from the stored one.
+int set_grad_mode(dgp_handle* h, int accumulate, float out_scale, cudaStream_t s) {
+  TrainState* ts = h->train;
+  if (ts->grad_mode_host.accumulate == accumulate && ts->grad_mode_host.out_scale == out_scale) return DGP_OK;
+  ts->grad_mode_host.accumulate = accumulate;
+  ts->grad_mode_host.out_scale = out_scale;
+  CU_OK(h, cudaMemcpyAsync(ts->grad_mode, &ts->grad_mode_host, sizeof(GradMode), cudaMemcpyHostToDevice, s));
   return DGP_OK;
 }
 
-int dgp_train_forward_backward(dgp_handle* h, const uint8_t* frames_dev, int nt, int H, int W, const dgp_loss_cfg* cfg,
-                               const dgp_loss_batch* batch, int visible_only, float* losses_dev, void* stream) {
-  if (!h) return DGP_ERR_INVALID;
-  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_forward_backward before dgp_train_enable");
-  if (!frames_dev || !cfg || !batch || !losses_dev || nt < 1 || H < 32 || W < 32)
-    return fail(h, DGP_ERR_INVALID, "dgp_train_forward_backward: bad argument");
-  CU_OK(h, cudaSetDevice(h->device));
-  cudaStream_t s = (cudaStream_t)stream;
+// A change of the weights makes every outstanding dgp_train_forward token stale.
+void drop_train_tokens(dgp_handle* h) {
+  for (auto& kv : h->train_plans) kv.second->fwd_token = 0;
+}
+
+// Loss scaling of the head gradients before the network backward (dgp_train_set_loss_scale).
+int scale_head_grads(dgp_handle* h, const Plan* pl, Backward* bw, cudaStream_t s) {
+  const float ls = h->train->loss_scale;
+  if (ls == 1.0f) return DGP_OK;
+  const size_t n = (size_t)pl->B * 4 * pl->hf * pl->wf * h->cfg.num_joints;
+  CU_OK(h, launch_scale_inplace(bw->g_logits, n, ls, s));
+  if (bw->g_locref) CU_OK(h, launch_scale_inplace(bw->g_locref, 2 * n, ls, s));
+  h->launches += bw->g_locref ? 2 : 1;
+  return DGP_OK;
+}
+
+// The network backward of `bw` from its g_logits / g_locref: eager on the first run of a plan, a captured graph afterwards.
+int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
   TrainState* ts = h->train;
-  Plan* pl = nullptr;
-  int rc = build_plan(h, nt, H, W, true, &pl);
-  if (rc) return rc;
-  if (!pl->bwd && (rc = build_backward(h, pl))) return rc;
-  Backward* bw = static_cast<Backward*>(pl->bwd.get());
-  if (batch->nt != nt || batch->H != 2 * pl->hf || batch->W != 2 * pl->wf)
-    return fail(h, DGP_ERR_INVALID, "dgp_train_forward_backward: batch dims (%d,%d,%d) do not match the network output (%d,%d,%d)",
-                batch->nt, batch->H, batch->W, nt, 2 * pl->hf, 2 * pl->wf);
-  if (!ts->wd_fresh && (rc = refresh_dgrad_weights(h, s))) return rc;
-  if ((rc = run_forward_plan(h, pl, frames_dev, pl->logits, pl->locref, s))) return rc;
-  dgp_loss_batch b = *batch;
-  b.pred_dev = pl->logits;
-  b.locref_dev = pl->locref;
-  if ((rc = dgp_run_loss_impl(h, cfg, &b, losses_dev, nullptr, bw->g_logits, bw->g_locref, visible_only, stream))) return rc;
-  if (ts->loss_scale != 1.0f) {
-    const size_t n = (size_t)nt * 4 * pl->hf * pl->wf * h->cfg.num_joints;
-    CU_OK(h, launch_scale_inplace(bw->g_logits, n, ts->loss_scale, s));
-    if (bw->g_locref) CU_OK(h, launch_scale_inplace(bw->g_locref, 2 * n, ts->loss_scale, s));
-    h->launches += bw->g_locref ? 2 : 1;
-  }
   const bool graphs = ts->use_graphs && !h->profiling && bw->runs > 0;
   if (graphs && (!bw->graph_exec || bw->graph_gen != ts->ws_gen)) {
     // (re)capture on the handle's private stream; the first step ran eagerly, so every lazy cudaFuncSetAttribute is done
@@ -765,6 +715,162 @@ int dgp_train_forward_backward(dgp_handle* h, const uint8_t* frames_dev, int nt,
   return DGP_OK;
 }
 
+}  // namespace
+}  // namespace dgp
+
+extern "C" {
+
+int dgp_train_enable(dgp_handle* h) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_train_enable before dgp_finalize_weights");
+  if (h->train) return DGP_OK;
+  CU_OK(h, cudaSetDevice(h->device));
+  TrainState* ts = new TrainState();
+  h->train = ts;
+  CU_OK(h, cudaMalloc(&ts->grads, h->n_params * sizeof(float)));
+  CU_OK(h, cudaMalloc(&ts->accum, h->n_params * sizeof(float)));
+  CU_OK(h, cudaMemset(ts->grads, 0, h->n_params * sizeof(float)));
+  CU_OK(h, cudaMemset(ts->accum, 0, h->n_params * sizeof(float)));
+  CU_OK(h, cudaMalloc(&ts->norm_partial, sqnorm_partials() * sizeof(float)));
+  CU_OK(h, cudaMalloc(&ts->norm_clip, 2 * sizeof(float)));
+  CU_OK(h, cudaMemset(ts->norm_clip, 0, 2 * sizeof(float)));
+  CU_OK(h, cudaMalloc(&ts->grad_mode, sizeof(GradMode)));
+  CU_OK(h, cudaMemcpy(ts->grad_mode, &ts->grad_mode_host, sizeof(GradMode), cudaMemcpyHostToDevice));
+  ts->wd.assign(h->layers.size(), nullptr);
+  std::vector<DgradWJob> jobs;
+  for (size_t i = 0; i < h->layers.size(); ++i) {
+    if ((int)i == h->conv1_layer || (int)i == h->head_layer) continue;
+    const ConvLayer& L = h->layers[i];
+    if (L.Cin % 32 || L.Cout % 32 || L.ch_off < 0) return fail(h, DGP_ERR_UNSUPPORTED, "%s: dgrad operand needs 32-aligned channels", L.scope.c_str());
+    CU_OK(h, cudaMalloc(&ts->wd[i], (size_t)L.Cin * L.R * L.S * L.Cout * sizeof(W16)));
+    DgradWJob jb;
+    jb.w_off = L.w_off; jb.wd = reinterpret_cast<uint16_t*>(ts->wd[i]); jb.ch_off = L.ch_off;
+    jb.Cout = L.Cout; jb.taps = L.R * L.S; jb.Cin = L.Cin; jb.tile_start = ts->wd_tiles;
+    ts->wd_tiles += (L.Cin / 32) * (L.Cout / 32) * L.R * L.S;
+    jobs.push_back(jb);
+  }
+  if (jobs.size() > (size_t)kDgradWMaxJobs)
+    return fail(h, DGP_ERR_UNSUPPORTED, "%zu conv layers exceed the %d of the one-launch dgrad operand rebuild", jobs.size(),
+                kDgradWMaxJobs);
+  ts->n_wd_jobs = (int)jobs.size();
+  CU_OK(h, cudaMalloc(&ts->wd_jobs, jobs.size() * sizeof(DgradWJob)));
+  CU_OK(h, cudaMemcpy(ts->wd_jobs, jobs.data(), jobs.size() * sizeof(DgradWJob), cudaMemcpyHostToDevice));
+  CU_OK(h, cudaEventCreateWithFlags(&ts->ev_early, cudaEventDisableTiming));
+  for (const UnitDesc& u : h->units)
+    if (u.scope.find("/block4/") != std::string::npos && u.shortcut >= 0) {
+      ts->early_off = h->layers[u.shortcut].w_off;
+      ts->early_cnt = h->n_w - ts->early_off;
+      break;
+    }
+  {
+    // bucket k = the weight gradients of one block (k = 0: block4 + heads ... k = 3: conv1 + block1 + the BN / bias tail)
+    const char* first[3] = {"/block4/unit_1/", "/block3/unit_1/", "/block2/unit_1/"};
+    ts->bucket_off[0] = h->n_w;
+    for (int k = 0; k < 3; ++k)
+      for (const UnitDesc& u : h->units)
+        if (u.scope.find(first[k]) != std::string::npos && u.shortcut >= 0) ts->bucket_off[k + 1] = h->layers[u.shortcut].w_off;
+    ts->bucket_off[4] = 0;
+    for (int k = 0; k < 3; ++k) CU_OK(h, cudaEventCreateWithFlags(&ts->ev_bucket[k], cudaEventDisableTiming));
+    CU_OK(h, cudaEventCreate(&ts->ev_bwd_done));
+    CU_OK(h, cudaEventCreate(&ts->ev_comm_done));
+    CU_OK(h, cudaStreamCreateWithFlags(&ts->comm_stream, cudaStreamNonBlocking));
+  }
+  ts->head_Kd = ceil_div(std::max(9 * h->ctot, h->layers[h->head_layer].Npad), 64) * 64;
+  CU_OK(h, cudaMalloc(&ts->head_wd, (size_t)2048 * ts->head_Kd * sizeof(W16)));
+  return DGP_OK;
+}
+
+int dgp_train_forward_backward(dgp_handle* h, const uint8_t* frames_dev, int nt, int H, int W, const dgp_loss_cfg* cfg,
+                               const dgp_loss_batch* batch, int visible_only, float* losses_dev, void* stream) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_forward_backward before dgp_train_enable");
+  if (!frames_dev || !cfg || !batch || !losses_dev || nt < 1 || H < 32 || W < 32)
+    return fail(h, DGP_ERR_INVALID, "dgp_train_forward_backward: bad argument");
+  CU_OK(h, cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  TrainState* ts = h->train;
+  Plan* pl = nullptr;
+  int rc = build_plan(h, nt, H, W, true, &pl);
+  if (rc) return rc;
+  if (!pl->bwd && (rc = build_backward(h, pl))) return rc;
+  Backward* bw = static_cast<Backward*>(pl->bwd.get());
+  if (batch->nt != nt || batch->H != 2 * pl->hf || batch->W != 2 * pl->wf)
+    return fail(h, DGP_ERR_INVALID, "dgp_train_forward_backward: batch dims (%d,%d,%d) do not match the network output (%d,%d,%d)",
+                batch->nt, batch->H, batch->W, nt, 2 * pl->hf, 2 * pl->wf);
+  if (!ts->wd_fresh && (rc = refresh_dgrad_weights(h, s))) return rc;
+  pl->fwd_token = 0;   // the activations are this step's from here on
+  if ((rc = run_forward_plan(h, pl, frames_dev, pl->logits, pl->locref, s))) return rc;
+  dgp_loss_batch b = *batch;
+  b.pred_dev = pl->logits;
+  b.locref_dev = pl->locref;
+  if ((rc = dgp_run_loss_impl(h, cfg, &b, losses_dev, nullptr, bw->g_logits, bw->g_locref, visible_only, stream))) return rc;
+  if ((rc = scale_head_grads(h, pl, bw, s))) return rc;
+  if ((rc = set_grad_mode(h, 0, 1.0f, s))) return rc;
+  if ((rc = run_backward(h, bw, s))) return rc;
+  ts->arena_scale = ts->loss_scale;
+  ts->arena_fused = true;
+  return DGP_OK;
+}
+
+int dgp_train_forward(dgp_handle* h, const uint8_t* frames_dev, int nt, int H, int W, float* logits_dev, float* locref_dev,
+                      uint64_t* token, void* stream) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_forward before dgp_train_enable");
+  if (!frames_dev || !logits_dev || !token || nt < 1 || H < 32 || W < 32)
+    return fail(h, DGP_ERR_INVALID, "dgp_train_forward: bad argument");
+  if (locref_dev && !h->cfg.location_refinement)
+    return fail(h, DGP_ERR_INVALID, "dgp_train_forward: locref_dev given but the network has no locref head");
+  CU_OK(h, cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  TrainState* ts = h->train;
+  Plan* pl = nullptr;
+  int rc = build_plan(h, nt, H, W, true, &pl);
+  if (rc) return rc;
+  if (!pl->bwd && (rc = build_backward(h, pl))) return rc;
+  if (!ts->wd_fresh && (rc = refresh_dgrad_weights(h, s))) return rc;
+  pl->fwd_token = 0;
+  // the head GEMM's col2im writes straight into the caller's buffers; the backward needs only the kept activations
+  if ((rc = run_forward_plan(h, pl, frames_dev, logits_dev, locref_dev, s))) return rc;
+  pl->fwd_token = ++ts->fwd_seq;
+  *token = pl->fwd_token;
+  return DGP_OK;
+}
+
+int dgp_train_backward(dgp_handle* h, uint64_t token, const float* g_logits_dev, const float* g_locref_dev, int accumulate,
+                       void* stream) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_backward before dgp_train_enable");
+  TrainState* ts = h->train;
+  Plan* pl = nullptr;
+  for (auto& kv : h->train_plans)
+    if (token != 0 && kv.second->fwd_token == token) pl = kv.second.get();
+  if (!pl)
+    return fail(h, DGP_ERR_STATE, "dgp_train_backward: stale token (a later training forward of this shape, a plan eviction or a "
+                                  "weight change has overwritten the activations of that forward)");
+  Backward* bw = static_cast<Backward*>(pl->bwd.get());
+  if (g_locref_dev && !bw->g_locref)
+    return fail(h, DGP_ERR_INVALID, "dgp_train_backward: g_locref_dev given but the network has no locref head");
+  if (accumulate && ts->arena_fused)
+    return fail(h, DGP_ERR_STATE, "dgp_train_backward: cannot accumulate onto the loss-scaled gradients of dgp_train_forward_backward");
+  CU_OK(h, cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t n = (size_t)pl->B * 4 * pl->hf * pl->wf * h->cfg.num_joints;
+  if (g_logits_dev) CU_OK(h, cudaMemcpyAsync(bw->g_logits, g_logits_dev, n * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  else CU_OK(h, cudaMemsetAsync(bw->g_logits, 0, n * sizeof(float), s));
+  if (bw->g_locref) {
+    if (g_locref_dev) CU_OK(h, cudaMemcpyAsync(bw->g_locref, g_locref_dev, 2 * n * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    else CU_OK(h, cudaMemsetAsync(bw->g_locref, 0, 2 * n * sizeof(float), s));
+  }
+  int rc;
+  if ((rc = scale_head_grads(h, pl, bw, s))) return rc;
+  // the loss scale is divided out again as the finished gradients are stored: the arena holds the true gradient
+  if ((rc = set_grad_mode(h, accumulate ? 1 : 0, 1.0f / ts->loss_scale, s))) return rc;
+  if ((rc = run_backward(h, bw, s))) return rc;
+  ts->arena_scale = 1.0f;
+  ts->arena_fused = false;
+  return DGP_OK;
+}
+
 int dgp_train_use_graphs(dgp_handle* h, int enable) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_use_graphs before dgp_train_enable");
@@ -797,13 +903,33 @@ int dgp_optimizer_step(dgp_handle* h, float lr, float momentum, float clip_norm,
   CU_OK(h, cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
   TrainState* ts = h->train;
-  grad_scale /= ts->loss_scale;  // the buffer holds loss_scale * gradient
+  grad_scale /= ts->arena_scale;  // the buffer holds arena_scale * gradient
   CU_OK(h, launch_global_norm(ts->grads, h->n_params, grad_scale, clip_norm, ts->norm_partial, ts->norm_clip, s));
   CU_OK(h, launch_momentum_step(h->master, ts->accum, ts->grads, h->n_params, lr, momentum, grad_scale, ts->norm_clip, s));
   h->launches += 3;
+  drop_train_tokens(h);
   int rc = refresh_operands(h, s);
   if (rc) return rc;
   return refresh_dgrad_weights(h, s);
+}
+
+int dgp_params_changed(dgp_handle* h, void* stream) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_params_changed before dgp_finalize_weights");
+  CU_OK(h, cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  drop_train_tokens(h);
+  int rc = refresh_operands(h, s);
+  if (rc || !h->train) return rc;
+  return refresh_dgrad_weights(h, s);
+}
+
+int dgp_get_param_buffer(dgp_handle* h, void** dev_ptr, size_t* bytes) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_get_param_buffer before dgp_finalize_weights");
+  if (dev_ptr) *dev_ptr = h->master;
+  if (bytes) *bytes = h->n_params * sizeof(float);
+  return DGP_OK;
 }
 
 int dgp_train_set_loss_scale(dgp_handle* h, float loss_scale) {
@@ -866,10 +992,10 @@ int dgp_get_variable(dgp_handle* h, const char* tf_var_name, int what, float* ho
   if (ndim) *ndim = nd;
   if (!host_out) return DGP_OK;
   if (n > max_elems) return fail(h, DGP_ERR_INVALID, "buffer too small for %s", tf_var_name);
-  struct Unscale {  // gradients are stored multiplied by the loss scale; hand back the true gradient
+  struct Unscale {  // gradients are stored multiplied by arena_scale; hand back the true gradient
     float* p; size_t n; float f;
     ~Unscale() { if (f != 1.0f) for (size_t i = 0; i < n; ++i) p[i] *= f; }
-  } unscale{host_out, n, what == 1 ? 1.0f / h->train->loss_scale : 1.0f};
+  } unscale{host_out, n, what == 1 ? 1.0f / h->train->arena_scale : 1.0f};
   CU_OK(h, cudaSetDevice(h->device));
   CU_OK(h, cudaDeviceSynchronize());
   if (r.kind == 2 || r.kind == 3) {
@@ -958,6 +1084,7 @@ int dgp_set_variable(dgp_handle* h, const char* tf_var_name, int what, const flo
     CU_OK(h, cudaMemcpy(arena + L.w_off, m.data(), m.size() * 4, cudaMemcpyHostToDevice));
   }
   if (what == 0) {  // the tensor-core operands are derived from the master copy
+    drop_train_tokens(h);
     int rc = refresh_operands(h, nullptr);
     if (rc) return rc;
     if (h->train) h->train->wd_fresh = false;

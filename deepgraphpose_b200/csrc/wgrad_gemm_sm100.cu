@@ -240,14 +240,15 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_gemm_kernel(const __grid_
   }
 }
 
-// grad[co][kk] = rowscale[co] * mask[co][kk] * sum_s partial[(m_blk, n_blk, s)][co % 128][kk % 256].
+// grad[co][kk] = rowscale[co] * mask[co][kk] * sum_s partial[(m_blk, n_blk, s)][co % 128][kk % 256], stored through `mode`
+// (scaled, then optionally added to what the arena holds).
 // SG threads share one float4 of the gradient: thread (e, sg) sums the splits sg, sg + SG, ...; the SG partial sums are
 // then added in index order by one thread (fixed order: bitwise reproducible, no atomics).
 template <int SG>
 __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restrict__ partials, int Cout, int Kw, int nnb,
                                                            int splits, const float* __restrict__ rowscale,
                                                            const float* __restrict__ mask, float* __restrict__ grad,
-                                                           int accumulate, const float* __restrict__ wmaster,
+                                                           const GradMode* __restrict__ mode, const float* __restrict__ wmaster,
                                                            float* __restrict__ rowdot_part) {
   constexpr int EPB = 256 / SG;  // float4 elements per block
   const int e = threadIdx.x % EPB, sg = threadIdx.x / EPB;
@@ -288,9 +289,13 @@ __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restri
     const float4 m = *reinterpret_cast<const float4*>(mask + (size_t)co * Kw + kk);
     acc.x *= m.x; acc.y *= m.y; acc.z *= m.z; acc.w *= m.w;
   }
-  if (accumulate) {
-    const float4 o = *g;
-    acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
+  if (mode != nullptr) {
+    const GradMode md = *mode;
+    acc.x *= md.out_scale; acc.y *= md.out_scale; acc.z *= md.out_scale; acc.w *= md.out_scale;
+    if (md.accumulate) {
+      const float4 o = *g;
+      acc.x = o.x + acc.x; acc.y = o.y + acc.y; acc.z = o.z + acc.z; acc.w = o.w + acc.w;
+    }
   }
   *g = acc;
 }
@@ -349,18 +354,18 @@ cudaError_t launch_wgrad_gemm(const WgradParams& p, int num_sms, cudaStream_t st
 }
 
 cudaError_t launch_wgrad_reduce(const WgradParams& p, const float* rowscale, const float* mask, float* grad,
-                                int accumulate, cudaStream_t stream, const float* wmaster, float* rowdot_part) {
+                                const GradMode* mode, cudaStream_t stream, const float* wmaster, float* rowdot_part) {
   const size_t total = (size_t)p.Cout * (p.Kw / 4);
   // few elements and many splits (the narrow, pixel-rich layers of block 1/2): spread the split loop over threads
   if (p.splits >= 32 && total <= 32768) {
     wgrad_reduce_kernel<16><<<(unsigned)((total + 15) / 16), 256, 0, stream>>>(p.partials, p.Cout, p.Kw, p.num_n_blocks,
-                                                                             p.splits, rowscale, mask, grad, accumulate, wmaster, rowdot_part);
+                                                                             p.splits, rowscale, mask, grad, mode, wmaster, rowdot_part);
   } else if (p.splits >= 8 && total <= 262144) {
     wgrad_reduce_kernel<4><<<(unsigned)((total + 63) / 64), 256, 0, stream>>>(p.partials, p.Cout, p.Kw, p.num_n_blocks,
-                                                                            p.splits, rowscale, mask, grad, accumulate, wmaster, rowdot_part);
+                                                                            p.splits, rowscale, mask, grad, mode, wmaster, rowdot_part);
   } else {
     wgrad_reduce_kernel<1><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(p.partials, p.Cout, p.Kw, p.num_n_blocks,
-                                                                              p.splits, rowscale, mask, grad, accumulate, wmaster, rowdot_part);
+                                                                              p.splits, rowscale, mask, grad, mode, wmaster, rowdot_part);
   }
   return cudaGetLastError();
 }

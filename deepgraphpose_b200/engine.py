@@ -382,6 +382,59 @@ class Engine:
         self._check(self.lib.dgp_get_grad_buffer(self.h, C.byref(p), C.byref(n)))
         return _device_view(p.value, (n.value // 4,), "<f4", self.device)
 
+    def param_buffer(self):
+        """The flat float32 parameter arena (fp32 master copy, same layout as grad_buffer) as a CUDA tensor VIEW.  After
+        changing it in place, call params_changed() before the next forward."""
+        p, n = C.c_void_p(), C.c_size_t()
+        self._check(self.lib.dgp_get_param_buffer(self.h, C.byref(p), C.byref(n)))
+        return _device_view(p.value, (n.value // 4,), "<f4", self.device)
+
+    def params_changed(self):
+        """Re-derive the 16-bit weights, BatchNorm scale / shift and dgrad operands from param_buffer() (dgp_params_changed)."""
+        self._check(self.lib.dgp_params_changed(self.h, _stream(self.device)))
+
+    def train_forward(self, frames, want_locref=None):
+        """Training forward (dgp_train_forward): frames uint8 cuda (nt,H,W,3) -> (logits, locref | None, token).  The outputs
+        are new float32 tensors; the token names the kept activations for train_backward."""
+        if frames.dtype != torch.uint8 or frames.dim() != 4 or frames.shape[-1] != 3 or not frames.is_cuda:
+            raise ValueError("frames must be a uint8 CUDA tensor of shape (B,H,W,3)")
+        self.train_enable()
+        frames = frames.contiguous()
+        B, H, W, _ = frames.shape
+        _, (ho, wo) = output_dims(H, W)
+        if want_locref is None:
+            want_locref = self.location_refinement
+        logits = torch.empty((B, ho, wo, self.nj), dtype=torch.float32, device=frames.device)
+        locref = torch.empty((B, ho, wo, 2 * self.nj), dtype=torch.float32, device=frames.device) if want_locref else None
+        token = C.c_uint64()
+        self._check(self.lib.dgp_train_forward(self.h, _ptr(frames), B, H, W, _ptr(logits), _ptr(locref), C.byref(token),
+                                               _stream(frames.device)))
+        # head shapes of the live token of each input shape (at most one: a new forward at a shape makes the old token stale)
+        live = self.__dict__.setdefault("_live_tokens", {})
+        for t in [t for t, v in live.items() if v[0] == tuple(frames.shape)]:
+            del live[t]
+        live[int(token.value)] = (tuple(frames.shape), tuple(logits.shape))
+        return logits, locref, int(token.value)
+
+    def train_backward(self, token, g_logits, g_locref=None, accumulate=False):
+        """Network backward of the train_forward named by ``token`` from the loss gradients w.r.t. its head outputs (float32
+        cuda, None = zeros) into grad_buffer(): overwrite, or add with ``accumulate``.  The buffer then holds the true
+        (unscaled) gradient.  A stale token raises DgpError (DGP_ERR_STATE)."""
+        for g in (g_logits, g_locref):
+            if g is not None and (g.dtype != torch.float32 or not g.is_cuda):
+                raise ValueError("head gradients must be float32 CUDA tensors")
+        live = self.__dict__.get("_live_tokens", {})
+        if token in live:   # the C side checks the token; the sizes of the caller's buffers can only be checked here
+            shp = live[token][1]
+            if g_logits is not None and tuple(g_logits.shape) != shp:
+                raise ValueError("g_logits must have the logits' shape %s" % (shp,))
+            if g_locref is not None and tuple(g_locref.shape) != shp[:3] + (2 * self.nj,):
+                raise ValueError("g_locref must have the locref shape %s" % (shp[:3] + (2 * self.nj,),))
+        g_logits = g_logits.contiguous() if g_logits is not None else None
+        g_locref = g_locref.contiguous() if g_locref is not None else None
+        self._check(self.lib.dgp_train_backward(self.h, C.c_uint64(token), _ptr(g_logits), _ptr(g_locref), int(bool(accumulate)),
+                                                _stream(self.device)))
+
     def use_graphs(self, enable=True):
         """Replay the network backward as a CUDA graph from the second step on (default) or launch it eagerly."""
         self.train_enable()

@@ -155,6 +155,63 @@ def loss_forward(engine, pred, locref, feed, cfg, edges, ws, ws_max, n_frames_to
     return dict(zip(LOSS_KEYS, [np.float32(v) for v in vals])), all_markers
 
 
+class _DgpLossFunction(torch.autograd.Function):
+    """dgp_loss_backward as an autograd node: the forward computes the six losses and the gradients of the differentiated
+    total w.r.t. the heads in one call; the backward scales those gradients by grad_output."""
+
+    @staticmethod
+    def forward(ctx, pred, locref, engine, feed, cfg, edges, ws, ws_max, n_frames_total, n_visible_frames_total, visible_only):
+        dev = pred.device
+        nt, H, W, nj = pred.shape
+        pred = pred.detach().contiguous()
+        locref = locref.detach().contiguous() if locref is not None else None
+        c, b, keep = _loss_args(dev, feed, cfg, edges, ws, ws_max, n_frames_total, n_visible_frames_total, nt, H, W, nj, pred,
+                                locref, engine=engine)
+        out = torch.empty(6, dtype=torch.float32, device=dev)
+        g_pred = torch.empty_like(pred)
+        g_loc = torch.empty_like(locref) if locref is not None else None
+        engine._check(engine.lib.dgp_loss_backward(engine.h, C.byref(c), C.byref(b), _ptr(out), _ptr(g_pred), _ptr(g_loc),
+                                                   int(visible_only), _stream(dev)))
+        ctx.keep = keep   # feed tensors (some produced on a side stream) outlive the asynchronous loss kernels
+        ctx.grads = (g_pred, g_loc)
+        vals = torch.cat([out, (out[0] + out[2]).view(1)])   # + total_loss_visible
+        ctx.mark_non_differentiable(vals)
+        return vals[6 if visible_only else 5].clone(), vals
+
+    @staticmethod
+    def backward(ctx, g_total, g_vals):
+        g_pred, g_loc = ctx.grads
+        return (g_pred * g_total, g_loc * g_total if g_loc is not None else None) + (None,) * 9
+
+
+def _loss_engine(dev, nj, cfg):
+    """A weight-less handle that runs the loss kernels, one per (device, joints, stride, locref_stdev)."""
+    key = (str(dev), int(nj), float(_get(cfg, "stride", 8.0)), float(_get(cfg, "locref_stdev", 7.2801)))
+    eng = _LOSS_ENGINES.get(key)
+    if eng is None:
+        eng = _LOSS_ENGINES[key] = Engine(nj, device=dev, stride=key[2], locref_stdev=key[3])
+    return eng
+
+
+_LOSS_ENGINES = {}
+
+
+def dgp_loss_function(pred, locref, feed, cfg, edges, ws, ws_max, n_frames_total, n_visible_frames_total, visible_only=False,
+                      engine=None):
+    """dgp_loss (fitdgp.py:934-1128) as a differentiable PyTorch function of the heads: pred float32 CUDA (nt,H,W,nj) and
+    locref (nt,H,W,2nj) or None, e.g. from ``autograd.TrainablePoseNet``; the other arguments as in ``loss_forward``.
+    Returns {LOSS_KEYS..., "total_loss_visible"} as 0-d tensors; ``total_loss`` (``total_loss_visible`` when visible_only)
+    is differentiable, the others are values only.  ``dgp_total + my_term`` then trains on the sum.  ``engine``: the handle
+    whose loss kernels run (default: a weight-less one per device and joint count)."""
+    if engine is None:
+        engine = _loss_engine(pred.device, pred.shape[-1], cfg)
+    total, vals = _DgpLossFunction.apply(pred, locref, engine, feed, cfg, edges, ws, ws_max, n_frames_total,
+                                         n_visible_frames_total, bool(visible_only))
+    out = {k: vals[i] for i, k in enumerate(LOSS_KEYS + ("total_loss_visible",))}
+    out["total_loss_visible" if visible_only else "total_loss"] = total
+    return out
+
+
 def train_forward_backward(engine, frames, feed, cfg, edges, ws, ws_max, n_frames_total, n_visible_frames_total,
                            visible_only=False, sync=True):
     """Forward + loss + full backward of one fit_dgp batch (fitdgp.py:817-818 without the apply step): fills the

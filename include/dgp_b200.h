@@ -270,15 +270,40 @@ int dgp_train_enable(dgp_handle* h);
  * members as in dgp_loss_forward.  losses_dev[6] as in dgp_loss_forward. */
 int dgp_train_forward_backward(dgp_handle* h, const uint8_t* frames_dev, int nt, int H, int W, const dgp_loss_cfg* cfg,
                                const dgp_loss_batch* batch, int visible_only, float* losses_dev, void* stream);
+/* The same step split in two, for a loss (and optimizer) written by the caller:
+ *  dgp_train_forward: the training forward of frames_dev uint8 (nt,H,W,3), keeping every activation.  The head outputs go to
+ *    logits_dev float32 (nt,2h,2w,nj) and locref_dev (nt,2h,2w,2nj); locref_dev may be NULL.  *token names this forward.
+ *    At most one forward per input shape is live: the next training forward at that shape (either entry), the eviction of
+ *    the shape's plan (more than 3 training shapes) or a weight change (dgp_set_variable, dgp_optimizer_step,
+ *    dgp_params_changed) makes the token stale.
+ *  dgp_train_backward: the network backward of that forward from the caller's loss gradients w.r.t. the head outputs
+ *    (float32, shapes as above; NULL = zeros).  They are loss-scaled like the fused step's, and the finished gradients are
+ *    divided by the loss scale again as they are stored, so the gradient buffer holds the TRUE gradient.  accumulate = 0
+ *    overwrites the buffer, 1 adds to it (the add comes after every fixed-order sum: batch A then B == gA + gB in fp32, bit
+ *    for bit); adding onto the loss-scaled buffer of dgp_train_forward_backward is DGP_ERR_STATE.  A stale token is
+ *    DGP_ERR_STATE and launches nothing.  The same token may be differentiated more than once.
+ * Readers of the gradient buffer (dgp_optimizer_step, dgp_get_variable(what = 1), dgp_get_grad_norm) divide by the scale
+ * the buffer holds: loss_scale after dgp_train_forward_backward, 1 after dgp_train_backward. */
+int dgp_train_forward(dgp_handle* h, const uint8_t* frames_dev, int nt, int H, int W, float* logits_dev, float* locref_dev,
+                      uint64_t* token, void* stream);
+int dgp_train_backward(dgp_handle* h, uint64_t token, const float* g_logits_dev, const float* g_locref_dev, int accumulate,
+                       void* stream);
 /* g' = g * grad_scale; g' *= clip_norm / max(||g'||, clip_norm) (clip_norm <= 0: no clipping);
  * accum = momentum * accum + g'; var -= lr * accum; then refreshes the 16-bit operands and BN scale/shift. */
 int dgp_optimizer_step(dgp_handle* h, float lr, float momentum, float clip_norm, float grad_scale, void* stream);
+/* Flat float32 parameter arena (fp32 master copy, kernel layouts: [weights | gamma | beta | head bias], the layout of the
+ * gradient buffer) for an optimizer outside the library.  After changing it in place, call dgp_params_changed: it re-derives
+ * the 16-bit weights, the BatchNorm scale / shift and the dgrad operands on `stream` (what dgp_optimizer_step does at its
+ * end).  Padding of the layouts (conv1's space-to-depth taps, head rows beyond 3nj) must stay 0. */
+int dgp_get_param_buffer(dgp_handle* h, void** dev_ptr, size_t* bytes);
+int dgp_params_changed(dgp_handle* h, void* stream);
 /* From its second run at a given input shape the network backward (about 280 launches with fixed arguments) is replayed as
  * one CUDA graph; enable = 0 goes back to eager launches (always used while dgp_set_profiling is on). Default 1. */
 int dgp_train_use_graphs(dgp_handle* h, int enable);
 /* Loss scaling for fp16 storage (precision = 1): the head gradients are multiplied by loss_scale before the network
  * backward so that small activation gradients stay above fp16's subnormal range; dgp_optimizer_step divides it out again and
- * dgp_get_variable(what = 1) returns unscaled gradients (the raw buffer of dgp_get_grad_buffer holds loss_scale * gradient).
+ * dgp_get_variable(what = 1) returns unscaled gradients (after dgp_train_forward_backward the raw buffer of
+ * dgp_get_grad_buffer holds loss_scale * gradient; after dgp_train_backward the gradient itself).
  * Default 1 (bf16 storage has fp32's exponent range and needs none). */
 int dgp_train_set_loss_scale(dgp_handle* h, float loss_scale);
 /* Flat float32 gradient buffer (kernel layouts: [weights | gamma | beta | head bias]) for ncclAllReduce. */
@@ -313,7 +338,8 @@ int dgp_allreduce_gradients(dgp_handle* h, void* stream, float* grad_scale);
 int dgp_allreduce_exposed_ms(dgp_handle* h, float* ms);
 /* Global gradient norm computed by the last dgp_optimizer_step (after grad_scale, before clipping). Synchronises. */
 int dgp_get_grad_norm(dgp_handle* h, float* norm_host);
-/* Device pointers of the head outputs (nt,2h,2w,nj) / (nt,2h,2w,2nj) written by the last training step at this shape. */
+/* Device pointers of the head outputs (nt,2h,2w,nj) / (nt,2h,2w,2nj) written by the last dgp_train_forward_backward at this
+ * shape (dgp_train_forward writes into the caller's buffers instead). */
 int dgp_train_outputs(dgp_handle* h, int nt, int H, int W, float** logits_dev, float** locref_dev);
 /* Replaces sess.run(variable) / TF.train.Saver.save (fitdgp.py:830-839): copies a trainable variable back to the host under
  * its TF name and TF layout.  what: 0 = value, 1 = gradient of the last step, 2 = momentum accumulator.
