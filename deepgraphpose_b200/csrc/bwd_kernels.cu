@@ -7,9 +7,11 @@
 //                   out = relu(shortcut + bn3(conv3)) conv3 and the projection shortcut share it).  dgamma is taken from the
 //                   weight gradient: sum_p dy*z = <W[c,:], dW_raw[c,:]> with z the conv output, so
 //                   dgamma = (<W, dW_raw> - mean * dbeta) / sigma -- exact for gamma = 0 too (wgrad_gemm_sm100.cu).
-//   maxpool_bwd   : gradient of slim.max_pool2d(3x3, stride 2, SAME), routed to the first maximum of each window.
+//                   It also adds the gradient of resnet_utils.subsample (identity shortcut of a stride-2 unit):
+//                   g_x[2p,2q] += d[p,q].
+//   maxpool_relu_bwd : gradient of slim.max_pool2d(3x3, stride 2, SAME), routed to the first maximum of each window,
+//                   with conv1's ReLU mask and dy sums.
 //   upsample2     : zero insertion that turns the stride-2 3x3 dgrad into a stride-1 conv.
-//   scatter_add2  : gradient of resnet_utils.subsample (identity shortcut of a stride-2 unit): g_x[2p,2q] += d[p,q].
 //   col2im_bwd    : gradient of the deconv heads' col2im (gather of the head gradients per (pixel, tap, channel)).
 // Reductions are two-stage with a fixed order (bitwise reproducible).
 #include "half_utils.cuh"
@@ -23,8 +25,8 @@ using h16::unpack8;
 __device__ __forceinline__ uint4 pack8v(const float* f, int fp16) { return h16::pack8(f, fp16); }
 
 // dy = g * [act > 0] in place + per-channel partial sums of dy (-> dbeta).  The same kernel serves plain ReLU layers and the
-// bottleneck junctions out = relu(shortcut + bn3(conv3)): dgamma no longer needs the BN output (see bn_gamma_grad_kernel in
-// wgrad_gemm_sm100.cu), so neither the shortcut tensor nor a division by gamma is involved.
+// bottleneck junctions out = relu(shortcut + bn3(conv3)): dgamma no longer needs the BN output (bn_finalize_all_kernel takes it
+// from the wgrad reduce's row-dot products <W, dW_raw>), so neither the shortcut tensor nor a division by gamma is involved.
 // d != nullptr: g first receives the gradient of resnet_utils.subsample (the identity shortcut of the stride-2 unit behind this
 // junction): g[n,2p,2q] += d[n,p,q] with g (N,H,W,C), d (N,P,Q,C) -- one pass instead of a scatter-add pass plus this one.
 __global__ void __launch_bounds__(256) relu_bn_bwd_kernel(uint4* __restrict__ g, const uint4* __restrict__ act, int M, int C8,
@@ -73,29 +75,6 @@ __global__ void __launch_bounds__(256) relu_bn_bwd_kernel(uint4* __restrict__ g,
   }
 }
 
-// dbeta[c] = sum of the partial rows (written to one or two layers: conv3 and the projection shortcut share dy at a junction).
-// Block = 8 channels x 128 row groups: row group r sums the partial rows r, r+128, ... (at most 5 dependent loads per thread --
-// this kernel is pure latency), then a fixed-order tree over the row groups.
-__global__ void __launch_bounds__(1024) bn_grad_finalize_kernel(const float* __restrict__ partial, int nblocks, int C,
-                                                                float* __restrict__ dbeta_a, float* __restrict__ dbeta_b) {
-  const int cl = threadIdx.x & 7, rg = threadIdx.x >> 3;
-  const int c = blockIdx.x * 8 + cl;
-  float s0 = 0.0f;
-  if (c < C)
-    for (int b = rg; b < nblocks; b += 128) s0 += partial[(size_t)b * C + c];
-  __shared__ float sm0[128][9];
-  sm0[rg][cl] = s0;
-  __syncthreads();
-  for (int st = 64; st > 0; st >>= 1) {
-    if (rg < st) sm0[rg][cl] += sm0[rg + st][cl];
-    __syncthreads();
-  }
-  if (rg == 0 && c < C) {
-    dbeta_a[c] = sm0[0][cl];
-    if (dbeta_b != nullptr) dbeta_b[c] = sm0[0][cl];
-  }
-}
-
 // All frozen-BN parameter gradients of the network in one launch (one block per 8 channels, 128 row groups x 8 channels):
 // dbeta = sum over the row blocks of the dy sums its mask site left, dgamma = (sum_kk <W, dW_raw> - mean * dbeta) / sigma.
 // Fixed summation order (strided partial sums, then a tree over the row groups): bitwise reproducible.
@@ -129,86 +108,6 @@ __global__ void __launch_bounds__(1024) bn_finalize_all_kernel(const BnGroup* __
     const float db = sm0[0][cl];
     store_grad(dbeta + c, db, mode);
     store_grad(dgamma + c, (sm1[0][cl] - mean[c] * db) * rsqrtf(var[c] + eps), mode);
-  }
-}
-
-// First-maximum position (0..8, row-major in the 3x3 window) of every pooled element: one byte per channel.
-__global__ void maxpool_argmax_kernel(const uint4* __restrict__ x, int N, int H, int W, int C8, int Ho, int Wo, int pad_t,
-                                      int pad_l, uint2* __restrict__ arg, int fp16) {
-  const size_t total = (size_t)N * Ho * Wo * C8;
-  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
-    const int c = (int)(t % C8);
-    size_t r = t / C8;
-    const int q = (int)(r % Wo);
-    r /= Wo;
-    const int p = (int)(r % Ho);
-    const int n = (int)(r / Ho);
-    float best[8];
-    uint32_t idx[8];
-    bool have = false;
-#pragma unroll
-    for (int dy = 0; dy < 3; ++dy) {
-      const int y = 2 * p - pad_t + dy;
-      if (y < 0 || y >= H) continue;
-#pragma unroll
-      for (int dx = 0; dx < 3; ++dx) {
-        const int xq = 2 * q - pad_l + dx;
-        if (xq < 0 || xq >= W) continue;
-        float v[8];
-        unpack8(__ldg(x + (((size_t)n * H + y) * W + xq) * C8 + c), v, fp16);
-        if (!have) {
-#pragma unroll
-          for (int j = 0; j < 8; ++j) { best[j] = v[j]; idx[j] = dy * 3 + dx; }
-          have = true;
-        } else {
-#pragma unroll
-          for (int j = 0; j < 8; ++j)
-            if (v[j] > best[j]) { best[j] = v[j]; idx[j] = dy * 3 + dx; }
-        }
-      }
-    }
-    uint2 o;
-    o.x = idx[0] | (idx[1] << 8) | (idx[2] << 16) | (idx[3] << 24);
-    o.y = idx[4] | (idx[5] << 8) | (idx[6] << 16) | (idx[7] << 24);
-    arg[t] = o;
-  }
-}
-
-// gx[n,y,x,c] = sum over the <= 4 windows (p,q) containing (y,x) of gout[n,p,q,c] * [arg[n,p,q,c] == position of (y,x)]
-__global__ void maxpool_bwd_kernel(const uint2* __restrict__ arg, const uint4* __restrict__ gout, int N, int H, int W, int C8,
-                                   int Ho, int Wo, int pad_t, int pad_l, uint4* __restrict__ gx, int fp16) {
-  const size_t total = (size_t)N * H * W * C8;
-  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
-    const int c = (int)(t % C8);
-    size_t r = t / C8;
-    const int xx = (int)(r % W);
-    r /= W;
-    const int yy = (int)(r % H);
-    const int n = (int)(r / H);
-    float acc[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] = 0.0f;
-    // windows containing (yy, xx): 2p - pad_t <= yy <= 2p - pad_t + 2
-    const int p_lo = (yy + pad_t - 2 + 1) >> 1 < 0 ? 0 : (yy + pad_t - 2 + 1) >> 1;
-    int p_hi = (yy + pad_t) >> 1;
-    if (p_hi > Ho - 1) p_hi = Ho - 1;
-    const int q_lo = (xx + pad_l - 2 + 1) >> 1 < 0 ? 0 : (xx + pad_l - 2 + 1) >> 1;
-    int q_hi = (xx + pad_l) >> 1;
-    if (q_hi > Wo - 1) q_hi = Wo - 1;
-    for (int p = p_lo; p <= p_hi; ++p)
-      for (int q = q_lo; q <= q_hi; ++q) {
-        const uint32_t mine = (uint32_t)((yy - (2 * p - pad_t)) * 3 + (xx - (2 * q - pad_l)));
-        const size_t o = (((size_t)n * Ho + p) * Wo + q) * C8 + c;
-        const uint2 a = __ldg(arg + o);
-        float gv[8];
-        unpack8(__ldg(gout + o), gv, fp16);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          if (((a.x >> (8 * j)) & 0xffu) == mine) acc[j] += gv[j];
-          if (((a.y >> (8 * j)) & 0xffu) == mine) acc[4 + j] += gv[4 + j];
-        }
-      }
-    gx[t] = pack8v(acc, fp16);
   }
 }
 
@@ -366,27 +265,6 @@ __global__ void upsample2_kernel(const uint4* __restrict__ in, int N, int P, int
   }
 }
 
-// gx (N,H,W,C)[n,2p,2q] += d (N,P,Q,C)[n,p,q]
-__global__ void scatter_add2_kernel(const uint4* __restrict__ d, int N, int P, int Q, int C8, uint4* __restrict__ gx, int H,
-                                    int W, int fp16) {
-  const size_t total = (size_t)N * P * Q * C8;
-  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
-    const int c = (int)(t % C8);
-    size_t r = t / C8;
-    const int q = (int)(r % Q);
-    r /= Q;
-    const int p = (int)(r % P);
-    const int n = (int)(r / P);
-    const size_t o = (((size_t)n * H + 2 * p) * W + 2 * q) * C8 + c;
-    float a[8], b[8];
-    unpack8(__ldg(d + t), a, fp16);
-    unpack8(gx[o], b, fp16);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) a[j] += b[j];
-    gx[o] = pack8v(a, fp16);
-  }
-}
-
 // dG[m][kk] (16-bit, Kd columns) = head gradient at (2i+kh, 2j+kw), kk = (kh*3+kw)*ctot + co; zero outside / padding.
 __global__ void col2im_bwd_kernel(const float* __restrict__ g_logits, const float* __restrict__ g_locref, int N, int h, int w,
                                   int ctot, int nj, uint16_t* __restrict__ dG, int Kd, int fp16) {
@@ -479,23 +357,6 @@ cudaError_t launch_bn_finalize_all(const BnGroup* table, int ngroups, const floa
   return cudaGetLastError();
 }
 
-cudaError_t launch_bn_grad_finalize(const float* partial, int nblocks, int C, float* dbeta_a, float* dbeta_b, cudaStream_t s) {
-  bn_grad_finalize_kernel<<<(C + 7) / 8, 1024, 0, s>>>(partial, nblocks, C, dbeta_a, dbeta_b);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_maxpool_bwd(const void* x, const void* gout, int N, int H, int W, int C, int Ho, int Wo, int pad_t,
-                               int pad_l, void* arg_ws, void* gx, int fp16, cudaStream_t s) {
-  const size_t tout = (size_t)N * Ho * Wo * (C / 8);
-  maxpool_argmax_kernel<<<flat_grid(tout, 256), 256, 0, s>>>(reinterpret_cast<const uint4*>(x), N, H, W, C / 8, Ho, Wo, pad_t,
-                                                             pad_l, reinterpret_cast<uint2*>(arg_ws), fp16);
-  const size_t total = (size_t)N * H * W * (C / 8);
-  maxpool_bwd_kernel<<<flat_grid(total, 256), 256, 0, s>>>(reinterpret_cast<const uint2*>(arg_ws),
-                                                           reinterpret_cast<const uint4*>(gout), N, H, W, C / 8, Ho, Wo,
-                                                           pad_t, pad_l, reinterpret_cast<uint4*>(gx), fp16);
-  return cudaGetLastError();
-}
-
 int maxpool_relu_bwd_rows(int N, int H, int W) {
   return N * ((H + kPoolTileH - 1) / kPoolTileH) * ((W + kPoolTileW - 1) / kPoolTileW);
 }
@@ -523,14 +384,6 @@ cudaError_t launch_upsample2(const void* in, int N, int P, int Q, int C, void* o
   const size_t total = (size_t)N * H * W * (C / 8);
   upsample2_kernel<<<flat_grid(total, 256), 256, 0, s>>>(reinterpret_cast<const uint4*>(in), N, P, Q, C / 8,
                                                          reinterpret_cast<uint4*>(out), H, W);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_scatter_add2(const void* d, int N, int P, int Q, int C, void* gx, int H, int W, int fp16,
-                                cudaStream_t s) {
-  const size_t total = (size_t)N * P * Q * (C / 8);
-  scatter_add2_kernel<<<flat_grid(total, 256), 256, 0, s>>>(reinterpret_cast<const uint4*>(d), N, P, Q, C / 8,
-                                                            reinterpret_cast<uint4*>(gx), H, W, fp16);
   return cudaGetLastError();
 }
 

@@ -279,13 +279,9 @@ int alloc_buf(dgp_handle* h, Plan* pl, size_t bytes, void** out) {
 }
 
 // Staging buffers per epilogue warp (2 KB each, 16 warps): the residual prefetch runs epi_bufs-1 units ahead.
-// DGP_EPI_BUFS_RES / DGP_EPI_BUFS override the defaults (A/B experiments).
 int epi_bufs_for(bool residual, int block_n) {
-  const char* e = getenv(residual ? "DGP_EPI_BUFS_RES" : "DGP_EPI_BUFS");
   // 64-wide layers (256-row tiles, one unit per warp and tile): a single buffer leaves room for a fourth smem stage
-  int v = e ? atoi(e) : ((!residual && block_n == 64) ? 1 : 2);
-  const int lo = residual ? 2 : 1;
-  return v < lo ? lo : (v > 4 ? 4 : v);
+  return (!residual && block_n == 64) ? 1 : 2;
 }
 
 // Epilogue configuration: bf16 outputs whose tile width is a multiple of 64 go through the TMA-staged epilogue
@@ -317,8 +313,8 @@ int setup_epilogue(dgp_handle* h, ConvGemmParams& g, const char* scope, int n_im
   // issue overhead of the single-warp producer / MMA loops (see DESIGN.md "BLOCK_M = 256")
   g.msub = (g.epi_mode == 1 && g.block_n <= 128 && g.M > kBlockM) ? 2 : 1;
   // 256-wide tiles of big layers run as CTA pairs (cta_group::2): a single-CTA M=128 x N=256 MMA reads 12 KB of operands
-  // from shared memory per K=16 step and is bound by that, the pair reads 8 KB per CTA.  DGP_NO_CTA2=1 disables (A/B).
-  g.cta2 = (g.epi_mode == 1 && g.block_n == 256 && g.M >= 4 * kBlockM && getenv("DGP_NO_CTA2") == nullptr) ? 1 : 0;
+  // from shared memory per K=16 step and is bound by that, the pair reads 8 KB per CTA.
+  g.cta2 = (g.epi_mode == 1 && g.block_n == 256 && g.M >= 4 * kBlockM) ? 1 : 0;
   g.num_m_blocks = ceil_div(g.M, g.cta2 ? 2 * kBlockM : kBlockM * g.msub);
   g.tmem_cols = tmem_cols_for(g.block_n * g.msub);
   g.num_stages = conv_gemm_pick_stages(g);
@@ -387,9 +383,9 @@ int make_gemm_step(dgp_handle* h, const ConvLayer& L, const void* x, int N, int 
   const char* e = nullptr;
   // 3x3 stride-1 convs over 64 channels (block 1 conv2 and its dgrad) run from a shared-memory resident input patch: the
   // im2col form re-reads every activation nine times from the L2 and is bound by the L2 -> SM fabric (~11 TB/s of
-  // distinct lines), not by the tensor pipe.  DGP_NO_PATCH_CONV=1 restores the im2col path (A/B, tests).
+  // distinct lines), not by the tensor pipe.
   const bool patch = L.R == 3 && L.S == 3 && L.stride == 1 && L.Cin == 64 && bn == 64 && L.Npad == 64 && !out_f32 && !residual &&
-                     lower_h == L.dil && lower_w == L.dil && getenv("DGP_NO_PATCH_CONV") == nullptr;
+                     lower_h == L.dil && lower_w == L.dil;
   if (patch) {
     g.a_mode = 3; g.epi_mode = 3; g.epi_bufs = 0; g.msub = 2;
     g.pt_rows = 14; g.pt_cols = 16;
@@ -471,7 +467,7 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
   // Inference plans run conv1 fused with pool1 (conv_gemm_kernel a_mode / epi_mode 2): conv1's output -- 20 MB per 747x832
   // frame, the largest tensor of the net -- never reaches HBM.  Training keeps it for the backward pass and debug runs
   // (dgp_debug_keep_activations) dump it: those plans (key -B for the debug one) run conv1 and the pool as two launches.
-  const bool unfused = train || h->debug_keep || getenv("DGP_NO_POOL_FUSION") != nullptr;
+  const bool unfused = train || h->debug_keep;
   auto key = std::make_tuple((!train && h->debug_keep) ? -B : B, H, W);
   auto& plans = train ? h->train_plans : h->plans;
   auto it = plans.find(key);
@@ -554,7 +550,6 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
     g.scale = L.scale; g.shift = L.shift; g.residual = nullptr; g.res_sub = 1; g.relu = 1;
     g.out_f32 = 0; g.ldc = 64; g.num_n_blocks = 1;
     uint32_t pixels_per_load;
-    bool resident = false;
     if (unfused) {
       g.a_mode = 1;
       g.out = c1;
@@ -566,32 +561,18 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
       g.epi_mode = 2; g.epi_bufs = 0; g.msub = 2;
       g.out = xa;
       g.pool_H = Hc; g.pool_W = Wc; g.pool_pad_t = pad_t; g.pool_pad_l = pad_l;
-      // Measured (profiles/r02_conv1_variants.md): both variants are bound by the SM's shared-memory port (UMMA operand reads
-      // of the 64-wide tile + the pooling epilogue's patch traffic), the resident one needs 20 % more tiles (48 instead of
-      // 56 pooled pixels per 256 accumulator rows) and is the slower of the two; it stays as DGP_CONV1_RESIDENT=1.
-      resident = getenv("DGP_CONV1_RESIDENT") != nullptr;
-      if (resident) {
-        // a tile = 4 x 12 pooled pixels <- 9 x 25 conv1 outputs <- a 12 x 28 patch of space-to-depth pixels that stays in
-        // shared memory: the accumulator rows run over the patch grid (9 x 28 = 252 of 256), every tap is a shifted view
-        g.a_mode = 4; g.pool_R = 4; g.pool_C = 12;
-        g.pt_wp = 2 * g.pool_C + 4;
-        g.pt_stage_bytes = ((256 + 3 * g.pt_wp + 3) * 32 + 1023) / 1024 * 1024;
-        g.num_stages = 3;
-      } else {
-        // a tile = the 15 x 17 patch of conv1 outputs (255 of the 256 accumulator rows) under 7 x 8 pooled pixels, loaded
-        // per filter row as one tiled box of overlapping 4-pixel windows (10x read amplification out of the L2)
-        g.a_mode = 2; g.pool_R = 7; g.pool_C = 8;
-      }
+      // a tile = the 15 x 17 patch of conv1 outputs (255 of the 256 accumulator rows) under 7 x 8 pooled pixels, loaded
+      // per filter row as one tiled box of overlapping 4-pixel windows (10x read amplification out of the L2).  Measured
+      // (profiles/r02_conv1_variants.md) against a since-removed variant that kept a patch of space-to-depth pixels resident
+      // in shared memory: both are bound by the SM's shared-memory port, and the resident one needed 20 % more tiles.
+      g.a_mode = 2; g.pool_R = 7; g.pool_C = 8;
       g.pool_tiles_i = ceil_div(Hc, g.pool_R); g.pool_tiles_j = ceil_div(Wc, g.pool_C);
       g.num_m_blocks = B * g.pool_tiles_i * g.pool_tiles_j;
       g.tmem_cols = tmem_cols_for(64 * g.msub);
-      if (!resident) g.num_stages = conv_gemm_pick_stages(g);
+      g.num_stages = conv_gemm_pick_stages(g);
       pixels_per_load = 0;
     }
-    const char* e = resident
-        ? make_tmap_tiled4d(&g.tmap_a, pl->s2d, 16, (uint64_t)pl->Ws, (uint64_t)pl->Hs, (uint64_t)B, 32, (uint64_t)pl->Ws * 32,
-                            (uint64_t)pl->Hs * pl->Ws * 32, (uint32_t)g.pt_wp, (uint32_t)(2 * g.pool_R + 4))
-        : unfused
+    const char* e = unfused
         ? make_tmap_im2col(&g.tmap_a, pl->s2d, 64, (uint64_t)pl->W1, (uint64_t)pl->Hs, (uint64_t)B, 32, (uint64_t)pl->Ws * 32,
                            (uint64_t)pl->Hs * pl->Ws * 32, 0, 0, 0, -3, 1, (uint64_t)B * pl->Hs * pl->Ws * 32, pixels_per_load)
         : make_tmap_tiled4d(&g.tmap_a, pl->s2d, 64, (uint64_t)pl->W1, (uint64_t)pl->Hs, (uint64_t)B, 32, (uint64_t)pl->Ws * 32,
@@ -1241,7 +1222,7 @@ int dgp_estimate_pose_host(dgp_handle* h, const uint8_t* frames_host, int T, int
     CU_OK(h, cudaStreamWaitEvent(s, h->ev_copied[slot], 0));
     // the tail batch of a multi-batch video reuses the full-batch plan (see dgp_estimate_pose_stream): surplus rows hold an
     // earlier batch's frames and their read-outs are not copied back
-    const int run_b = (b < batch && it > 0 && getenv("DGP_STREAM_NO_PAD") == nullptr) ? batch : b;
+    const int run_b = (b < batch && it > 0) ? batch : b;
     if ((rc = dgp_forward(h, (const uint8_t*)h->st_frames2[slot].p, run_b, H, W, (float*)h->st_logits.p, nullptr, s))) return rc;
     CU_OK(h, cudaEventRecord(h->ev_consumed[slot], s));
     if ((rc = dgp_softargmax(h, (const float*)h->st_logits.p, nullptr, run_b, ho, wo, nj, gamma, gauss_len,

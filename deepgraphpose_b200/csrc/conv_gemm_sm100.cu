@@ -162,11 +162,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int stages = p.num_stages;
   const int msub = p.msub;                     // 128-row sub-tiles per CTA tile (BLOCK_M = 128 * msub)
-  const int a_bytes = p.a_mode >= 3 ? p.pt_stage_bytes : msub * kABytes;
+  const int a_bytes = p.a_mode == 3 ? p.pt_stage_bytes : msub * kABytes;
   const int b_bytes = (kCta2 ? p.block_n / 2 : p.block_n) * kBlockK * 2;   // a CTA pair splits the weight tile
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem + stages * a_bytes;
-  uint8_t* smem_epi = smem_b + (p.a_mode >= 3 ? p.num_k_blocks : stages) * b_bytes;  // [16 warps][epi_bufs][2 KiB], 1024 B aligned
+  uint8_t* smem_epi = smem_b + (p.a_mode == 3 ? p.num_k_blocks : stages) * b_bytes;  // [16 warps][epi_bufs][2 KiB], 1024 B aligned
   const int epi_bufs = p.epi_mode == 1 ? p.epi_bufs : 0;
   float* smem_ss = reinterpret_cast<float*>(smem_epi + (p.epi_mode == 2 ? 2 * kPatchBytes : kEpiWarps * epi_bufs * kEpiUnitBytes));  // [16 warps][2 sets][scale 32 | shift 32]
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_ss + kEpiWarps * 128);
@@ -253,32 +253,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
         if (lane == 0) {
           ptx::mbar_arrive_expect_tx(&full_bar[stage], box_bytes);
           ptx::tma_load_4d(smem_a + stage * a_bytes, &p.tmap_a, &full_bar[stage], 0, tj * p.pt_cols - dil, ti * p.pt_rows - dil, img);
-        }
-        __syncwarp();
-        if (++stage == stages) {
-          stage = 0;
-          phase ^= 1;
-        }
-      }
-    } else if (!kCta2 && a_mode == 4) {
-      // conv1 + pool1 from a resident space-to-depth patch: all weights once, then one tiled box per tile
-      const int tiles_j = p.pool_tiles_j, tiles_ij = p.pool_tiles_i * tiles_j;
-      const uint32_t box_bytes = (uint32_t)(p.pt_wp * (2 * p.pool_R + 4) * 32);
-      if (lane == 0) {
-        ptx::mbar_arrive_expect_tx(b_bar, (uint32_t)(nkb * b_bytes));
-        for (int kb = 0; kb < nkb; ++kb) ptx::tma_load_2d(smem_b + kb * b_bytes, &p.tmap_b, b_bar, kb * kBlockK, 0);
-      }
-      __syncwarp();
-      for (int tile = tile0; tile < num_tiles; tile += tstep) {
-        const int img = tile / tiles_ij;
-        const int rem = tile - img * tiles_ij;
-        const int ti = rem / tiles_j;
-        const int tj = rem - ti * tiles_j;
-        const int ra = max(0, 2 * ti * p.pool_R - p.pool_pad_t), ca = max(0, 2 * tj * p.pool_C - p.pool_pad_l);
-        ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (lane == 0) {
-          ptx::mbar_arrive_expect_tx(&full_bar[stage], box_bytes);
-          ptx::tma_load_4d(smem_a + stage * a_bytes, &p.tmap_a, &full_bar[stage], 0, ca, ra, img);
         }
         __syncwarp();
         if (++stage == stages) {
@@ -464,43 +438,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
         acc ^= 1;
         if (acc == 0) acc_phase ^= 1;
       }
-    } else if (!kCta2 && p.a_mode == 4) {
-      // conv1: 4 x 4 taps of 16 (space-to-depth) channels = sixteen K=16 MMAs per 128-row sub-tile; tap (kr, ks) reads
-      // patch rows m + kr*Wp + ks (32 B each, SWIZZLE_32B) and the weight slab at k-block kr, +ks*32 B
-      const int Wp = p.pt_wp;
-      const uint32_t a0 = ptx::smem_u32(smem_a);
-      ptx::mbar_wait(b_bar, 0);
-      ptx::tc_fence_after();
-      for (int tile = tile0; tile < num_tiles; tile += tstep) {
-        ptx::mbar_wait(&tmem_empty_bar[acc], acc_phase ^ 1);
-        ptx::mbar_wait(&full_bar[stage], phase);
-        ptx::tc_fence_after();
-        if (ptx::elect_one()) {
-          const uint32_t tmem_d = tmem_base + (uint32_t)acc * acc_cols;
-          const uint32_t abase = a0 + (uint32_t)(stage * a_bytes);
-#pragma unroll
-          for (int kr = 0; kr < 4; ++kr) {
-#pragma unroll
-            for (int ks = 0; ks < 4; ++ks) {
-              const uint64_t bdesc = bdesc0 + (uint64_t)(kr * b_step + ks * 2);
-#pragma unroll
-              for (int sub = 0; sub < 2; ++sub) {
-                const uint64_t adesc = ptx::make_desc_k_sw32(abase + (uint32_t)((kr * Wp + ks + sub * 128) * 32));
-                ptx::umma_bf16(tmem_d + (uint32_t)(sub * block_n), adesc, bdesc, idesc, (kr | ks) != 0);
-              }
-            }
-          }
-          ptx::umma_commit(&empty_bar[stage]);
-          ptx::umma_commit(&tmem_full_bar[acc]);
-        }
-        __syncwarp();
-        if (++stage == stages) {
-          stage = 0;
-          phase ^= 1;
-        }
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1;
-      }
     } else if (!kCta2 && msub == 2) run(std::integral_constant<int, 2>{});
     else run(std::integral_constant<int, 1>{});
     }  // leader CTA (or single-CTA kernel)
@@ -652,7 +589,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_gemm_kernel(const __grid_con
     }
     __syncwarp();
     const int R = p.pool_R, Cp = p.pool_C, H1 = p.P, W1 = p.Q;
-    const int Cw = p.a_mode == 4 ? p.pt_wp : 2 * p.pool_C + 1;   // accumulator rows per patch row
+    const int Cw = 2 * p.pool_C + 1;   // accumulator rows per patch row
     const int tiles_i = p.pool_tiles_i, tiles_j = p.pool_tiles_j;
     uint8_t* patch = smem_epi + grp * kPatchBytes;
     const uint32_t bar_id = 1u + (uint32_t)grp;
@@ -1028,10 +965,10 @@ const char* make_tmap_im2col(CUtensorMap* out, const void* base, uint64_t C, uin
 }
 
 size_t conv_gemm_smem_bytes(const ConvGemmParams& p) {
-  const size_t a_bytes = p.a_mode >= 3 ? (size_t)p.pt_stage_bytes : (size_t)p.msub * kABytes;
+  const size_t a_bytes = p.a_mode == 3 ? (size_t)p.pt_stage_bytes : (size_t)p.msub * kABytes;
   const size_t b_bytes = (size_t)(p.cta2 ? p.block_n / 2 : p.block_n) * kBlockK * 2;
   const size_t epi = p.epi_mode == 2 ? (size_t)2 * kPatchBytes : (p.epi_mode == 1 ? (size_t)kEpiWarps * p.epi_bufs * kEpiUnitBytes : 0);
-  return 1024 + (size_t)p.num_stages * a_bytes + (size_t)(p.a_mode >= 3 ? p.num_k_blocks : p.num_stages) * b_bytes + epi +
+  return 1024 + (size_t)p.num_stages * a_bytes + (size_t)(p.a_mode == 3 ? p.num_k_blocks : p.num_stages) * b_bytes + epi +
          kEpiWarps * 128 * sizeof(float) + (2 * kMaxStages + 4 + kEpiWarps * kMaxEpiBufs + 1) * 8 + 16;
 }
 
@@ -1052,7 +989,7 @@ const char* make_tmap_tiled4d(CUtensorMap* out, const void* base, uint64_t C, ui
                               uint64_t stride_w_bytes, uint64_t stride_h_bytes, uint64_t stride_n_bytes, uint32_t box_w,
                               uint32_t box_h) {
   if (const char* e = tma_init()) return e;
-  if (C != 64 && C != 16) return "make_tmap_tiled4d: 64 or 16 channels expected";
+  if (C != 64) return "make_tmap_tiled4d: 64 channels expected";
   cuuint64_t dims[4] = {C, W, H, N};
   cuuint64_t strides[3] = {stride_w_bytes, stride_h_bytes, stride_n_bytes};
   cuuint32_t box[4] = {(cuuint32_t)C, box_w, box_h, 1};
@@ -1060,7 +997,7 @@ const char* make_tmap_tiled4d(CUtensorMap* out, const void* base, uint64_t C, ui
   if (box_w > 256 || box_h > 256) return "make_tmap_tiled4d: box too large";
   CUresult r = g_encode_tiled(out, g_tmap_fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims,
                               strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                              C == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_32B,
+                              CU_TENSOR_MAP_SWIZZLE_128B,
                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     snprintf(g_err, sizeof(g_err), "cuTensorMapEncodeTiled (4-D) failed: %d", (int)r);

@@ -38,9 +38,7 @@ struct ConvGemmParams {
   int num_k_blocks;  // K / 64
   int a_mode;        // 0 = tiled [M,K], 1 = im2col, 2 = im2col by 2-D patches (conv1 fused with the 3x3/2 max-pool),
                      // 3 = shared-memory resident input patch (3x3 stride-1 convs with 64 input channels): ONE tiled TMA box
-                     //     per tile, the nine taps are row-shifted UMMA descriptors over it, all weights stay resident,
-                     // 4 = the same for conv1 fused with pool1: the space-to-depth input patch (32 B per pixel, SWIZZLE_32B)
-                     //     is resident, the 4x4 taps are K=16 MMAs over 32 B-shifted descriptors
+                     //     per tile, the nine taps are row-shifted UMMA descriptors over it, all weights stay resident
   int fp16;          // 0 = bf16 activations/weights (default), 1 = fp16 storage (same kind::f16 MMA, fp32 accumulate)
   // im2col geometry (a_mode == 1)
   int P, Q;          // output height / width
@@ -55,7 +53,7 @@ struct ConvGemmParams {
   int epi_mode;      // 0 = direct register->global stores (fp32 head GEMM), 1 = TMA-staged 16-bit (+ TMA residual),
                      // 2 = BN + ReLU + 3x3 stride-2 max-pool of a 2-D patch (a_mode 2), pooled pixels stored directly,
                      // 3 = direct masked 16-bit stores of a patch tile (a_mode 3)
-  int epi_bufs;      // 2 KB staging buffers per epilogue warp (epi_mode 1): 2..4; the residual prefetch runs epi_bufs-1 units ahead
+  int epi_bufs;      // 2 KB staging buffers per epilogue warp (epi_mode 1): 1 or 2; the residual prefetch runs epi_bufs-1 units ahead
   const __nv_bfloat16* residual;  // nullptr = none
   int res_sub;       // 1 = same pixel grid as the output, 2 = residual grid is (res_H, res_W), read at (2p, 2q)
   int res_H, res_W;
@@ -104,9 +102,6 @@ cudaError_t launch_wgrad_gemm(const WgradParams& p, int num_sms, cudaStream_t st
 cudaError_t launch_wgrad_reduce(const WgradParams& p, const float* rowscale, const float* mask, float* grad,
                                 const GradMode* mode, cudaStream_t stream, const float* wmaster = nullptr,
                                 float* rowdot_part = nullptr);
-// dgamma = (row sums of rowdot_part - mean * dbeta) / sqrt(var + eps)  (frozen BN; exact, no division by gamma)
-cudaError_t launch_bn_gamma_grad(const float* rowdot_part, int Cout, int Kw, const float* mean, const float* var, float eps,
-                                 const float* dbeta, float* dgamma, cudaStream_t stream);
 
 // Host helpers (conv_gemm_sm100.cu)
 void tmap_set_fp16(int fp16);  // element type of subsequently encoded tensor maps
@@ -121,7 +116,7 @@ const char* make_tmap_im2col(CUtensorMap* out, const void* base, uint64_t C, uin
                              uint32_t pixels_per_column = kBlockM, uint32_t channels_per_pixel = kBlockK);
 // a_mode 3: patch stage bytes (1024-aligned) for a tile geometry, and the tiled 4-D activation map (box = whole input patch)
 int conv_patch_stage_bytes(int pt_wp, int dil);
-// C = 64 channels per pixel (128 B rows, SWIZZLE_128B) or 16 (32 B rows, SWIZZLE_32B)
+// C = 64 channels per pixel (128 B rows, SWIZZLE_128B)
 const char* make_tmap_tiled4d(CUtensorMap* out, const void* base, uint64_t C, uint64_t W, uint64_t H, uint64_t N,
                               uint64_t stride_w_bytes, uint64_t stride_h_bytes, uint64_t stride_n_bytes, uint32_t box_w,
                               uint32_t box_h);

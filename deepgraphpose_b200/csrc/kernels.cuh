@@ -123,17 +123,11 @@ int relu_bn_bwd_blocks(int M, int C);  // rows of `partial` ([blocks][C])
 // scatter_d != nullptr: g (N,H,W,C) += zero-inserted scatter_d (N,P,Q,C) first (gradient of the stride-2 identity shortcut)
 cudaError_t launch_relu_bn_bwd(void* g, const void* act, int M, int C, float* partial, int fp16, cudaStream_t s,
                                const void* scatter_d = nullptr, int H = 0, int W = 0, int P = 0, int Q = 0);
-cudaError_t launch_bn_grad_finalize(const float* partial, int nblocks, int C, float* dbeta_a, float* dbeta_b, cudaStream_t s);
-// arg_ws: N*Ho*Wo*C bytes (first-maximum position of every pooled element)
 // fused root of the backward: max-pool gradient + conv1 ReLU mask + dy sums ([maxpool_relu_bwd_rows][64] partial rows)
 int maxpool_relu_bwd_rows(int N, int H, int W);
 cudaError_t launch_maxpool_relu_bwd(const void* x, const void* gout, int N, int H, int W, int C, int Ho, int Wo, int pad_t,
                                     int pad_l, void* gx, float* partial, int fp16, cudaStream_t s);
-cudaError_t launch_maxpool_bwd(const void* x, const void* gout, int N, int H, int W, int C, int Ho, int Wo, int pad_t,
-                               int pad_l, void* arg_ws, void* gx, int fp16, cudaStream_t s);
 cudaError_t launch_upsample2(const void* in, int N, int P, int Q, int C, void* out, int H, int W, cudaStream_t s);
-cudaError_t launch_scatter_add2(const void* d, int N, int P, int Q, int C, void* gx, int H, int W, int fp16,
-                                cudaStream_t s);
 cudaError_t launch_col2im_bwd(const float* g_logits, const float* g_locref, int N, int h, int w, int ctot, int nj,
                               void* dG, int Kd, int fp16, cudaStream_t s);
 int head_bias_blocks();

@@ -299,17 +299,6 @@ __device__ __forceinline__ uint64_t make_desc_k_sw128(uint32_t smem_addr, uint32
   return d;
 }
 
-// K-major, SWIZZLE_32B descriptor: rows of 32 B (one K = 16 slab of 16-bit elements), 8-row groups 256 B apart.
-__device__ __forceinline__ uint64_t make_desc_k_sw32(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(256 >> 4) << 32;   // SBO = 256 B between 8-row groups
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)6 << 61;            // SWIZZLE_32B
-  return d;
-}
-
 // Instruction descriptor for kind::f16, A=B=bf16 (K-major both), D=fp32, M x N tile.
 // Bit layout: cute::UMMA::InstrDescriptor.
 __host__ __device__ __forceinline__ uint32_t make_idesc_bf16_f32(int M, int N, int fp16 = 0) {

@@ -6,7 +6,6 @@
 #include "../../include/dgp_b200.h"
 
 #include <cuda_runtime.h>
-#include <stdlib.h>
 
 #include <condition_variable>
 #include <deque>
@@ -151,7 +150,6 @@ int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user,
   int64_t t0 = 0;
   int it = 0;
   bool full_batch_seen = false;
-  const bool no_pad = getenv("DGP_STREAM_NO_PAD") != nullptr;   // A/B switch for the short-batch rule below
   int status = DGP_OK;
   cudaError_t ce = cudaSuccess;
   for (;;) {
@@ -175,7 +173,7 @@ int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user,
     // every frame's arithmetic is independent of its batch, the surplus rows of the device slot hold an earlier batch's
     // frames, and only the first f.n read-outs are copied back.  Building a second plan for it would cost far more than the
     // surplus frames (allocation of every activation, tensor maps, first-use kernel loads).
-    const int run_n = (f.n < batch && full_batch_seen && !no_pad) ? batch : f.n;
+    const int run_n = (f.n < batch && full_batch_seen) ? batch : f.n;
     if (f.n == batch) full_batch_seen = true;
     if ((status = dgp_forward(h, (const uint8_t*)h->st_frames2[dslot].p, run_n, H, W, (float*)h->st_logits.p, nullptr, s))) break;
     if ((ce = cudaEventRecord(h->ev_consumed[dslot], s)) != cudaSuccess) break;

@@ -18,8 +18,6 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
-#include <limits.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <dlfcn.h>
@@ -148,15 +146,6 @@ namespace nccl {
 typedef struct { char internal[128]; } UniqueId;     // ncclUniqueId (NCCL_UNIQUE_ID_BYTES = 128)
 typedef int (*GetUniqueIdFn)(UniqueId*);
 typedef int (*CommInitRankFn)(void**, int, UniqueId, int);
-// ncclConfig_t as of NCCL 2.14 (the prefix every later version keeps; `size` / `version` tell the library which fields are set)
-struct ConfigV21400 {
-  size_t size;
-  unsigned int magic;
-  unsigned int version;
-  int blocking, cgaClusterSize, minCTAs, maxCTAs;
-  const char* netName;
-};
-typedef int (*CommInitRankConfigFn)(void**, int, UniqueId, int, ConfigV21400*);
 typedef int (*CommDestroyFn)(void*);
 typedef int (*CommCountFn)(void*, int*);
 typedef int (*AllReduceFn)(const void*, void*, size_t, int, int, void*, cudaStream_t);
@@ -166,7 +155,6 @@ constexpr int kFloat = 7, kSum = 0;                  // ncclFloat32, ncclSum
 struct Api {
   GetUniqueIdFn get_unique_id = nullptr;
   CommInitRankFn comm_init_rank = nullptr;
-  CommInitRankConfigFn comm_init_rank_config = nullptr;   // optional (NCCL >= 2.14)
   CommDestroyFn comm_destroy = nullptr;
   CommCountFn comm_count = nullptr;
   AllReduceFn all_reduce = nullptr;
@@ -185,7 +173,6 @@ const Api& api() {
   if (!lib) return a;
   a.get_unique_id = (GetUniqueIdFn)dlsym(lib, "ncclGetUniqueId");
   a.comm_init_rank = (CommInitRankFn)dlsym(lib, "ncclCommInitRank");
-  a.comm_init_rank_config = (CommInitRankConfigFn)dlsym(lib, "ncclCommInitRankConfig");
   a.comm_destroy = (CommDestroyFn)dlsym(lib, "ncclCommDestroy");
   a.comm_count = (CommCountFn)dlsym(lib, "ncclCommCount");
   a.all_reduce = (AllReduceFn)dlsym(lib, "ncclAllReduce");
@@ -219,10 +206,29 @@ int refresh_dgrad_weights(dgp_handle* h, cudaStream_t s) {
   return DGP_OK;
 }
 
+// Pushes the dgrad GEMM `gp`, which writes `out`.  mask_act != nullptr: `out` is the gradient w.r.t. the post-ReLU tensor
+// mask_act (same shape); when the GEMM runs the staged epilogue, that epilogue also applies its consumer's dy = g * [act > 0]
+// and leaves the per-channel sums of dy (conv_gemm_kernel kMask) in a [ceil(M/32)][N] region of bw->bn_part reserved here.
+// Returns the region's offset, or -1 when the caller has to add the stand-alone mask pass.
+long long push_dgrad_gemm(dgp_handle* h, Backward* bw, ConvGemmParams gp, void* out, const void* mask_act) {
+  long long off = -1;
+  if (mask_act != nullptr && gp.epi_mode == 1) {
+    off = (long long)bw->bn_part_floats;
+    bw->bn_part_floats += (size_t)ceil_div(gp.M, 32) * gp.N;
+    gp.mask_act = mask_act;
+  }
+  const int sms = h->num_sms;
+  bw->steps.push_back({5, 1, [gp, sms, bw, off](cudaStream_t s) {
+                         ConvGemmParams g = gp;
+                         if (off >= 0) g.colsum_part = bw->bn_part + off;
+                         return launch_conv_gemm(g, sms, s);
+                       }});
+  bw->steps.back().wr = out;
+  return off;
+}
+
 // dgrad of layer L as a stride-1 conv of dy (N,H,W,L.Cout) with the transposed / flipped operand -> out (N,H,W,L.Cin).
-// mask_act != nullptr: `out` is the gradient w.r.t. the post-ReLU tensor mask_act (same shape); its consumer's
-// dy = g * [act > 0] and the per-channel sums of dy are produced by this GEMM's epilogue (conv_gemm_kernel kMask) when the layer
-// runs the staged epilogue.  Returns through *fused whether that happened (else the caller adds the stand-alone mask pass).
+// mask_act / *site: see push_dgrad_gemm.
 int add_dgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, W16* wd, const void* dy, int N, int H, int W, void* out,
               const void* residual, const void* mask_act = nullptr, long long* site = nullptr) {
   ConvLayer D;
@@ -237,22 +243,8 @@ int add_dgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, W16* wd, const vo
   int rc = make_gemm_step(h, D, dy, N, H, W, (L.R == 1 && L.S == 1) ? 0 : 1, out, false, (const __nv_bfloat16*)residual, 1, H,
                           W, 0, &st, &Ho, &Wo);
   if (rc) return rc;
-  const bool fuse = mask_act != nullptr && st.gp.epi_mode == 1 && getenv("DGP_NO_MASK_FUSION") == nullptr;
-  long long off = -1;
-  if (fuse) {
-    off = (long long)bw->bn_part_floats;                                   // this site's [ceil(M/32)][N] region
-    bw->bn_part_floats += (size_t)ceil_div(st.gp.M, 32) * st.gp.N;
-    st.gp.mask_act = mask_act;
-  }
+  const long long off = push_dgrad_gemm(h, bw, st.gp, out, mask_act);
   if (site) *site = off;
-  const ConvGemmParams gp = st.gp;
-  const int sms = h->num_sms;
-  bw->steps.push_back({5, 1, [gp, sms, bw, off](cudaStream_t s) {
-                         ConvGemmParams g = gp;
-                         if (off >= 0) g.colsum_part = bw->bn_part + off;
-                         return launch_conv_gemm(g, sms, s);
-                       }});
-  bw->steps.back().wr = out;
   return DGP_OK;
 }
 
@@ -400,21 +392,7 @@ int build_backward(dgp_handle* h, Plan* pl) {
     rc = make_gemm_step(h, D, dG, B, hf, wf, 0, gbuf[0], false, nullptr, 1, 0, 0, 0, &st, &Ho, &Wo);
     if (rc) return rc;
     // gbuf[0] is the gradient w.r.t. block4's output: the last unit's junction mask rides in this GEMM's epilogue
-    if (st.gp.epi_mode == 1 && getenv("DGP_NO_MASK_FUSION") == nullptr) {
-      st.gp.mask_act = pl->feat;
-      g_site = (long long)bw->bn_part_floats;
-      bw->bn_part_floats += (size_t)ceil_div(st.gp.M, 32) * st.gp.N;
-    }
-    const ConvGemmParams gp = st.gp;
-    const int sms = h->num_sms;
-    const long long off = g_site;
-    Backward* bwp = bw.get();
-    bw->steps.push_back({5, 1, [gp, sms, bwp, off](cudaStream_t s) {
-                           ConvGemmParams g = gp;
-                           if (off >= 0) g.colsum_part = bwp->bn_part + off;
-                           return launch_conv_gemm(g, sms, s);
-                         }});
-    bw->steps.back().wr = gbuf[0];
+    g_site = push_dgrad_gemm(h, bw.get(), st.gp, gbuf[0], pl->feat);
   }
 
   // ---- bottleneck units, last to first.  G = gradient w.r.t. the unit output (then d in place).
@@ -454,7 +432,7 @@ int build_backward(dgp_handle* h, Plan* pl) {
     if ((rc = add_wgrad(h, bw.get(), L1, ub.x, B, ub.H, ub.W, 0, gt1, &ws_need))) return rc;
     // the GEMM that completes Gx (gradient w.r.t. this unit's input = the previous unit's post-ReLU output) also applies that
     // unit's junction mask -- except for the first unit (its input is the max-pool output) and the stride-2 identity shortcuts
-    // (scatter_add2 still adds into Gx afterwards)
+    // (their scatter-add into Gx rides in the previous unit's stand-alone junction mask)
     const void* junction_act = i > 0 ? ub.x : nullptr;
     g_site = -1;
     if (Ls) {
@@ -464,16 +442,13 @@ int build_backward(dgp_handle* h, Plan* pl) {
     } else if (u.stride == 1) {
       if ((rc = add_dgrad(h, bw.get(), L1, ts->wd[u.conv1], gt1, B, ub.H, ub.W, Gx, G, junction_act, &g_site))) return rc;
     } else {
+      if (i == 0)
+        return fail(h, DGP_ERR_STATE, "backward plan: %s: a stride-2 identity shortcut in the first unit is not supported",
+                    u.scope.c_str());
       if ((rc = add_dgrad(h, bw.get(), L1, ts->wd[u.conv1], gt1, B, ub.H, ub.W, Gx, nullptr))) return rc;
-      const int P = ub.Ho, Q = ub.Wo, H = ub.H, W = ub.W, C = u.depth;
-      if (i > 0 && getenv("DGP_NO_SCATTER_FUSION") == nullptr) {
-        // Gx[n,2p,2q] += G[n,p,q] rides in the previous unit's junction mask (the next step of this plan; G stays intact until
-        // then: it is that unit's third buffer, written only after its mask)
-        scatter.d = G; scatter.H = H; scatter.W = W; scatter.P = P; scatter.Q = Q;
-      } else {
-        bw->steps.push_back({7, 1, [=](cudaStream_t s) { return launch_scatter_add2(G, B, P, Q, C, Gx, H, W, fp16, s); }});
-        bw->steps.back().wr = Gx;
-      }
+      // Gx[n,2p,2q] += G[n,p,q] rides in the previous unit's junction mask (the next step of this plan; G stays intact until
+      // then: it is that unit's third buffer, written only after its mask)
+      scatter.d = G; scatter.H = ub.H; scatter.W = ub.W; scatter.P = ub.Ho; scatter.Q = ub.Wo;
     }
     gi = (gi + 1) % 3;
     if (ts->early_cnt > 0 && u.shortcut >= 0 && h->layers[u.shortcut].w_off == ts->early_off) bw->early_step = (int)bw->steps.size();
@@ -487,24 +462,16 @@ int build_backward(dgp_handle* h, Plan* pl) {
     const void* c1 = pl->c1;
     const int H1 = pl->H1, W1 = pl->W1, Hp = pl->Hp, Wp = pl->Wp, pt = pl->pool_pad_t, plft = pl->pool_pad_l;
     const ConvLayer& L = h->layers[h->conv1_layer];
-    if (getenv("DGP_NO_POOL_BWD_FUSION") == nullptr) {
-      // max-pool gradient + conv1's ReLU mask + dy sums in one pass (bwd_kernels.cu: maxpool_relu_bwd_kernel)
-      const long long site = (long long)bw->bn_part_floats;
-      const int rows = maxpool_relu_bwd_rows(B, H1, W1);
-      bw->bn_part_floats += (size_t)rows * 64;
-      Backward* bwp = bw.get();
-      bw->steps.push_back({7, 1, [=](cudaStream_t s) {
-                             return launch_maxpool_relu_bwd(c1, Gp, B, H1, W1, 64, Hp, Wp, pt, plft, g_c1, bwp->bn_part + site, fp16, s);
-                           }});
-      bw->steps.back().wr = g_c1;
-      add_mask(h, bw.get(), g_c1, c1, B * H1 * W1, 64, &L, nullptr, site, rows);
-    } else {
-      void* arg_ws = nullptr;
-      if ((rc = alloc_buf(h, pl, (size_t)B * Hp * Wp * 64 + 1024, &arg_ws))) return rc;
-      bw->steps.push_back({7, 2, [=](cudaStream_t s) { return launch_maxpool_bwd(c1, Gp, B, H1, W1, 64, Hp, Wp, pt, plft, arg_ws, g_c1, fp16, s); }});
-      bw->steps.back().wr = g_c1;
-      add_mask(h, bw.get(), g_c1, c1, B * H1 * W1, 64, &L, nullptr);
-    }
+    // max-pool gradient + conv1's ReLU mask + dy sums in one pass (bwd_kernels.cu: maxpool_relu_bwd_kernel)
+    const long long site = (long long)bw->bn_part_floats;
+    const int rows = maxpool_relu_bwd_rows(B, H1, W1);
+    bw->bn_part_floats += (size_t)rows * 64;
+    Backward* bwp = bw.get();
+    bw->steps.push_back({7, 1, [=](cudaStream_t s) {
+                           return launch_maxpool_relu_bwd(c1, Gp, B, H1, W1, 64, Hp, Wp, pt, plft, g_c1, bwp->bn_part + site, fp16, s);
+                         }});
+    bw->steps.back().wr = g_c1;
+    add_mask(h, bw.get(), g_c1, c1, B * H1 * W1, 64, &L, nullptr, site, rows);
     WgradParams wp;
     memset(&wp, 0, sizeof(wp));
     tmap_set_fp16(h->fp16);
@@ -627,8 +594,7 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
     // tail hide under the dgrad GEMMs instead of being serialised between them.  Joins: before a main-branch step that
     // overwrites the buffer a pending wgrad reads, before every bucket event, before the final gamma/beta pass.
     cudaError_t ce = cudaSuccess;
-    const bool two = getenv("DGP_BWD_ONE_STREAM") == nullptr;
-    if (two && !ts->side_stream) ce = cudaStreamCreateWithFlags(&ts->side_stream, cudaStreamNonBlocking);
+    if (!ts->side_stream) ce = cudaStreamCreateWithFlags(&ts->side_stream, cudaStreamNonBlocking);
     size_t ev_next = 0;
     auto next_event = [&](cudaEvent_t* out) -> cudaError_t {
       if (ev_next == ts->branch_events.size()) {
@@ -650,7 +616,7 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
     int k = 0;
     for (const BStep& st : bw->steps) {
       if (ce != cudaSuccess) break;
-      if (two && st.kind == 6 && st.rd != nullptr) {
+      if (st.kind == 6 && st.rd != nullptr) {
         cudaEvent_t fork = nullptr, done = nullptr;
         if ((ce = next_event(&fork)) != cudaSuccess || (ce = next_event(&done)) != cudaSuccess) break;
         if ((ce = cudaEventRecord(fork, h->stream)) != cudaSuccess) break;
@@ -1120,25 +1086,7 @@ int dgp_comm_init_rank(dgp_handle* h, const char* id128, int nranks, int rank) {
   nccl::UniqueId id;
   memcpy(id.internal, id128, 128);
   void* comm = nullptr;
-  // DGP_NCCL_MAX_CTAS > 0 caps the communicator's CTAs (ncclConfig_t::maxCTAs).  The all-reduce is hidden behind the backward
-  // pass and needs little bandwidth (94 MB in ~5 ms), so fewer CTAs could mean fewer SMs taken from the GEMMs it runs beside;
-  // measured on 2 and 8 B200 the cap (2 / 4 / 8 / 16) changes nothing (8.13-8.20 ms per step at dp8 either way: the 4 % over
-  // dp1 are the slowest of eight power-capped GPUs plus the HBM / NVLink traffic itself), so the default is NCCL's own choice.
-  int max_ctas = 0;
-  if (const char* e = getenv("DGP_NCCL_MAX_CTAS")) max_ctas = atoi(e);
-  if (max_ctas > 0 && nccl::api().comm_init_rank_config) {
-    nccl::ConfigV21400 cfg;
-    cfg.size = sizeof(cfg);
-    cfg.magic = 0xcafebeef;
-    cfg.version = 21400;                      // NCCL_VERSION(2, 14, 0)
-    cfg.blocking = cfg.cgaClusterSize = cfg.minCTAs = INT_MIN;   // NCCL_CONFIG_UNDEF_INT
-    cfg.maxCTAs = max_ctas;
-    cfg.netName = nullptr;                    // NCCL_CONFIG_UNDEF_PTR
-    const int rc_cfg = nccl::api().comm_init_rank_config(&comm, nranks, id, rank, &cfg);
-    if (rc_cfg != 0) return fail(h, DGP_ERR_CUDA, "ncclCommInitRankConfig(maxCTAs=%d): %s", max_ctas, nccl::api().err_str(rc_cfg));
-  } else {
-    NCCL_OK(h, nccl::api().comm_init_rank(&comm, nranks, id, rank));
-  }
+  NCCL_OK(h, nccl::api().comm_init_rank(&comm, nranks, id, rank));
   h->train->comm = comm;
   h->train->comm_owned = true;
   h->train->comm_world = nranks;

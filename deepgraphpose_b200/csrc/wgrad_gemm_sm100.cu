@@ -300,23 +300,6 @@ __global__ void __launch_bounds__(256) wgrad_reduce_kernel(const float* __restri
   *g = acc;
 }
 
-// dgamma[c] = (sum_kk rowdot_part[c][kk] - mean[c] * dbeta[c]) / sqrt(var[c] + eps): one warp per channel, lane-strided sums
-// then a fixed shuffle tree (bitwise reproducible).  No division by gamma: channels with gamma = 0 get their true gradient.
-__global__ void __launch_bounds__(256) bn_gamma_grad_kernel(const float* __restrict__ rowdot_part, int Cout, int K4,
-                                                            const float* __restrict__ mean, const float* __restrict__ var,
-                                                            float eps, const float* __restrict__ dbeta,
-                                                            float* __restrict__ dgamma) {
-  const int c = blockIdx.x * 8 + (threadIdx.x >> 5);
-  const int lane = threadIdx.x & 31;
-  if (c >= Cout) return;
-  const float* row = rowdot_part + (size_t)c * K4;
-  float a = 0.0f;
-  for (int i = lane; i < K4; i += 32) a += row[i];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-  if (lane == 0) dgamma[c] = (a - mean[c] * dbeta[c]) * rsqrtf(var[c] + eps);
-}
-
 }  // namespace
 
 void wgrad_plan(WgradParams* p, int num_sms) {
@@ -367,12 +350,6 @@ cudaError_t launch_wgrad_reduce(const WgradParams& p, const float* rowscale, con
     wgrad_reduce_kernel<1><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(p.partials, p.Cout, p.Kw, p.num_n_blocks,
                                                                               p.splits, rowscale, mask, grad, mode, wmaster, rowdot_part);
   }
-  return cudaGetLastError();
-}
-
-cudaError_t launch_bn_gamma_grad(const float* rowdot_part, int Cout, int Kw, const float* mean, const float* var, float eps,
-                                 const float* dbeta, float* dgamma, cudaStream_t stream) {
-  bn_gamma_grad_kernel<<<(Cout + 7) / 8, 256, 0, stream>>>(rowdot_part, Cout, Kw / 4, mean, var, eps, dbeta, dgamma);
   return cudaGetLastError();
 }
 

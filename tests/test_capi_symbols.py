@@ -58,6 +58,17 @@ def test_product_never_imports_oracle():
             assert not re.search(r"^\s*(from|import)\s+oracle", src, flags=re.M), fn
 
 
+def test_library_reads_only_the_plan_printing_env_var():
+    """What the library computes depends on its inputs alone: the one environment variable it reads prints the plan."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    csrc = os.path.join(root, "deepgraphpose_b200", "csrc")
+    args = []
+    for fn in sorted(os.listdir(csrc)):
+        src = open(os.path.join(csrc, fn)).read()
+        args += [(fn, a.strip()) for a in re.findall(r"\bgetenv\s*\(([^)]*)\)", src)]
+    assert [a for _, a in args] == ['"DGP_DEBUG_PLAN"'], args
+
+
 def test_ctypes_structs_match_the_header(tmp_path):
     """sizeof / offsetof of every struct of include/dgp_b200.h (compiled with gcc) against the ctypes mirrors in _lib.py."""
     import ctypes as C
