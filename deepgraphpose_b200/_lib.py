@@ -54,6 +54,11 @@ class DgpCyclicSource(C.Structure):
                 ("frame_bytes", C.c_size_t)]
 
 
+class DgpFrameTransform(C.Structure):
+    _fields_ = [("resize_h", C.c_int32), ("resize_w", C.c_int32), ("crop_x0", C.c_int32), ("crop_y0", C.c_int32),
+                ("crop_x1", C.c_int32), ("crop_y1", C.c_int32)]
+
+
 # reader(user, slot, max_frames, &direct) -> frames delivered (0 = end of video, < 0 = error)
 FRAME_READER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p))
 
@@ -84,6 +89,13 @@ SIGNATURES = {
     "dgp_estimate_pose_host": (_i, [_vp, _vp, _i, _i, _i, _i, _f, _f, _vp, _vp, _vp]),
     "dgp_estimate_pose_stream": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, _f, C.c_int64, _vp, _vp, _vp, _i64p]),
     "dgp_cyclic_reader": (_i, [_vp, _vp, _i, C.POINTER(_vp)]),
+    "dgp_transform_dims": (_i, [_i, _i, C.POINTER(DgpFrameTransform), C.POINTER(_i), C.POINTER(_i)]),
+    "dgp_resize_coefficients": (_i, [_i, _i, _i, _vp, _vp, _vp]),
+    "dgp_resize_crop": (_i, [_vp, _vp, _i, _i, _i, C.POINTER(DgpFrameTransform), _vp, _vp]),
+    "dgp_estimate_pose_host_transform": (_i, [_vp, _vp, _i, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f, _vp, _vp,
+                                              _vp]),
+    "dgp_estimate_pose_stream_transform": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f, C.c_int64,
+                                                _vp, _vp, _vp, _i64p]),
     "dgp_debug_keep_activations": (_i, [_vp, _i]),
     "dgp_debug_get_activation": (_i, [_vp, C.c_char_p, _vp, _sz, _i64p]),
     "dgp_conv2d": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _vp,

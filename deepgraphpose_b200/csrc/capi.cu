@@ -831,6 +831,9 @@ void dgp_destroy(dgp_handle* h) {
   cudaFree(h->st_mu.p);
   cudaFree(h->st_peak.p);
   cudaFree(h->st_lik.p);
+  cudaFree(h->st_xf.p);
+  cudaFree(h->resize_tmp.p);
+  for (auto& kv : h->resize_tables) cudaFree(kv.second.dev);
   for (auto& r : h->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
   for (auto e : h->ev_pool) cudaEventDestroy(e);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -1186,18 +1189,30 @@ int dgp_potentials(dgp_handle* h, const float* mu_dev, const float* mu_halo_next
 
 int dgp_estimate_pose_host(dgp_handle* h, const uint8_t* frames_host, int T, int H, int W, int batch, float gamma,
                            float gauss_len, float* mu_host, int32_t* peak_host, float* lik_host) {
+  return dgp_estimate_pose_host_transform(h, frames_host, T, H, W, nullptr, batch, gamma, gauss_len, mu_host, peak_host,
+                                          lik_host);
+}
+
+int dgp_estimate_pose_host_transform(dgp_handle* h, const uint8_t* frames_host, int T, int H0, int W0,
+                                     const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                     float* mu_host, int32_t* peak_host, float* lik_host) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_estimate_pose_host before dgp_finalize_weights");
   if (!frames_host || T < 0 || batch < 1 || !mu_host) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_host: bad argument");
+  int H, W;
+  bool identity;
+  if (transform_dims(H0, W0, transform, &H, &W, &identity))
+    return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_host: invalid frame size or transform");
   if (T == 0) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
   const int nj = h->cfg.num_joints;
   int hf, wf, ho, wo;
   dgp_output_dims(H, W, &hf, &wf, &ho, &wo);
-  const size_t frame_bytes = (size_t)H * W * 3;
+  const size_t frame_bytes = (size_t)H0 * W0 * 3;
   int rc;
   if ((rc = ensure(h, &h->st_frames2[0], frame_bytes * batch))) return rc;
   if ((rc = ensure(h, &h->st_frames2[1], frame_bytes * batch))) return rc;
+  if (!identity && (rc = ensure(h, &h->st_xf, (size_t)H * W * 3 * batch))) return rc;
   if ((rc = ensure(h, &h->st_logits, (size_t)batch * ho * wo * nj * 4))) return rc;
   if ((rc = ensure(h, &h->st_mu, (size_t)batch * nj * 2 * 4))) return rc;
   if ((rc = ensure(h, &h->st_peak, (size_t)batch * nj * 2 * 4))) return rc;
@@ -1223,7 +1238,12 @@ int dgp_estimate_pose_host(dgp_handle* h, const uint8_t* frames_host, int T, int
     // the tail batch of a multi-batch video reuses the full-batch plan (see dgp_estimate_pose_stream): surplus rows hold an
     // earlier batch's frames and their read-outs are not copied back
     const int run_b = (b < batch && it > 0) ? batch : b;
-    if ((rc = dgp_forward(h, (const uint8_t*)h->st_frames2[slot].p, run_b, H, W, (float*)h->st_logits.p, nullptr, s))) return rc;
+    const uint8_t* frames = (const uint8_t*)h->st_frames2[slot].p;
+    if (!identity) {
+      if ((rc = resize_crop_impl(h, frames, b, H0, W0, transform, (uint8_t*)h->st_xf.p, s))) return rc;
+      frames = (const uint8_t*)h->st_xf.p;
+    }
+    if ((rc = dgp_forward(h, frames, run_b, H, W, (float*)h->st_logits.p, nullptr, s))) return rc;
     CU_OK(h, cudaEventRecord(h->ev_consumed[slot], s));
     if ((rc = dgp_softargmax(h, (const float*)h->st_logits.p, nullptr, run_b, ho, wo, nj, gamma, gauss_len,
                              (float*)h->st_mu.p, (int32_t*)h->st_peak.p, (float*)h->st_lik.p, nullptr, nullptr, s)))

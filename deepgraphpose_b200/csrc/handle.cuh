@@ -13,6 +13,7 @@
 #include <memory>
 #include <string>
 #include <tuple>
+#include <utility>
 #include <vector>
 
 #include "conv_gemm_sm100.cuh"
@@ -91,6 +92,14 @@ struct Plan {
   uint64_t fwd_token = 0;     // train.cu: token of the dgp_train_forward whose activations the plan holds (0 = none)
 };
 
+// Pillow's fixed-point resample table of one (in, out) size pair (resize_kernels.cu): dev holds first[out] | count[out] |
+// weights[out][ksize] as int32; first / count are kept on the host for the launch geometry.
+struct ResizeTable {
+  int ksize = 0;
+  std::vector<int32_t> first, count;
+  int32_t* dev = nullptr;
+};
+
 }  // namespace dgp
 
 using namespace dgp;  // internal header: the handle's members are dgp:: types
@@ -149,6 +158,10 @@ struct dgp_handle {
   cudaStream_t copy_stream = nullptr;  // H2D of the next batch overlaps the current batch's kernels
   cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr};
   DevBuf st_frames2[2], st_logits, st_mu, st_peak, st_lik;
+  DevBuf st_xf;      // transformed (resized / cropped) batch that dgp_forward consumes when a frame transform is given
+  // dgp_resize_crop: tables per (in, out) size pair and the uint8 intermediate of the horizontal pass
+  std::map<std::pair<int, int>, ResizeTable> resize_tables;
+  DevBuf resize_tmp;
   // dgp_estimate_pose_stream: pinned host ring the reader thread decodes into (stream.cu)
   void* ring_slot[3] = {nullptr, nullptr, nullptr};
   size_t ring_bytes = 0;
@@ -191,6 +204,11 @@ int run_forward_plan(dgp_handle* h, Plan* pl, const uint8_t* frames_dev, float* 
 int ensure(dgp_handle* h, DevBuf* b, size_t bytes);
 int refresh_operands(dgp_handle* h, cudaStream_t s);
 void train_destroy(dgp_handle* h);  // train.cu
+// Size of a transformed frame (DGP_ERR_INVALID for an invalid transform); *identity: the transform leaves frames unchanged.
+int transform_dims(int H0, int W0, const dgp_frame_transform* t, int* H, int* W, bool* identity);
+// dgp_resize_crop without the device switch (resize_kernels.cu)
+int resize_crop_impl(dgp_handle* h, const uint8_t* src, int N, int H0, int W0, const dgp_frame_transform* t, uint8_t* dst,
+                     cudaStream_t s);
 
 inline cudaEvent_t prof_event(dgp_handle* h) {
   if (!h->ev_pool.empty()) {

@@ -67,19 +67,33 @@ int dgp_cyclic_reader(void* user, uint8_t* slot, int max_frames, const uint8_t**
 int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user, int H, int W, int batch, float gamma,
                              float gauss_len, int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
                              int64_t* frames_done) {
+  return dgp_estimate_pose_stream_transform(h, reader, user, H, W, nullptr, batch, gamma, gauss_len, max_frames, mu_host,
+                                            peak_host, lik_host, frames_done);
+}
+
+int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                       const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                       int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                       int64_t* frames_done) {
   if (!h) return DGP_ERR_INVALID;
   if (frames_done) *frames_done = 0;
   if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_estimate_pose_stream before dgp_finalize_weights");
   if (!reader || batch < 1 || max_frames < 0 || !mu_host) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: bad argument");
+  int H, W;
+  bool identity;
+  if (transform_dims(H0, W0, transform, &H, &W, &identity))
+    return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: invalid frame size or transform");
   if (max_frames == 0) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
   const int nj = h->cfg.num_joints;
   int hf, wf, ho, wo;
   dgp_output_dims(H, W, &hf, &wf, &ho, &wo);
-  const size_t frame_bytes = (size_t)H * W * 3;
+  // the ring, the H2D copy and st_frames2 carry source-size frames; the transform writes st_xf on the compute stream
+  const size_t frame_bytes = (size_t)H0 * W0 * 3;
   int rc;
   if ((rc = ensure(h, &h->st_frames2[0], frame_bytes * batch))) return rc;
   if ((rc = ensure(h, &h->st_frames2[1], frame_bytes * batch))) return rc;
+  if (!identity && (rc = ensure(h, &h->st_xf, (size_t)H * W * 3 * batch))) return rc;
   if ((rc = ensure(h, &h->st_logits, (size_t)batch * ho * wo * nj * 4))) return rc;
   if ((rc = ensure(h, &h->st_mu, (size_t)batch * nj * 2 * 4))) return rc;
   if ((rc = ensure(h, &h->st_peak, (size_t)batch * nj * 2 * 4))) return rc;
@@ -175,7 +189,12 @@ int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user,
     // surplus frames (allocation of every activation, tensor maps, first-use kernel loads).
     const int run_n = (f.n < batch && full_batch_seen) ? batch : f.n;
     if (f.n == batch) full_batch_seen = true;
-    if ((status = dgp_forward(h, (const uint8_t*)h->st_frames2[dslot].p, run_n, H, W, (float*)h->st_logits.p, nullptr, s))) break;
+    const uint8_t* frames = (const uint8_t*)h->st_frames2[dslot].p;
+    if (!identity) {
+      if ((status = resize_crop_impl(h, frames, f.n, H0, W0, transform, (uint8_t*)h->st_xf.p, s))) break;
+      frames = (const uint8_t*)h->st_xf.p;
+    }
+    if ((status = dgp_forward(h, frames, run_n, H, W, (float*)h->st_logits.p, nullptr, s))) break;
     if ((ce = cudaEventRecord(h->ev_consumed[dslot], s)) != cudaSuccess) break;
     if ((status = dgp_softargmax(h, (const float*)h->st_logits.p, nullptr, run_n, ho, wo, nj, gamma, gauss_len, (float*)h->st_mu.p,
                                  (int32_t*)h->st_peak.p, (float*)h->st_lik.p, nullptr, nullptr, s)))

@@ -24,6 +24,35 @@ def output_dims(H, W):
     return (a.value, b.value), (c.value, d.value)
 
 
+def frame_transform(new_size=None, crop_size=None):
+    """The dgp_frame_transform of estimate_pose's options, or None for neither: ``new_size`` = (height, width) of
+    PIL's ``resize(size=(new_size[1], new_size[0]))`` (eval.py:319), ``crop_size`` = the PIL box (x0, y0, x1, y1) of
+    ``crop(crop_size)`` taken on the resized frame (eval.py:322)."""
+    if new_size is None and crop_size is None:
+        return None
+    t = _lib.DgpFrameTransform()
+    if new_size is not None:
+        t.resize_h, t.resize_w = int(new_size[0]), int(new_size[1])
+        if t.resize_h < 1 or t.resize_w < 1:
+            raise ValueError("new_size must be two positive sizes (height, width), got %r" % (tuple(new_size),))
+    if crop_size is not None:
+        x0, y0, x1, y1 = (int(v) for v in crop_size)
+        if x1 <= x0 or y1 <= y0:
+            raise ValueError("crop_size must be a box (x0, y0, x1, y1) with x1 > x0 and y1 > y0, got %r" % (tuple(crop_size),))
+        t.crop_x0, t.crop_y0, t.crop_x1, t.crop_y1 = x0, y0, x1, y1
+    return t
+
+
+def transform_dims(H0, W0, new_size=None, crop_size=None):
+    """(H, W) of an H0 x W0 frame after estimate_pose's resize / crop (dgp_transform_dims); ValueError if invalid."""
+    lib = _lib.load()
+    t = frame_transform(new_size, crop_size)
+    H, W = C.c_int(), C.c_int()
+    if lib.dgp_transform_dims(int(H0), int(W0), C.byref(t) if t is not None else None, C.byref(H), C.byref(W)) != 0:
+        raise ValueError("invalid frame size %dx%d or transform new_size=%r crop_size=%r" % (H0, W0, new_size, crop_size))
+    return H.value, W.value
+
+
 def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3)):
     """Frames per batch that minimise wave quantisation of the persistent conv-GEMM grid (one CTA per SM).
 
@@ -289,20 +318,40 @@ class Engine:
         return {"skel": skel, "temporal": temporal[:n_t], "e_skel": e_skel, "e_temp": e_temp, "_temporal_full": temporal,
                 "_T": T, "_nl": nl}
 
-    def estimate_pose_host(self, frames_host, batch=16, gamma=1.0, gauss_len=1.0):
-        """End-to-end with HOST buffers (H2D + forward + soft-argmax + D2H inside). frames_host: uint8 (T,H,W,3) CPU tensor."""
-        if frames_host.is_cuda or frames_host.dtype != torch.uint8:
-            raise ValueError("frames_host must be a uint8 CPU tensor (pinned for async copies)")
+    def resize_crop(self, frames_dev, new_size=None, crop_size=None):
+        """estimate_pose's per-frame ``PIL.Image.resize(size=(new_size[1], new_size[0]))`` + ``.crop(crop_size)`` on the
+        device, bit-exact (dgp_resize_crop): uint8 cuda (N,H0,W0,3) -> new uint8 cuda (N,H,W,3)."""
+        if frames_dev.dtype != torch.uint8 or frames_dev.dim() != 4 or frames_dev.shape[-1] != 3 or not frames_dev.is_cuda:
+            raise ValueError("frames must be a uint8 CUDA tensor of shape (N,H,W,3)")
+        frames_dev = frames_dev.contiguous()
+        N, H0, W0, _ = frames_dev.shape
+        H, W = transform_dims(H0, W0, new_size, crop_size)
+        t = frame_transform(new_size, crop_size)
+        out = torch.empty((N, H, W, 3), dtype=torch.uint8, device=frames_dev.device)
+        self._check(self.lib.dgp_resize_crop(self.h, _ptr(frames_dev), N, H0, W0, C.byref(t) if t is not None else None,
+                                             _ptr(out), _stream(frames_dev.device)))
+        return out
+
+    def estimate_pose_host(self, frames_host, batch=16, gamma=1.0, gauss_len=1.0, new_size=None, crop_size=None):
+        """End-to-end with HOST buffers (H2D + forward + soft-argmax + D2H inside). frames_host: uint8 (T,H0,W0,3) CPU tensor.
+        ``new_size`` / ``crop_size`` (estimate_pose's options, see ``frame_transform``) resize / crop every frame on the
+        device after the H2D copy, which carries the frames at their source size."""
+        if frames_host.is_cuda or frames_host.dtype != torch.uint8 or frames_host.dim() != 4 or frames_host.shape[-1] != 3:
+            raise ValueError("frames_host must be a uint8 CPU tensor (T,H,W,3) (pinned for async copies)")
         frames_host = frames_host.contiguous()
-        T, H, W, _ = frames_host.shape
+        T, H0, W0, _ = frames_host.shape
+        transform_dims(H0, W0, new_size, crop_size)
+        t = frame_transform(new_size, crop_size)
         mu = torch.empty((T, self.nj, 2), dtype=torch.float32).pin_memory()
         peak = torch.empty((T, self.nj, 2), dtype=torch.int32).pin_memory()
         lik = torch.empty((T, self.nj), dtype=torch.float32).pin_memory()
-        self._check(self.lib.dgp_estimate_pose_host(self.h, _ptr(frames_host), T, H, W, int(batch), float(gamma), float(gauss_len),
-                                                    _ptr(mu), _ptr(peak), _ptr(lik)))
+        self._check(self.lib.dgp_estimate_pose_host_transform(self.h, _ptr(frames_host), T, H0, W0,
+                                                              C.byref(t) if t is not None else None, int(batch), float(gamma),
+                                                              float(gauss_len), _ptr(mu), _ptr(peak), _ptr(lik)))
         return mu, peak, lik
 
-    def estimate_pose_stream(self, source, H, W, max_frames, batch=16, gamma=1.0, gauss_len=1.0, start=0):
+    def estimate_pose_stream(self, source, H, W, max_frames, batch=16, gamma=1.0, gauss_len=1.0, start=0, new_size=None,
+                             crop_size=None):
         """Streaming estimate_pose (dgp_estimate_pose_stream): host memory is bounded by a ring of 3 pinned slots of `batch`
         frames, whatever the length of the video.  ``source`` is either
 
@@ -313,8 +362,13 @@ class Engine:
           ``start`` is the index of the first frame to serve (frame t of the video is ``source[t % P]``), which lets every
           rank of a sharded run read its own contiguous range of the same video.
 
+        ``H``, ``W`` are the size of the source frames.  ``new_size`` / ``crop_size`` (estimate_pose's options, see
+        ``frame_transform``) resize / crop every frame on the device: the ring and the H2D copy carry source-size frames.
+
         Returns (mu (T,nj,2) f32, peak (T,nj,2) i32, lik (T,nj) f32) as CPU tensors, T = frames actually delivered."""
         T = int(max_frames)
+        transform_dims(H, W, new_size, crop_size)
+        tf = frame_transform(new_size, crop_size)
         mu = torch.empty((T, self.nj, 2), dtype=torch.float32).pin_memory()
         peak = torch.empty((T, self.nj, 2), dtype=torch.int32).pin_memory()
         lik = torch.empty((T, self.nj), dtype=torch.float32).pin_memory()
@@ -352,8 +406,10 @@ class Engine:
 
             cb = _lib.FRAME_READER(_read)
             reader, user, keep = C.cast(cb, C.c_void_p), C.c_void_p(0), (cb, state)
-        status = self.lib.dgp_estimate_pose_stream(self.h, reader, user, int(H), int(W), int(batch), float(gamma),
-                                                   float(gauss_len), T, _ptr(mu), _ptr(peak), _ptr(lik), C.byref(done))
+        status = self.lib.dgp_estimate_pose_stream_transform(self.h, reader, user, int(H), int(W),
+                                                             C.byref(tf) if tf is not None else None, int(batch),
+                                                             float(gamma), float(gauss_len), T, _ptr(mu), _ptr(peak),
+                                                             _ptr(lik), C.byref(done))
         if not isinstance(source, torch.Tensor) and keep[1]["error"] is not None:
             raise keep[1]["error"]
         self._check(status)

@@ -95,14 +95,17 @@ def _iter_video(video_file):
     cap.release()
 
 
-def estimate_pose_frames(engine, frames, batch=16, gamma=1.0, gauss_len=1.0, stride=None):
+def estimate_pose_frames(engine, frames, batch=16, gamma=1.0, gauss_len=1.0, stride=None, new_size=None, crop_size=None):
     """The estimate_pose frame loop (eval.py:306-357) on in-memory frames: uint8 (T,H,W,3), numpy or CPU tensor.
 
     Host buffers in, host arrays out; the H2D copy of every batch and the D2H copy of its results happen inside.
+    ``new_size`` (height, width) / ``crop_size`` (x0, y0, x1, y1) resize / crop every frame on the device exactly as the
+    reference's PIL calls do (eval.py:319-322); the coordinates returned are those of the transformed frames.
     Returns dict(x, y, likelihoods, mu_likelihoods, markers) with the reference's shapes.
     """
     ft = frames if isinstance(frames, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(frames))
-    mu, peak, lik = engine.estimate_pose_host(ft, batch=batch, gamma=gamma, gauss_len=gauss_len)
+    mu, peak, lik = engine.estimate_pose_host(ft, batch=batch, gamma=gamma, gauss_len=gauss_len, new_size=new_size,
+                                              crop_size=crop_size)
     stride = engine.stride if stride is None else stride
     markers = mu.numpy().astype(np.float64)
     xr = markers[:, :, 1] * stride + 0.5 * stride
@@ -117,22 +120,26 @@ def _readout_dict(mu, peak, lik, stride):
             "likelihoods": lik.numpy().astype(np.float64), "mu_likelihoods": peak.numpy().astype("int"), "markers": markers}
 
 
-def estimate_pose_stream(engine, source, H, W, n_frames=None, batch=16, gamma=1.0, gauss_len=1.0, chunk=65536):
+def estimate_pose_stream(engine, source, H, W, n_frames=None, batch=16, gamma=1.0, gauss_len=1.0, chunk=65536, new_size=None,
+                         crop_size=None):
     """The estimate_pose frame loop (eval.py:306-357) over a frame SOURCE instead of an in-memory array: an iterator of uint8
     (H,W,3) RGB frames (video decoder) or a pinned uint8 tensor (P,H,W,3) cycled for ``n_frames`` frames.  Frames stream
     through a pinned ring of 3 x ``batch`` frames (Engine.estimate_pose_stream): host memory does not grow with the video.
-    ``n_frames`` may be None for iterators of unknown length (results are collected ``chunk`` frames at a time)."""
+    ``n_frames`` may be None for iterators of unknown length (results are collected ``chunk`` frames at a time).
+    ``H``, ``W`` are the source frame size; ``new_size`` / ``crop_size`` transform each frame on the device as in
+    ``estimate_pose_frames``."""
     parts = []
+    kw = dict(new_size=new_size, crop_size=crop_size)
     if isinstance(source, torch.Tensor):
         if n_frames is None:
             n_frames = source.shape[0]
-        parts.append(engine.estimate_pose_stream(source, H, W, n_frames, batch, gamma, gauss_len))
+        parts.append(engine.estimate_pose_stream(source, H, W, n_frames, batch, gamma, gauss_len, **kw))
     else:
         it = iter(source)
         left = None if n_frames is None else int(n_frames)
         while left is None or left > 0:
             want = chunk if left is None else min(chunk, left)
-            mu, peak, lik = engine.estimate_pose_stream(it, H, W, want, batch, gamma, gauss_len)
+            mu, peak, lik = engine.estimate_pose_stream(it, H, W, want, batch, gamma, gauss_len, **kw)
             parts.append((mu, peak, lik))
             if left is not None:
                 left -= mu.shape[0]
@@ -143,7 +150,7 @@ def estimate_pose_stream(engine, source, H, W, n_frames=None, batch=16, gamma=1.
 
 
 def estimate_pose_sharded(engine, source, T, H, W, edges=(), ws=None, ws_max=None, wt_max=0.0, batch=16, gamma=1.0,
-                          gauss_len=1.0, group=None, gather=True, timings=None):
+                          gauss_len=1.0, group=None, gather=True, timings=None, new_size=None, crop_size=None):
     """estimate_pose over a T-frame video sharded contiguously by frame over the ranks of ``group`` (SURVEY.md 8e; one process
     per GPU): rank r streams frames [a_r, b_r) (``sharding.shard_range``) through its own engine, the ranks exchange the
     soft-argmax of their first frame (one all_gather of nj*8 bytes per rank) so that the temporal potential at every shard
@@ -155,7 +162,9 @@ def estimate_pose_sharded(engine, source, T, H, W, edges=(), ws=None, ws_max=Non
     ``(start, stop) -> iterator of frames`` that opens the rank's own range of a real video.
     Returns the estimate_pose dict plus 'skel' (T,nl), 'temporal' (T,nj; last row 0), 'e_skel', 'e_temp' (T) -- for the
     whole video on every rank when ``gather`` (else for the rank's shard) -- and 'shard' = (a_r, b_r).
-    ``timings``: an optional dict that receives the wall-clock seconds of the phases ('stream', 'potentials', 'gather')."""
+    ``timings``: an optional dict that receives the wall-clock seconds of the phases ('stream', 'potentials', 'gather').
+    ``H``, ``W`` are the source frame size; ``new_size`` / ``crop_size`` transform each frame on the device as in
+    ``estimate_pose_frames``."""
     import time
     import torch.distributed as dist
     from . import sharding
@@ -167,9 +176,11 @@ def estimate_pose_sharded(engine, source, T, H, W, edges=(), ws=None, ws_max=Non
     a, b = sharding.shard_range(T, rank, world)
     t_start = time.perf_counter()
     if isinstance(source, torch.Tensor):
-        mu, peak, lik = engine.estimate_pose_stream(source, H, W, b - a, batch, gamma, gauss_len, start=a)
+        mu, peak, lik = engine.estimate_pose_stream(source, H, W, b - a, batch, gamma, gauss_len, start=a, new_size=new_size,
+                                                    crop_size=crop_size)
     else:
-        mu, peak, lik = engine.estimate_pose_stream(source(a, b), H, W, b - a, batch, gamma, gauss_len)
+        mu, peak, lik = engine.estimate_pose_stream(source(a, b), H, W, b - a, batch, gamma, gauss_len, new_size=new_size,
+                                                    crop_size=crop_size)
     if mu.shape[0] != b - a:
         raise RuntimeError("rank %d: the source delivered %d of its %d frames" % (rank, mu.shape[0], b - a))
     dev = engine.device
@@ -199,9 +210,10 @@ def estimate_pose_sharded(engine, source, T, H, W, edges=(), ws=None, ws_max=Non
     return out
 
 
-def _video_source(video_file, new_size=None, crop_size=None):
-    """(frame iterator, H, W, frame count or None, scale_x, scale_y) for a video file: frames are decoded one at a time
-    (OpenCV), resized / cropped the way the reference does per frame (eval.py:309-326), and never held beyond the ring."""
+def _video_source(video_file, new_size=None):
+    """(frame iterator, H0, W0, frame count or None, scale_x, scale_y) for a video file: frames are decoded one at a time
+    (OpenCV) at their source size and never held beyond the ring; the reference's per-frame resize / crop (eval.py:309-326)
+    runs on the device.  The scales map coordinates of the resized frame back to the video (eval.py:312-313)."""
     import cv2
     cap = cv2.VideoCapture(str(video_file))
     if not cap.isOpened():
@@ -210,27 +222,9 @@ def _video_source(video_file, new_size=None, crop_size=None):
     count = int(cap.get(cv2.CAP_PROP_FRAME_COUNT))
     cap.release()
     scale_x = scale_y = 1.0
-    H, W = h0, w0
     if new_size is not None:
         scale_x, scale_y = w0 / new_size[1], h0 / new_size[0]
-        H, W = int(new_size[0]), int(new_size[1])
-    if crop_size is not None:
-        W, H = int(crop_size[2] - crop_size[0]), int(crop_size[3] - crop_size[1])
-
-    def frames():
-        if new_size is None and crop_size is None:
-            yield from _iter_video(video_file)
-            return
-        from PIL import Image
-        for fr in _iter_video(video_file):
-            im = Image.fromarray(np.ascontiguousarray(fr))
-            if new_size is not None:
-                im = im.resize(size=(new_size[1], new_size[0]))
-            if crop_size is not None:
-                im = im.crop(crop_size)
-            yield np.asarray(im)
-
-    return frames(), H, W, (count if count > 0 else None), scale_x, scale_y
+    return _iter_video(video_file), h0, w0, (count if count > 0 else None), scale_x, scale_y
 
 
 def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle=1, save_pose=True, save_str="",
@@ -239,6 +233,8 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
     ``bodyparts``; ``video_file`` a path or a uint8 array (T,H,W,3).  Returns {'x','y','likelihoods'} (T,nj) each.
     A video file is STREAMED: decoded frame by frame (as the reference's ``clip.iter_frames()``, eval.py:306) into a pinned
     ring that the GPU drains batch by batch, so a 100 k-frame clip needs no more host memory than a 100-frame one.
+    ``new_size`` (height, width) and ``crop_size`` (x0, y0, x1, y1) resize and crop every frame on the device, bit-exact to
+    the reference's ``PIL.Image.resize`` (Pillow's default filter, BICUBIC) and ``crop``.
     The backbone (ResNet-50, -101 or -152) is the one the weights' names describe, as the reference's estimate_pose tries
     each snapshot scope (eval.py:271-276)."""
     if isinstance(proj_cfg_file, (dict,)) or hasattr(proj_cfg_file, "num_joints"):
@@ -256,27 +252,16 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
         if os.path.exists(save_file + ".csv"):
             print("labels already exist! video at %s will not be processed" % video_file)
             return save_file + ".csv"
-        source, H, W, n_frames, scale_x, scale_y = _video_source(video_file, new_size, crop_size)
+        source, H0, W0, n_frames, scale_x, scale_y = _video_source(video_file, new_size)
         sess, mu_n, _, scmap, _, inputs = _setup_eval_graph(dlc_cfg, dgp_model_file, None)
         # the container's frame count is a hint only (it can be off by a few frames): read until the decoder runs dry
-        res = estimate_pose_stream(sess.engine, source, H, W, None, batch=batch)
+        res = estimate_pose_stream(sess.engine, source, H0, W0, None, batch=batch, new_size=new_size, crop_size=crop_size)
     else:
         frames = np.asarray(video_file)
-        if new_size is not None or crop_size is not None:
-            from PIL import Image
-            out = []
-            for fr in frames:
-                im = Image.fromarray(fr)
-                if new_size is not None:
-                    scale_x = im.width / new_size[1]
-                    scale_y = im.height / new_size[0]
-                    im = im.resize(size=(new_size[1], new_size[0]))
-                if crop_size is not None:
-                    im = im.crop(crop_size)
-                out.append(np.asarray(im))
-            frames = np.stack(out)
+        if new_size is not None:
+            scale_x, scale_y = frames.shape[2] / new_size[1], frames.shape[1] / new_size[0]
         sess, mu_n, _, scmap, _, inputs = _setup_eval_graph(dlc_cfg, dgp_model_file, None)
-        res = estimate_pose_frames(sess.engine, frames, batch=batch)
+        res = estimate_pose_frames(sess.engine, frames, batch=batch, new_size=new_size, crop_size=crop_size)
     sess.close()
     labels = {"x": res["x"] * scale_x, "y": res["y"] * scale_y, "likelihoods": res["likelihoods"]}
     if save_pose and save_file is not None:

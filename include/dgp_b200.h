@@ -227,11 +227,40 @@ int dgp_loss_forward(dgp_handle* h, const dgp_loss_cfg* cfg, const dgp_loss_batc
 int dgp_loss_backward(dgp_handle* h, const dgp_loss_cfg* cfg, const dgp_loss_batch* batch, float* losses_dev,
                       float* grad_pred_dev, float* grad_locref_dev, int visible_only, void* stream);
 
+/* ---- frame resize + crop (estimate_pose's new_size / crop_size, eval.py:309-326) ----
+ * The reference resizes each frame with PIL's Image.resize((resize_w, resize_h)) -- Pillow's default filter for RGB images,
+ * BICUBIC (a = -0.5) since Pillow 7.0 -- and then crops it with Image.crop((crop_x0, crop_y0, crop_x1, crop_y1)).  The
+ * entries below compute the same bytes on the device: Pillow's 8-bit resample is integer arithmetic on fixed-point weights
+ * (22 fraction bits) computed in double, horizontal pass first, a pass skipped when its size does not change, and the
+ * crop taken on the resized frame with box pixels outside that frame set to 0.
+ *  resize_h = resize_w = 0: no resize (else both > 0).  All four crop fields 0: no crop (else crop_x1 > crop_x0 and
+ *  crop_y1 > crop_y0; the box may extend past the resized frame).  Anything else is DGP_ERR_INVALID and launches nothing. */
+typedef struct dgp_frame_transform {
+  int32_t resize_h, resize_w;
+  int32_t crop_x0, crop_y0, crop_x1, crop_y1;
+} dgp_frame_transform;
+/* Size (H, W) of a transformed H0 x W0 frame; `t` NULL = identity.  Handle-free, like dgp_output_dims. */
+int dgp_transform_dims(int H0, int W0, const dgp_frame_transform* t, int* H, int* W);
+/* Pillow's resample table for one axis, in_size -> out_size (handle-free; what the device passes use): output index i reads
+ * count[i] inputs from first[i] with int32 weights[i * max_taps + k] (weights past count[i] are 0).  ceil(2 * max(in_size /
+ * out_size, 1)) * 2 + 1 taps always suffice; a max_taps below some count[i] is DGP_ERR_INVALID. */
+int dgp_resize_coefficients(int in_size, int out_size, int max_taps, int32_t* first, int32_t* count, int32_t* weights);
+/* src_dev uint8 (N,H0,W0,3) RGB -> dst_dev uint8 (N,H,W,3), (H, W) from dgp_transform_dims.  Asynchronous on `stream`.
+ * The size tables are built on the host at the first use of a size pair and kept on the handle. */
+int dgp_resize_crop(dgp_handle* h, const uint8_t* src_dev, int N, int H0, int W0, const dgp_frame_transform* t,
+                    uint8_t* dst_dev, void* stream);
+
 /* Replaces the estimate_pose frame loop (eval.py:306-345) end to end with HOST buffers: per batch of `batch`
  * frames H2D copy, dgp_forward, dgp_softargmax, D2H of the results.  frames_host uint8 (T,H,W,3) (pinned memory
  * gives asynchronous copies); mu_host float32 (T,nj,2); peak_host int32 (T,nj,2); lik_host float32 (T,nj). */
 int dgp_estimate_pose_host(dgp_handle* h, const uint8_t* frames_host, int T, int H, int W, int batch, float gamma,
                            float gauss_len, float* mu_host, int32_t* peak_host, float* lik_host);
+/* dgp_estimate_pose_host on frames that `transform` resizes / crops on the device first (NULL = identity, which is
+ * dgp_estimate_pose_host): frames_host holds (T,H0,W0,3) source frames, the H2D copy carries them at that size, and
+ * dgp_resize_crop turns each batch into the (H,W) frames of dgp_transform_dims on the compute stream. */
+int dgp_estimate_pose_host_transform(dgp_handle* h, const uint8_t* frames_host, int T, int H0, int W0,
+                                     const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                     float* mu_host, int32_t* peak_host, float* lik_host);
 
 /* Streaming form of the estimate_pose frame loop (eval.py:256, 306-345: `for frame in clip.iter_frames()`), for videos that
  * do not fit in host memory.  A reader thread owned by the call asks `reader` for up to `max_frames` frames at a time and
@@ -246,6 +275,13 @@ typedef int (*dgp_frame_reader)(void* user, uint8_t* slot, int max_frames, const
 int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user, int H, int W, int batch, float gamma,
                              float gauss_len, int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
                              int64_t* frames_done);
+/* dgp_estimate_pose_stream on (H0,W0,3) source frames that `transform` resizes / crops on the device (NULL = identity):
+ * the reader delivers source-size frames, the pinned ring and the H2D copy carry them, and dgp_resize_crop runs on the
+ * compute stream into the device buffer that dgp_forward consumes. */
+int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                       const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                       int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                       int64_t* frames_done);
 /* A ready-made reader for frames already resident in (pinned) host memory, e.g. a decoded clip kept in RAM or bench.py's
  * synthetic video: serves `total_frames` frames by cycling over pool[0 .. pool_frames) in direct (zero-copy) mode. */
 typedef struct dgp_cyclic_source {
