@@ -59,6 +59,12 @@ class DgpFrameTransform(C.Structure):
                 ("crop_x1", C.c_int32), ("crop_y1", C.c_int32)]
 
 
+class DgpAugmentParams(C.Structure):
+    _fields_ = [("rotate_deg", C.c_double), ("blur_k", C.c_int32), ("blur_angle_deg", C.c_double),
+                ("blur_direction", C.c_double), ("drop_p", C.c_double), ("drop_size_percent", C.c_double),
+                ("elastic_alpha", C.c_double), ("elastic_sigma", C.c_double), ("seed", C.c_uint64)]
+
+
 # reader(user, slot, max_frames, &direct) -> frames delivered (0 = end of video, < 0 = error)
 FRAME_READER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p))
 
@@ -96,6 +102,9 @@ SIGNATURES = {
                                               _vp]),
     "dgp_estimate_pose_stream_transform": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f, C.c_int64,
                                                 _vp, _vp, _vp, _i64p]),
+    "dgp_motion_blur_kernel": (_i, [_i, C.c_double, C.c_double, _vp]),
+    "dgp_elastic_field": (_i, [_vp, _i, _i, C.c_double, C.c_double, C.c_uint64, _vp, _vp, _vp]),
+    "dgp_augment": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, C.POINTER(DgpAugmentParams), _vp, C.c_double, _vp]),
     "dgp_debug_keep_activations": (_i, [_vp, _i]),
     "dgp_debug_get_activation": (_i, [_vp, C.c_char_p, _vp, _sz, _i64p]),
     "dgp_conv2d": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _vp,

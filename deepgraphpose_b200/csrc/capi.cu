@@ -834,6 +834,10 @@ void dgp_destroy(dgp_handle* h) {
   cudaFree(h->st_xf.p);
   cudaFree(h->resize_tmp.p);
   for (auto& kv : h->resize_tables) cudaFree(kv.second.dev);
+  cudaFree(h->aug_scratch[0].p);
+  cudaFree(h->aug_scratch[1].p);
+  cudaFree(h->aug_fields.p);
+  cudaFree(h->aug_tmp.p);
   for (auto& r : h->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
   for (auto e : h->ev_pool) cudaEventDestroy(e);
   if (h->stream) cudaStreamDestroy(h->stream);

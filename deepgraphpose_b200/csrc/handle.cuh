@@ -162,6 +162,9 @@ struct dgp_handle {
   // dgp_resize_crop: tables per (in, out) size pair and the uint8 intermediate of the horizontal pass
   std::map<std::pair<int, int>, ResizeTable> resize_tables;
   DevBuf resize_tmp;
+  // dgp_augment: two scratch frame sets of the ping-pong between passes, elastic fields (dx | dy per frame) and the
+  // intermediate of the field's horizontal pass
+  DevBuf aug_scratch[2], aug_fields, aug_tmp;
   // dgp_estimate_pose_stream: pinned host ring the reader thread decodes into (stream.cu)
   void* ring_slot[3] = {nullptr, nullptr, nullptr};
   size_t ring_bytes = 0;

@@ -332,6 +332,46 @@ class Engine:
                                              _ptr(out), _stream(frames_dev.device)))
         return out
 
+    def augment(self, frames_dev, positions, joint_loc, params, stride=None):
+        """fit_dgp's augmentation of labelled frames on the device (dgp_augment): rotation, motion blur, coarse dropout and
+        elastic deformation of ``frames_dev`` (uint8 contiguous CUDA (nt,H,W,3), modified in place) at the batch
+        ``positions``, frame ``positions[k]`` with ``params[k]`` (a dict of dgp_augment_params fields, missing ones 0, or a
+        ``_lib.DgpAugmentParams``).  ``joint_loc``: the (n, nj, 2) scoremap (row, col) labels of those frames, a float64
+        contiguous CUDA tensor moved in place (or a host array, uploaded), or None; ``stride``: scoremap stride of the labels
+        (default: the engine's).  Returns the device labels (or None)."""
+        if frames_dev.dtype != torch.uint8 or frames_dev.dim() != 4 or frames_dev.shape[-1] != 3 or not frames_dev.is_cuda:
+            raise ValueError("frames must be a uint8 CUDA tensor of shape (nt,H,W,3)")
+        if not frames_dev.is_contiguous():
+            raise ValueError("frames must be contiguous: they are augmented in place")
+        nt, H, W, _ = frames_dev.shape
+        idx = np.ascontiguousarray(np.asarray(positions, dtype=np.int32).reshape(-1))
+        n = idx.shape[0]
+        if len(params) != n:
+            raise ValueError("one parameter set per augmented frame is required")
+        par = (_lib.DgpAugmentParams * max(n, 1))()
+        for k, p in enumerate(params):
+            par[k] = p if isinstance(p, _lib.DgpAugmentParams) else _lib.DgpAugmentParams(**p)
+        jl = None
+        if joint_loc is not None:
+            jl = joint_loc
+            if not isinstance(jl, torch.Tensor):
+                jl = torch.from_numpy(np.ascontiguousarray(np.asarray(joint_loc, dtype=np.float64))).to(frames_dev.device)
+            if jl.dtype != torch.float64 or not jl.is_cuda or not jl.is_contiguous() or tuple(jl.shape) != (n, self.nj, 2):
+                raise ValueError("joint_loc must be a contiguous float64 CUDA tensor (%d, %d, 2)" % (n, self.nj))
+        self._check(self.lib.dgp_augment(self.h, _ptr(frames_dev), nt, H, W, idx.ctypes.data_as(C.c_void_p), n, par,
+                                          _ptr(jl) if jl is not None and jl.numel() else None,
+                                          float(self.stride if stride is None else stride),
+                                          _stream(frames_dev.device)))
+        return jl
+
+    def elastic_field(self, H, W, alpha, sigma, seed):
+        """The elastic displacement fields dgp_augment samples with (dgp_elastic_field): float32 CUDA (dx, dy), each (H, W)."""
+        dx = torch.empty((H, W), dtype=torch.float32, device=self.device)
+        dy = torch.empty_like(dx)
+        self._check(self.lib.dgp_elastic_field(self.h, int(H), int(W), float(alpha), float(sigma), int(seed), _ptr(dx), _ptr(dy),
+                                               _stream(self.device)))
+        return dx, dy
+
     def estimate_pose_host(self, frames_host, batch=16, gamma=1.0, gauss_len=1.0, new_size=None, crop_size=None):
         """End-to-end with HOST buffers (H2D + forward + soft-argmax + D2H inside). frames_host: uint8 (T,H0,W0,3) CPU tensor.
         ``new_size`` / ``crop_size`` (estimate_pose's options, see ``frame_transform``) resize / crop every frame on the
@@ -547,12 +587,16 @@ class Engine:
     def locref_targets(self, joint_loc, visible_frame_within_batch, nt, H, W, pos_dist_thresh=17.0, locref_stdev=7.2801):
         """Device-side coord2map + batch scatter (dataset.py:246-271, fitdgp.py:781-795): joint_loc (n_vis,nj,2) float64
         scoremap (row,col) labels (NaN = missing).  Returns float32 CUDA tensors (locref_map, locref_mask) (nt,H,W,2nj)."""
-        jl = np.ascontiguousarray(np.asarray(joint_loc, dtype=np.float64).reshape(-1, self.nj, 2))
-        idx = np.ascontiguousarray(np.asarray(visible_frame_within_batch, dtype=np.int32).reshape(-1))
-        if jl.shape[0] != idx.shape[0]:
-            raise ValueError("one batch position per labelled frame is required")
         dev = self.device
-        jl_d = torch.from_numpy(jl).to(dev) if jl.size else None
+        if isinstance(joint_loc, torch.Tensor):     # labels already on the device (fitdgp_util.data_aug) are read in place
+            jl_d = joint_loc.to(device=dev, dtype=torch.float64).reshape(-1, self.nj, 2).contiguous()
+        else:
+            jl_d = torch.from_numpy(np.ascontiguousarray(np.asarray(joint_loc, dtype=np.float64).reshape(-1, self.nj, 2))).to(dev)
+        idx = np.ascontiguousarray(np.asarray(visible_frame_within_batch, dtype=np.int32).reshape(-1))
+        if jl_d.shape[0] != idx.shape[0]:
+            raise ValueError("one batch position per labelled frame is required")
+        if not jl_d.numel():
+            jl_d = None
         idx_d = torch.from_numpy(idx).to(dev) if idx.size else None
         lmap = torch.empty((nt, H, W, 2 * self.nj), dtype=torch.float32, device=dev)
         lmask = torch.empty_like(lmap)

@@ -81,7 +81,8 @@ def _loss_args(dev, feed, cfg, edges, ws, ws_max, n_frames_total, n_visible_fram
         if isinstance(a, torch.Tensor):
             return a.to(device=dev, dtype=torch.int32).contiguous()
         return torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32), device=dev)
-    targets = f32(np.asarray(feed["targets"]).reshape(-1, nj, 2))
+    tg = feed["targets"]
+    targets = f32(tg if isinstance(tg, torch.Tensor) else np.asarray(tg)).reshape(-1, nj, 2)
     vis, hid, vit = i32(feed["visible_marker_pl"]), i32(feed["hidden_marker_pl"]), i32(feed["visible_marker_in_targets_pl"])
     keep = [targets, vis, hid, vit]
     b = _lib.DgpLossBatch()
@@ -328,10 +329,16 @@ class TrainSession:
                 flat.append(f)
         collect(fetches)
         g = flat[0].graph
-        frames = np.asarray(feed["inputs"])
-        if frames.dtype != np.uint8:
-            frames = np.clip(np.round(frames), 0, 255).astype(np.uint8)
-        frames = torch.from_numpy(np.ascontiguousarray(frames)).to(g.engine.device)
+        frames = feed["inputs"]
+        if isinstance(frames, torch.Tensor):           # frames already on the device (fitdgp_util.data_aug)
+            if frames.dtype != torch.uint8:
+                raise ValueError("a tensor fed as inputs must hold uint8 frames")
+            frames = frames.to(g.engine.device).contiguous()
+        else:
+            frames = np.asarray(frames)
+            if frames.dtype != np.uint8:
+                frames = np.clip(np.round(frames), 0, 255).astype(np.uint8)
+            frames = torch.from_numpy(np.ascontiguousarray(frames)).to(g.engine.device)
         train_ops = [f for f in flat if f.kind == "train_op"]
         if train_ops:
             op = train_ops[0]
@@ -393,13 +400,16 @@ def gen_batch(visible_frame_total, hidden_frame_total, all_frame_total, dgp_cfg,
 
 
 def _fit_loop(data_batcher, dgp_cfg, variables, visible_frame_total, hidden_frame_total, all_frame_total, maxiters, step,
-              saveiters, displayiters, debug, labeled_only, device, batch_ind_all=None, snapshot_fn=None, verbose=True):
+              saveiters, displayiters, debug, labeled_only, device, batch_ind_all=None, snapshot_fn=None, verbose=True,
+              aug_pipeline=None):
     """The training loop both drivers share (fitdgp.py:727-845 / 431-546): batch schedule, per-batch feeds (learn_wt flow field
     when wt > 0, coord2map locref targets -- built on the device --, 2-D grids), ``sess.run([loss, train_op])`` and snapshots.
+    With ``aug_pipeline`` (fitdgp_util.build_aug) the batch is uploaded once and its labelled frames and their labels are
+    augmented on the device (fitdgp_util.data_aug, fitdgp.py:773-779) before they are fed.
     Returns the list of per-iteration loss dicts (the reference only prints them)."""
     import time
     from random import randint
-    from .fitdgp_util import learn_wt
+    from .fitdgp_util import data_aug, learn_wt
     loss, total_loss, total_loss_visible, placeholders = dgp_loss(data_batcher, dgp_cfg, variables=variables, device=device)
     learning_rate = learning_rate_placeholder()
     train_op = momentum_train_op(total_loss_visible if labeled_only else total_loss, learning_rate)   # fitdgp.py:706-713
@@ -440,6 +450,9 @@ def _fit_loop(data_batcher, dgp_cfg, variables, visible_frame_total, hidden_fram
         visible_marker, hidden_marker, visible_marker_in_targets = addn_batch_info
         all_frame = np.sort(list(visible_frame) + list(hidden_frame))
         visible_frame_within_batch = [int(np.where(all_frame == i)[0][0]) for i in visible_frame]
+        if aug_pipeline is not None:
+            all_data_batch, joint_loc = data_aug(all_data_batch, visible_frame_within_batch, joint_loc, aug_pipeline, dgp_cfg,
+                                                 engine=engine)
         # Farneback flow on the GPU, on a side stream: it overlaps the forward pass of this step (the loss waits for its event)
         vector_field = learn_wt(all_data_batch, engine=engine, overlap=True) if wt > 0 else np.zeros((1, 1, 1))
         feed = {
@@ -493,30 +506,34 @@ _PROJECT_READER_MSG = (
 def fit_dgp(snapshot, dlcpath, batch_size=10, shuffle=1, step=2, saveiters=1000, displayiters=5, maxiters=200000, ns=10,
             nc=2048, n_max_frames=2000, gm2=0, gm3=0, nepoch=100, wt=0, aug=True, debug="", trainingsetindex=0, *,
             data_batcher=None, dgp_cfg=None, frame_lists=None, variables=None, device=None, batch_ind_all=None,
-            snapshot_fn=None, verbose=True):
+            snapshot_fn=None, verbose=True, aug_pipeline=None):
     """fitdgp.py:549-845 with the reference's argument list.  The keyword-only arguments carry what the reference derives from
     the DLC project on the host: ``data_batcher`` (MultiDataset interface), ``dgp_cfg`` (the merged training config; gm2 / gm3 /
     wt / batch_size given here override it like fitdgp.py:640-660), ``frame_lists`` = (visible_frame_total, hidden_frame_total,
     all_frame_total) and ``variables`` (what ``restorer.restore(sess, init_weights)`` would load; defaults to
-    dgp_cfg.init_weights or ``snapshot``)."""
+    dgp_cfg.init_weights or ``snapshot``).  ``aug_pipeline`` (``fitdgp_util.build_aug(...)``): where the reference augments
+    (``aug`` and ``wt == 0``, fitdgp.py:773-779) the labelled frames of every batch are augmented on the device with it;
+    None trains on the frames as they are."""
     if data_batcher is None or dgp_cfg is None or frame_lists is None:
         raise NotImplementedError(_PROJECT_READER_MSG % "fit_dgp")
     cfg = SimpleNamespace(**(dict(dgp_cfg) if isinstance(dgp_cfg, dict) else vars(dgp_cfg)))
     cfg.batch_size, cfg.gm2, cfg.gm3, cfg.wt = batch_size, gm2, gm3, wt
-    if aug and wt == 0 and verbose:
+    if aug and wt == 0 and verbose and aug_pipeline is None:
         print("note: imgaug augmentation of visible frames (fitdgp.py:773-775) is a host feeder outside this library")
     if variables is None:
         variables = _get(cfg, "init_weights", None) or snapshot
     vis, hid, allf = frame_lists
     return _fit_loop(data_batcher, cfg, variables, vis, hid, allf, maxiters, step, saveiters, displayiters, debug, False, device,
-                     batch_ind_all, snapshot_fn, verbose)
+                     batch_ind_all, snapshot_fn, verbose, aug_pipeline if aug and wt == 0 else None)
 
 
 def fit_dgp_labeledonly(snapshot, dlcpath, shuffle=1, step=1, saveiters=1000, displayiters=5, maxiters=50000, ns=10, nc=2048,
                         n_max_frames=2000, aug=True, trainingsetindex=0, *, data_batcher=None, dgp_cfg=None,
-                        frame_lists=None, variables=None, device=None, batch_ind_all=None, snapshot_fn=None, verbose=True):
+                        frame_lists=None, variables=None, device=None, batch_ind_all=None, snapshot_fn=None, verbose=True,
+                        aug_pipeline=None):
     """fitdgp.py:257-546: the same loop on the labelled frames only -- no hidden frames in a batch, and the optimizer follows
-    ``total_loss_visible`` (visible cross-entropy + locref Huber), fitdgp.py:406-414."""
+    ``total_loss_visible`` (visible cross-entropy + locref Huber), fitdgp.py:406-414.  ``aug_pipeline`` as in ``fit_dgp``
+    (used when ``aug``)."""
     if data_batcher is None or dgp_cfg is None or frame_lists is None:
         raise NotImplementedError(_PROJECT_READER_MSG % "fit_dgp_labeledonly")
     cfg = SimpleNamespace(**(dict(dgp_cfg) if isinstance(dgp_cfg, dict) else vars(dgp_cfg)))
@@ -527,4 +544,4 @@ def fit_dgp_labeledonly(snapshot, dlcpath, shuffle=1, step=1, saveiters=1000, di
         variables = _get(cfg, "init_weights", None) or snapshot
     vis, hid, allf = frame_lists
     return _fit_loop(data_batcher, cfg, variables, vis, hid, allf, maxiters, step, saveiters, displayiters, "", True, device,
-                     batch_ind_all, snapshot_fn, verbose)
+                     batch_ind_all, snapshot_fn, verbose, aug_pipeline if aug else None)

@@ -136,3 +136,85 @@ def learn_wt(all_data_batch, engine=None, overlap=False):
     gray = [cv2.cvtColor(f.astype(np.uint8), cv2.COLOR_BGR2GRAY) for f in frames]
     fields = [np.abs(cv2.calcOpticalFlowFarneback(a, b, None, 0.5, 3, 15, 3, 5, 1.2, 0)).sum(2) for a, b in zip(gray[:-1], gray[1:])]
     return np.array(fields)
+
+
+class AugPipeline:
+    """The pipeline of ``build_aug``: per frame, rotation, motion blur, coarse dropout and elastic deformation (in that order),
+    each switched on with probability ``apply_prob`` (imgaug's ``Sometimes``), their parameters drawn from the pipeline's own
+    ``np.random.Generator``.  ``sample(n)`` gives the n ``dgp_augment_params`` dicts of the next n frames; every frame
+    consumes the same number of draws whichever ops it switches on."""
+
+    def __init__(self, apply_prob, rotation, motion_blur_k, motion_blur_angle, dropout_p, dropout_size_percent, elastic_alpha,
+                 elastic_sigma, seed):
+        self.apply_prob = float(apply_prob)
+        self.rotation = float(rotation)
+        self.motion_blur_k = int(motion_blur_k)
+        self.motion_blur_angle = tuple(float(v) for v in motion_blur_angle)
+        self.dropout_p = tuple(float(v) for v in dropout_p)
+        self.dropout_size_percent = tuple(float(v) for v in dropout_size_percent)
+        self.elastic_alpha = tuple(float(v) for v in elastic_alpha)
+        self.elastic_sigma = float(elastic_sigma)
+        if self.motion_blur_k and (self.motion_blur_k < 3 or self.motion_blur_k % 2 == 0):
+            raise ValueError("motion_blur_k must be 0 (off) or odd >= 3")
+        self.rng = np.random.default_rng(seed)
+
+    def sample(self, n):
+        out = []
+        for _ in range(int(n)):
+            on = self.rng.random(4) < self.apply_prob
+            rot = self.rng.uniform(-self.rotation, self.rotation)
+            angle = self.rng.uniform(*self.motion_blur_angle)
+            direction = self.rng.uniform(-1.0, 1.0)
+            p = self.rng.uniform(*self.dropout_p)
+            sp = self.rng.uniform(*self.dropout_size_percent)
+            alpha = self.rng.uniform(*self.elastic_alpha)
+            seed = int(self.rng.integers(0, 2 ** 63))
+            out.append(dict(rotate_deg=rot if on[0] else 0.0, blur_k=self.motion_blur_k if on[1] else 0,
+                            blur_angle_deg=angle, blur_direction=direction, drop_p=p if on[2] else 0.0,
+                            drop_size_percent=sp if on[2] else 0.0, elastic_alpha=alpha if on[3] else 0.0,
+                            elastic_sigma=self.elastic_sigma, seed=seed))
+        return out
+
+
+def build_aug(apply_prob=0.5, rotation=25, motion_blur_k=7, motion_blur_angle=(-90, 90), dropout_p=(0, 0.02),
+              dropout_size_percent=(0.01, 0.05), elastic_alpha=(0, 40), elastic_sigma=5, seed=None):
+    """fitdgp_util.py:412-451: the augmenters DeepLabCut's imgaug pipeline builds by default, each under
+    ``iaa.Sometimes(apply_prob)``: ``Affine(rotate=(-rotation, rotation))``, ``MotionBlur(k=motion_blur_k,
+    angle=motion_blur_angle)``, ``CoarseDropout(dropout_p, size_percent=dropout_size_percent)`` and
+    ``ElasticTransformation(alpha=elastic_alpha, sigma=elastic_sigma)``.  Returns the sampler ``data_aug`` takes; the
+    transforms run on the device (``dgp_augment``, bilinear elastic sampling -- see DESIGN.md)."""
+    return AugPipeline(apply_prob, rotation, motion_blur_k, motion_blur_angle, dropout_p, dropout_size_percent, elastic_alpha,
+                       elastic_sigma, seed)
+
+
+def data_aug(all_data_batch, visible_frame_within_batch, joint_loc, pipeline, dlc_cfg, engine=None):
+    """fitdgp_util.py data_aug, as called at fitdgp.py:773-779: augments the frames of the batch at the positions
+    ``visible_frame_within_batch`` and moves their labels ``joint_loc`` ((n_vis, nj, 2) scoremap (row, col), stride
+    ``dlc_cfg.stride``) with them.  ``all_data_batch``: (nt,H,W,3) frames on the host (non-uint8 values are rounded and
+    clipped as ``TrainSession.run`` does) or a CUDA tensor; neither is modified.  Returns (uint8 CUDA frames, float64 CUDA
+    joint_loc), ready to feed as ``inputs`` / ``targets``."""
+    from .fitdgp import _get
+    fr = all_data_batch
+    dev = engine.device if engine is not None else (fr.device if isinstance(fr, torch.Tensor) and fr.is_cuda
+                                                    else torch.device("cuda", torch.cuda.current_device()))
+    if isinstance(fr, torch.Tensor):
+        if fr.dtype != torch.uint8:
+            raise ValueError("a tensor batch must hold uint8 frames")
+        fr = fr.to(dev).clone(memory_format=torch.contiguous_format)
+    else:
+        fr = np.asarray(fr)
+        if fr.dtype != np.uint8:
+            fr = np.clip(np.round(fr), 0, 255).astype(np.uint8)
+        fr = torch.from_numpy(np.ascontiguousarray(fr)).to(dev)
+    if isinstance(joint_loc, torch.Tensor):
+        jl = joint_loc.to(device=dev, dtype=torch.float64).clone(memory_format=torch.contiguous_format)
+    else:
+        jl = torch.from_numpy(np.ascontiguousarray(np.asarray(joint_loc, dtype=np.float64))).to(dev)
+    pos = np.asarray(visible_frame_within_batch, dtype=np.int64).reshape(-1)
+    if jl.dim() != 3 or jl.shape[0] != pos.shape[0] or jl.shape[2] != 2:
+        raise ValueError("joint_loc must be (n_vis, nj, 2) with one label set per visible frame")
+    if pos.shape[0] == 0:
+        return fr, jl
+    eng = engine if engine is not None else _engine_for(jl.shape[1], dev)
+    eng.augment(fr, pos, jl, pipeline.sample(pos.shape[0]), stride=float(_get(dlc_cfg, "stride", 8.0)))
+    return fr, jl

@@ -250,6 +250,59 @@ int dgp_resize_coefficients(int in_size, int out_size, int max_taps, int32_t* fi
 int dgp_resize_crop(dgp_handle* h, const uint8_t* src_dev, int N, int H0, int W0, const dgp_frame_transform* t,
                     uint8_t* dst_dev, void* stream);
 
+/* ---- augmentation of labelled training frames (fit_dgp's data_aug, fitdgp.py:773-779; pipeline of build_aug,
+ * fitdgp_util.py:412-451) ----
+ * Per frame, in this order, each op switched on by its parameters:
+ *  1. rotation by rotate_deg (0 = off) about the frame centre: forward matrix, in double, with t = rotate_deg * (pi / 180),
+ *     c = cos t, s = sin t, cx = W / 2 - 0.5, cy = H / 2 - 0.5:  M = [[c, -s, cx - c cx + s cy], [s, c, cy - s cx - c cy]].
+ *     Pixels: bit-exact to cv2.warpAffine(img, M, (W, H), INTER_LINEAR, BORDER_CONSTANT, 0) -- OpenCV's fixed-point path
+ *     (M inverted in double; X0 = rint((M1 y + M2) 1024) + 16 per row, X = (X0 + rint(M0 x 1024)) >> 5 per column; 5
+ *     fraction bits select 2x2 int16 weights summing to 2^15; (sum w p + 2^14) >> 15, saturated; taps outside read 0).
+ *  2. motion blur with the k x k table of dgp_motion_blur_kernel(blur_k, blur_angle_deg, blur_direction) (blur_k 0 = off,
+ *     else odd in [3, 15]): (sum w p + 2^13) >> 14 per channel, saturated, correlation with a reflect-101 border.
+ *  3. coarse dropout (drop_p = 0 or drop_size_percent = 0: off): grid gh = max(1, rint(H sp)), gw = max(1, rint(W sp)),
+ *     sp = drop_size_percent; cell (i, j) is dropped when u01(seed, 2, i, j) < drop_p; pixel (y, x) lies in cell
+ *     (min(floor(y * (1 / (H / gh))), gh - 1), min(floor(x * (1 / (W / gw))), gw - 1)), in double -- the indexing of
+ *     cv2.resize(mask, (W, H), INTER_NEAREST); the pixels of dropped cells become 0 in all channels.
+ *  4. elastic deformation (elastic_alpha 0 = off) with the fields of dgp_elastic_field(alpha, sigma, seed):
+ *     out(x, y) = in(x + dx, y + dy), bit-exact to cv2.remap(img, x + dx, y + dy, INTER_LINEAR, BORDER_CONSTANT, 0) fed
+ *     the same float32 maps (map = float32(x) + dx in float32; X = rint(map * 32); the weights of rotation).
+ * Counter hash (splitmix64) of (seed, plane, row, col):
+ *     c = plane << 48 | row << 24 | col;  z = seed + (c + 1) * 0x9E3779B97F4A7C15;
+ *     z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9;  z = (z ^ z >> 27) * 0x94D049BB133111EB;  z ^= z >> 31;  b = z >> 40
+ *   (all mod 2^64); noise(seed, plane, row, col) = (b + 0.5) / 2^23 - 1 (float32, exact), u01 = (b + 0.5) / 2^24 (double). */
+typedef struct dgp_augment_params {
+  double rotate_deg;
+  int32_t blur_k;
+  double blur_angle_deg;
+  double blur_direction;     /* in [-1, 1] */
+  double drop_p;             /* in [0, 1] */
+  double drop_size_percent;  /* in [0, 1] */
+  double elastic_alpha;
+  double elastic_sigma;      /* in (0, 16] when elastic_alpha != 0 */
+  uint64_t seed;             /* of the dropout cells and the elastic noise */
+} dgp_augment_params;
+/* The motion-blur table (handle-free): a k x k float64 image whose middle column is numpy.linspace(d, 1 - d, k),
+ * d = (direction + 1) / 2, rotated by angle_deg about its centre c = (k - 1) / 2 with bilinear sampling (constant 0 outside):
+ * out(i, j) = img at (x, y) = (ca u + sa v + c, -sa u + ca v + c), u = j - c, v = i - c, ca = cos, sa = sin of
+ * angle_deg * (pi / 180); divided by its sum (row-major, sequential); w = rint(out * 2^14) and 2^14 - sum(w) added to the
+ * first largest weight, so the k * k int32 weights (row-major) sum to exactly 2^14.  k odd in [3, 15]. */
+int dgp_motion_blur_kernel(int k, double angle_deg, double direction, int32_t* weights);
+/* Elastic displacement fields of one H x W frame into float32 dx_dev, dy_dev (H, W): the noise planes 0 (dx) and 1 (dy) of
+ * `seed` are smoothed by a separable float32 Gaussian of radius R = ceil(4 sigma) (weights exp(-k^2 / (2 sigma^2)) divided
+ * by their sum in double, reflect-101 border, rows then columns) and multiplied by alpha.  sigma in (0, 16]. */
+int dgp_elastic_field(dgp_handle* h, int H, int W, double alpha, double sigma, uint64_t seed, float* dx_dev, float* dy_dev,
+                      void* stream);
+/* Augments frames_dev uint8 (nt, H, W, 3) in place: frame frame_idx_host[k] (k < n, distinct, in [0, nt)) with
+ * params_host[k]; other frames are not touched.  joint_loc_dev (NULL = no labels): float64 (n, nj) (row, col) scoremap
+ * labels of those frames, moved in place -- to pixels x = col stride + stride / 2, by M under rotation, under elastic by the
+ * inverse of the backward map (p <- q - d(p) from p = q, 20 iterations, d bilinear in the frame's float32 fields with
+ * coordinates clamped to the frame), and back; NaN labels stay NaN, labels leaving the frame are kept.  Blur and dropout
+ * leave labels alone.  Asynchronous on `stream`: per-frame matrices and tables travel as kernel arguments; a pass no frame
+ * needs is not launched.  Invalid arguments return DGP_ERR_INVALID before anything is launched. */
+int dgp_augment(dgp_handle* h, uint8_t* frames_dev, int nt, int H, int W, const int32_t* frame_idx_host, int n,
+                const dgp_augment_params* params_host, double* joint_loc_dev, double stride, void* stream);
+
 /* Replaces the estimate_pose frame loop (eval.py:306-345) end to end with HOST buffers: per batch of `batch`
  * frames H2D copy, dgp_forward, dgp_softargmax, D2H of the results.  frames_host uint8 (T,H,W,3) (pinned memory
  * gives asynchronous copies); mu_host float32 (T,nj,2); peak_host int32 (T,nj,2); lik_host float32 (T,nj). */
