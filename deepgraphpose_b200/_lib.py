@@ -107,6 +107,7 @@ SIGNATURES = {
     "dgp_augment": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, C.POINTER(DgpAugmentParams), _vp, C.c_double, _vp]),
     "dgp_debug_keep_activations": (_i, [_vp, _i]),
     "dgp_debug_get_activation": (_i, [_vp, C.c_char_p, _vp, _sz, _i64p]),
+    "dgp_debug_live_resources": (_i, [_i64p, _i64p]),
     "dgp_conv2d": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _vp,
                         _i, _i, _vp]),
     "dgp_conv2d_wgrad": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),

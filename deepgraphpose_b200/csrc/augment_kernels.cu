@@ -434,7 +434,7 @@ int dgp_elastic_field(dgp_handle* h, int H, int W, double alpha, double sigma, u
     return fail(h, DGP_ERR_INVALID, "dgp_elastic_field: bad argument");
   CU_OK(h, cudaSetDevice(h->device));
   if (int rc = ensure(h, &h->aug_tmp, (size_t)2 * H * W * sizeof(float))) return rc;
-  float* t = (float*)h->aug_tmp.p;
+  float* t = h->aug_tmp.get<float>();
   return launch_field(h, H, W, alpha, sigma, seed, t, t + (size_t)H * W, dx_dev, dy_dev, (cudaStream_t)stream);
 }
 
@@ -485,9 +485,9 @@ int dgp_augment(dgp_handle* h, uint8_t* frames_dev, int nt, int H, int W, const 
     if ((rc = ensure(h, &h->aug_fields, plane * 2 * n_el * sizeof(float)))) return rc;
     if ((rc = ensure(h, &h->aug_tmp, plane * 2 * sizeof(float)))) return rc;
   }
-  uint8_t* B = (uint8_t*)h->aug_scratch[0].p;
-  uint8_t* Cb = (uint8_t*)h->aug_scratch[1].p;
-  float* fields = (float*)h->aug_fields.p;
+  uint8_t* B = h->aug_scratch[0].get<uint8_t>();
+  uint8_t* Cb = h->aug_scratch[1].get<uint8_t>();
+  float* fields = h->aug_fields.get<float>();
   for (int k = 0; k < n; ++k) {
     Plan& f = plan[k];
     uint8_t* A = frames_dev + (size_t)frame_idx_host[k] * fb;
@@ -504,7 +504,7 @@ int dgp_augment(dgp_handle* h, uint8_t* frames_dev, int nt, int H, int W, const 
     const dgp_augment_params& p = params_host[k];
     if (!plan[k].el) continue;
     float* dx = fields + (size_t)plan[k].field * 2 * plane;
-    float* t = (float*)h->aug_tmp.p;
+    float* t = h->aug_tmp.get<float>();
     if ((rc = launch_field(h, H, W, p.elastic_alpha, p.elastic_sigma, p.seed, t, t + plane, dx, dx + plane, s))) return rc;
   }
   std::vector<int> step(n, 0);  // passes each frame has run so far

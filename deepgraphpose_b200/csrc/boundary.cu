@@ -40,27 +40,19 @@ int dgp_prediction_layers(dgp_handle* h, const float* net_dev, int B, int hf, in
   cudaStream_t s = (cudaStream_t)stream;
   const ConvLayer& L = h->layers[h->head_layer];
   const size_t npix = (size_t)B * hf * wf;
-  void* x16 = nullptr;
-  float* contrib = nullptr;
-  CU_OK(h, cudaMalloc(&x16, npix * 2048 * 2 + 1024));
-  cudaError_t e = cudaMalloc(&contrib, npix * L.Npad * 4);
-  if (e != cudaSuccess) { cudaFree(x16); return fail(h, DGP_ERR_NOMEM, "dgp_prediction_layers: %s", cudaGetErrorString(e)); }
-  int rc = DGP_OK;
+  DevBuf x16, contrib;
+  CU_OK(h, x16.alloc(npix * 2048 * 2 + 1024));
+  CU_OK(h, contrib.alloc(npix * L.Npad * 4));
   Step st;
   int dh, dw;
-  e = launch_f32_to_cvt16(net_dev, x16, npix * 2048, h->fp16, s);
-  if (e == cudaSuccess) {
-    rc = make_gemm_step(h, L, x16, B, hf, wf, 0, contrib, true, nullptr, 1, 0, 0, 0, &st, &dh, &dw);
-    if (rc == DGP_OK) e = launch_conv_gemm(st.gp, h->num_sms, s);
-  }
-  if (rc == DGP_OK && e == cudaSuccess)
-    e = launch_deconv_col2im(contrib, B, hf, wf, L.Npad, h->ctot, h->cfg.num_joints, h->head_bias, logits_dev, locref_dev, s);
-  h->launches += 3;
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  cudaFree(x16);
-  cudaFree(contrib);
+  CU_OK(h, launch_f32_to_cvt16(net_dev, x16.get(), npix * 2048, h->fp16, s));
+  int rc = make_gemm_step(h, L, x16.get(), B, hf, wf, 0, contrib.get(), true, nullptr, 1, 0, 0, 0, &st, &dh, &dw);
   if (rc) return rc;
-  if (e != cudaSuccess) return fail(h, DGP_ERR_CUDA, "dgp_prediction_layers: %s", cudaGetErrorString(e));
+  h->launches += 3;
+  CU_OK(h, launch_conv_gemm(st.gp, h->num_sms, s));
+  CU_OK(h, launch_deconv_col2im(contrib.get<float>(), B, hf, wf, L.Npad, h->ctot, h->cfg.num_joints, h->head_bias, logits_dev,
+                                locref_dev, s));
+  CU_OK(h, cudaStreamSynchronize(s));
   return DGP_OK;
 }
 
@@ -97,33 +89,23 @@ int dgp_deconv2d(dgp_handle* h, const float* x_dev, int N, int H, int W, int Cin
       for (int c = 0; c < Cin; ++c) d[c] = cvt16(h, src[c]);
     }
   const size_t npix = (size_t)N * H * W;
-  void *x16 = nullptr, *w16 = nullptr;
-  float *contrib = nullptr, *bias = nullptr;
-  cudaError_t e = cudaMalloc(&x16, npix * Cin * 2 + 1024);
-  if (e == cudaSuccess) e = cudaMalloc(&w16, wm.size() * 2);
-  if (e == cudaSuccess) e = cudaMalloc(&contrib, npix * L.Npad * 4);
-  if (e == cudaSuccess && bias_host) e = cudaMalloc(&bias, (size_t)Cout * 4);
-  int rc = DGP_OK;
-  if (e == cudaSuccess) e = cudaMemcpyAsync(w16, wm.data(), wm.size() * 2, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess && bias_host) e = cudaMemcpyAsync(bias, bias_host, (size_t)Cout * 4, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) e = launch_f32_to_cvt16(x_dev, x16, npix * Cin, h->fp16, s);
-  if (e == cudaSuccess) {
-    L.w = (__nv_bfloat16*)w16;
-    Step st;
-    int dh, dw;
-    rc = make_gemm_step(h, L, x16, N, H, W, 0, contrib, true, nullptr, 1, 0, 0, 0, &st, &dh, &dw);
-    if (rc == DGP_OK) e = launch_conv_gemm(st.gp, h->num_sms, s);
-  }
-  if (rc == DGP_OK && e == cudaSuccess)
-    e = launch_deconv_col2im(contrib, N, H, W, L.Npad, Cout, Cout, bias, out_dev, nullptr, s);
-  h->launches += 3;
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  cudaFree(x16);
-  cudaFree(w16);
-  cudaFree(contrib);
-  cudaFree(bias);
+  DevBuf x16, w16, contrib, bias;
+  CU_OK(h, x16.alloc(npix * Cin * 2 + 1024));
+  CU_OK(h, w16.alloc(wm.size() * 2));
+  CU_OK(h, contrib.alloc(npix * L.Npad * 4));
+  if (bias_host) CU_OK(h, bias.alloc((size_t)Cout * 4));
+  CU_OK(h, cudaMemcpyAsync(w16.get(), wm.data(), wm.size() * 2, cudaMemcpyHostToDevice, s));
+  if (bias_host) CU_OK(h, cudaMemcpyAsync(bias.get(), bias_host, (size_t)Cout * 4, cudaMemcpyHostToDevice, s));
+  CU_OK(h, launch_f32_to_cvt16(x_dev, x16.get(), npix * Cin, h->fp16, s));
+  L.w = w16.get<__nv_bfloat16>();
+  Step st;
+  int dh, dw;
+  int rc = make_gemm_step(h, L, x16.get(), N, H, W, 0, contrib.get(), true, nullptr, 1, 0, 0, 0, &st, &dh, &dw);
   if (rc) return rc;
-  if (e != cudaSuccess) return fail(h, DGP_ERR_CUDA, "dgp_deconv2d: %s", cudaGetErrorString(e));
+  h->launches += 3;
+  CU_OK(h, launch_conv_gemm(st.gp, h->num_sms, s));
+  CU_OK(h, launch_deconv_col2im(contrib.get<float>(), N, H, W, L.Npad, Cout, Cout, bias.get<float>(), out_dev, nullptr, s));
+  CU_OK(h, cudaStreamSynchronize(s));
   return DGP_OK;
 }
 

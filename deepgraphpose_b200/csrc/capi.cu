@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <atomic>
 #include <map>
 #include <memory>
 #include <string>
@@ -24,6 +25,7 @@ using namespace dgp;
 namespace dgp {
 
 char g_create_error[512] = "";
+std::atomic<int64_t> g_live_objects{0}, g_live_device_bytes{0};
 
 
 W16 cvt16(const dgp_handle* h, float f) {
@@ -85,26 +87,13 @@ const HostVar* find_var(dgp_handle* h, const std::string& name) {
   return it == h->host_vars.end() ? nullptr : &it->second;
 }
 
-int upload_layer(dgp_handle* h, ConvLayer& L, const std::vector<__nv_bfloat16>& wmat, const std::vector<float>* scale,
-                 const std::vector<float>* shift) {
-  CU_OK(h, cudaMalloc(&L.w, wmat.size() * sizeof(__nv_bfloat16)));
-  CU_OK(h, cudaMemcpy(L.w, wmat.data(), wmat.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
-  if (scale) {
-    CU_OK(h, cudaMalloc(&L.scale, scale->size() * sizeof(float)));
-    CU_OK(h, cudaMemcpy(L.scale, scale->data(), scale->size() * sizeof(float), cudaMemcpyHostToDevice));
-  }
-  if (shift) {
-    CU_OK(h, cudaMalloc(&L.shift, shift->size() * sizeof(float)));
-    CU_OK(h, cudaMemcpy(L.shift, shift->data(), shift->size() * sizeof(float), cudaMemcpyHostToDevice));
-  }
-  return DGP_OK;
-}
-
 // master fp32 -> 16-bit GEMM operands + BN scale/shift (after loading and after every optimizer step)
 int refresh_operands(dgp_handle* h, cudaStream_t s) {
-  CU_OK(h, launch_refresh_w16(h->master, h->w16, h->n_w, h->fp16, s));
-  CU_OK(h, launch_refresh_bn(h->master + h->n_w, h->master + h->n_w + h->n_ch, h->bn_mean, h->bn_var, h->cfg.bn_epsilon,
-                             (int)h->n_ch, h->bn_ss, h->bn_ss + h->n_ch, s));
+  const float* master = h->master.get<float>();
+  float* bn_ss = h->bn_ss.get<float>();
+  CU_OK(h, launch_refresh_w16(master, h->w16.get<W16>(), h->n_w, h->fp16, s));
+  CU_OK(h, launch_refresh_bn(master + h->n_w, master + h->n_w + h->n_ch, h->bn_mean.get<float>(), h->bn_var.get<float>(),
+                             h->cfg.bn_epsilon, (int)h->n_ch, bn_ss, bn_ss + h->n_ch, s));
   h->launches += 2;
   return DGP_OK;
 }
@@ -241,27 +230,29 @@ int upload_arena(dgp_handle* h) {
   h->n_bias = h->host_bias.size();
   h->n_params = h->n_w + 2 * h->n_ch + h->n_bias;
   if (h->n_w % 8 || h->n_ch % 4) return fail(h, DGP_ERR_STATE, "parameter arena is not vector aligned");
-  CU_OK(h, cudaMalloc(&h->master, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMalloc(&h->w16, h->n_w * sizeof(W16)));
-  CU_OK(h, cudaMalloc(&h->bn_mean, h->n_ch * sizeof(float)));
-  CU_OK(h, cudaMalloc(&h->bn_var, h->n_ch * sizeof(float)));
-  CU_OK(h, cudaMalloc(&h->bn_ss, 2 * h->n_ch * sizeof(float)));
-  CU_OK(h, cudaMemcpy(h->master, h->host_master.data(), h->n_w * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->master + h->n_w, h->host_gamma.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->master + h->n_w + h->n_ch, h->host_beta.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->master + h->n_w + 2 * h->n_ch, h->host_bias.data(), h->n_bias * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->bn_mean, h->host_mean.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->bn_var, h->host_var.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMalloc(&h->conv1_mask, h->host_conv1_mask.size() * 4));
-  CU_OK(h, cudaMemcpy(h->conv1_mask, h->host_conv1_mask.data(), h->host_conv1_mask.size() * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, h->master.alloc(h->n_params * sizeof(float)));
+  CU_OK(h, h->w16.alloc(h->n_w * sizeof(W16)));
+  CU_OK(h, h->bn_mean.alloc(h->n_ch * sizeof(float)));
+  CU_OK(h, h->bn_var.alloc(h->n_ch * sizeof(float)));
+  CU_OK(h, h->bn_ss.alloc(2 * h->n_ch * sizeof(float)));
+  float* master = h->master.get<float>();
+  CU_OK(h, cudaMemcpy(master, h->host_master.data(), h->n_w * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(master + h->n_w, h->host_gamma.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(master + h->n_w + h->n_ch, h->host_beta.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(master + h->n_w + 2 * h->n_ch, h->host_bias.data(), h->n_bias * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(h->bn_mean.get(), h->host_mean.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(h->bn_var.get(), h->host_var.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, h->conv1_mask.alloc(h->host_conv1_mask.size() * 4));
+  CU_OK(h, cudaMemcpy(h->conv1_mask.get(), h->host_conv1_mask.data(), h->host_conv1_mask.size() * 4, cudaMemcpyHostToDevice));
+  float* bn_ss = h->bn_ss.get<float>();
   for (ConvLayer& L : h->layers) {
-    L.w = h->w16 + L.w_off;
+    L.w = h->w16.get<W16>() + L.w_off;
     if (L.ch_off >= 0) {
-      L.scale = h->bn_ss + L.ch_off;
-      L.shift = h->bn_ss + h->n_ch + L.ch_off;
+      L.scale = bn_ss + L.ch_off;
+      L.shift = bn_ss + h->n_ch + L.ch_off;
     }
   }
-  h->head_bias = h->master + h->n_w + 2 * h->n_ch;
+  h->head_bias = master + h->n_w + 2 * h->n_ch;
   int rc = refresh_operands(h, nullptr);
   if (rc) return rc;
   CU_OK(h, cudaDeviceSynchronize());
@@ -269,12 +260,11 @@ int upload_arena(dgp_handle* h) {
   return DGP_OK;
 }
 
-int alloc_buf(dgp_handle* h, Plan* pl, size_t bytes, void** out) {
+int alloc_buf(dgp_handle* h, std::vector<DevBuf>* bufs, size_t bytes, void** out) {
   DevBuf b;
-  b.bytes = bytes;
-  CU_OK(h, cudaMalloc(&b.p, bytes));
-  pl->bufs.push_back(b);
-  *out = b.p;
+  CU_OK(h, b.alloc(bytes));
+  *out = b.get();
+  bufs->push_back(std::move(b));
   return DGP_OK;
 }
 
@@ -484,7 +474,6 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
     auto victim = plans.begin();
     for (auto jt = plans.begin(); jt != plans.end(); ++jt)
       if (jt->second->last_use < victim->second->last_use) victim = jt;
-    for (auto& b : victim->second->bufs) cudaFree(b.p);
     plans.erase(victim);
   }
   std::unique_ptr<Plan> pl(new Plan());
@@ -496,7 +485,7 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
   int rc;
   void* p = nullptr;
   // ---- conv1 (s2d + windowed im2col GEMM)
-  rc = alloc_buf(h, pl.get(), (size_t)B * pl->Hs * pl->Ws * 16 * 2, &p);
+  rc = alloc_buf(h, &pl->bufs, (size_t)B * pl->Hs * pl->Ws * 16 * 2, &p);
   if (rc) return rc;
   pl->s2d = (__nv_bfloat16*)p;
   {
@@ -523,19 +512,19 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
   const size_t x_bytes = (size_t)B * max_x * 2 + 1024, t_bytes = (size_t)B * max_t * 2 + 1024,
                sc_bytes = (size_t)B * max_sc * 2 + 1024;
   void *c1 = nullptr, *xa = nullptr, *xb = nullptr, *t1 = nullptr, *t2 = nullptr, *sc = nullptr;
-  if (unfused && (rc = alloc_buf(h, pl.get(), big, &c1))) return rc;
+  if (unfused && (rc = alloc_buf(h, &pl->bufs, big, &c1))) return rc;
   int Hc, Wc, pad_t, pad_l;
   same_pad(pl->H1, 3, 2, 1, &pad_t, &Hc);
   same_pad(pl->W1, 3, 2, 1, &pad_l, &Wc);
   if (!train) {
-    if ((rc = alloc_buf(h, pl.get(), x_bytes, &xa))) return rc;
-    if ((rc = alloc_buf(h, pl.get(), x_bytes, &xb))) return rc;
-    if ((rc = alloc_buf(h, pl.get(), sc_bytes, &sc))) return rc;
-    if ((rc = alloc_buf(h, pl.get(), t_bytes, &t1))) return rc;
-    if ((rc = alloc_buf(h, pl.get(), t_bytes, &t2))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, x_bytes, &xa))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, x_bytes, &xb))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, sc_bytes, &sc))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, t_bytes, &t1))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, t_bytes, &t2))) return rc;
   } else {
     // training keeps every activation for the backward pass: each tensor gets its own buffer
-    if ((rc = alloc_buf(h, pl.get(), (size_t)B * Hc * Wc * 64 * 2 + 1024, &xa))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * Hc * Wc * 64 * 2 + 1024, &xa))) return rc;
   }
   pl->c1 = c1; pl->pool = xa; pl->Hp = Hc; pl->Wp = Wc; pl->pool_pad_t = pad_t; pl->pool_pad_l = pad_l;
   {
@@ -610,10 +599,10 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
     if (train) {
       const int ho = ceil_div(Hc, u.stride), wo = ceil_div(Wc, u.stride);
       sc = nullptr;
-      if (u.shortcut >= 0 && (rc = alloc_buf(h, pl.get(), (size_t)B * Hc * Wc * u.depth * 2 + 1024, &sc))) return rc;
-      if ((rc = alloc_buf(h, pl.get(), (size_t)B * Hc * Wc * u.base * 2 + 1024, &t1))) return rc;
-      if ((rc = alloc_buf(h, pl.get(), (size_t)B * ho * wo * u.base * 2 + 1024, &t2))) return rc;
-      if ((rc = alloc_buf(h, pl.get(), (size_t)B * ho * wo * u.depth * 2 + 1024, &y))) return rc;
+      if (u.shortcut >= 0 && (rc = alloc_buf(h, &pl->bufs, (size_t)B * Hc * Wc * u.depth * 2 + 1024, &sc))) return rc;
+      if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * Hc * Wc * u.base * 2 + 1024, &t1))) return rc;
+      if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * ho * wo * u.base * 2 + 1024, &t2))) return rc;
+      if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * ho * wo * u.depth * 2 + 1024, &y))) return rc;
       Plan::UnitBufs ub;
       ub.x = x; ub.sc = sc; ub.t1 = t1; ub.t2 = t2; ub.out = y; ub.H = Hc; ub.W = Wc; ub.Ho = ho; ub.Wo = wo; ub.Cin = Cin;
       pl->ub.push_back(ub);
@@ -660,7 +649,7 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
   // ---- heads: GEMM over feature pixels + col2im
   {
     const ConvLayer& L = h->layers[h->head_layer];
-    if ((rc = alloc_buf(h, pl.get(), (size_t)B * Hc * Wc * L.Npad * 4, &p))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * Hc * Wc * L.Npad * 4, &p))) return rc;
     pl->contrib = (float*)p;
     pl->contrib_ld = L.Npad;
     Step st;
@@ -674,10 +663,10 @@ int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {
   }
   if (train) {
     const int nj = h->cfg.num_joints;
-    if ((rc = alloc_buf(h, pl.get(), (size_t)B * 4 * Hc * Wc * nj * 4, &p))) return rc;
+    if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * 4 * Hc * Wc * nj * 4, &p))) return rc;
     pl->logits = (float*)p;
     if (h->cfg.location_refinement) {
-      if ((rc = alloc_buf(h, pl.get(), (size_t)B * 4 * Hc * Wc * 2 * nj * 4, &p))) return rc;
+      if ((rc = alloc_buf(h, &pl->bufs, (size_t)B * 4 * Hc * Wc * 2 * nj * 4, &p))) return rc;
       pl->locref = (float*)p;
     }
   }
@@ -738,26 +727,73 @@ int run_forward_plan(dgp_handle* h, Plan* pl, const uint8_t* frames_dev, float* 
 int keep_activation(dgp_handle* h, const Step& st, cudaStream_t s) {
   if (!h->debug_keep || st.end_point.empty() || !st.out_ptr) return DGP_OK;
   const size_t bytes = (size_t)st.oN * st.oH * st.oW * st.oC * 2;
-  auto it = h->kept.find(st.end_point);
-  if (it != h->kept.end()) {
-    cudaFree(it->second.p);
-    h->kept.erase(it);
-  }
+  h->kept.erase(st.end_point);
   dgp_handle::Kept k;
   k.N = st.oN; k.H = st.oH; k.W = st.oW; k.C = st.oC;
-  CU_OK(h, cudaMalloc(&k.p, bytes));
-  CU_OK(h, cudaMemcpyAsync(k.p, st.out_ptr, bytes, cudaMemcpyDeviceToDevice, s));
-  h->kept[st.end_point] = k;
+  CU_OK(h, k.buf.alloc(bytes));
+  CU_OK(h, cudaMemcpyAsync(k.buf.get(), st.out_ptr, bytes, cudaMemcpyDeviceToDevice, s));
+  h->kept[st.end_point] = std::move(k);
   return DGP_OK;
 }
 
 int ensure(dgp_handle* h, DevBuf* b, size_t bytes) {
-  if (b->bytes >= bytes) return DGP_OK;
-  if (b->p) cudaFree(b->p);
-  b->p = nullptr;
-  b->bytes = 0;
-  CU_OK(h, cudaMalloc(&b->p, bytes));
-  b->bytes = bytes;
+  if (b->bytes() >= bytes) return DGP_OK;
+  CU_OK(h, b->alloc(bytes));
+  return DGP_OK;
+}
+
+// The ring of dgp_estimate_pose_stream, the H2D copies and `frames` carry source-size frames; the transform writes `xf`
+// on the compute stream.
+int PoseStaging::reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W, bool identity) {
+  const int nj = h->cfg.num_joints;
+  int hf, wf, ho, wo;
+  dgp_output_dims(H, W, &hf, &wf, &ho, &wo);
+  const size_t frame_bytes = (size_t)H0 * W0 * 3;
+  int rc;
+  if ((rc = ensure(h, &frames[0], frame_bytes * batch))) return rc;
+  if ((rc = ensure(h, &frames[1], frame_bytes * batch))) return rc;
+  if (!identity && (rc = ensure(h, &xf, (size_t)H * W * 3 * batch))) return rc;
+  if ((rc = ensure(h, &logits, (size_t)batch * ho * wo * nj * 4))) return rc;
+  if ((rc = ensure(h, &mu, (size_t)batch * nj * 2 * 4))) return rc;
+  if ((rc = ensure(h, &peak, (size_t)batch * nj * 2 * 4))) return rc;
+  if ((rc = ensure(h, &lik, (size_t)batch * nj * 4))) return rc;
+  if (!copy_stream) CU_OK(h, create(&copy_stream, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; ++i) {
+    if (!ev_copied[i]) CU_OK(h, create(&ev_copied[i], cudaEventDisableTiming));
+    if (!ev_consumed[i]) CU_OK(h, create(&ev_consumed[i], cudaEventDisableTiming));
+  }
+  return DGP_OK;
+}
+
+int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
+                           cudaHostFn_t release, void* release_arg) {
+  const int nj = h->cfg.num_joints;
+  int hf, wf, ho, wo;
+  dgp_output_dims(j.H, j.W, &hf, &wf, &ho, &wo);
+  cudaStream_t s = h->stream.get(), cs = copy_stream.get();
+  const int slot = it & 1;
+  // H2D of this batch on the copy stream, as soon as the batch that last used this slot has been consumed
+  if (it >= 2) CU_OK(h, cudaStreamWaitEvent(cs, ev_consumed[slot].get(), 0));
+  CU_OK(h, cudaMemcpyAsync(frames[slot].get(), host_frames, (size_t)j.H0 * j.W0 * 3 * n, cudaMemcpyHostToDevice, cs));
+  if (release) CU_OK(h, cudaLaunchHostFunc(cs, release, release_arg));
+  CU_OK(h, cudaEventRecord(ev_copied[slot].get(), cs));
+  CU_OK(h, cudaStreamWaitEvent(s, ev_copied[slot].get(), 0));
+  const uint8_t* x = frames[slot].get<uint8_t>();
+  int rc;
+  if (!j.identity) {
+    if ((rc = resize_crop_impl(h, x, n, j.H0, j.W0, j.transform, xf.get<uint8_t>(), s))) return rc;
+    x = xf.get<uint8_t>();
+  }
+  if ((rc = dgp_forward(h, x, run_n, j.H, j.W, logits.get<float>(), nullptr, s))) return rc;
+  CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), s));
+  if ((rc = dgp_softargmax(h, logits.get<float>(), nullptr, run_n, ho, wo, nj, j.gamma, j.gauss_len, mu.get<float>(),
+                           peak.get<int32_t>(), lik.get<float>(), nullptr, nullptr, s)))
+    return rc;
+  CU_OK(h, cudaMemcpyAsync(j.mu_host + (size_t)t0 * nj * 2, mu.get(), (size_t)n * nj * 2 * 4, cudaMemcpyDeviceToHost, s));
+  if (j.peak_host)
+    CU_OK(h, cudaMemcpyAsync(j.peak_host + (size_t)t0 * nj * 2, peak.get(), (size_t)n * nj * 2 * 4, cudaMemcpyDeviceToHost, s));
+  if (j.lik_host)
+    CU_OK(h, cudaMemcpyAsync(j.lik_host + (size_t)t0 * nj, lik.get(), (size_t)n * nj * 4, cudaMemcpyDeviceToHost, s));
   return DGP_OK;
 }
 
@@ -790,7 +826,7 @@ int dgp_create(const dgp_config* cfg, dgp_handle** out) {
   if (h->cfg.bn_epsilon <= 0) h->cfg.bn_epsilon = 1e-5f;
   h->device = cfg->device;
   h->num_sms = prop.multiProcessorCount;
-  e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
+  e = create(&h->stream, cudaStreamNonBlocking);
   if (e != cudaSuccess) {
     delete h;
     return fail(nullptr, DGP_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
@@ -802,45 +838,7 @@ int dgp_create(const dgp_config* cfg, dgp_handle** out) {
 void dgp_destroy(dgp_handle* h) {
   if (!h) return;
   cudaSetDevice(h->device);
-  cudaDeviceSynchronize();
-  train_destroy(h);
-  cudaFree(h->master);
-  cudaFree(h->w16);
-  cudaFree(h->bn_mean);
-  cudaFree(h->bn_var);
-  cudaFree(h->bn_ss);
-  cudaFree(h->conv1_mask);
-  for (auto& kv : h->plans)
-    for (auto& b : kv.second->bufs) cudaFree(b.p);
-  for (auto& kv : h->train_plans)
-    for (auto& b : kv.second->bufs) cudaFree(b.p);
-  for (auto& kv : h->kept) cudaFree(kv.second.p);
-  cudaFree(h->sa_ws);
-  cudaFree(h->flow_ws.p);
-  cudaFree(h->loss_ws.p);
-  cudaFree(h->st_frames2[0].p);
-  cudaFree(h->st_frames2[1].p);
-  for (int i = 0; i < 3; ++i)
-    if (h->ring_slot[i]) cudaFreeHost(h->ring_slot[i]);
-  for (int i = 0; i < 2; ++i) {
-    if (h->ev_copied[i]) cudaEventDestroy(h->ev_copied[i]);
-    if (h->ev_consumed[i]) cudaEventDestroy(h->ev_consumed[i]);
-  }
-  if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-  cudaFree(h->st_logits.p);
-  cudaFree(h->st_mu.p);
-  cudaFree(h->st_peak.p);
-  cudaFree(h->st_lik.p);
-  cudaFree(h->st_xf.p);
-  cudaFree(h->resize_tmp.p);
-  for (auto& kv : h->resize_tables) cudaFree(kv.second.dev);
-  cudaFree(h->aug_scratch[0].p);
-  cudaFree(h->aug_scratch[1].p);
-  cudaFree(h->aug_fields.p);
-  cudaFree(h->aug_tmp.p);
-  for (auto& r : h->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
-  for (auto e : h->ev_pool) cudaEventDestroy(e);
-  if (h->stream) cudaStreamDestroy(h->stream);
+  cudaDeviceSynchronize();  // nothing in flight uses what the owners release
   delete h;
 }
 
@@ -969,17 +967,10 @@ int dgp_softargmax(dgp_handle* h, const float* logits_dev, const float* locref_d
     return fail(h, DGP_ERR_UNSUPPORTED, "dgp_softargmax: num_joints must be <= 128 with num_joints / gcd(num_joints, 4) <= 32");
   CU_OK(h, cudaSetDevice(h->device));
   const int splits = softargmax_splits(H, W, nj);
-  const size_t need = (size_t)B * splits * nj * sizeof(SaPartial);
-  if (need > h->sa_ws_bytes) {
-    if (h->sa_ws) CU_OK(h, cudaFree(h->sa_ws));
-    h->sa_ws = nullptr;
-    h->sa_ws_bytes = 0;
-    CU_OK(h, cudaMalloc(&h->sa_ws, need));
-    h->sa_ws_bytes = need;
-  }
+  if (int rc = ensure(h, &h->sa_ws, (size_t)B * splits * nj * sizeof(SaPartial))) return rc;
   ProfScope prof(h, 4, (cudaStream_t)stream);
   CU_OK(h, launch_softargmax(logits_dev, locref_dev, B, H, W, nj, gamma, gauss_len, h->cfg.stride, h->cfg.locref_stdev,
-                             h->sa_ws, splits, mu_dev, peak_dev, lik_dev, dlc_peak_dev, dlc_pose_dev, nullptr,
+                             h->sa_ws.get<SaPartial>(), splits, mu_dev, peak_dev, lik_dev, dlc_peak_dev, dlc_pose_dev, nullptr,
                              (cudaStream_t)stream));
   h->launches += 2;
   return DGP_OK;
@@ -994,16 +985,11 @@ int dgp_softmax_map(dgp_handle* h, const float* logits_dev, int B, int H, int W,
   CU_OK(h, cudaSetDevice(h->device));
   const int splits = softargmax_splits(H, W, nj);
   const size_t need = (size_t)B * splits * nj * sizeof(SaPartial) + (size_t)B * nj * 2 * sizeof(float);
-  if (need > h->sa_ws_bytes) {
-    if (h->sa_ws) CU_OK(h, cudaFree(h->sa_ws));
-    h->sa_ws = nullptr;
-    h->sa_ws_bytes = 0;
-    CU_OK(h, cudaMalloc(&h->sa_ws, need));
-    h->sa_ws_bytes = need;
-  }
-  float* norm = reinterpret_cast<float*>(h->sa_ws + (size_t)B * splits * nj);
-  CU_OK(h, launch_softargmax(logits_dev, nullptr, B, H, W, nj, gamma, gauss_len, h->cfg.stride, h->cfg.locref_stdev,
-                             h->sa_ws, splits, nullptr, nullptr, nullptr, nullptr, nullptr, norm, (cudaStream_t)stream));
+  if (int rc = ensure(h, &h->sa_ws, need)) return rc;
+  SaPartial* ws = h->sa_ws.get<SaPartial>();
+  float* norm = reinterpret_cast<float*>(ws + (size_t)B * splits * nj);
+  CU_OK(h, launch_softargmax(logits_dev, nullptr, B, H, W, nj, gamma, gauss_len, h->cfg.stride, h->cfg.locref_stdev, ws, splits,
+                             nullptr, nullptr, nullptr, nullptr, nullptr, norm, (cudaStream_t)stream));
   CU_OK(h, launch_softmax_map(logits_dev, norm, B, H, W, nj, gamma, gauss_len, map_dev, h->num_sms, (cudaStream_t)stream));
   h->launches += 3;
   return DGP_OK;
@@ -1032,7 +1018,7 @@ int dgp_run_loss_impl(dgp_handle* h, const dgp_loss_cfg* cfg, const dgp_loss_bat
   const size_t need = (size_t)nm * 2 * 4 * 3 + (size_t)(b->nbv + b->nbh + 1) * 16 + (size_t)nm * 4 + (size_t)nm * 16 + 512 + flow_part_bytes;
   int rc = ensure(h, &h->loss_ws, need);
   if (rc) return rc;
-  char* w = (char*)h->loss_ws.p;
+  char* w = h->loss_ws.get<char>();
   float* mu = (float*)w; w += (size_t)nm * 2 * 4;
   float* all = (float*)w; w += (size_t)nm * 2 * 4;
   float* norm = (float*)w; w += (size_t)nm * 2 * 4;
@@ -1046,17 +1032,10 @@ int dgp_run_loss_impl(dgp_handle* h, const dgp_loss_cfg* cfg, const dgp_loss_bat
     return fail(h, DGP_ERR_INVALID, "dgp_loss: scoremap dims must be even, gauss_len in [1,5), gamma > 0");
   {
     const int splits = softargmax_splits(b->H, b->W, nj);
-    const size_t sa_need = (size_t)b->nt * splits * nj * sizeof(SaPartial);
-    if (sa_need > h->sa_ws_bytes) {
-      if (h->sa_ws) CU_OK(h, cudaFree(h->sa_ws));
-      h->sa_ws = nullptr;
-      h->sa_ws_bytes = 0;
-      CU_OK(h, cudaMalloc(&h->sa_ws, sa_need));
-      h->sa_ws_bytes = sa_need;
-    }
+    if ((rc = ensure(h, &h->sa_ws, (size_t)b->nt * splits * nj * sizeof(SaPartial)))) return rc;
     CU_OK(h, launch_softargmax(b->pred_dev, nullptr, b->nt, b->H, b->W, nj, cfg->gamma, cfg->gauss_len, h->cfg.stride,
-                               h->cfg.locref_stdev, h->sa_ws, splits, mu, nullptr, nullptr, nullptr, nullptr, norm,
-                               (cudaStream_t)stream));
+                               h->cfg.locref_stdev, h->sa_ws.get<SaPartial>(), splits, mu, nullptr, nullptr, nullptr, nullptr,
+                               norm, (cudaStream_t)stream));
     h->launches += 2;
   }
   LossArgs a;
@@ -1151,7 +1130,7 @@ int dgp_learn_wt(dgp_handle* h, const uint8_t* frames_dev, int T, int H, int W, 
   CU_OK(h, cudaSetDevice(h->device));
   if (int rc = ensure(h, &h->flow_ws, learn_wt_workspace_bytes(T, H, W))) return rc;
   int nl = 0;
-  CU_OK(h, launch_learn_wt(frames_dev, T, H, W, field_dev, h->flow_ws.p, &nl, (cudaStream_t)stream));
+  CU_OK(h, launch_learn_wt(frames_dev, T, H, W, field_dev, h->flow_ws.get(), &nl, (cudaStream_t)stream));
   h->launches += nl;
   return DGP_OK;
 }
@@ -1209,56 +1188,19 @@ int dgp_estimate_pose_host_transform(dgp_handle* h, const uint8_t* frames_host, 
     return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_host: invalid frame size or transform");
   if (T == 0) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
-  const int nj = h->cfg.num_joints;
-  int hf, wf, ho, wo;
-  dgp_output_dims(H, W, &hf, &wf, &ho, &wo);
+  int rc = h->pose.reserve(h, batch, H0, W0, H, W, identity);
+  if (rc) return rc;
+  const PoseJob job = {H0, W0, H, W, identity, transform, gamma, gauss_len, mu_host, peak_host, lik_host};
   const size_t frame_bytes = (size_t)H0 * W0 * 3;
-  int rc;
-  if ((rc = ensure(h, &h->st_frames2[0], frame_bytes * batch))) return rc;
-  if ((rc = ensure(h, &h->st_frames2[1], frame_bytes * batch))) return rc;
-  if (!identity && (rc = ensure(h, &h->st_xf, (size_t)H * W * 3 * batch))) return rc;
-  if ((rc = ensure(h, &h->st_logits, (size_t)batch * ho * wo * nj * 4))) return rc;
-  if ((rc = ensure(h, &h->st_mu, (size_t)batch * nj * 2 * 4))) return rc;
-  if ((rc = ensure(h, &h->st_peak, (size_t)batch * nj * 2 * 4))) return rc;
-  if ((rc = ensure(h, &h->st_lik, (size_t)batch * nj * 4))) return rc;
-  if (!h->copy_stream) {
-    CU_OK(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-      CU_OK(h, cudaEventCreateWithFlags(&h->ev_copied[i], cudaEventDisableTiming));
-      CU_OK(h, cudaEventCreateWithFlags(&h->ev_consumed[i], cudaEventDisableTiming));
-    }
-  }
-  cudaStream_t s = h->stream, cs = h->copy_stream;
   int it = 0;
   for (int t0 = 0; t0 < T; t0 += batch, ++it) {
     const int b = (T - t0) < batch ? (T - t0) : batch;
-    const int slot = it & 1;
-    // H2D of this batch on the copy stream, as soon as the batch that last used this slot has been consumed
-    if (it >= 2) CU_OK(h, cudaStreamWaitEvent(cs, h->ev_consumed[slot], 0));
-    CU_OK(h, cudaMemcpyAsync(h->st_frames2[slot].p, frames_host + (size_t)t0 * frame_bytes, frame_bytes * b,
-                             cudaMemcpyHostToDevice, cs));
-    CU_OK(h, cudaEventRecord(h->ev_copied[slot], cs));
-    CU_OK(h, cudaStreamWaitEvent(s, h->ev_copied[slot], 0));
     // the tail batch of a multi-batch video reuses the full-batch plan (see dgp_estimate_pose_stream): surplus rows hold an
     // earlier batch's frames and their read-outs are not copied back
     const int run_b = (b < batch && it > 0) ? batch : b;
-    const uint8_t* frames = (const uint8_t*)h->st_frames2[slot].p;
-    if (!identity) {
-      if ((rc = resize_crop_impl(h, frames, b, H0, W0, transform, (uint8_t*)h->st_xf.p, s))) return rc;
-      frames = (const uint8_t*)h->st_xf.p;
-    }
-    if ((rc = dgp_forward(h, frames, run_b, H, W, (float*)h->st_logits.p, nullptr, s))) return rc;
-    CU_OK(h, cudaEventRecord(h->ev_consumed[slot], s));
-    if ((rc = dgp_softargmax(h, (const float*)h->st_logits.p, nullptr, run_b, ho, wo, nj, gamma, gauss_len,
-                             (float*)h->st_mu.p, (int32_t*)h->st_peak.p, (float*)h->st_lik.p, nullptr, nullptr, s)))
-      return rc;
-    CU_OK(h, cudaMemcpyAsync(mu_host + (size_t)t0 * nj * 2, h->st_mu.p, (size_t)b * nj * 2 * 4, cudaMemcpyDeviceToHost, s));
-    if (peak_host)
-      CU_OK(h, cudaMemcpyAsync(peak_host + (size_t)t0 * nj * 2, h->st_peak.p, (size_t)b * nj * 2 * 4, cudaMemcpyDeviceToHost, s));
-    if (lik_host)
-      CU_OK(h, cudaMemcpyAsync(lik_host + (size_t)t0 * nj, h->st_lik.p, (size_t)b * nj * 4, cudaMemcpyDeviceToHost, s));
+    if ((rc = h->pose.run_batch(h, job, frames_host + (size_t)t0 * frame_bytes, b, run_b, it, t0, nullptr, nullptr))) return rc;
   }
-  CU_OK(h, cudaStreamSynchronize(s));
+  CU_OK(h, cudaStreamSynchronize(h->stream.get()));
   return DGP_OK;
 }
 
@@ -1280,7 +1222,7 @@ int dgp_debug_get_activation(dgp_handle* h, const char* end_point, float* host_o
   CU_OK(h, cudaSetDevice(h->device));
   CU_OK(h, cudaDeviceSynchronize());
   std::vector<__nv_bfloat16> tmp(n);
-  CU_OK(h, cudaMemcpy(tmp.data(), k.p, n * 2, cudaMemcpyDeviceToHost));
+  CU_OK(h, cudaMemcpy(tmp.data(), k.buf.get(), n * 2, cudaMemcpyDeviceToHost));
   for (size_t i = 0; i < n; ++i) host_out[i] = cvt16_to_float(h, tmp[i]);
   return DGP_OK;
 }
@@ -1305,25 +1247,29 @@ int dgp_conv2d(dgp_handle* h, const void* x_dev, int N, int H, int W, int Cin, c
     for (int c = 0; c < Cin; ++c)
       for (int o = 0; o < Cout; ++o)
         wm[(size_t)o * L.K + (size_t)t * Cin + c] = cvt16(h, w_host[((size_t)t * Cin + c) * Cout + o]);
-  std::vector<float> sc, sh;
-  if (scale_host) sc.assign(scale_host, scale_host + Cout);
-  if (shift_host) sh.assign(shift_host, shift_host + Cout);
-  int rc = upload_layer(h, L, wm, scale_host ? &sc : nullptr, shift_host ? &sh : nullptr);
-  if (rc) return rc;
+  DevBuf w, scale, shift;
+  CU_OK(h, w.alloc(wm.size() * sizeof(__nv_bfloat16)));
+  CU_OK(h, cudaMemcpy(w.get(), wm.data(), wm.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
+  if (scale_host) {
+    CU_OK(h, scale.alloc(Cout * sizeof(float)));
+    CU_OK(h, cudaMemcpy(scale.get(), scale_host, Cout * sizeof(float), cudaMemcpyHostToDevice));
+  }
+  if (shift_host) {
+    CU_OK(h, shift.alloc(Cout * sizeof(float)));
+    CU_OK(h, cudaMemcpy(shift.get(), shift_host, Cout * sizeof(float), cudaMemcpyHostToDevice));
+  }
+  L.w = w.get<__nv_bfloat16>();
+  L.scale = scale.get<float>();
+  L.shift = shift.get<float>();
   Step st;
   int Ho, Wo;
-  rc = make_gemm_step(h, L, x_dev, N, H, W, pad_mode, out_dev, out_f32 != 0, (const __nv_bfloat16*)residual_dev,
-                      res_sub > 0 ? res_sub : 1, res_H, res_W, 0, &st, &Ho, &Wo);
-  if (rc == DGP_OK) {
-    cudaError_t e = launch_conv_gemm(st.gp, h->num_sms, (cudaStream_t)stream);
-    h->launches++;
-    if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);
-    if (e != cudaSuccess) rc = fail(h, DGP_ERR_CUDA, "dgp_conv2d launch: %s", cudaGetErrorString(e));
-  }
-  cudaFree(L.w);
-  cudaFree(L.scale);
-  cudaFree(L.shift);
-  return rc;
+  int rc = make_gemm_step(h, L, x_dev, N, H, W, pad_mode, out_dev, out_f32 != 0, (const __nv_bfloat16*)residual_dev,
+                          res_sub > 0 ? res_sub : 1, res_H, res_W, 0, &st, &Ho, &Wo);
+  if (rc) return rc;
+  h->launches++;
+  CU_OK(h, launch_conv_gemm(st.gp, h->num_sms, (cudaStream_t)stream));
+  CU_OK(h, cudaStreamSynchronize((cudaStream_t)stream));
+  return DGP_OK;
 }
 
 int dgp_conv2d_wgrad(dgp_handle* h, const void* x_dev, int N, int H, int W, int Cin, const void* dy_dev, int R, int S,
@@ -1336,15 +1282,13 @@ int dgp_conv2d_wgrad(dgp_handle* h, const void* x_dev, int N, int H, int W, int 
   int rc = make_wgrad_params(h, "dgp_conv2d_wgrad", R, S, Cin, Cout, stride, dilation, x_dev, N, H, W, pad_mode, dy_dev, &wp);
   if (rc) return rc;
   if (dbg3) { wp.dbg_lbo = (uint32_t)dbg3[0]; wp.dbg_sbo = (uint32_t)dbg3[1]; wp.dbg_kstep = (uint32_t)dbg3[2]; }
-  void* ws = nullptr;
-  CU_OK(h, cudaMalloc(&ws, wgrad_workspace_bytes(wp)));
-  wp.partials = (float*)ws;
-  cudaError_t e = launch_wgrad_gemm(wp, h->num_sms, (cudaStream_t)stream);
-  if (e == cudaSuccess) e = launch_wgrad_reduce(wp, nullptr, nullptr, dw_dev, nullptr, (cudaStream_t)stream);
+  DevBuf ws;
+  CU_OK(h, ws.alloc(wgrad_workspace_bytes(wp)));
+  wp.partials = ws.get<float>();
   h->launches += 2;
-  if (e == cudaSuccess) e = cudaStreamSynchronize((cudaStream_t)stream);
-  cudaFree(ws);
-  if (e != cudaSuccess) return fail(h, DGP_ERR_CUDA, "dgp_conv2d_wgrad launch: %s", cudaGetErrorString(e));
+  CU_OK(h, launch_wgrad_gemm(wp, h->num_sms, (cudaStream_t)stream));
+  CU_OK(h, launch_wgrad_reduce(wp, nullptr, nullptr, dw_dev, nullptr, (cudaStream_t)stream));
+  CU_OK(h, cudaStreamSynchronize((cudaStream_t)stream));
   return DGP_OK;
 }
 
@@ -1362,12 +1306,12 @@ int dgp_get_profile(dgp_handle* h, double* ms_by_kind, int64_t* count_by_kind, i
   for (int i = 0; i < nkinds; ++i) { ms_by_kind[i] = 0.0; count_by_kind[i] = 0; }
   for (auto& r : h->prof) {
     float ms = 0.0f;
-    if (cudaEventElapsedTime(&ms, r.a, r.b) == cudaSuccess && r.kind < nkinds) {
+    if (cudaEventElapsedTime(&ms, r.a.get(), r.b.get()) == cudaSuccess && r.kind < nkinds) {
       ms_by_kind[r.kind] += ms;
       count_by_kind[r.kind] += r.count;
     }
-    h->ev_pool.push_back(r.a);
-    h->ev_pool.push_back(r.b);
+    h->ev_pool.push_back(std::move(r.a));
+    h->ev_pool.push_back(std::move(r.b));
   }
   h->prof.clear();
   return DGP_OK;
@@ -1380,13 +1324,13 @@ int dgp_get_profile_records(dgp_handle* h, float* ms, int32_t* kind, int max_rec
   int n = 0;
   for (auto& r : h->prof) {
     float t = 0.0f;
-    if (n < max_records && cudaEventElapsedTime(&t, r.a, r.b) == cudaSuccess) {
+    if (n < max_records && cudaEventElapsedTime(&t, r.a.get(), r.b.get()) == cudaSuccess) {
       ms[n] = t;
       kind[n] = r.kind;
       ++n;
     }
-    h->ev_pool.push_back(r.a);
-    h->ev_pool.push_back(r.b);
+    h->ev_pool.push_back(std::move(r.a));
+    h->ev_pool.push_back(std::move(r.b));
   }
   h->prof.clear();
   *n_records = n;
@@ -1413,5 +1357,11 @@ uint32_t dgp_crc32c(const void* data, size_t n) {
 
 int64_t dgp_launch_count(const dgp_handle* h) { return h ? h->launches : 0; }
 int dgp_num_sms(const dgp_handle* h) { return h ? h->num_sms : 0; }
+
+int dgp_debug_live_resources(int64_t* objects, int64_t* device_bytes) {
+  if (objects) *objects = g_live_objects;
+  if (device_bytes) *device_bytes = g_live_device_bytes;
+  return DGP_OK;
+}
 
 }  // extern "C"

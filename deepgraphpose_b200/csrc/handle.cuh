@@ -18,20 +18,19 @@
 
 #include "conv_gemm_sm100.cuh"
 #include "kernels.cuh"
+#include "owned.cuh"
 
 namespace dgp {
 
 struct TrainState;  // train.cu
+struct TrainStateDeleter {
+  void operator()(TrainState* ts) const;  // train.cu
+};
 typedef __nv_bfloat16 W16;  // opaque 16-bit storage element (bf16 or fp16 bits)
 
 struct HostVar {
   std::vector<float> data;
   std::vector<int64_t> shape;
-};
-
-struct DevBuf {
-  void* p = nullptr;
-  size_t bytes = 0;
 };
 
 struct ConvLayer {
@@ -97,7 +96,32 @@ struct Plan {
 struct ResizeTable {
   int ksize = 0;
   std::vector<int32_t> first, count;
-  int32_t* dev = nullptr;
+  DevBuf dev;
+};
+
+// What one dgp_estimate_pose_host / _stream call reads and writes, besides its frames.
+struct PoseJob {
+  int H0, W0;       // source frame size
+  int H, W;         // size of the frames the network sees (after the transform)
+  bool identity;    // the transform leaves frames unchanged
+  const dgp_frame_transform* transform;
+  float gamma, gauss_len;
+  float* mu_host;
+  int32_t* peak_host;
+  float* lik_host;
+};
+
+// estimate_pose staging: source frames double-buffered between the H2D of the copy stream and the compute stream (slot =
+// batch index & 1), the transformed batch that dgp_forward consumes when a frame transform is given, and the read-outs.
+struct PoseStaging {
+  Stream copy_stream;  // H2D of the next batch overlaps the current batch's kernels
+  Event ev_copied[2], ev_consumed[2];
+  DevBuf frames[2], xf, logits, mu, peak, lik;
+  int reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W, bool identity);
+  // Batch number `it` (n frames at host_frames, output rows [t0, t0 + n)): H2D, transform, forward + soft-argmax of run_n
+  // rows, D2H of n read-outs.  release(release_arg) runs on the copy stream once host_frames has been copied.
+  int run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
+                cudaHostFn_t release, void* release_arg);
 };
 
 }  // namespace dgp
@@ -105,7 +129,7 @@ struct ResizeTable {
 using namespace dgp;  // internal header: the handle's members are dgp:: types
 
 struct dgp_handle {
-  dgp::TrainState* train = nullptr;  // allocated by dgp_train_enable
+  std::unique_ptr<TrainState, TrainStateDeleter> train;  // set by dgp_train_enable
   dgp_config cfg;
   int device = 0;
   int num_sms = 0;
@@ -121,19 +145,19 @@ struct dgp_handle {
   float* head_bias = nullptr;  // points into the arena
   int ctot = 0;
   // Parameter arena (fp32 master, kernel layouts): [weights n_w | gamma n_ch | beta n_ch | head bias n_bias]
-  float* master = nullptr;
-  dgp::W16* w16 = nullptr;       // 16-bit copy of the weight part (tensor-core operands)
-  float* bn_mean = nullptr;      // frozen moving statistics [n_ch]
-  float* bn_var = nullptr;
-  float* bn_ss = nullptr;        // [scale n_ch | shift n_ch]
-  float* conv1_mask = nullptr;   // [64][256] 1 = real 7x7x3 tap of the space-to-depth conv1 matrix
+  DevBuf master;
+  DevBuf w16;          // W16: 16-bit copy of the weight part (tensor-core operands)
+  DevBuf bn_mean;      // frozen moving statistics [n_ch]
+  DevBuf bn_var;
+  DevBuf bn_ss;        // [scale n_ch | shift n_ch]
+  DevBuf conv1_mask;   // [64][256] 1 = real 7x7x3 tap of the space-to-depth conv1 matrix
   size_t n_w = 0, n_ch = 0, n_bias = 0, n_params = 0;
   std::vector<float> host_master, host_gamma, host_beta, host_mean, host_var, host_bias, host_conv1_mask;
   std::map<std::tuple<int, int, int>, std::unique_ptr<Plan>> plans, train_plans;  // inference key (-B,..) = unchunked debug plan
   uint64_t plan_clock = 0;
   bool debug_keep = false;
   struct Kept {
-    void* p;
+    DevBuf buf;
     int N, H, W, C;
   };
   std::map<std::string, Kept> kept;
@@ -143,22 +167,16 @@ struct dgp_handle {
   struct ProfRec {
     int kind;
     int count = 1;   // launches bracketed by the event pair (> 1 in bracket mode)
-    cudaEvent_t a, b;
+    Event a, b;
   };
   bool profile_brackets = false;  // dgp_set_profiling(h, 2): one event pair around every RUN of same-kind launches
   std::vector<ProfRec> prof;
-  std::vector<cudaEvent_t> ev_pool;
-  // softargmax workspace
+  std::vector<Event> ev_pool;
   DevBuf flow_ws;   // dgp_learn_wt workspace
-  SaPartial* sa_ws = nullptr;
-  size_t sa_ws_bytes = 0;
+  DevBuf sa_ws;     // SaPartial: softargmax workspace
   DevBuf loss_ws;
-  // estimate_pose_host staging
-  cudaStream_t stream = nullptr;       // compute stream of dgp_estimate_pose_host
-  cudaStream_t copy_stream = nullptr;  // H2D of the next batch overlaps the current batch's kernels
-  cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr};
-  DevBuf st_frames2[2], st_logits, st_mu, st_peak, st_lik;
-  DevBuf st_xf;      // transformed (resized / cropped) batch that dgp_forward consumes when a frame transform is given
+  Stream stream;    // the handle's own stream: estimate_pose computes and the backward graph is captured on it
+  PoseStaging pose;
   // dgp_resize_crop: tables per (in, out) size pair and the uint8 intermediate of the horizontal pass
   std::map<std::pair<int, int>, ResizeTable> resize_tables;
   DevBuf resize_tmp;
@@ -166,8 +184,7 @@ struct dgp_handle {
   // intermediate of the field's horizontal pass
   DevBuf aug_scratch[2], aug_fields, aug_tmp;
   // dgp_estimate_pose_stream: pinned host ring the reader thread decodes into (stream.cu)
-  void* ring_slot[3] = {nullptr, nullptr, nullptr};
-  size_t ring_bytes = 0;
+  PinnedBuf ring_slot[3];
 };
 
 // loss forward (+ optional loss-side backward) shared by dgp_loss_forward / dgp_loss_backward / the training step
@@ -200,27 +217,26 @@ int make_gemm_step(dgp_handle* h, const ConvLayer& L, const void* x, int N, int 
                    Step* st, int* Ho, int* Wo);
 int make_wgrad_params(dgp_handle* h, const char* scope, int R, int S, int Cin, int Cout, int stride, int dil,
                       const void* x, int N, int H, int W, int pad_mode, const void* dy, WgradParams* wp);
-int alloc_buf(dgp_handle* h, Plan* pl, size_t bytes, void** out);
+int alloc_buf(dgp_handle* h, std::vector<DevBuf>* bufs, size_t bytes, void** out);
 int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out);
 int run_forward_plan(dgp_handle* h, Plan* pl, const uint8_t* frames_dev, float* logits_dev, float* locref_dev,
                      cudaStream_t s, int first_step = 0, int last_step = -1);
 int ensure(dgp_handle* h, DevBuf* b, size_t bytes);
 int refresh_operands(dgp_handle* h, cudaStream_t s);
-void train_destroy(dgp_handle* h);  // train.cu
 // Size of a transformed frame (DGP_ERR_INVALID for an invalid transform); *identity: the transform leaves frames unchanged.
 int transform_dims(int H0, int W0, const dgp_frame_transform* t, int* H, int* W, bool* identity);
 // dgp_resize_crop without the device switch (resize_kernels.cu)
 int resize_crop_impl(dgp_handle* h, const uint8_t* src, int N, int H0, int W0, const dgp_frame_transform* t, uint8_t* dst,
                      cudaStream_t s);
 
-inline cudaEvent_t prof_event(dgp_handle* h) {
+inline Event prof_event(dgp_handle* h) {
+  Event e;
   if (!h->ev_pool.empty()) {
-    cudaEvent_t e = h->ev_pool.back();
+    e = std::move(h->ev_pool.back());
     h->ev_pool.pop_back();
-    return e;
+  } else {
+    create(&e, cudaEventDefault);
   }
-  cudaEvent_t e = nullptr;
-  cudaEventCreate(&e);
   return e;
 }
 
@@ -235,12 +251,12 @@ struct ProfScope {
     r.count = count;
     r.a = prof_event(h);
     r.b = prof_event(h);
-    cudaEventRecord(r.a, s);
+    cudaEventRecord(r.a.get(), s);
     idx = (int)h->prof.size();
-    h->prof.push_back(r);
+    h->prof.push_back(std::move(r));
   }
   ~ProfScope() {
-    if (idx >= 0) cudaEventRecord(h->prof[idx].b, s);
+    if (idx >= 0) cudaEventRecord(h->prof[idx].b.get(), s);
   }
 };
 

@@ -243,13 +243,9 @@ static int resize_table(dgp_handle* h, int in_size, int out_size, const ResizeTa
     pillow_coeffs(in_size, out_size, t.ksize, host.data(), host.data() + out_size, host.data() + 2 * (size_t)out_size);
     t.first.assign(host.begin(), host.begin() + out_size);
     t.count.assign(host.begin() + out_size, host.begin() + 2 * out_size);
-    CU_OK(h, cudaMalloc(&t.dev, host.size() * 4));
-    const cudaError_t e = cudaMemcpy(t.dev, host.data(), host.size() * 4, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-      cudaFree(t.dev);
-      return fail(h, DGP_ERR_CUDA, "resize table upload: %s", cudaGetErrorString(e));
-    }
-    it = h->resize_tables.emplace(key, std::move(t)).first;
+    CU_OK(h, t.dev.alloc(host.size() * 4));
+    CU_OK(h, cudaMemcpy(t.dev.get(), host.data(), host.size() * 4, cudaMemcpyHostToDevice));
+    it =h->resize_tables.emplace(key, std::move(t)).first;
   }
   *out = &it->second;
   return DGP_OK;
@@ -272,9 +268,9 @@ int resize_crop_impl(dgp_handle* h, const uint8_t* src, int N, int H0, int W0, c
   a.first = a.count = a.weights = nullptr;
   a.ksize = 0;
   if (vpass) {
-    a.first = tv->dev;
-    a.count = tv->dev + g.Hr;
-    a.weights = tv->dev + 2 * (size_t)g.Hr;
+    a.first = tv->dev.get<int32_t>();
+    a.count = a.first + g.Hr;
+    a.weights = a.first + 2 * (size_t)g.Hr;
     a.ksize = tv->ksize;
   }
   a.out = dst;
@@ -310,12 +306,13 @@ int resize_crop_impl(dgp_handle* h, const uint8_t* src, int N, int H0, int W0, c
     if ((rc = ensure(h, &h->resize_tmp, (size_t)N * R * pitch))) return rc;
     if (smem > 48 * 1024)
       CU_OK(h, cudaFuncSetAttribute(resize_h_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    resize_h_kernel<<<R * N, kHThreads, smem, s>>>(src, H0, W0, r0, R, th->dev + g.cx0, th->dev + g.Wr + g.cx0,
-                                                   th->dev + 2 * (size_t)g.Wr + (size_t)g.cx0 * th->ksize, th->ksize, Wv,
-                                                   span0, span_bytes, (uint8_t*)h->resize_tmp.p, pitch);
+    const int32_t* tab = th->dev.get<int32_t>();
+    resize_h_kernel<<<R * N, kHThreads, smem, s>>>(src, H0, W0, r0, R, tab + g.cx0, tab + g.Wr + g.cx0,
+                                                   tab + 2 * (size_t)g.Wr + (size_t)g.cx0 * th->ksize, th->ksize, Wv,
+                                                   span0, span_bytes, h->resize_tmp.get<uint8_t>(), pitch);
     CU_OK(h, cudaGetLastError());
     h->launches++;
-    a.in = (const uint8_t*)h->resize_tmp.p;
+    a.in = h->resize_tmp.get<uint8_t>();
     a.in_frame = (size_t)R * pitch;
     a.in_pitch = pitch;
     a.in_readable = pitch;

@@ -85,36 +85,12 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
     return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: invalid frame size or transform");
   if (max_frames == 0) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
-  const int nj = h->cfg.num_joints;
-  int hf, wf, ho, wo;
-  dgp_output_dims(H, W, &hf, &wf, &ho, &wo);
-  // the ring, the H2D copy and st_frames2 carry source-size frames; the transform writes st_xf on the compute stream
+  int rc = h->pose.reserve(h, batch, H0, W0, H, W, identity);
+  if (rc) return rc;
   const size_t frame_bytes = (size_t)H0 * W0 * 3;
-  int rc;
-  if ((rc = ensure(h, &h->st_frames2[0], frame_bytes * batch))) return rc;
-  if ((rc = ensure(h, &h->st_frames2[1], frame_bytes * batch))) return rc;
-  if (!identity && (rc = ensure(h, &h->st_xf, (size_t)H * W * 3 * batch))) return rc;
-  if ((rc = ensure(h, &h->st_logits, (size_t)batch * ho * wo * nj * 4))) return rc;
-  if ((rc = ensure(h, &h->st_mu, (size_t)batch * nj * 2 * 4))) return rc;
-  if ((rc = ensure(h, &h->st_peak, (size_t)batch * nj * 2 * 4))) return rc;
-  if ((rc = ensure(h, &h->st_lik, (size_t)batch * nj * 4))) return rc;
-  if (h->ring_bytes < frame_bytes * batch) {
-    for (int i = 0; i < kSlots; ++i) {
-      if (h->ring_slot[i]) cudaFreeHost(h->ring_slot[i]);
-      h->ring_slot[i] = nullptr;
-    }
-    h->ring_bytes = 0;
-    for (int i = 0; i < kSlots; ++i) CU_OK(h, cudaHostAlloc(&h->ring_slot[i], frame_bytes * batch, cudaHostAllocDefault));
-    h->ring_bytes = frame_bytes * batch;
-  }
-  if (!h->copy_stream) {
-    CU_OK(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-      CU_OK(h, cudaEventCreateWithFlags(&h->ev_copied[i], cudaEventDisableTiming));
-      CU_OK(h, cudaEventCreateWithFlags(&h->ev_consumed[i], cudaEventDisableTiming));
-    }
-  }
-  cudaStream_t s = h->stream, cs = h->copy_stream;
+  for (PinnedBuf& r : h->ring_slot)
+    if (r.bytes() < frame_bytes * batch) CU_OK(h, r.alloc(frame_bytes * batch));
+  const PoseJob job = {H0, W0, H, W, identity, transform, gamma, gauss_len, mu_host, peak_host, lik_host};
 
   Ring ring;
   for (int i = 0; i < kSlots; ++i) ring.slot_free[i] = true;
@@ -123,7 +99,7 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
 
   // ---- reader thread: source -> pinned ring
   uint8_t* slots[kSlots];
-  for (int i = 0; i < kSlots; ++i) slots[i] = static_cast<uint8_t*>(h->ring_slot[i]);
+  for (int i = 0; i < kSlots; ++i) slots[i] = h->ring_slot[i].get<uint8_t>();
   std::thread producer([&ring, &slots, reader, user, batch, max_frames]() {
     int64_t produced = 0;
     while (produced < max_frames) {
@@ -165,7 +141,6 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
   int it = 0;
   bool full_batch_seen = false;
   int status = DGP_OK;
-  cudaError_t ce = cudaSuccess;
   for (;;) {
     Ring::Filled f;
     {
@@ -175,36 +150,14 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
       f = ring.filled.front();
       ring.filled.pop_front();
     }
-    const int dslot = it & 1;
-    if (it >= 2) ce = cudaStreamWaitEvent(cs, h->ev_consumed[dslot], 0);
-    if (ce == cudaSuccess)
-      ce = cudaMemcpyAsync(h->st_frames2[dslot].p, f.src, frame_bytes * f.n, cudaMemcpyHostToDevice, cs);
-    if (ce == cudaSuccess) ce = cudaLaunchHostFunc(cs, release_slot, &rel[f.slot]);   // the host slot is reusable after the copy
-    if (ce == cudaSuccess) ce = cudaEventRecord(h->ev_copied[dslot], cs);
-    if (ce == cudaSuccess) ce = cudaStreamWaitEvent(s, h->ev_copied[dslot], 0);
-    if (ce != cudaSuccess) break;
     // A short batch (the tail of the video, or the wrap of a cyclic source) reuses the full-batch plan once one exists:
     // every frame's arithmetic is independent of its batch, the surplus rows of the device slot hold an earlier batch's
     // frames, and only the first f.n read-outs are copied back.  Building a second plan for it would cost far more than the
     // surplus frames (allocation of every activation, tensor maps, first-use kernel loads).
     const int run_n = (f.n < batch && full_batch_seen) ? batch : f.n;
     if (f.n == batch) full_batch_seen = true;
-    const uint8_t* frames = (const uint8_t*)h->st_frames2[dslot].p;
-    if (!identity) {
-      if ((status = resize_crop_impl(h, frames, f.n, H0, W0, transform, (uint8_t*)h->st_xf.p, s))) break;
-      frames = (const uint8_t*)h->st_xf.p;
-    }
-    if ((status = dgp_forward(h, frames, run_n, H, W, (float*)h->st_logits.p, nullptr, s))) break;
-    if ((ce = cudaEventRecord(h->ev_consumed[dslot], s)) != cudaSuccess) break;
-    if ((status = dgp_softargmax(h, (const float*)h->st_logits.p, nullptr, run_n, ho, wo, nj, gamma, gauss_len, (float*)h->st_mu.p,
-                                 (int32_t*)h->st_peak.p, (float*)h->st_lik.p, nullptr, nullptr, s)))
-      break;
-    ce = cudaMemcpyAsync(mu_host + (size_t)t0 * nj * 2, h->st_mu.p, (size_t)f.n * nj * 2 * 4, cudaMemcpyDeviceToHost, s);
-    if (ce == cudaSuccess && peak_host)
-      ce = cudaMemcpyAsync(peak_host + (size_t)t0 * nj * 2, h->st_peak.p, (size_t)f.n * nj * 2 * 4, cudaMemcpyDeviceToHost, s);
-    if (ce == cudaSuccess && lik_host)
-      ce = cudaMemcpyAsync(lik_host + (size_t)t0 * nj, h->st_lik.p, (size_t)f.n * nj * 4, cudaMemcpyDeviceToHost, s);
-    if (ce != cudaSuccess) break;
+    // the host slot is reusable once its frames have been copied
+    if ((status = h->pose.run_batch(h, job, f.src, f.n, run_n, it, t0, release_slot, &rel[f.slot]))) break;
     t0 += f.n;
     ++it;
   }
@@ -214,12 +167,11 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
   }
   ring.cv.notify_all();
   // pending release callbacks reference `ring`: drain both streams before it goes out of scope
-  cudaError_t e1 = cudaStreamSynchronize(cs);
-  cudaError_t e2 = cudaStreamSynchronize(s);
+  cudaError_t e1 = cudaStreamSynchronize(h->pose.copy_stream.get());
+  cudaError_t e2 = cudaStreamSynchronize(h->stream.get());
   producer.join();
   if (frames_done) *frames_done = t0;
   if (status) return status;
-  if (ce != cudaSuccess) return fail(h, DGP_ERR_CUDA, "dgp_estimate_pose_stream: %s", cudaGetErrorString(ce));
   if (e1 != cudaSuccess || e2 != cudaSuccess)
     return fail(h, DGP_ERR_CUDA, "dgp_estimate_pose_stream: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
   if (ring.reader_error) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: the frame reader failed (%d)", ring.reader_error);

@@ -44,6 +44,7 @@ struct BStep {
 };
 
 struct Backward {
+  std::vector<DevBuf> bufs;  // gradient buffers (declared first: the graph exec that references them goes before them)
   std::vector<BStep> steps;
   float *g_logits = nullptr, *g_locref = nullptr;
   // Deferred frozen-BN gradients: every mask site leaves its per-row-block sums of dy in its own region of `bn_part`, every
@@ -61,20 +62,16 @@ struct Backward {
   int runs = 0;
   int launches = 0;
   uint64_t graph_gen = 0;
-  cudaGraphExec_t graph_exec = nullptr;
-  ~Backward() {
-    if (graph_exec) cudaGraphExecDestroy(graph_exec);
-  }
+  GraphExec graph_exec;
 };
 
 struct TrainState {
-  float* grads = nullptr;
-  float* accum = nullptr;
-  float* norm_partial = nullptr;
-  float* norm_clip = nullptr;  // [0] = global norm of the last step, [1] = clip factor
+  DevBuf grads, accum;  // float, n_params each
+  DevBuf norm_partial;
+  DevBuf norm_clip;     // float [0] = global norm of the last step, [1] = clip factor
   DevBuf bn_partial, wgrad_ws;
-  std::vector<W16*> wd;  // per layer: dgrad operand [Cin][taps*Cout] (nullptr for conv1 / head)
-  W16* head_wd = nullptr;
+  std::vector<DevBuf> wd;  // per layer: W16 dgrad operand [Cin][taps*Cout] (empty for conv1 / head)
+  DevBuf head_wd;
   int head_Kd = 0;
   bool wd_fresh = false;
   uint64_t ws_gen = 1;           // bumped whenever a shared workspace is reallocated (captured graphs hold its address)
@@ -85,15 +82,15 @@ struct TrainState {
   // (GradMode), grad_mode_host the value last stored there.
   float arena_scale = 1.0f;
   bool arena_fused = false;      // the last backward was dgp_train_forward_backward's (no accumulation onto it)
-  GradMode* grad_mode = nullptr;
+  DevBuf grad_mode;              // GradMode
   GradMode grad_mode_host = {0, 1.0f};
   uint64_t fwd_seq = 0;          // tokens handed out by dgp_train_forward
-  DgradWJob* wd_jobs = nullptr;  // device table for the one-launch rebuild of every dgrad operand
+  DevBuf wd_jobs;                // DgradWJob: device table for the one-launch rebuild of every dgrad operand
   int n_wd_jobs = 0, wd_tiles = 0;
   // Early all-reduce bucket: the weight gradients of block4 and the heads (two thirds of the arena, contiguous at the end of
   // its weight part) are complete after a quarter of the backward pass; `ev_early` is recorded there so a data-parallel
   // caller can start their all-reduce on a side stream while blocks 3..1 are still running.
-  cudaEvent_t ev_early = nullptr;
+  Event ev_early;
   size_t early_off = 0, early_cnt = 0;
   // Data-parallel all-reduce owned by the library (dgp_attach_comm / dgp_comm_init_rank + dgp_allreduce_gradients): the
   // weight gradients of a block are final once the backward has passed its first unit, so the arena is reduced in four
@@ -101,44 +98,22 @@ struct TrainState {
   // communication stream behind an event recorded at that point of the backward (ev_bucket[0] == ev_early's position).
   static constexpr int kBuckets = 4;
   size_t bucket_off[kBuckets + 1] = {0, 0, 0, 0, 0};   // weight-part offsets: bucket k = [bucket_off[k+1], bucket_off[k])
-  cudaEvent_t ev_bucket[kBuckets - 1] = {nullptr, nullptr, nullptr};
+  Event ev_bucket[kBuckets - 1];
   void* comm = nullptr;           // ncclComm_t
   bool comm_owned = false;
   int comm_world = 1;
-  cudaStream_t comm_stream = nullptr;
-  cudaEvent_t ev_bwd_done = nullptr, ev_comm_done = nullptr;   // timing enabled: exposed all-reduce time
+  Stream comm_stream;
+  Event ev_bwd_done, ev_comm_done;   // timing enabled: exposed all-reduce time
   bool bwd_ran = false;           // a backward has recorded the bucket events on some stream
   // second branch of the captured backward: the wgrad chain (see dgp_train_forward_backward)
-  cudaStream_t side_stream = nullptr;
-  std::vector<cudaEvent_t> branch_events;
+  Stream side_stream;
+  std::vector<Event> branch_events;
+
+  void release_comm();
+  ~TrainState() { release_comm(); }
 };
 
-void comm_release(dgp_handle* h);
-
-void train_destroy(dgp_handle* h) {
-  TrainState* ts = h->train;
-  if (!ts) return;
-  cudaFree(ts->grads);
-  cudaFree(ts->accum);
-  cudaFree(ts->norm_partial);
-  cudaFree(ts->norm_clip);
-  cudaFree(ts->bn_partial.p);
-  cudaFree(ts->wgrad_ws.p);
-  for (W16* p : ts->wd) cudaFree(p);
-  cudaFree(ts->head_wd);
-  cudaFree(ts->wd_jobs);
-  cudaFree(ts->grad_mode);
-  if (ts->ev_early) cudaEventDestroy(ts->ev_early);
-  for (cudaEvent_t e : ts->ev_bucket) if (e) cudaEventDestroy(e);
-  if (ts->ev_bwd_done) cudaEventDestroy(ts->ev_bwd_done);
-  if (ts->ev_comm_done) cudaEventDestroy(ts->ev_comm_done);
-  comm_release(h);
-  if (ts->comm_stream) cudaStreamDestroy(ts->comm_stream);
-  if (ts->side_stream) cudaStreamDestroy(ts->side_stream);
-  for (cudaEvent_t e : ts->branch_events) cudaEventDestroy(e);
-  delete ts;
-  h->train = nullptr;
-}
+void TrainStateDeleter::operator()(TrainState* ts) const { delete ts; }
 
 // ---- NCCL, resolved at run time from the process (the copy PyTorch loaded, if any) or the system library: the .so has no
 // link-time NCCL dependency, and a host that never calls dgp_attach_comm / dgp_comm_init_rank never needs it.
@@ -185,22 +160,23 @@ const Api& api() {
 }
 }  // namespace nccl
 
-void comm_release(dgp_handle* h) {
-  TrainState* ts = h->train;
-  if (!ts || !ts->comm) return;
-  if (ts->comm_owned && nccl::api().ok) nccl::api().comm_destroy(ts->comm);
-  ts->comm = nullptr;
-  ts->comm_owned = false;
-  ts->comm_world = 1;
+void TrainState::release_comm() {
+  if (!comm) return;
+  if (comm_owned && nccl::api().ok) nccl::api().comm_destroy(comm);
+  comm = nullptr;
+  comm_owned = false;
+  comm_world = 1;
 }
 
 namespace {
 
 int refresh_dgrad_weights(dgp_handle* h, cudaStream_t s) {
-  TrainState* ts = h->train;
-  CU_OK(h, launch_build_dgrad_w(ts->wd_jobs, ts->n_wd_jobs, ts->wd_tiles, h->master, h->bn_ss, h->fp16, s));
+  TrainState* ts = h->train.get();
+  const float* master = h->master.get<float>();
+  CU_OK(h, launch_build_dgrad_w(ts->wd_jobs.get<DgradWJob>(), ts->n_wd_jobs, ts->wd_tiles, master, h->bn_ss.get<float>(), h->fp16,
+                                s));
   const ConvLayer& Lh = h->layers[h->head_layer];
-  CU_OK(h, launch_build_head_dgrad_w(h->master + Lh.w_off, 9 * h->ctot, 2048, ts->head_wd, ts->head_Kd, h->fp16, s));
+  CU_OK(h, launch_build_head_dgrad_w(master + Lh.w_off, 9 * h->ctot, 2048, ts->head_wd.get<W16>(), ts->head_Kd, h->fp16, s));
   h->launches += 2;
   ts->wd_fresh = true;
   return DGP_OK;
@@ -229,7 +205,7 @@ long long push_dgrad_gemm(dgp_handle* h, Backward* bw, ConvGemmParams gp, void* 
 
 // dgrad of layer L as a stride-1 conv of dy (N,H,W,L.Cout) with the transposed / flipped operand -> out (N,H,W,L.Cin).
 // mask_act / *site: see push_dgrad_gemm.
-int add_dgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, W16* wd, const void* dy, int N, int H, int W, void* out,
+int add_dgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, const DevBuf& wd, const void* dy, int N, int H, int W, void* out,
               const void* residual, const void* mask_act = nullptr, long long* site = nullptr) {
   ConvLayer D;
   D.scope = L.scope + "/dgrad";
@@ -237,7 +213,7 @@ int add_dgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, W16* wd, const vo
   D.K = L.R * L.S * L.Cout;
   D.Npad = L.Cin;
   D.block_n = L.Cin >= 256 ? 256 : L.Cin;
-  D.w = wd;
+  D.w = wd.get<W16>();
   Step st;
   int Ho, Wo;
   int rc = make_gemm_step(h, D, dy, N, H, W, (L.R == 1 && L.S == 1) ? 0 : 1, out, false, (const __nv_bfloat16*)residual, 1, H,
@@ -252,11 +228,11 @@ int add_dgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, W16* wd, const vo
 // (-> dgamma in the final bn_finalize_all pass), or nullptr (heads)
 int add_wgrad_params(dgp_handle* h, Backward* bw, const WgradParams& wp0, const void* dy_buf, const float* rowscale,
                      const float* mask, float* grad, size_t* ws_need, const ConvLayer* bn_layer = nullptr) {
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   const size_t need = wgrad_workspace_bytes(wp0);
   if (need > *ws_need) *ws_need = need;
   const int sms = h->num_sms;
-  const float* wmaster = bn_layer ? h->master + bn_layer->w_off : nullptr;
+  const float* wmaster = bn_layer ? h->master.get<float>() + bn_layer->w_off : nullptr;
   const size_t rd_off = bn_layer ? bn_layer->w_off / 4 : 0;
   if (bn_layer) {
     for (int c = 0; c < wp0.Cout; c += 8) {
@@ -267,10 +243,10 @@ int add_wgrad_params(dgp_handle* h, Backward* bw, const WgradParams& wp0, const 
   }
   bw->steps.push_back({6, 2, [=](cudaStream_t s) {
                          WgradParams wp = wp0;
-                         wp.partials = (float*)ts->wgrad_ws.p;
+                         wp.partials = ts->wgrad_ws.get<float>();
                          cudaError_t e = launch_wgrad_gemm(wp, sms, s);
                          if (e != cudaSuccess) return e;
-                         return launch_wgrad_reduce(wp, rowscale, mask, grad, ts->grad_mode, s, wmaster,
+                         return launch_wgrad_reduce(wp, rowscale, mask, grad, ts->grad_mode.get<GradMode>(), s, wmaster,
                                                     wmaster ? bw->rowdot + rd_off : nullptr);
                        }});
   bw->steps.back().rd = dy_buf;
@@ -282,7 +258,7 @@ int add_wgrad(dgp_handle* h, Backward* bw, const ConvLayer& L, const void* x, in
   WgradParams wp;
   int rc = make_wgrad_params(h, L.scope.c_str(), L.R, L.S, L.Cin, L.Cout, L.stride, L.dil, x, N, H, W, pad_mode, dy, &wp);
   if (rc) return rc;
-  return add_wgrad_params(h, bw, wp, dy, L.scale, nullptr, h->train->grads + L.w_off, ws_need, &L);
+  return add_wgrad_params(h, bw, wp, dy, L.scale, nullptr, h->train->grads.get<float>() + L.w_off, ws_need, &L);
 }
 
 // dy = g * [act > 0] in place and the dy sums of up to two layers (conv3 and the projection shortcut share dy at a junction).
@@ -320,7 +296,7 @@ void add_mask(dgp_handle* h, Backward* bw, void* g, const void* act, int M, int 
 }
 
 int build_backward(dgp_handle* h, Plan* pl) {
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   std::shared_ptr<Backward> bw(new Backward());
   const int B = pl->B, nj = h->cfg.num_joints, fp16 = h->fp16;
   const int hf = pl->hf, wf = pl->wf;
@@ -342,18 +318,18 @@ int build_backward(dgp_handle* h, Plan* pl) {
   }
   void *gbuf[3], *gt1 = nullptr, *gt2 = nullptr, *gup = nullptr, *g_c1 = nullptr, *dG = nullptr;
   for (int i = 0; i < 3; ++i)
-    if ((rc = alloc_buf(h, pl, (size_t)B * max_unit * 2 + 1024, &gbuf[i]))) return rc;
-  if ((rc = alloc_buf(h, pl, (size_t)B * max_t1 * 2 + 1024, &gt1))) return rc;
-  if ((rc = alloc_buf(h, pl, (size_t)B * max_t2 * 2 + 1024, &gt2))) return rc;
-  if (max_up && (rc = alloc_buf(h, pl, (size_t)B * max_up * 2 + 1024, &gup))) return rc;
-  if ((rc = alloc_buf(h, pl, (size_t)B * pl->H1 * pl->W1 * 64 * 2 + 1024, &g_c1))) return rc;
+    if ((rc = alloc_buf(h, &bw->bufs, (size_t)B * max_unit * 2 + 1024, &gbuf[i]))) return rc;
+  if ((rc = alloc_buf(h, &bw->bufs, (size_t)B * max_t1 * 2 + 1024, &gt1))) return rc;
+  if ((rc = alloc_buf(h, &bw->bufs, (size_t)B * max_t2 * 2 + 1024, &gt2))) return rc;
+  if (max_up && (rc = alloc_buf(h, &bw->bufs, (size_t)B * max_up * 2 + 1024, &gup))) return rc;
+  if ((rc = alloc_buf(h, &bw->bufs, (size_t)B * pl->H1 * pl->W1 * 64 * 2 + 1024, &g_c1))) return rc;
   const int Kd = ts->head_Kd;
   const int Mf = B * hf * wf;
-  if ((rc = alloc_buf(h, pl, (size_t)Mf * Kd * 2 + 1024, &dG))) return rc;
-  if ((rc = alloc_buf(h, pl, (size_t)B * 4 * hf * wf * nj * 4, &p))) return rc;
+  if ((rc = alloc_buf(h, &bw->bufs, (size_t)Mf * Kd * 2 + 1024, &dG))) return rc;
+  if ((rc = alloc_buf(h, &bw->bufs, (size_t)B * 4 * hf * wf * nj * 4, &p))) return rc;
   bw->g_logits = (float*)p;
   if (pl->locref) {
-    if ((rc = alloc_buf(h, pl, (size_t)B * 4 * hf * wf * 2 * nj * 4, &p))) return rc;
+    if ((rc = alloc_buf(h, &bw->bufs, (size_t)B * 4 * hf * wf * 2 * nj * 4, &p))) return rc;
     bw->g_locref = (float*)p;
   }
   float* g_logits = bw->g_logits;
@@ -364,14 +340,15 @@ int build_backward(dgp_handle* h, Plan* pl) {
   bw->steps.push_back({7, 1, [=](cudaStream_t s) { return launch_col2im_bwd(g_logits, g_locref, B, hf, wf, ctot, nj, dG, Kd, fp16, s); }});
   bw->steps.back().wr = dG;
   {
-    float* dbias = ts->grads + h->n_w + 2 * h->n_ch;
+    float* dbias = ts->grads.get<float>() + h->n_w + 2 * h->n_ch;
     const size_t npix = (size_t)B * 4 * hf * wf;
     bn_need = std::max(bn_need, (size_t)head_bias_blocks() * 256 * sizeof(float));
     bw->steps.push_back({7, g_locref ? 4 : 2, [=](cudaStream_t s) {
-                           float* partial = (float*)ts->bn_partial.p;
-                           cudaError_t e = launch_head_bias_grad(g_logits, npix, nj, partial, dbias, ts->grad_mode, s);
+                           float* partial = ts->bn_partial.get<float>();
+                           const GradMode* mode = ts->grad_mode.get<GradMode>();
+                           cudaError_t e = launch_head_bias_grad(g_logits, npix, nj, partial, dbias, mode, s);
                            if (e == cudaSuccess && g_locref)
-                             e = launch_head_bias_grad(g_locref, npix, 2 * nj, partial, dbias + nj, ts->grad_mode, s);
+                             e = launch_head_bias_grad(g_locref, npix, 2 * nj, partial, dbias + nj, mode, s);
                            return e;
                          }});
   }
@@ -383,10 +360,10 @@ int build_backward(dgp_handle* h, Plan* pl) {
     if (rc) return rc;
     wp.Cout = Lh.Npad;
     wgrad_plan(&wp, h->num_sms);
-    if ((rc = add_wgrad_params(h, bw.get(), wp, dG, nullptr, nullptr, ts->grads + Lh.w_off, &ws_need))) return rc;
+    if ((rc = add_wgrad_params(h, bw.get(), wp, dG, nullptr, nullptr, ts->grads.get<float>() + Lh.w_off, &ws_need))) return rc;
     ConvLayer D;
     D.scope = "pose/heads/dgrad"; D.R = 1; D.S = 1; D.Cin = Kd; D.Cout = 2048; D.relu = false;
-    D.K = Kd; D.Npad = 2048; D.block_n = 256; D.w = ts->head_wd;
+    D.K = Kd; D.Npad = 2048; D.block_n = 256; D.w = ts->head_wd.get<W16>();
     Step st;
     int Ho, Wo;
     rc = make_gemm_step(h, D, dG, B, hf, wf, 0, gbuf[0], false, nullptr, 1, 0, 0, 0, &st, &Ho, &Wo);
@@ -485,36 +462,38 @@ int build_backward(dgp_handle* h, Plan* pl) {
                          (uint64_t)pl->Hs * pl->Ws * 32, 0, 0, 0, -3, 1, (uint64_t)B * pl->Hs * pl->Ws * 32, 64);
     if (e) return fail(h, DGP_ERR_CUDA, "conv1 wgrad (x map): %s", e);
     wgrad_plan(&wp, h->num_sms);
-    if ((rc = add_wgrad_params(h, bw.get(), wp, g_c1, L.scale, h->conv1_mask, ts->grads + L.w_off, &ws_need, &L))) return rc;
+    if ((rc = add_wgrad_params(h, bw.get(), wp, g_c1, L.scale, h->conv1_mask.get<float>(), ts->grads.get<float>() + L.w_off,
+                               &ws_need, &L)))
+      return rc;
   }
   // ---- every channel's dbeta / dgamma in one pass at the end
   {
-    if ((rc = alloc_buf(h, pl, bw->bn_part_floats * sizeof(float) + 1024, &p))) return rc;
+    if ((rc = alloc_buf(h, &bw->bufs, bw->bn_part_floats * sizeof(float) + 1024, &p))) return rc;
     bw->bn_part = (float*)p;
-    if ((rc = alloc_buf(h, pl, (h->n_w / 4 + 64) * sizeof(float), &p))) return rc;
+    if ((rc = alloc_buf(h, &bw->bufs, (h->n_w / 4 + 64) * sizeof(float), &p))) return rc;
     bw->rowdot = (float*)p;
-    if ((rc = alloc_buf(h, pl, bw->bn_groups.size() * sizeof(BnGroup), &p))) return rc;
+    if ((rc = alloc_buf(h, &bw->bufs, bw->bn_groups.size() * sizeof(BnGroup), &p))) return rc;
     bw->bn_table = (BnGroup*)p;
     for (const BnGroup& g : bw->bn_groups)
       if (g.rows <= 0 || g.K4 <= 0) return fail(h, DGP_ERR_STATE, "backward plan: a BatchNorm channel group has no gradient source");
     CU_OK(h, cudaMemcpy(bw->bn_table, bw->bn_groups.data(), bw->bn_groups.size() * sizeof(BnGroup), cudaMemcpyHostToDevice));
     const int ngroups = (int)bw->bn_groups.size();
     Backward* bwp = bw.get();
-    const float *mean = h->bn_mean, *var = h->bn_var;
+    const float *mean = h->bn_mean.get<float>(), *var = h->bn_var.get<float>();
     const float eps = h->cfg.bn_epsilon;
-    float* dgam = ts->grads + h->n_w;
-    float* dbet = ts->grads + h->n_w + h->n_ch;
-    const GradMode* mode = ts->grad_mode;
+    float* dgam = ts->grads.get<float>() + h->n_w;
+    float* dbet = ts->grads.get<float>() + h->n_w + h->n_ch;
+    const GradMode* mode = ts->grad_mode.get<GradMode>();
     bw->steps.push_back({7, 1, [=](cudaStream_t s) {
                            return launch_bn_finalize_all(bwp->bn_table, ngroups, bwp->bn_part, bwp->rowdot, mean, var, eps, dgam, dbet,
                                                          mode, s);
                          }});
     bw->steps.back().join = true;
   }
-  const void *p0 = ts->wgrad_ws.p, *p1 = ts->bn_partial.p;
+  const void *p0 = ts->wgrad_ws.get(), *p1 = ts->bn_partial.get();
   if ((rc = ensure(h, &ts->wgrad_ws, ws_need))) return rc;
   if ((rc = ensure(h, &ts->bn_partial, bn_need))) return rc;
-  if (p0 != ts->wgrad_ws.p || p1 != ts->bn_partial.p) ++ts->ws_gen;
+  if (p0 != ts->wgrad_ws.get() || p1 != ts->bn_partial.get()) ++ts->ws_gen;
   for (const BStep& st : bw->steps) bw->launches += st.launches;
   pl->bwd = bw;
   return DGP_OK;
@@ -554,11 +533,11 @@ bool find_variable(dgp_handle* h, const std::string& name, VarRef* r) {
 
 // Stores the arena write mode the backward kernels read (GradMode) on `s`, when it differs from the stored one.
 int set_grad_mode(dgp_handle* h, int accumulate, float out_scale, cudaStream_t s) {
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   if (ts->grad_mode_host.accumulate == accumulate && ts->grad_mode_host.out_scale == out_scale) return DGP_OK;
   ts->grad_mode_host.accumulate = accumulate;
   ts->grad_mode_host.out_scale = out_scale;
-  CU_OK(h, cudaMemcpyAsync(ts->grad_mode, &ts->grad_mode_host, sizeof(GradMode), cudaMemcpyHostToDevice, s));
+  CU_OK(h, cudaMemcpyAsync(ts->grad_mode.get(), &ts->grad_mode_host, sizeof(GradMode), cudaMemcpyHostToDevice, s));
   return DGP_OK;
 }
 
@@ -580,13 +559,13 @@ int scale_head_grads(dgp_handle* h, const Plan* pl, Backward* bw, cudaStream_t s
 
 // The network backward of `bw` from its g_logits / g_locref: eager on the first run of a plan, a captured graph afterwards.
 int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   const bool graphs = ts->use_graphs && !h->profiling && bw->runs > 0;
   if (graphs && (!bw->graph_exec || bw->graph_gen != ts->ws_gen)) {
     // (re)capture on the handle's private stream; the first step ran eagerly, so every lazy cudaFuncSetAttribute is done
-    if (bw->graph_exec) { cudaGraphExecDestroy(bw->graph_exec); bw->graph_exec = nullptr; }
-    cudaGraph_t graph = nullptr;
-    CU_OK(h, cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
+    bw->graph_exec.reset();
+    cudaStream_t hs = h->stream.get();
+    CU_OK(h, cudaStreamBeginCapture(hs, cudaStreamCaptureModeThreadLocal));
     // Two branches: the wgrad GEMMs only read a gradient buffer that the dgrad chain has finished writing, and nothing
     // downstream of them is needed before the end of the pass (or the bucket boundaries of the data-parallel all-reduce), so
     // they are captured on a side stream forked from the main branch.  A wgrad of blocks 2-3 is a short kernel (a few k-blocks
@@ -594,22 +573,23 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
     // tail hide under the dgrad GEMMs instead of being serialised between them.  Joins: before a main-branch step that
     // overwrites the buffer a pending wgrad reads, before every bucket event, before the final gamma/beta pass.
     cudaError_t ce = cudaSuccess;
-    if (!ts->side_stream) ce = cudaStreamCreateWithFlags(&ts->side_stream, cudaStreamNonBlocking);
+    if (!ts->side_stream) ce = create(&ts->side_stream, cudaStreamNonBlocking);
+    cudaStream_t ss = ts->side_stream.get();
     size_t ev_next = 0;
     auto next_event = [&](cudaEvent_t* out) -> cudaError_t {
       if (ev_next == ts->branch_events.size()) {
-        cudaEvent_t e = nullptr;
-        cudaError_t r = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+        Event e;
+        cudaError_t r = create(&e, cudaEventDisableTiming);
         if (r != cudaSuccess) return r;
-        ts->branch_events.push_back(e);
+        ts->branch_events.push_back(std::move(e));
       }
-      *out = ts->branch_events[ev_next++];
+      *out = ts->branch_events[ev_next++].get();
       return cudaSuccess;
     };
     struct Pending { const void* rd; cudaEvent_t done; };
     std::vector<Pending> pending;   // in side-stream order: waiting for entry i covers entries 0..i
     auto join_through = [&](size_t i) -> cudaError_t {
-      cudaError_t r = cudaStreamWaitEvent(h->stream, pending[i].done, 0);
+      cudaError_t r = cudaStreamWaitEvent(hs, pending[i].done, 0);
       pending.erase(pending.begin(), pending.begin() + i + 1);
       return r;
     };
@@ -619,17 +599,17 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
       if (st.kind == 6 && st.rd != nullptr) {
         cudaEvent_t fork = nullptr, done = nullptr;
         if ((ce = next_event(&fork)) != cudaSuccess || (ce = next_event(&done)) != cudaSuccess) break;
-        if ((ce = cudaEventRecord(fork, h->stream)) != cudaSuccess) break;
-        if ((ce = cudaStreamWaitEvent(ts->side_stream, fork, 0)) != cudaSuccess) break;
-        if ((ce = st.run(ts->side_stream)) != cudaSuccess) break;
-        if ((ce = cudaEventRecord(done, ts->side_stream)) != cudaSuccess) break;
+        if ((ce = cudaEventRecord(fork, hs)) != cudaSuccess) break;
+        if ((ce = cudaStreamWaitEvent(ss, fork, 0)) != cudaSuccess) break;
+        if ((ce = st.run(ss)) != cudaSuccess) break;
+        if ((ce = cudaEventRecord(done, ss)) != cudaSuccess) break;
         pending.push_back({st.rd, done});
       } else {
         if (st.join && !pending.empty()) ce = join_through(pending.size() - 1);
         if (ce == cudaSuccess && st.wr != nullptr)
           for (size_t i = pending.size(); i-- > 0;)
             if (pending[i].rd == st.wr) { ce = join_through(i); break; }
-        if (ce == cudaSuccess) ce = st.run(h->stream);
+        if (ce == cudaSuccess) ce = st.run(hs);
         if (ce != cudaSuccess) break;
       }
       ++k;
@@ -637,30 +617,33 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
       for (int b = 0; b < 3; ++b) boundary = boundary || k == bw->bucket_step[b];
       if (boundary && !pending.empty() && (ce = join_through(pending.size() - 1)) != cudaSuccess) break;
       if (k == bw->early_step) {
-        ce = cudaEventRecordWithFlags(ts->ev_early, h->stream, cudaEventRecordExternal);
+        ce = cudaEventRecordWithFlags(ts->ev_early.get(), hs, cudaEventRecordExternal);
         if (ce != cudaSuccess) break;
       }
       for (int b = 0; b < 3 && ce == cudaSuccess; ++b)
-        if (k == bw->bucket_step[b]) ce = cudaEventRecordWithFlags(ts->ev_bucket[b], h->stream, cudaEventRecordExternal);
+        if (k == bw->bucket_step[b]) ce = cudaEventRecordWithFlags(ts->ev_bucket[b].get(), hs, cudaEventRecordExternal);
       if (ce != cudaSuccess) break;
     }
     if (!pending.empty()) {
       cudaError_t je = join_through(pending.size() - 1);   // every forked branch rejoins before the capture ends
       if (ce == cudaSuccess) ce = je;
     }
-    cudaError_t ee = cudaStreamEndCapture(h->stream, &graph);
+    cudaGraph_t g = nullptr;
+    cudaError_t ee = cudaStreamEndCapture(hs, &g);
+    Graph graph;
+    if (g) adopt(&graph, g);
     if (ce == cudaSuccess) ce = ee;
-    if (ce == cudaSuccess) ce = cudaGraphInstantiate(&bw->graph_exec, graph, 0);
-    if (graph) cudaGraphDestroy(graph);
+    cudaGraphExec_t exec = nullptr;
+    if (ce == cudaSuccess) ce = cudaGraphInstantiate(&exec, g, 0);
     if (ce != cudaSuccess) {
-      bw->graph_exec = nullptr;
       cudaGetLastError();
       return fail(h, DGP_ERR_CUDA, "capturing the backward graph failed: %s", cudaGetErrorString(ce));
     }
+    adopt(&bw->graph_exec, exec);
     bw->graph_gen = ts->ws_gen;
   }
   if (graphs) {
-    CU_OK(h, cudaGraphLaunch(bw->graph_exec, s));
+    CU_OK(h, cudaGraphLaunch(bw->graph_exec.get(), s));
     h->launches += bw->launches;
   } else {
     int k = 0;
@@ -671,9 +654,9 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
       }
       h->launches += st.launches;
       ++k;
-      if (k == bw->early_step) CU_OK(h, cudaEventRecord(ts->ev_early, s));
+      if (k == bw->early_step) CU_OK(h, cudaEventRecord(ts->ev_early.get(), s));
       for (int b = 0; b < 3; ++b)
-        if (k == bw->bucket_step[b]) CU_OK(h, cudaEventRecord(ts->ev_bucket[b], s));
+        if (k == bw->bucket_step[b]) CU_OK(h, cudaEventRecord(ts->ev_bucket[b].get(), s));
     }
   }
   ts->bwd_ran = bw->early_step > 0;
@@ -691,26 +674,25 @@ int dgp_train_enable(dgp_handle* h) {
   if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_train_enable before dgp_finalize_weights");
   if (h->train) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
-  TrainState* ts = new TrainState();
-  h->train = ts;
-  CU_OK(h, cudaMalloc(&ts->grads, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->accum, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMemset(ts->grads, 0, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMemset(ts->accum, 0, h->n_params * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->norm_partial, sqnorm_partials() * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->norm_clip, 2 * sizeof(float)));
-  CU_OK(h, cudaMemset(ts->norm_clip, 0, 2 * sizeof(float)));
-  CU_OK(h, cudaMalloc(&ts->grad_mode, sizeof(GradMode)));
-  CU_OK(h, cudaMemcpy(ts->grad_mode, &ts->grad_mode_host, sizeof(GradMode), cudaMemcpyHostToDevice));
-  ts->wd.assign(h->layers.size(), nullptr);
+  std::unique_ptr<TrainState, TrainStateDeleter> ts(new TrainState());
+  CU_OK(h, ts->grads.alloc(h->n_params * sizeof(float)));
+  CU_OK(h, ts->accum.alloc(h->n_params * sizeof(float)));
+  CU_OK(h, cudaMemset(ts->grads.get(), 0, h->n_params * sizeof(float)));
+  CU_OK(h, cudaMemset(ts->accum.get(), 0, h->n_params * sizeof(float)));
+  CU_OK(h, ts->norm_partial.alloc(sqnorm_partials() * sizeof(float)));
+  CU_OK(h, ts->norm_clip.alloc(2 * sizeof(float)));
+  CU_OK(h, cudaMemset(ts->norm_clip.get(), 0, 2 * sizeof(float)));
+  CU_OK(h, ts->grad_mode.alloc(sizeof(GradMode)));
+  CU_OK(h, cudaMemcpy(ts->grad_mode.get(), &ts->grad_mode_host, sizeof(GradMode), cudaMemcpyHostToDevice));
+  ts->wd.resize(h->layers.size());
   std::vector<DgradWJob> jobs;
   for (size_t i = 0; i < h->layers.size(); ++i) {
     if ((int)i == h->conv1_layer || (int)i == h->head_layer) continue;
     const ConvLayer& L = h->layers[i];
     if (L.Cin % 32 || L.Cout % 32 || L.ch_off < 0) return fail(h, DGP_ERR_UNSUPPORTED, "%s: dgrad operand needs 32-aligned channels", L.scope.c_str());
-    CU_OK(h, cudaMalloc(&ts->wd[i], (size_t)L.Cin * L.R * L.S * L.Cout * sizeof(W16)));
+    CU_OK(h, ts->wd[i].alloc((size_t)L.Cin * L.R * L.S * L.Cout * sizeof(W16)));
     DgradWJob jb;
-    jb.w_off = L.w_off; jb.wd = reinterpret_cast<uint16_t*>(ts->wd[i]); jb.ch_off = L.ch_off;
+    jb.w_off = L.w_off; jb.wd = ts->wd[i].get<uint16_t>(); jb.ch_off = L.ch_off;
     jb.Cout = L.Cout; jb.taps = L.R * L.S; jb.Cin = L.Cin; jb.tile_start = ts->wd_tiles;
     ts->wd_tiles += (L.Cin / 32) * (L.Cout / 32) * L.R * L.S;
     jobs.push_back(jb);
@@ -719,9 +701,9 @@ int dgp_train_enable(dgp_handle* h) {
     return fail(h, DGP_ERR_UNSUPPORTED, "%zu conv layers exceed the %d of the one-launch dgrad operand rebuild", jobs.size(),
                 kDgradWMaxJobs);
   ts->n_wd_jobs = (int)jobs.size();
-  CU_OK(h, cudaMalloc(&ts->wd_jobs, jobs.size() * sizeof(DgradWJob)));
-  CU_OK(h, cudaMemcpy(ts->wd_jobs, jobs.data(), jobs.size() * sizeof(DgradWJob), cudaMemcpyHostToDevice));
-  CU_OK(h, cudaEventCreateWithFlags(&ts->ev_early, cudaEventDisableTiming));
+  CU_OK(h, ts->wd_jobs.alloc(jobs.size() * sizeof(DgradWJob)));
+  CU_OK(h, cudaMemcpy(ts->wd_jobs.get(), jobs.data(), jobs.size() * sizeof(DgradWJob), cudaMemcpyHostToDevice));
+  CU_OK(h, create(&ts->ev_early, cudaEventDisableTiming));
   for (const UnitDesc& u : h->units)
     if (u.scope.find("/block4/") != std::string::npos && u.shortcut >= 0) {
       ts->early_off = h->layers[u.shortcut].w_off;
@@ -736,13 +718,14 @@ int dgp_train_enable(dgp_handle* h) {
       for (const UnitDesc& u : h->units)
         if (u.scope.find(first[k]) != std::string::npos && u.shortcut >= 0) ts->bucket_off[k + 1] = h->layers[u.shortcut].w_off;
     ts->bucket_off[4] = 0;
-    for (int k = 0; k < 3; ++k) CU_OK(h, cudaEventCreateWithFlags(&ts->ev_bucket[k], cudaEventDisableTiming));
-    CU_OK(h, cudaEventCreate(&ts->ev_bwd_done));
-    CU_OK(h, cudaEventCreate(&ts->ev_comm_done));
-    CU_OK(h, cudaStreamCreateWithFlags(&ts->comm_stream, cudaStreamNonBlocking));
+    for (int k = 0; k < 3; ++k) CU_OK(h, create(&ts->ev_bucket[k], cudaEventDisableTiming));
+    CU_OK(h, create(&ts->ev_bwd_done, cudaEventDefault));
+    CU_OK(h, create(&ts->ev_comm_done, cudaEventDefault));
+    CU_OK(h, create(&ts->comm_stream, cudaStreamNonBlocking));
   }
   ts->head_Kd = ceil_div(std::max(9 * h->ctot, h->layers[h->head_layer].Npad), 64) * 64;
-  CU_OK(h, cudaMalloc(&ts->head_wd, (size_t)2048 * ts->head_Kd * sizeof(W16)));
+  CU_OK(h, ts->head_wd.alloc((size_t)2048 * ts->head_Kd * sizeof(W16)));
+  h->train = std::move(ts);
   return DGP_OK;
 }
 
@@ -754,7 +737,7 @@ int dgp_train_forward_backward(dgp_handle* h, const uint8_t* frames_dev, int nt,
     return fail(h, DGP_ERR_INVALID, "dgp_train_forward_backward: bad argument");
   CU_OK(h, cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   Plan* pl = nullptr;
   int rc = build_plan(h, nt, H, W, true, &pl);
   if (rc) return rc;
@@ -788,7 +771,7 @@ int dgp_train_forward(dgp_handle* h, const uint8_t* frames_dev, int nt, int H, i
     return fail(h, DGP_ERR_INVALID, "dgp_train_forward: locref_dev given but the network has no locref head");
   CU_OK(h, cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   Plan* pl = nullptr;
   int rc = build_plan(h, nt, H, W, true, &pl);
   if (rc) return rc;
@@ -806,7 +789,7 @@ int dgp_train_backward(dgp_handle* h, uint64_t token, const float* g_logits_dev,
                        void* stream) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_backward before dgp_train_enable");
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   Plan* pl = nullptr;
   for (auto& kv : h->train_plans)
     if (token != 0 && kv.second->fwd_token == token) pl = kv.second.get();
@@ -859,7 +842,7 @@ int dgp_train_wait_early_bucket(dgp_handle* h, void* stream) {
     return fail(h, DGP_ERR_STATE, "dgp_train_wait_early_bucket: no backward pass has recorded the early-bucket event (waiting on a "
                                   "never-recorded event would not order anything)");
   CU_OK(h, cudaSetDevice(h->device));
-  CU_OK(h, cudaStreamWaitEvent((cudaStream_t)stream, h->train->ev_early, 0));
+  CU_OK(h, cudaStreamWaitEvent((cudaStream_t)stream, h->train->ev_early.get(), 0));
   return DGP_OK;
 }
 
@@ -868,10 +851,12 @@ int dgp_optimizer_step(dgp_handle* h, float lr, float momentum, float clip_norm,
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_optimizer_step before dgp_train_enable");
   CU_OK(h, cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   grad_scale /= ts->arena_scale;  // the buffer holds arena_scale * gradient
-  CU_OK(h, launch_global_norm(ts->grads, h->n_params, grad_scale, clip_norm, ts->norm_partial, ts->norm_clip, s));
-  CU_OK(h, launch_momentum_step(h->master, ts->accum, ts->grads, h->n_params, lr, momentum, grad_scale, ts->norm_clip, s));
+  float *grads = ts->grads.get<float>(), *norm_clip = ts->norm_clip.get<float>();
+  CU_OK(h, launch_global_norm(grads, h->n_params, grad_scale, clip_norm, ts->norm_partial.get<float>(), norm_clip, s));
+  CU_OK(h, launch_momentum_step(h->master.get<float>(), ts->accum.get<float>(), grads, h->n_params, lr, momentum, grad_scale,
+                                norm_clip, s));
   h->launches += 3;
   drop_train_tokens(h);
   int rc = refresh_operands(h, s);
@@ -893,7 +878,7 @@ int dgp_params_changed(dgp_handle* h, void* stream) {
 int dgp_get_param_buffer(dgp_handle* h, void** dev_ptr, size_t* bytes) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_get_param_buffer before dgp_finalize_weights");
-  if (dev_ptr) *dev_ptr = h->master;
+  if (dev_ptr) *dev_ptr = h->master.get();
   if (bytes) *bytes = h->n_params * sizeof(float);
   return DGP_OK;
 }
@@ -909,7 +894,7 @@ int dgp_train_set_loss_scale(dgp_handle* h, float loss_scale) {
 int dgp_get_grad_buffer(dgp_handle* h, void** dev_ptr, size_t* bytes) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_get_grad_buffer before dgp_train_enable");
-  if (dev_ptr) *dev_ptr = h->train->grads;
+  if (dev_ptr) *dev_ptr = h->train->grads.get();
   if (bytes) *bytes = h->n_params * sizeof(float);
   return DGP_OK;
 }
@@ -919,7 +904,7 @@ int dgp_get_grad_norm(dgp_handle* h, float* norm_host) {
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_get_grad_norm before dgp_train_enable");
   CU_OK(h, cudaSetDevice(h->device));
   CU_OK(h, cudaDeviceSynchronize());
-  CU_OK(h, cudaMemcpy(norm_host, h->train->norm_clip, sizeof(float), cudaMemcpyDeviceToHost));
+  CU_OK(h, cudaMemcpy(norm_host, h->train->norm_clip.get(), sizeof(float), cudaMemcpyDeviceToHost));
   return DGP_OK;
 }
 
@@ -940,7 +925,8 @@ int dgp_get_variable(dgp_handle* h, const char* tf_var_name, int what, float* ho
   if (what > 0 && !h->train) return fail(h, DGP_ERR_STATE, "dgp_get_variable: gradients need dgp_train_enable");
   VarRef r;
   if (!find_variable(h, tf_var_name, &r)) return fail(h, DGP_ERR_INVALID, "unknown variable %s", tf_var_name);
-  const float* arena = what == 0 ? h->master : (what == 1 ? h->train->grads : h->train->accum);
+  const DevBuf& buf = what == 0 ? h->master : (what == 1 ? h->train->grads : h->train->accum);
+  const float* arena = buf.get<float>();
   const ConvLayer& L = *r.L;
   const int nj = h->cfg.num_joints;
   int64_t shp[4] = {0, 0, 0, 0};
@@ -1004,7 +990,7 @@ int dgp_set_variable(dgp_handle* h, const char* tf_var_name, int what, const flo
   if (what == 2 && !h->train) return fail(h, DGP_ERR_STATE, "dgp_set_variable: momentum needs dgp_train_enable");
   VarRef r;
   if (!find_variable(h, tf_var_name, &r)) return fail(h, DGP_ERR_INVALID, "unknown variable %s", tf_var_name);
-  float* arena = what == 0 ? h->master : h->train->accum;
+  float* arena = (what == 0 ? h->master : h->train->accum).get<float>();
   const ConvLayer& L = *r.L;
   const int nj = h->cfg.num_joints;
   CU_OK(h, cudaSetDevice(h->device));
@@ -1082,7 +1068,7 @@ int dgp_comm_init_rank(dgp_handle* h, const char* id128, int nranks, int rank) {
   if (!id128 || nranks < 1 || rank < 0 || rank >= nranks) return fail(h, DGP_ERR_INVALID, "dgp_comm_init_rank: bad argument");
   if (!nccl::api().ok) return fail(h, DGP_ERR_UNSUPPORTED, "dgp_comm_init_rank: libnccl.so.2 could not be loaded");
   CU_OK(h, cudaSetDevice(h->device));
-  comm_release(h);
+  h->train->release_comm();
   nccl::UniqueId id;
   memcpy(id.internal, id128, 128);
   void* comm = nullptr;
@@ -1096,7 +1082,7 @@ int dgp_comm_init_rank(dgp_handle* h, const char* id128, int nranks, int rank) {
 int dgp_attach_comm(dgp_handle* h, void* nccl_comm) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_attach_comm before dgp_train_enable");
-  comm_release(h);
+  h->train->release_comm();
   if (!nccl_comm) return DGP_OK;   // detach
   if (!nccl::api().ok) return fail(h, DGP_ERR_UNSUPPORTED, "dgp_attach_comm: libnccl.so.2 could not be loaded");
   int n = 0;
@@ -1112,28 +1098,29 @@ int dgp_comm_world_size(dgp_handle* h) { return (h && h->train && h->train->comm
 int dgp_allreduce_gradients(dgp_handle* h, void* stream, float* grad_scale) {
   if (!h) return DGP_ERR_INVALID;
   if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_allreduce_gradients before dgp_train_enable");
-  TrainState* ts = h->train;
+  TrainState* ts = h->train.get();
   if (grad_scale) *grad_scale = 1.0f / (float)ts->comm_world;
   if (!ts->comm || ts->comm_world == 1) return DGP_OK;
   if (!ts->bwd_ran) return fail(h, DGP_ERR_STATE, "dgp_allreduce_gradients: no backward pass has run");
   CU_OK(h, cudaSetDevice(h->device));
-  cudaStream_t s = (cudaStream_t)stream, cs = ts->comm_stream;
+  cudaStream_t s = (cudaStream_t)stream, cs = ts->comm_stream.get();
   const nccl::Api& nc = nccl::api();
-  CU_OK(h, cudaEventRecord(ts->ev_bwd_done, s));                    // the end of the backward on the caller's stream
+  float* grads = ts->grads.get<float>();
+  CU_OK(h, cudaEventRecord(ts->ev_bwd_done.get(), s));                    // the end of the backward on the caller's stream
   for (int k = 0; k < 3; ++k) {                                      // buckets that were final before the backward ended
     const size_t lo = ts->bucket_off[k + 1], hi = ts->bucket_off[k];
     if (hi <= lo) continue;
-    CU_OK(h, cudaStreamWaitEvent(cs, ts->ev_bucket[k], 0));
-    NCCL_OK(h, nc.all_reduce(ts->grads + lo, ts->grads + lo, hi - lo, nccl::kFloat, nccl::kSum, ts->comm, cs));
+    CU_OK(h, cudaStreamWaitEvent(cs, ts->ev_bucket[k].get(), 0));
+    NCCL_OK(h, nc.all_reduce(grads + lo, grads + lo, hi - lo, nccl::kFloat, nccl::kSum, ts->comm, cs));
   }
-  CU_OK(h, cudaStreamWaitEvent(cs, ts->ev_bwd_done, 0));             // conv1 + block1 weights, then gamma / beta / head bias
+  CU_OK(h, cudaStreamWaitEvent(cs, ts->ev_bwd_done.get(), 0));       // conv1 + block1 weights, then gamma / beta / head bias
   NCCL_OK(h, nc.group_start());
   if (ts->bucket_off[3] > 0)
-    NCCL_OK(h, nc.all_reduce(ts->grads, ts->grads, ts->bucket_off[3], nccl::kFloat, nccl::kSum, ts->comm, cs));
-  NCCL_OK(h, nc.all_reduce(ts->grads + h->n_w, ts->grads + h->n_w, h->n_params - h->n_w, nccl::kFloat, nccl::kSum, ts->comm, cs));
+    NCCL_OK(h, nc.all_reduce(grads, grads, ts->bucket_off[3], nccl::kFloat, nccl::kSum, ts->comm, cs));
+  NCCL_OK(h, nc.all_reduce(grads + h->n_w, grads + h->n_w, h->n_params - h->n_w, nccl::kFloat, nccl::kSum, ts->comm, cs));
   NCCL_OK(h, nc.group_end());
-  CU_OK(h, cudaEventRecord(ts->ev_comm_done, cs));
-  CU_OK(h, cudaStreamWaitEvent(s, ts->ev_comm_done, 0));             // the optimizer step on `s` follows the reduced gradients
+  CU_OK(h, cudaEventRecord(ts->ev_comm_done.get(), cs));
+  CU_OK(h, cudaStreamWaitEvent(s, ts->ev_comm_done.get(), 0));       // the optimizer step on `s` follows the reduced gradients
   return DGP_OK;
 }
 
@@ -1143,8 +1130,8 @@ int dgp_allreduce_exposed_ms(dgp_handle* h, float* ms) {
   *ms = 0.0f;
   if (!h->train->comm || h->train->comm_world == 1) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
-  CU_OK(h, cudaEventSynchronize(h->train->ev_comm_done));
-  CU_OK(h, cudaEventElapsedTime(ms, h->train->ev_bwd_done, h->train->ev_comm_done));
+  CU_OK(h, cudaEventSynchronize(h->train->ev_comm_done.get()));
+  CU_OK(h, cudaEventElapsedTime(ms, h->train->ev_bwd_done.get(), h->train->ev_comm_done.get()));
   return DGP_OK;
 }
 

@@ -447,6 +447,10 @@ int dgp_debug_keep_activations(dgp_handle* h, int enable);
 /* Copy a kept end_point to host as float32 NHWC; shape4 receives (N,H,W,C). Returns DGP_ERR_INVALID if unknown. */
 int dgp_debug_get_activation(dgp_handle* h, const char* end_point, float* host_out, size_t max_elems,
                              int64_t* shape4);
+/* Process-wide count of the CUDA resources the library holds (buffers, pinned host memory, events, streams, graphs) and
+ * of their device bytes, over all handles.  Either pointer may be NULL.  A handle's dgp_destroy returns both counts to
+ * their value before its dgp_create. */
+int dgp_debug_live_resources(int64_t* objects, int64_t* device_bytes);
 /* One conv layer through the tcgen05 implicit-GEMM kernel (unit tests): x_dev bf16 NHWC (N,H,W,Cin), w_host float32
  * HWIO, scale/shift host float32 [Cout] or NULL, residual_dev bf16 or NULL (res_sub 1|2), out_dev bf16 or fp32.
  * pad_mode: 0 = TF SAME (stride 1), 1 = slim conv2d_same explicit padding, 2 = VALID. */
