@@ -119,9 +119,6 @@ SIGNATURES = {
     "dgp_get_param_buffer": (_i, [_vp, C.POINTER(_vp), C.POINTER(_sz)]),
     "dgp_params_changed": (_i, [_vp, _vp]),
     "dgp_get_grad_buffer": (_i, [_vp, C.POINTER(_vp), C.POINTER(_sz)]),
-    "dgp_train_early_bucket": (_i, [_vp, C.POINTER(_sz), C.POINTER(_sz)]),
-    "dgp_train_wait_early_bucket": (_i, [_vp, _vp]),
-    "dgp_train_use_graphs": (_i, [_vp, _i]),
     "dgp_train_set_loss_scale": (_i, [_vp, _f]),
     "dgp_comm_unique_id": (_i, [C.c_char_p]),
     "dgp_comm_init_rank": (_i, [_vp, C.c_char_p, _i, _i]),

@@ -56,7 +56,6 @@ struct Backward {
   size_t bn_part_floats = 0;
   std::vector<BnGroup> bn_groups;   // host copy, one entry per 8 channels
   int bucket_step[3] = {-1, -1, -1};  // steps after which buckets 0 (block4 + heads), 1 (block3), 2 (block2) are final
-  int early_step = -1;  // number of steps after which the gradients of block4 + heads (the arena's tail) are final
   // The ~280 launches of the network backward have fixed arguments per plan: after the first (eager) step they are
   // replayed as one CUDA graph, which removes the launch gaps between the many small bandwidth-class kernels.
   int runs = 0;
@@ -75,7 +74,6 @@ struct TrainState {
   int head_Kd = 0;
   bool wd_fresh = false;
   uint64_t ws_gen = 1;           // bumped whenever a shared workspace is reallocated (captured graphs hold its address)
-  bool use_graphs = true;
   float loss_scale = 1.0f;       // head gradients are multiplied by this before the network backward (fp16 storage)
   // What the gradient arena holds: arena_scale x the true gradient (loss_scale after dgp_train_forward_backward, 1 after
   // dgp_train_backward); every reader divides by it.  grad_mode is the device word the arena-writing kernels read
@@ -87,15 +85,11 @@ struct TrainState {
   uint64_t fwd_seq = 0;          // tokens handed out by dgp_train_forward
   DevBuf wd_jobs;                // DgradWJob: device table for the one-launch rebuild of every dgrad operand
   int n_wd_jobs = 0, wd_tiles = 0;
-  // Early all-reduce bucket: the weight gradients of block4 and the heads (two thirds of the arena, contiguous at the end of
-  // its weight part) are complete after a quarter of the backward pass; `ev_early` is recorded there so a data-parallel
-  // caller can start their all-reduce on a side stream while blocks 3..1 are still running.
-  Event ev_early;
-  size_t early_off = 0, early_cnt = 0;
   // Data-parallel all-reduce owned by the library (dgp_attach_comm / dgp_comm_init_rank + dgp_allreduce_gradients): the
   // weight gradients of a block are final once the backward has passed its first unit, so the arena is reduced in four
   // buckets in backward order -- [block4 + heads], [block3], [block2], [conv1 + block1 + gamma/beta/bias] -- each on the
-  // communication stream behind an event recorded at that point of the backward (ev_bucket[0] == ev_early's position).
+  // communication stream behind an event recorded at that point of the backward.  Bucket 0 holds about two thirds of the
+  // arena and is final after the first quarter of the backward pass.
   static constexpr int kBuckets = 4;
   size_t bucket_off[kBuckets + 1] = {0, 0, 0, 0, 0};   // weight-part offsets: bucket k = [bucket_off[k+1], bucket_off[k])
   Event ev_bucket[kBuckets - 1];
@@ -428,7 +422,6 @@ int build_backward(dgp_handle* h, Plan* pl) {
       scatter.d = G; scatter.H = ub.H; scatter.W = ub.W; scatter.P = ub.Ho; scatter.Q = ub.Wo;
     }
     gi = (gi + 1) % 3;
-    if (ts->early_cnt > 0 && u.shortcut >= 0 && h->layers[u.shortcut].w_off == ts->early_off) bw->early_step = (int)bw->steps.size();
     if (u.shortcut >= 0)
       for (int k = 0; k < 3; ++k)
         if (h->layers[u.shortcut].w_off == ts->bucket_off[k + 1]) bw->bucket_step[k] = (int)bw->steps.size();
@@ -560,7 +553,7 @@ int scale_head_grads(dgp_handle* h, const Plan* pl, Backward* bw, cudaStream_t s
 // The network backward of `bw` from its g_logits / g_locref: eager on the first run of a plan, a captured graph afterwards.
 int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
   TrainState* ts = h->train.get();
-  const bool graphs = ts->use_graphs && !h->profiling && bw->runs > 0;
+  const bool graphs = !h->profiling && bw->runs > 0;
   if (graphs && (!bw->graph_exec || bw->graph_gen != ts->ws_gen)) {
     // (re)capture on the handle's private stream; the first step ran eagerly, so every lazy cudaFuncSetAttribute is done
     bw->graph_exec.reset();
@@ -613,13 +606,8 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
         if (ce != cudaSuccess) break;
       }
       ++k;
-      bool boundary = k == bw->early_step;
-      for (int b = 0; b < 3; ++b) boundary = boundary || k == bw->bucket_step[b];
+      const bool boundary = k == bw->bucket_step[0] || k == bw->bucket_step[1] || k == bw->bucket_step[2];
       if (boundary && !pending.empty() && (ce = join_through(pending.size() - 1)) != cudaSuccess) break;
-      if (k == bw->early_step) {
-        ce = cudaEventRecordWithFlags(ts->ev_early.get(), hs, cudaEventRecordExternal);
-        if (ce != cudaSuccess) break;
-      }
       for (int b = 0; b < 3 && ce == cudaSuccess; ++b)
         if (k == bw->bucket_step[b]) ce = cudaEventRecordWithFlags(ts->ev_bucket[b].get(), hs, cudaEventRecordExternal);
       if (ce != cudaSuccess) break;
@@ -654,12 +642,11 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
       }
       h->launches += st.launches;
       ++k;
-      if (k == bw->early_step) CU_OK(h, cudaEventRecord(ts->ev_early.get(), s));
       for (int b = 0; b < 3; ++b)
         if (k == bw->bucket_step[b]) CU_OK(h, cudaEventRecord(ts->ev_bucket[b].get(), s));
     }
   }
-  ts->bwd_ran = bw->early_step > 0;
+  ts->bwd_ran = bw->bucket_step[0] > 0;
   bw->runs++;
   return DGP_OK;
 }
@@ -703,13 +690,6 @@ int dgp_train_enable(dgp_handle* h) {
   ts->n_wd_jobs = (int)jobs.size();
   CU_OK(h, ts->wd_jobs.alloc(jobs.size() * sizeof(DgradWJob)));
   CU_OK(h, cudaMemcpy(ts->wd_jobs.get(), jobs.data(), jobs.size() * sizeof(DgradWJob), cudaMemcpyHostToDevice));
-  CU_OK(h, create(&ts->ev_early, cudaEventDisableTiming));
-  for (const UnitDesc& u : h->units)
-    if (u.scope.find("/block4/") != std::string::npos && u.shortcut >= 0) {
-      ts->early_off = h->layers[u.shortcut].w_off;
-      ts->early_cnt = h->n_w - ts->early_off;
-      break;
-    }
   {
     // bucket k = the weight gradients of one block (k = 0: block4 + heads ... k = 3: conv1 + block1 + the BN / bias tail)
     const char* first[3] = {"/block4/unit_1/", "/block3/unit_1/", "/block2/unit_1/"};
@@ -817,32 +797,6 @@ int dgp_train_backward(dgp_handle* h, uint64_t token, const float* g_logits_dev,
   if ((rc = run_backward(h, bw, s))) return rc;
   ts->arena_scale = 1.0f;
   ts->arena_fused = false;
-  return DGP_OK;
-}
-
-int dgp_train_use_graphs(dgp_handle* h, int enable) {
-  if (!h) return DGP_ERR_INVALID;
-  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_use_graphs before dgp_train_enable");
-  h->train->use_graphs = enable != 0;
-  return DGP_OK;
-}
-
-int dgp_train_early_bucket(dgp_handle* h, size_t* offset_floats, size_t* count_floats) {
-  if (!h) return DGP_ERR_INVALID;
-  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_early_bucket before dgp_train_enable");
-  if (offset_floats) *offset_floats = h->train->early_off;
-  if (count_floats) *count_floats = h->train->early_cnt;
-  return DGP_OK;
-}
-
-int dgp_train_wait_early_bucket(dgp_handle* h, void* stream) {
-  if (!h) return DGP_ERR_INVALID;
-  if (!h->train) return fail(h, DGP_ERR_STATE, "dgp_train_wait_early_bucket before dgp_train_enable");
-  if (!h->train->bwd_ran)
-    return fail(h, DGP_ERR_STATE, "dgp_train_wait_early_bucket: no backward pass has recorded the early-bucket event (waiting on a "
-                                  "never-recorded event would not order anything)");
-  CU_OK(h, cudaSetDevice(h->device));
-  CU_OK(h, cudaStreamWaitEvent((cudaStream_t)stream, h->train->ev_early.get(), 0));
   return DGP_OK;
 }
 

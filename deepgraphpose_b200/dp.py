@@ -1,7 +1,9 @@
 """Data-parallel training plumbing (SURVEY.md 8e, training): one process per GPU, replicas draw their own batches, and the
 only exchange is a SUM all-reduce of the flat float32 gradient buffer, scaled by 1/world before clipping -- the tower
 averaging of the reference's multi-GPU helper (src/deepgraphpose/helpers/utils_tf.py:4-39: average_gradients).  Frozen
-BatchNorm means there is no other cross-replica state.  Works with NCCL (CUDA tensors) and gloo (CPU tensors, tests).
+BatchNorm means there is no other cross-replica state.  The backend of the process group picks the exchange: over NCCL the
+engine's C handle owns a communicator and reduces its gradient arena itself (``dgp_allreduce_gradients``, overlapped with
+the backward pass); over gloo (CPU tensors, tests) the buffer goes through ``allreduce_flat_``.
 """
 import torch
 import torch.distributed as dist
@@ -49,55 +51,29 @@ def attach_comm(engine, group=None):
     return world
 
 
-def ensure_comm(engine, group=None):
-    """attach_comm once per engine, when the process group runs on NCCL (CUDA ranks); gloo / CPU groups keep the
-    torch.distributed path."""
-    if getattr(engine, "_c_comm", None) is not None:
-        return
-    engine._c_comm = False
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1 and \
-            "nccl" in str(dist.get_backend(group)).lower():
-        attach_comm(engine, group)
+def _ensure_comm(engine, group):
+    """attach_comm once per engine when the process group runs on NCCL; True when the C handle owns the all-reduce."""
+    if getattr(engine, "_c_comm", None) is None:
+        engine._c_comm = False
+        if "nccl" in str(dist.get_backend(group)).lower():
+            attach_comm(engine, group)
+    return engine._c_comm
 
 
-def allreduce_gradients(engine, group=None, overlap=True):
+def allreduce_gradients(engine, group=None):
     """All-reduce the engine's gradient buffer across ranks; returns grad_scale for Engine.optimizer_step.
 
-    With a communicator attached to the C handle (``attach_comm``) this is ``dgp_allreduce_gradients``; otherwise the
-    torch.distributed path below (NCCL or, for the CPU tests, gloo).
-
-    With ``overlap`` the slice holding block4 + the heads (two thirds of the buffer, final after the first quarter of the
-    backward pass) is reduced on a side stream that waits on the handle's early-bucket event, i.e. while the GPU is still
-    differentiating blocks 3..1; the rest follows on the compute stream once the backward is done."""
-    if getattr(engine, "_c_comm", False):
-        import ctypes as C
-        from .engine import _stream
-        scale = C.c_float(1.0)
-        engine._check(engine.lib.dgp_allreduce_gradients(engine.h, _stream(engine.device), C.byref(scale)))
-        return float(scale.value)
+    Over NCCL this is ``dgp_allreduce_gradients`` (the communicator is attached on first use); over gloo it is
+    ``allreduce_flat_`` of the buffer."""
     if not dist.is_available() or not dist.is_initialized() or dist.get_world_size(group) == 1:
         return 1.0
-    buf = engine.grad_buffer()
-    world = dist.get_world_size(group)
-    if not overlap or not buf.is_cuda:
-        # the training kernels ran on torch's current stream; NCCL orders its work after it
-        return allreduce_flat_(buf, group)
-    off, cnt = engine.early_bucket()
-    side = engine.__dict__.get("_dp_stream")
-    if side is None:
-        side = engine.__dict__["_dp_stream"] = torch.cuda.Stream(device=engine.device)
-    works = []
-    if cnt > 0:
-        with torch.cuda.stream(side):
-            engine.wait_early_bucket(side)
-            works.append(dist.all_reduce(buf[off:off + cnt], op=dist.ReduceOp.SUM, group=group, async_op=True))
-    if off > 0:
-        works.append(dist.all_reduce(buf[:off], op=dist.ReduceOp.SUM, group=group, async_op=True))
-    if off + cnt < buf.numel():
-        works.append(dist.all_reduce(buf[off + cnt:], op=dist.ReduceOp.SUM, group=group, async_op=True))
-    for w in works:
-        w.wait()   # the compute stream waits for the NCCL streams; the host does not block
-    return 1.0 / world
+    if not _ensure_comm(engine, group):
+        return allreduce_flat_(engine.grad_buffer(), group)
+    import ctypes as C
+    from .engine import _stream
+    scale = C.c_float(1.0)
+    engine._check(engine.lib.dgp_allreduce_gradients(engine.h, _stream(engine.device), C.byref(scale)))
+    return float(scale.value)
 
 
 def allreduce_mean_scalars(values, group=None):

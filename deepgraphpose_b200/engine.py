@@ -531,26 +531,10 @@ class Engine:
         self._check(self.lib.dgp_train_backward(self.h, C.c_uint64(token), _ptr(g_logits), _ptr(g_locref), int(bool(accumulate)),
                                                 _stream(self.device)))
 
-    def use_graphs(self, enable=True):
-        """Replay the network backward as a CUDA graph from the second step on (default) or launch it eagerly."""
-        self.train_enable()
-        self._check(self.lib.dgp_train_use_graphs(self.h, int(enable)))
-
     def set_loss_scale(self, loss_scale):
         """Loss scaling for fp16-storage training (no effect on the update; see dgp_train_set_loss_scale)."""
         self.train_enable()
         self._check(self.lib.dgp_train_set_loss_scale(self.h, float(loss_scale)))
-
-    def early_bucket(self):
-        """(offset, count) in floats of the gradient-buffer slice that is final early in the backward pass (block4 + heads)."""
-        self.train_enable()
-        o, c = C.c_size_t(), C.c_size_t()
-        self._check(self.lib.dgp_train_early_bucket(self.h, C.byref(o), C.byref(c)))
-        return int(o.value), int(c.value)
-
-    def wait_early_bucket(self, stream):
-        """Make the torch.cuda.Stream `stream` wait until the early bucket of the last training step is final."""
-        self._check(self.lib.dgp_train_wait_early_bucket(self.h, C.c_void_p(stream.cuda_stream)))
 
     def allreduce_exposed_ms(self):
         """Milliseconds between the end of the last backward pass and the end of its C-side gradient all-reduce."""

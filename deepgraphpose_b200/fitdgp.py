@@ -348,11 +348,11 @@ class TrainSession:
                 if not lr:
                     raise ValueError("feed_dict must provide the learning_rate placeholder")
                 lr = lr[0]
-            # nothing blocks the host between the backward, the gradient all-reduce (whose first bucket overlaps the rest of
-            # the backward on a side stream) and the optimizer: the six loss values are read only after all three are enqueued
+            # nothing blocks the host between the backward, the gradient all-reduce (whose first buckets overlap the rest of
+            # the backward on the handle's communication stream) and the optimizer: the six loss values are read only after
+            # all three are enqueued
             out = train_forward_backward(g.engine, frames, feed, g.cfg, g.edges, g.ws, g.ws_max, g.n_frames_total,
                                          g.n_visible_frames_total, visible_only=op.visible_only, sync=False)
-            dp.ensure_comm(g.engine, op.group)      # NCCL process group: the C handle owns the all-reduce from here on
             scale = dp.allreduce_gradients(g.engine, op.group)
             g.engine.optimizer_step(float(lr), op.momentum, op.clip_norm, scale)
             vals = dict(zip(LOSS_KEYS, [np.float32(v) for v in out.cpu().numpy()]))

@@ -352,7 +352,9 @@ int dgp_cyclic_reader(void* user, uint8_t* slot, int max_frames, const uint8_t**
  * (conv weights, BatchNorm gamma/beta with frozen moving statistics, deconv weights + biases); dgp_optimizer_step applies
  * tf.clip_by_global_norm(clip_norm) + MomentumOptimizer(lr, momentum).  Between the two calls a data-parallel caller
  * all-reduces (sums) the flat gradient buffer of dgp_get_grad_buffer with NCCL and passes grad_scale = 1 / world_size
- * (the tower averaging of src/deepgraphpose/helpers/utils_tf.py:4-39). */
+ * (the tower averaging of src/deepgraphpose/helpers/utils_tf.py:4-39).
+ * From its second run at a given input shape the network backward (about 280 launches with fixed arguments) is replayed as
+ * one CUDA graph; it is launched kernel by kernel while dgp_set_profiling is on. */
 /* Allocates gradients, momentum accumulators and the transposed (dgrad) weight operands. Call after finalize. */
 int dgp_train_enable(dgp_handle* h);
 /* frames_dev uint8 (nt,H,W,3); batch->pred_dev / locref_dev are ignored (the handle's own head outputs are used), all other
@@ -386,9 +388,6 @@ int dgp_optimizer_step(dgp_handle* h, float lr, float momentum, float clip_norm,
  * end).  Padding of the layouts (conv1's space-to-depth taps, head rows beyond 3nj) must stay 0. */
 int dgp_get_param_buffer(dgp_handle* h, void** dev_ptr, size_t* bytes);
 int dgp_params_changed(dgp_handle* h, void* stream);
-/* From its second run at a given input shape the network backward (about 280 launches with fixed arguments) is replayed as
- * one CUDA graph; enable = 0 goes back to eager launches (always used while dgp_set_profiling is on). Default 1. */
-int dgp_train_use_graphs(dgp_handle* h, int enable);
 /* Loss scaling for fp16 storage (precision = 1): the head gradients are multiplied by loss_scale before the network
  * backward so that small activation gradients stay above fp16's subnormal range; dgp_optimizer_step divides it out again and
  * dgp_get_variable(what = 1) returns unscaled gradients (after dgp_train_forward_backward the raw buffer of
@@ -397,12 +396,6 @@ int dgp_train_use_graphs(dgp_handle* h, int enable);
 int dgp_train_set_loss_scale(dgp_handle* h, float loss_scale);
 /* Flat float32 gradient buffer (kernel layouts: [weights | gamma | beta | head bias]) for ncclAllReduce. */
 int dgp_get_grad_buffer(dgp_handle* h, void** dev_ptr, size_t* bytes);
-/* Overlap of the gradient all-reduce with the backward pass: the gradients of block4 and the heads -- floats
- * [offset, offset + count) of the gradient buffer, about two thirds of it -- are final after the first quarter of the backward
- * pass.  dgp_train_wait_early_bucket makes `stream` (a side stream) wait for that point of the LAST
- * dgp_train_forward_backward, so their ncclAllReduce can run while blocks 3..1 are still being differentiated. */
-int dgp_train_early_bucket(dgp_handle* h, size_t* offset_floats, size_t* count_floats);
-int dgp_train_wait_early_bucket(dgp_handle* h, void* stream);
 /* ---- data-parallel training inside the C ABI (SURVEY 8b: dgp_attach_comm).  The reference's only multi-GPU design averages
  * tower gradients (src/deepgraphpose/helpers/utils_tf.py:4-39, average_gradients); here one process per GPU owns a handle and
  * an NCCL communicator, and the library itself all-reduces the flat gradient arena -- no Python, no torch.distributed on the

@@ -45,17 +45,13 @@ def test_bucketed_allreduce_equals_mean_gradient():
 
 
 class _FakeEngine:
-    """The four members dp.allreduce_gradients touches, on CPU tensors (the real Engine's buffer lives on the GPU)."""
+    """The gradient buffer dp.allreduce_gradients reduces over gloo, on CPU tensors (the real Engine's buffer lives on the GPU)."""
 
     def __init__(self, grads):
         self._g = grads
-        self.device = grads.device
 
     def grad_buffer(self):
         return self._g
-
-    def early_bucket(self):
-        return 6000, 4007
 
 
 def _engine_worker(rank, world, port, q):
@@ -65,7 +61,7 @@ def _engine_worker(rank, world, port, q):
     dist.init_process_group("gloo", rank=rank, world_size=world)
     grads = [torch.randn(10007, generator=torch.Generator().manual_seed(7 + r)) for r in range(world)]
     eng = _FakeEngine(grads[rank].clone())
-    scale = dp.allreduce_gradients(eng)          # CPU buffer: falls back to the bucketed path, same result
+    scale = dp.allreduce_gradients(eng)          # gloo group: the bucketed torch.distributed path, no C communicator
     ok = torch.allclose(eng.grad_buffer() * scale, sum(grads) / world, rtol=1e-6, atol=1e-6)
     q.put((rank, bool(ok)))
     dist.barrier()

@@ -115,7 +115,7 @@ def _train_setup(rank_seed):
     return T, W, frames, batch, edges, cfg, ws, ws_max
 
 
-def _train_worker(rank, world, port, out_dir, c_comm=True):
+def _train_worker(rank, world, port, out_dir, attach=True):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     torch.cuda.set_device(rank)
@@ -125,13 +125,14 @@ def _train_worker(rank, world, port, out_dir, c_comm=True):
     T, W, frames, batch, edges, cfg, ws, ws_max = _train_setup(rank)
     eng = Engine(T.NJ, device=rank)
     eng.load_weights(W)
-    if c_comm:
+    if attach:
         assert dp.attach_comm(eng) == world      # the C handle owns the communicator and the bucketed all-reduce
     fr = torch.from_numpy(frames).cuda(rank)
     for _ in range(2):
         fitdgp.train_forward_backward(eng, fr, batch, cfg, edges, ws, ws_max, 200, 20)
         scale = dp.allreduce_gradients(eng)
         eng.optimizer_step(0.005, 0.9, 10.0, scale)
+    assert eng.lib.dgp_comm_world_size(eng.h) == world      # without attach_comm: attached by the first allreduce_gradients
     same = dp.broadcast_check(eng, CHECK_VARS)
     if rank == 0:
         np.savez(os.path.join(out_dir, "dp.npz"), same=np.array(same), **{k.replace("/", "."): eng.get_variable(k) for k in CHECK_VARS})
@@ -140,16 +141,16 @@ def _train_worker(rank, world, port, out_dir, c_comm=True):
     eng.close()
 
 
-@pytest.mark.parametrize("c_comm", [True, False], ids=["c-abi-comm", "torch-distributed"])
-def test_two_gpu_data_parallel_training_matches_mean_gradient(tmp_path, c_comm):
-    """2 NCCL replicas with different batches, all-reduced gradients (dgp_allreduce_gradients inside the C ABI, or the
-    torch.distributed path), replicated clip + Momentum == one process that averages the two batches' gradients itself
-    (bit for bit: a two-rank sum is order independent)."""
+@pytest.mark.parametrize("attach", [True, False], ids=["c-abi-comm", "attach-on-first-use"])
+def test_two_gpu_data_parallel_training_matches_mean_gradient(tmp_path, attach):
+    """2 NCCL replicas with different batches, all-reduced gradients (dgp_allreduce_gradients inside the C ABI, with the
+    communicator attached up front or, as fit_dgp does, by the first dp.allreduce_gradients), replicated clip + Momentum ==
+    one process that averages the two batches' gradients itself (bit for bit: a two-rank sum is order independent)."""
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
     from deepgraphpose_b200 import fitdgp
     from deepgraphpose_b200.engine import Engine
-    mp.spawn(_train_worker, args=(2, 29541 + int(c_comm), str(tmp_path), c_comm), nprocs=2, join=True)
+    mp.spawn(_train_worker, args=(2, 29541 + int(attach), str(tmp_path), attach), nprocs=2, join=True)
     got = np.load(os.path.join(str(tmp_path), "dp.npz"))
     assert bool(got["same"])
     engs, frs = [], []

@@ -59,7 +59,6 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
     args = _a.Namespace(steps=steps, warmup=warmup, nt=nt, height=height, width=width)
     import torch.distributed as dist
     from deepgraphpose_b200 import dp, fitdgp, fitdgp_util, synthetic
-    no_overlap = os.environ.get("DGP_NO_FLOW_OVERLAP", "0") == "1"   # A/B: learn_wt in front of the step instead of beside it
     from deepgraphpose_b200.engine import Engine, output_dims
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
@@ -78,10 +77,6 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
     ws, ws_max = fitdgp.spatial_clique_params([labels], S0, 8.0, 1000.0, 1.2)
     eng = Engine(NJ, location_refinement=True, device=local_rank, precision=precision)
     eng.load_weights(synthetic.make_weights(NJ, seed=0, net_type=net_type))
-    eng.use_graphs(os.environ.get("DGP_TRAIN_GRAPHS", "1") != "0")
-    c_comm = world > 1 and os.environ.get("DGP_DP_TORCH", "0") != "1"
-    if c_comm:
-        dp.attach_comm(eng)     # the C handle owns its NCCL communicator: dgp_allreduce_gradients, 4 buckets in backward order
     frames_host = bench.make_frame_pool(nt, seed=1234 + rank) if (H, W) == (bench.H, bench.W) else \
         synthetic.make_video(nt, H, W, NJ, seed=1234 + rank)[0]
     frames = torch.from_numpy(frames_host).to(dev)
@@ -100,7 +95,7 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
 
     def step():
         out = fitdgp.train_forward_backward(eng, frames, batch, cfg, edges, ws, ws_max, 1000, 100, sync=False)
-        scale = dp.allreduce_gradients(eng, overlap=os.environ.get("DGP_DP_OVERLAP", "1") != "0")
+        scale = dp.allreduce_gradients(eng)
         eng.optimizer_step(0.005, 0.9, 10.0, scale)
         return out
 
@@ -137,9 +132,9 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
         # wt > 0: the flow-magnitude field of THIS batch, computed on the device from the frames just copied (dgp_learn_wt: the
         # reference's learn_wt = cv2 Farneback on the host, 175 ms per frame pair)
         # -- on the engine's side stream, as fit_dgp does: it overlaps the forward pass, the loss waits for its event
-        b2 = batch if flow_pinned is None else dict(batch, vector_field_tf=fitdgp_util.learn_wt(fr, engine=eng, overlap=not no_overlap))
+        b2 = batch if flow_pinned is None else dict(batch, vector_field_tf=fitdgp_util.learn_wt(fr, engine=eng, overlap=True))
         out = fitdgp.train_forward_backward(eng, fr, b2, cfg, edges, ws, ws_max, 1000, 100, sync=False)
-        scale = dp.allreduce_gradients(eng, overlap=os.environ.get("DGP_DP_OVERLAP", "1") != "0")
+        scale = dp.allreduce_gradients(eng)
         eng.optimizer_step(0.005, 0.9, 10.0, scale)
         return out.cpu()      # [loss_eval, _] = sess.run([loss, train_op]) hands the losses to the host
 
@@ -171,7 +166,7 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
         eng.set_profiling(False)
         prof = eng.get_profile()
     loss = float(out.cpu()[5])
-    exposed_ms = eng.allreduce_exposed_ms() if c_comm else None
+    exposed_ms = eng.allreduce_exposed_ms() if world > 1 else None
     line = None
     if rank == 0:
         peaks, src = bench.load_peaks()
@@ -187,10 +182,9 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
             "higher_is_better": True, "scaling": "weak", "dtype": precision, "data": "synthetic",
             "config": {"workload": "configs[3]: DGP training step, %dx%d, nt=%d frames per replica (%d visible), nj=%d + locref, gm2=1 gm3=3 ws=1000 wt=%g (temporal + skeleton cliques)"
                                    % (H, W, nt, len(vis), NJ, wt), "parallelism": ("dp%d, dgp_allreduce_gradients: NCCL SUM all-reduce of the 94 MB fp32 gradient arena inside the C ABI, 4 buckets in backward order "
-                                       "(block4+heads, block3, block2, rest) overlapped with the backward pass" % world) if c_comm else
-                                      "dp%d, torch.distributed NCCL all-reduce of the 94 MB fp32 gradient buffer" % world,
+                                       "(block4+heads, block3, block2, rest) overlapped with the backward pass" % world) if world > 1 else "single GPU",
                        "feeds": "device-timed value: frames and a (nt-1,H,W) flow-magnitude field resident on the device; e2e: frames from the host, the field from dgp_learn_wt (Farneback on the GPU); labels and marker index vectors fed from the host every step; locref maps built by dgp_locref_targets"},
-            "allreduce": {"exposed_ms_last_step": exposed_ms, "path": "C ABI (dgp_allreduce_gradients)" if c_comm else ("torch.distributed" if world > 1 else "none"),
+            "allreduce": {"exposed_ms_last_step": exposed_ms, "path": "C ABI (dgp_allreduce_gradients)" if world > 1 else "none",
                           "note": "time between the end of the backward pass and the end of the gradient all-reduce on rank 0"},
             "clocks": clocks, "gpu_launches": launches, "loss_after": loss, "finite": bool(np.isfinite(loss)),
             "e2e": {"value": world * nt * e2e_steps / e2e_dt, "unit": "frames/s", "ms_per_step": 1e3 * e2e_dt / e2e_steps,

@@ -20,8 +20,8 @@ for idx in 0 3 4 26 45 46; do
   timeout 600 ncu --set full --clock-control none --import-source on -k regex:conv_gemm -s $((162 + idx)) -c 1 \
     -o $O/${R}_gemm_$idx $B > $O/ncu_gemm_$idx.log 2>&1
 done
-# 5. training step: launch list of one step (graphs off so that every kernel is a launch)
-DGP_TRAIN_GRAPHS=0 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -s 900 -c 700 --csv \
+# 5. training step: launch list of one step
+timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -s 900 -c 700 --csv \
   --log-file $O/${R}_train_launches.csv python tools/bench_train.py --steps 2 --warmup 3 > /dev/null 2>&1
 timeout 300 python tools/bench_train.py --steps 20 --warmup 3 > $O/${R}_bench_train_1gpu.json 2>>$O/bench_${R}.err
 ls -la $O | tail -20
