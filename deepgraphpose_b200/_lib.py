@@ -65,8 +65,15 @@ class DgpAugmentParams(C.Structure):
                 ("elastic_alpha", C.c_double), ("elastic_sigma", C.c_double), ("seed", C.c_uint64)]
 
 
+class DgpMarkerStyle(C.Structure):
+    _fields_ = [("dotsize", C.c_int32), ("mask_threshold", C.c_double), ("scale_x", C.c_double), ("scale_y", C.c_double),
+                ("colors", C.c_void_p)]
+
+
 # reader(user, slot, max_frames, &direct) -> frames delivered (0 = end of video, < 0 = error)
 FRAME_READER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p))
+# writer(user, frames, n) -> < 0 aborts
+FRAME_WRITER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int)
 
 
 # name -> (restype, argtypes); kept in one table so the CPU test-suite can check every exported symbol.
@@ -102,6 +109,9 @@ SIGNATURES = {
                                               _vp]),
     "dgp_estimate_pose_stream_transform": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f, C.c_int64,
                                                 _vp, _vp, _vp, _i64p]),
+    "dgp_draw_markers": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, C.POINTER(DgpMarkerStyle), _vp]),
+    "dgp_estimate_pose_stream_render": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f, C.c_int64,
+                                             _vp, _vp, _vp, _i64p, C.POINTER(DgpMarkerStyle), _vp, _vp]),
     "dgp_motion_blur_kernel": (_i, [_i, C.c_double, C.c_double, _vp]),
     "dgp_elastic_field": (_i, [_vp, _i, _i, C.c_double, C.c_double, C.c_uint64, _vp, _vp, _vp]),
     "dgp_augment": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, C.POINTER(DgpAugmentParams), _vp, C.c_double, _vp]),

@@ -765,8 +765,15 @@ int PoseStaging::reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W,
   return DGP_OK;
 }
 
+int PoseStaging::reserve_render(dgp_handle* h) {
+  if (!d2h_stream) CU_OK(h, create(&d2h_stream, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; ++i)
+    if (!ev_drawn[i]) CU_OK(h, create(&ev_drawn[i], cudaEventDisableTiming));
+  return DGP_OK;
+}
+
 int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
-                           cudaHostFn_t release, void* release_arg) {
+                           cudaHostFn_t release, void* release_arg, const RenderBatch* render) {
   const int nj = h->cfg.num_joints;
   int hf, wf, ho, wo;
   dgp_output_dims(j.H, j.W, &hf, &wf, &ho, &wo);
@@ -785,10 +792,22 @@ int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_
     x = xf.get<uint8_t>();
   }
   if ((rc = dgp_forward(h, x, run_n, j.H, j.W, logits.get<float>(), nullptr, s))) return rc;
-  CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), s));
+  if (!render) CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), s));
   if ((rc = dgp_softargmax(h, logits.get<float>(), nullptr, run_n, ho, wo, nj, j.gamma, j.gauss_len, mu.get<float>(),
                            peak.get<int32_t>(), lik.get<float>(), nullptr, nullptr, s)))
     return rc;
+  if (render) {
+    // the next H2D into this slot waits for ev_consumed, so it must follow the copy of the annotated frames, not the forward
+    cudaStream_t ds = d2h_stream.get();
+    if ((rc = draw_markers_fused(h, frames[slot].get<uint8_t>(), n, j.H0, j.W0, mu.get<float>(), lik.get<float>(),
+                                 *render->args, s)))
+      return rc;
+    CU_OK(h, cudaEventRecord(ev_drawn[slot].get(), s));
+    CU_OK(h, cudaStreamWaitEvent(ds, ev_drawn[slot].get(), 0));
+    CU_OK(h, cudaMemcpyAsync(render->dst, frames[slot].get(), (size_t)j.H0 * j.W0 * 3 * n, cudaMemcpyDeviceToHost, ds));
+    CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), ds));
+    CU_OK(h, cudaLaunchHostFunc(ds, render->handoff, render->handoff_arg));
+  }
   CU_OK(h, cudaMemcpyAsync(j.mu_host + (size_t)t0 * nj * 2, mu.get(), (size_t)n * nj * 2 * 4, cudaMemcpyDeviceToHost, s));
   if (j.peak_host)
     CU_OK(h, cudaMemcpyAsync(j.peak_host + (size_t)t0 * nj * 2, peak.get(), (size_t)n * nj * 2 * 4, cudaMemcpyDeviceToHost, s));

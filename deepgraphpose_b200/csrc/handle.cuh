@@ -111,17 +111,47 @@ struct PoseJob {
   float* lik_host;
 };
 
+// Kernel argument of the marker drawing (render_kernels.cu): the style of dgp_marker_style with its colour table by value,
+// so a launch needs no allocation.
+constexpr int kMaxDotsize = 64;
+struct MarkerArgs {
+  int nj, dotsize;
+  double mask_threshold, scale_x, scale_y, stride, half_stride;
+  uint8_t colors[3 * 256];
+};
+// Validates `st` and fills `a` for the handle's joints and stride.
+int marker_args(dgp_handle* h, const dgp_marker_style* st, MarkerArgs* a);
+// Markers of N frames from the soft-argmax read-outs mu (N,nj,2) / lik (N,nj) of an estimate_pose batch.
+int draw_markers_fused(dgp_handle* h, uint8_t* frames, int N, int H, int W, const float* mu, const float* lik,
+                       const MarkerArgs& a, cudaStream_t s);
+
+// The rendering half of a dgp_estimate_pose_stream_render batch: markers drawn into the batch's source frames, the n real
+// frames copied to the pinned writer slot `dst`, then handoff(handoff_arg) on the D2H stream.
+struct RenderBatch {
+  const MarkerArgs* args;
+  uint8_t* dst;
+  cudaHostFn_t handoff;
+  void* handoff_arg;
+};
+
 // estimate_pose staging: source frames double-buffered between the H2D of the copy stream and the compute stream (slot =
 // batch index & 1), the transformed batch that dgp_forward consumes when a frame transform is given, and the read-outs.
 struct PoseStaging {
   Stream copy_stream;  // H2D of the next batch overlaps the current batch's kernels
   Event ev_copied[2], ev_consumed[2];
   DevBuf frames[2], xf, logits, mu, peak, lik;
+  // rendering: the annotated frames leave on their own stream so that their D2H overlaps the next batch's forward
+  Stream d2h_stream;
+  Event ev_drawn[2];
   int reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W, bool identity);
   // Batch number `it` (n frames at host_frames, output rows [t0, t0 + n)): H2D, transform, forward + soft-argmax of run_n
-  // rows, D2H of n read-outs.  release(release_arg) runs on the copy stream once host_frames has been copied.
+  // rows, D2H of n read-outs.  release(release_arg) runs on the copy stream once host_frames has been copied.  With
+  // `render`, the slot's source frames are annotated and copied out as well, and the slot counts as consumed only after that
+  // copy.
   int run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
-                cudaHostFn_t release, void* release_arg);
+                cudaHostFn_t release, void* release_arg, const RenderBatch* render = nullptr);
+  // the D2H stream and events of run_batch's `render` step (created at the first rendering call)
+  int reserve_render(dgp_handle* h);
 };
 
 }  // namespace dgp
@@ -185,6 +215,8 @@ struct dgp_handle {
   DevBuf aug_scratch[2], aug_fields, aug_tmp;
   // dgp_estimate_pose_stream: pinned host ring the reader thread decodes into (stream.cu)
   PinnedBuf ring_slot[3];
+  // dgp_estimate_pose_stream_render: pinned host ring of annotated frames the writer thread drains (stream.cu)
+  PinnedBuf writer_slot[3];
 };
 
 // loss forward (+ optional loss-side backward) shared by dgp_loss_forward / dgp_loss_backward / the training step

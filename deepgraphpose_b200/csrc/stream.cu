@@ -45,36 +45,39 @@ void CUDART_CB release_slot(void* p) {
   a->ring->cv.notify_all();
 }
 
-}  // namespace
+// Annotated frames on their way to the writer (dgp_estimate_pose_stream_render): the calling thread takes a free slot before
+// it enqueues a batch, the D2H stream hands the slot over once the frames are in it (stream order = video order), and the
+// writer thread frees it again after the writer returns.
+struct WriterRing {
+  std::mutex mu;
+  std::condition_variable cv;
+  bool slot_free[kSlots];
+  struct Ready { int slot; int n; };
+  std::deque<Ready> ready;
+  bool done = false;  // nothing more will be handed over
+  int error = 0;      // first negative return of the writer
+};
 
-extern "C" {
+struct HandoffArg {
+  WriterRing* ring;
+  int slot;
+  int n;
+};
 
-int dgp_cyclic_reader(void* user, uint8_t* slot, int max_frames, const uint8_t** direct) {
-  (void)slot;
-  dgp_cyclic_source* s = static_cast<dgp_cyclic_source*>(user);
-  if (!s || !s->pool || s->pool_frames < 1 || s->frame_bytes == 0) return -1;
-  const int64_t left = s->total_frames - s->position;
-  if (left <= 0) return 0;
-  const int64_t at = s->position % s->pool_frames;
-  int64_t n = s->pool_frames - at;
-  if (n > max_frames) n = max_frames;
-  if (n > left) n = left;
-  *direct = s->pool + (size_t)at * s->frame_bytes;
-  s->position += n;
-  return (int)n;
+void CUDART_CB handoff_slot(void* p) {
+  HandoffArg* a = static_cast<HandoffArg*>(p);
+  {
+    std::lock_guard<std::mutex> lk(a->ring->mu);
+    a->ring->ready.push_back({a->slot, a->n});
+  }
+  a->ring->cv.notify_all();
 }
 
-int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user, int H, int W, int batch, float gamma,
-                             float gauss_len, int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
-                             int64_t* frames_done) {
-  return dgp_estimate_pose_stream_transform(h, reader, user, H, W, nullptr, batch, gamma, gauss_len, max_frames, mu_host,
-                                            peak_host, lik_host, frames_done);
-}
-
-int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
-                                       const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
-                                       int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
-                                       int64_t* frames_done) {
+// The body of dgp_estimate_pose_stream_transform; with a writer, also that of dgp_estimate_pose_stream_render.
+int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0, const dgp_frame_transform* transform,
+                int batch, float gamma, float gauss_len, int64_t max_frames, float* mu_host, int32_t* peak_host,
+                float* lik_host, int64_t* frames_done, const dgp_marker_style* style, dgp_frame_writer writer,
+                void* writer_user) {
   if (!h) return DGP_ERR_INVALID;
   if (frames_done) *frames_done = 0;
   if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_estimate_pose_stream before dgp_finalize_weights");
@@ -83,6 +86,12 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
   bool identity;
   if (transform_dims(H0, W0, transform, &H, &W, &identity))
     return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: invalid frame size or transform");
+  const bool render = writer != nullptr;
+  MarkerArgs marker;
+  if (render) {
+    int rc = marker_args(h, style, &marker);
+    if (rc) return rc;
+  }
   if (max_frames == 0) return DGP_OK;
   CU_OK(h, cudaSetDevice(h->device));
   int rc = h->pose.reserve(h, batch, H0, W0, H, W, identity);
@@ -90,6 +99,11 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
   const size_t frame_bytes = (size_t)H0 * W0 * 3;
   for (PinnedBuf& r : h->ring_slot)
     if (r.bytes() < frame_bytes * batch) CU_OK(h, r.alloc(frame_bytes * batch));
+  if (render) {
+    if ((rc = h->pose.reserve_render(h))) return rc;
+    for (PinnedBuf& r : h->writer_slot)
+      if (r.bytes() < frame_bytes * batch) CU_OK(h, r.alloc(frame_bytes * batch));
+  }
   const PoseJob job = {H0, W0, H, W, identity, transform, gamma, gauss_len, mu_host, peak_host, lik_host};
 
   Ring ring;
@@ -136,6 +150,41 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
     ring.cv.notify_all();
   });
 
+  // ---- writer thread (rendering only): pinned writer slots -> writer, in video order
+  WriterRing wring;
+  for (int i = 0; i < kSlots; ++i) wring.slot_free[i] = true;
+  HandoffArg hand[kSlots];
+  for (int i = 0; i < kSlots; ++i) { hand[i].ring = &wring; hand[i].slot = i; hand[i].n = 0; }
+  uint8_t* wslots[kSlots];
+  for (int i = 0; i < kSlots; ++i) wslots[i] = h->writer_slot[i].get<uint8_t>();
+  std::thread writer_thread;
+  if (render) {
+    writer_thread = std::thread([&wring, &wslots, writer, writer_user]() {
+      for (;;) {
+        WriterRing::Ready r;
+        {
+          std::unique_lock<std::mutex> lk(wring.mu);
+          wring.cv.wait(lk, [&] { return !wring.ready.empty() || wring.done; });
+          if (wring.ready.empty()) break;
+          r = wring.ready.front();
+          wring.ready.pop_front();
+          if (wring.error) {  // after a failure the remaining slots are released unwritten
+            wring.slot_free[r.slot] = true;
+            wring.cv.notify_all();
+            continue;
+          }
+        }
+        const int rc = writer(writer_user, wslots[r.slot], r.n);
+        {
+          std::lock_guard<std::mutex> lk(wring.mu);
+          if (rc < 0 && !wring.error) wring.error = rc;
+          wring.slot_free[r.slot] = true;
+        }
+        wring.cv.notify_all();
+      }
+    });
+  }
+
   // ---- consumer: H2D (copy stream) -> forward + soft-argmax (compute stream) -> D2H of the read-outs
   int64_t t0 = 0;
   int it = 0;
@@ -156,8 +205,26 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
     // surplus frames (allocation of every activation, tensor maps, first-use kernel loads).
     const int run_n = (f.n < batch && full_batch_seen) ? batch : f.n;
     if (f.n == batch) full_batch_seen = true;
+    RenderBatch rb;
+    if (render) {
+      int ws = -1;
+      {
+        std::unique_lock<std::mutex> lk(wring.mu);
+        wring.cv.wait(lk, [&] {
+          if (wring.error) return true;
+          for (int i = 0; i < kSlots; ++i) if (wring.slot_free[i]) return true;
+          return false;
+        });
+        if (wring.error) break;
+        for (int i = 0; i < kSlots; ++i) if (wring.slot_free[i]) { ws = i; break; }
+        wring.slot_free[ws] = false;
+      }
+      hand[ws].n = f.n;
+      rb = {&marker, wslots[ws], handoff_slot, &hand[ws]};
+    }
     // the host slot is reusable once its frames have been copied
-    if ((status = h->pose.run_batch(h, job, f.src, f.n, run_n, it, t0, release_slot, &rel[f.slot]))) break;
+    if ((status = h->pose.run_batch(h, job, f.src, f.n, run_n, it, t0, release_slot, &rel[f.slot], render ? &rb : nullptr)))
+      break;
     t0 += f.n;
     ++it;
   }
@@ -166,16 +233,72 @@ int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, v
     ring.abort = true;
   }
   ring.cv.notify_all();
-  // pending release callbacks reference `ring`: drain both streams before it goes out of scope
+  // pending release / hand-off callbacks reference `ring` and `wring`: drain the streams before they go out of scope
   cudaError_t e1 = cudaStreamSynchronize(h->pose.copy_stream.get());
   cudaError_t e2 = cudaStreamSynchronize(h->stream.get());
+  const cudaError_t e3 = render ? cudaStreamSynchronize(h->pose.d2h_stream.get()) : cudaSuccess;
+  if (e2 == cudaSuccess) e2 = e3;
   producer.join();
+  if (render) {
+    {
+      std::lock_guard<std::mutex> lk(wring.mu);
+      wring.done = true;
+    }
+    wring.cv.notify_all();
+    writer_thread.join();
+  }
   if (frames_done) *frames_done = t0;
   if (status) return status;
   if (e1 != cudaSuccess || e2 != cudaSuccess)
     return fail(h, DGP_ERR_CUDA, "dgp_estimate_pose_stream: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
   if (ring.reader_error) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: the frame reader failed (%d)", ring.reader_error);
+  if (wring.error) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render: the frame writer failed (%d)", wring.error);
   return DGP_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dgp_cyclic_reader(void* user, uint8_t* slot, int max_frames, const uint8_t** direct) {
+  (void)slot;
+  dgp_cyclic_source* s = static_cast<dgp_cyclic_source*>(user);
+  if (!s || !s->pool || s->pool_frames < 1 || s->frame_bytes == 0) return -1;
+  const int64_t left = s->total_frames - s->position;
+  if (left <= 0) return 0;
+  const int64_t at = s->position % s->pool_frames;
+  int64_t n = s->pool_frames - at;
+  if (n > max_frames) n = max_frames;
+  if (n > left) n = left;
+  *direct = s->pool + (size_t)at * s->frame_bytes;
+  s->position += n;
+  return (int)n;
+}
+
+int dgp_estimate_pose_stream(dgp_handle* h, dgp_frame_reader reader, void* user, int H, int W, int batch, float gamma,
+                             float gauss_len, int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                             int64_t* frames_done) {
+  return dgp_estimate_pose_stream_transform(h, reader, user, H, W, nullptr, batch, gamma, gauss_len, max_frames, mu_host,
+                                            peak_host, lik_host, frames_done);
+}
+
+int dgp_estimate_pose_stream_transform(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                       const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                       int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                       int64_t* frames_done) {
+  return stream_impl(h, reader, user, H0, W0, transform, batch, gamma, gauss_len, max_frames, mu_host, peak_host, lik_host,
+                     frames_done, nullptr, nullptr, nullptr);
+}
+
+int dgp_estimate_pose_stream_render(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                    const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                    int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                    int64_t* frames_done, const dgp_marker_style* style, dgp_frame_writer writer,
+                                    void* writer_user) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!writer) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render: no frame writer");
+  return stream_impl(h, reader, user, H0, W0, transform, batch, gamma, gauss_len, max_frames, mu_host, peak_host, lik_host,
+                     frames_done, style, writer, writer_user);
 }
 
 }  // extern "C"

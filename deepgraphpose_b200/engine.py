@@ -53,6 +53,40 @@ def transform_dims(H0, W0, new_size=None, crop_size=None):
     return H.value, W.value
 
 
+MAX_DOTSIZE = 64  # kMaxDotsize of csrc/handle.cuh
+
+
+def marker_colors(nj, colormap="cool"):
+    """The (nj, 3) uint8 RGB marker colours of plot_dgp's default colormap, sampled as matplotlib's
+    ``ScalarMappable(cmap='cool').to_rgba(linspace(0, 1, nj))`` does: idx_j = min(255, floor(256 j / (nj - 1))) (0 when
+    nj == 1), colour (idx_j, 255 - idx_j, 255).  'cool' is the only colormap name; anything else is a ValueError."""
+    if not isinstance(colormap, str) or colormap != "cool":
+        raise ValueError("unknown colormap %r: 'cool' is the only named colormap (or pass an (nj, 3) uint8 table)" % (colormap,))
+    nj = int(nj)
+    if nj < 1:
+        raise ValueError("nj must be positive")
+    j = np.arange(nj, dtype=np.int64)
+    idx = np.zeros(nj, np.int64) if nj == 1 else np.minimum(255, (256 * j) // (nj - 1))
+    return np.stack([idx, 255 - idx, np.full(nj, 255)], axis=1).astype(np.uint8)
+
+
+def marker_style(nj, dotsize=3, mask_threshold=0.1, colors=None, scale_x=1.0, scale_y=1.0):
+    """(dgp_marker_style, colour table) of a drawing call; the table must stay alive while the style is in use.  ``colors``:
+    None (the 'cool' table), a colormap name, or an (nj, 3) table of values in [0, 255].  ValueError for a dotsize outside
+    [0, 64] or a table of another shape."""
+    if isinstance(dotsize, bool) or not isinstance(dotsize, (int, np.integer)) or not 0 <= int(dotsize) <= MAX_DOTSIZE:
+        raise ValueError("dotsize must be an integer in [0, %d], got %r" % (MAX_DOTSIZE, dotsize))
+    if colors is None or isinstance(colors, str):
+        table = marker_colors(nj, "cool" if colors is None else colors)
+    else:
+        arr = np.asarray(colors)
+        if arr.shape != (int(nj), 3) or not (np.issubdtype(arr.dtype, np.integer) and arr.min() >= 0 and arr.max() <= 255):
+            raise ValueError("colors must be an (%d, 3) table of RGB values in [0, 255], got %s %s" % (nj, arr.dtype, arr.shape))
+        table = np.ascontiguousarray(arr, dtype=np.uint8)
+    st = _lib.DgpMarkerStyle(int(dotsize), float(mask_threshold), float(scale_x), float(scale_y), table.ctypes.data)
+    return st, table
+
+
 def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3)):
     """Frames per batch that minimise wave quantisation of the persistent conv-GEMM grid (one CTA per SM).
 
@@ -390,6 +424,65 @@ class Engine:
                                                               float(gauss_len), _ptr(mu), _ptr(peak), _ptr(lik)))
         return mu, peak, lik
 
+    def draw_markers(self, frames_dev, x, y, lik, dotsize=3, mask_threshold=0.1, colors=None):
+        """plot_dgp's markers drawn into ``frames_dev`` (uint8 contiguous CUDA (N,H,W,3) RGB, modified in place;
+        dgp_draw_markers): joint j of frame t where ``lik[t, j] > mask_threshold``, a disc of radius ``dotsize`` at the
+        video-pixel coordinates ``x[t, j]``, ``y[t, j]`` in ``colors[j]`` (see ``marker_style``).  ``x``, ``y``, ``lik``:
+        (N, nj) float64 CUDA tensors, or host arrays (uploaded).  Asynchronous on the current stream."""
+        if frames_dev.dtype != torch.uint8 or frames_dev.dim() != 4 or frames_dev.shape[-1] != 3 or not frames_dev.is_cuda:
+            raise ValueError("frames must be a uint8 CUDA tensor of shape (N,H,W,3)")
+        if not frames_dev.is_contiguous():
+            raise ValueError("frames must be contiguous: markers are drawn in place")
+        N, H, W, _ = frames_dev.shape
+        st, table = marker_style(self.nj, dotsize, mask_threshold, colors)
+        cols = []
+        for v in (x, y, lik):
+            if not isinstance(v, torch.Tensor):
+                v = torch.from_numpy(np.ascontiguousarray(np.asarray(v, dtype=np.float64)))
+            v = v.to(device=frames_dev.device, dtype=torch.float64).contiguous()
+            if tuple(v.shape) != (N, self.nj):
+                raise ValueError("x, y and lik must be (%d, %d)" % (N, self.nj))
+            cols.append(v)
+        self._check(self.lib.dgp_draw_markers(self.h, _ptr(frames_dev), N, H, W, _ptr(cols[0]), _ptr(cols[1]), _ptr(cols[2]),
+                                              C.byref(st), _stream(frames_dev.device)))
+        return frames_dev
+
+    def _frame_reader(self, source, H, W, T, start):
+        """(reader, user, keep, state) of a stream source (see estimate_pose_stream); state["error"] holds an exception the
+        source raised."""
+        frame_bytes = int(H) * int(W) * 3
+        state = {"error": None}
+        if isinstance(source, torch.Tensor):
+            if source.is_cuda or source.dtype != torch.uint8 or source.dim() != 4 or tuple(source.shape[1:]) != (H, W, 3):
+                raise ValueError("a tensor source must be a uint8 CPU tensor (P,%d,%d,3)" % (H, W))
+            pool = source.contiguous()
+            src = _lib.DgpCyclicSource(pool.data_ptr(), pool.shape[0], int(start) + T, int(start), frame_bytes)
+            return C.cast(self.lib.dgp_cyclic_reader, C.c_void_p), C.cast(C.pointer(src), C.c_void_p), (pool, src), state
+        it = iter(source)
+
+        def _read(user_, slot, want, direct):
+            try:
+                dst = np.ctypeslib.as_array(C.cast(slot, C.POINTER(C.c_uint8)), shape=(want, H, W, 3))
+                n = 0
+                for n in range(1, want + 1):
+                    try:
+                        fr = next(it)
+                    except StopIteration:
+                        n -= 1
+                        break
+                    fr = np.asarray(fr)
+                    if fr.shape != (H, W, 3) or fr.dtype != np.uint8:
+                        raise ValueError("the source must yield uint8 frames of shape (%d, %d, 3), got %s %s"
+                                         % (H, W, fr.dtype, fr.shape))
+                    dst[n - 1] = fr
+                return n
+            except Exception as ex:  # never unwind through the C frame
+                state["error"] = ex
+                return -1
+
+        cb = _lib.FRAME_READER(_read)
+        return C.cast(cb, C.c_void_p), C.c_void_p(0), cb, state
+
     def estimate_pose_stream(self, source, H, W, max_frames, batch=16, gamma=1.0, gauss_len=1.0, start=0, new_size=None,
                              crop_size=None):
         """Streaming estimate_pose (dgp_estimate_pose_stream): host memory is bounded by a ring of 3 pinned slots of `batch`
@@ -413,45 +506,56 @@ class Engine:
         peak = torch.empty((T, self.nj, 2), dtype=torch.int32).pin_memory()
         lik = torch.empty((T, self.nj), dtype=torch.float32).pin_memory()
         done = C.c_int64(0)
-        frame_bytes = int(H) * int(W) * 3
-        if isinstance(source, torch.Tensor):
-            if source.is_cuda or source.dtype != torch.uint8 or source.dim() != 4 or tuple(source.shape[1:]) != (H, W, 3):
-                raise ValueError("a tensor source must be a uint8 CPU tensor (P,%d,%d,3)" % (H, W))
-            pool = source.contiguous()
-            src = _lib.DgpCyclicSource(pool.data_ptr(), pool.shape[0], int(start) + T, int(start), frame_bytes)
-            reader, user, keep = C.cast(self.lib.dgp_cyclic_reader, C.c_void_p), C.cast(C.pointer(src), C.c_void_p), (pool, src)
-        else:
-            it = iter(source)
-            state = {"error": None}
-
-            def _read(user_, slot, want, direct):
-                try:
-                    dst = np.ctypeslib.as_array(C.cast(slot, C.POINTER(C.c_uint8)), shape=(want, H, W, 3))
-                    n = 0
-                    for n in range(1, want + 1):
-                        try:
-                            fr = next(it)
-                        except StopIteration:
-                            n -= 1
-                            break
-                        fr = np.asarray(fr)
-                        if fr.shape != (H, W, 3) or fr.dtype != np.uint8:
-                            raise ValueError("the source must yield uint8 frames of shape (%d, %d, 3), got %s %s"
-                                             % (H, W, fr.dtype, fr.shape))
-                        dst[n - 1] = fr
-                    return n
-                except Exception as ex:  # never unwind through the C frame
-                    state["error"] = ex
-                    return -1
-
-            cb = _lib.FRAME_READER(_read)
-            reader, user, keep = C.cast(cb, C.c_void_p), C.c_void_p(0), (cb, state)
+        reader, user, keep, state = self._frame_reader(source, H, W, T, start)
         status = self.lib.dgp_estimate_pose_stream_transform(self.h, reader, user, int(H), int(W),
                                                              C.byref(tf) if tf is not None else None, int(batch),
                                                              float(gamma), float(gauss_len), T, _ptr(mu), _ptr(peak),
                                                              _ptr(lik), C.byref(done))
-        if not isinstance(source, torch.Tensor) and keep[1]["error"] is not None:
-            raise keep[1]["error"]
+        if state["error"] is not None:
+            raise state["error"]
+        self._check(status)
+        n = int(done.value)
+        return mu[:n], peak[:n], lik[:n]
+
+    def estimate_pose_render_stream(self, source, H, W, max_frames, writer, dotsize=3, mask_threshold=0.1, colors=None,
+                                    new_size=None, crop_size=None, batch=16, gamma=1.0, gauss_len=1.0, start=0):
+        """estimate_pose_stream that renders plot_dgp's labelled video in the same pass (dgp_estimate_pose_stream_render):
+        after each batch's soft-argmax the markers are drawn on the device into the batch's source frames (coordinates
+        converted to video pixels as eval.estimate_pose does, scale W / new_size[1], H / new_size[0] under ``new_size``) and
+        the annotated frames are handed to ``writer(frames)`` -- a uint8 (n,H,W,3) RGB array valid only during the call --
+        from a writer thread, in video order.  An exception the writer raises aborts the pass and is re-raised here; a
+        negative integer it returns aborts it with DgpError, as in the C ABI.
+        Sources and return value as in estimate_pose_stream; style arguments as in draw_markers."""
+        T = int(max_frames)
+        transform_dims(H, W, new_size, crop_size)
+        tf = frame_transform(new_size, crop_size)
+        sx, sy = (1.0, 1.0) if new_size is None else (W / new_size[1], H / new_size[0])
+        st, table = marker_style(self.nj, dotsize, mask_threshold, colors, sx, sy)
+        if not callable(writer):
+            raise ValueError("writer must be callable")
+        mu = torch.empty((T, self.nj, 2), dtype=torch.float32).pin_memory()
+        peak = torch.empty((T, self.nj, 2), dtype=torch.int32).pin_memory()
+        lik = torch.empty((T, self.nj), dtype=torch.float32).pin_memory()
+        done = C.c_int64(0)
+        reader, user, keep, state = self._frame_reader(source, H, W, T, start)
+        werr = {"error": None}
+
+        def _write(user_, frames, n):
+            try:
+                rc = writer(np.ctypeslib.as_array(C.cast(frames, C.POINTER(C.c_uint8)), shape=(n, H, W, 3)))
+                return int(rc) if isinstance(rc, (int, np.integer)) and rc < 0 else 0
+            except Exception as ex:  # never unwind through the C frame
+                werr["error"] = ex
+                return -1
+
+        wcb = _lib.FRAME_WRITER(_write)
+        status = self.lib.dgp_estimate_pose_stream_render(self.h, reader, user, int(H), int(W),
+                                                          C.byref(tf) if tf is not None else None, int(batch), float(gamma),
+                                                          float(gauss_len), T, _ptr(mu), _ptr(peak), _ptr(lik), C.byref(done),
+                                                          C.byref(st), C.cast(wcb, C.c_void_p), None)
+        for err in (state["error"], werr["error"]):
+            if err is not None:
+                raise err
         self._check(status)
         n = int(done.value)
         return mu[:n], peak[:n], lik[:n]

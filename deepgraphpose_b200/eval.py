@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import synthetic
-from .engine import Engine
+from .engine import Engine, marker_colors, marker_style  # noqa: F401  (marker_colors: eval's public name)
 from .session import Handle, Session
 
 
@@ -237,13 +237,7 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
     the reference's ``PIL.Image.resize`` (Pillow's default filter, BICUBIC) and ``crop``.
     The backbone (ResNet-50, -101 or -152) is the one the weights' names describe, as the reference's estimate_pose tries
     each snapshot scope (eval.py:271-276)."""
-    if isinstance(proj_cfg_file, (dict,)) or hasattr(proj_cfg_file, "num_joints"):
-        dlc_cfg = proj_cfg_file
-    else:
-        import yaml
-        with open(proj_cfg_file, "r") as stream:
-            proj = yaml.safe_load(stream)
-        dlc_cfg = {"num_joints": len(proj["bodyparts"]), "all_joints_names": list(proj["bodyparts"]), "stride": 8.0}
+    dlc_cfg = _load_dlc_cfg(proj_cfg_file)
     save_file = None
     scale_x = scale_y = 1.0
     if isinstance(video_file, (str, os.PathLike)):
@@ -265,11 +259,25 @@ def estimate_pose(proj_cfg_file, dgp_model_file, video_file, output_dir, shuffle
     sess.close()
     labels = {"x": res["x"] * scale_x, "y": res["y"] * scale_y, "likelihoods": res["likelihoods"]}
     if save_pose and save_file is not None:
-        os.makedirs(os.path.dirname(save_file) or ".", exist_ok=True)
-        names = _cfg_get(dlc_cfg, "all_joints_names", ["joint%d" % i for i in range(labels["x"].shape[1])])
-        scorer = os.path.basename(str(dgp_model_file)) if isinstance(dgp_model_file, (str, os.PathLike)) else "dgp_b200"
-        export_pose_like_dlc(labels, scorer, list(names), save_file)
+        _save_labels(labels, dlc_cfg, dgp_model_file, save_file)
     return labels
+
+
+def _load_dlc_cfg(proj_cfg_file):
+    """A dict-like dlc_cfg as given, or the one of a DLC project yaml (its bodyparts)."""
+    if isinstance(proj_cfg_file, (dict,)) or hasattr(proj_cfg_file, "num_joints"):
+        return proj_cfg_file
+    import yaml
+    with open(proj_cfg_file, "r") as stream:
+        proj = yaml.safe_load(stream)
+    return {"num_joints": len(proj["bodyparts"]), "all_joints_names": list(proj["bodyparts"]), "stride": 8.0}
+
+
+def _save_labels(labels, dlc_cfg, dgp_model_file, save_file):
+    os.makedirs(os.path.dirname(save_file) or ".", exist_ok=True)
+    names = _cfg_get(dlc_cfg, "all_joints_names", ["joint%d" % i for i in range(labels["x"].shape[1])])
+    scorer = os.path.basename(str(dgp_model_file)) if isinstance(dgp_model_file, (str, os.PathLike)) else "dgp_b200"
+    export_pose_like_dlc(labels, scorer, list(names), save_file)
 
 
 def export_pose_like_dlc(labels, scorer, joints_names, save_file):
@@ -294,6 +302,152 @@ def load_pose_from_dlc_to_dict(filename):
     """eval.py:648-653: read a DLC csv back into {'x', 'y', 'likelihoods'} (T, nj) arrays."""
     body = np.genfromtxt(filename, delimiter=",", skip_header=3)[:, 1:]   # missing values (empty cells) become NaN
     return {"x": body[:, 0::3], "y": body[:, 1::3], "likelihoods": body[:, 2::3]}
+
+
+def _video_writer(filename, fourcc, fps, H, W):
+    import cv2
+    os.makedirs(os.path.dirname(str(filename)) or ".", exist_ok=True)
+    vw = cv2.VideoWriter(str(filename), cv2.VideoWriter_fourcc(*fourcc), float(fps), (int(W), int(H)))
+    if not vw.isOpened():
+        raise IOError("cannot open a %r video writer for %s" % (fourcc, filename))
+    return vw
+
+
+def _write_rgb(vw, frames):
+    for fr in frames:
+        vw.write(np.ascontiguousarray(fr[:, :, ::-1]))  # RGB -> BGR, what OpenCV encodes
+
+
+def _check_fourcc(fourcc):
+    if not isinstance(fourcc, str) or len(fourcc) != 4:
+        raise ValueError("fourcc must be a four-character code such as 'mp4v' or 'FFV1', got %r" % (fourcc,))
+
+
+def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colormap="cool", filename="movie.mp4", fps=None,
+                           fourcc="mp4v", batch=16, engine=None):
+    """plot_dgp's renderer (src/deepgraphpose/models/eval.py): a video of ``clip`` with joint j of frame t marked by a disc
+    of radius ``dotsize`` at (``df_x[t, j]``, ``df_y[t, j]``) (video pixels) where ``mask_array[t, j]`` (None: every joint),
+    coloured by ``colormap`` (the name 'cool' or an (nj, 3) uint8 RGB table) -- the drawing contract of dgp_draw_markers.
+    ``clip``: a video path (decoded with OpenCV) or a uint8 (T,H,W,3) RGB array.  Frames are drawn on the device in batches
+    of ``batch`` (``engine``: an Engine with nj joints, else one is created for the call) and written with
+    ``cv2.VideoWriter(filename, fourcc, fps)``; ``fps`` None = the video's own rate (required for an array).  Every frame
+    the decoder yields is written, one label row per frame.  The reference writes ``int(duration * fps)`` frames with
+    moviepy (libx264) and draws with matplotlib / skimage on the host; bitstream and anti-aliasing parity are not goals."""
+    x = np.asarray(df_x, dtype=np.float64)
+    y = np.asarray(df_y, dtype=np.float64)
+    if x.ndim != 2 or y.shape != x.shape:
+        raise ValueError("df_x and df_y must be (T, nj) arrays of one shape")
+    nj = x.shape[1]
+    mask = np.ones(x.shape, np.float64) if mask_array is None else np.asarray(mask_array, dtype=bool).astype(np.float64)
+    if mask.shape != x.shape:
+        raise ValueError("mask_array must be (T, nj) like df_x")
+    marker_style(nj, dotsize, 0.5, colormap)  # validates dotsize and colours before any decode or device work
+    _check_fourcc(fourcc)
+    if isinstance(clip, (str, os.PathLike)):
+        if fps is None:
+            import cv2
+            cap = cv2.VideoCapture(str(clip))
+            fps = cap.get(cv2.CAP_PROP_FPS)
+            cap.release()
+        frames_iter = _iter_video(clip)
+    else:
+        arr = np.asarray(clip)
+        if arr.dtype != np.uint8 or arr.ndim != 4 or arr.shape[-1] != 3:
+            raise ValueError("clip must be a video path or a uint8 (T,H,W,3) array")
+        if fps is None:
+            raise ValueError("fps is required when clip is an array")
+        frames_iter = iter(arr)
+    own = engine is None
+    eng = Engine(nj) if own else engine
+    vw = None
+    try:
+        t0 = 0
+        while True:
+            chunk = []
+            for fr in frames_iter:
+                chunk.append(fr)
+                if len(chunk) == batch:
+                    break
+            if not chunk:
+                break
+            n = len(chunk)
+            if t0 + n > x.shape[0]:
+                raise ValueError("the clip has more frames than the %d label rows" % x.shape[0])
+            host = torch.from_numpy(np.ascontiguousarray(np.stack(chunk)))
+            if vw is None:
+                vw = _video_writer(filename, fourcc, fps, host.shape[1], host.shape[2])
+            dev = host.to(eng.device)
+            eng.draw_markers(dev, x[t0:t0 + n], y[t0:t0 + n], mask[t0:t0 + n], dotsize, 0.5, colormap)
+            _write_rgb(vw, dev.cpu().numpy())
+            t0 += n
+    finally:
+        if vw is not None:
+            vw.release()
+        if own:
+            eng.close()
+    return filename
+
+
+def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_model_file=None, shuffle=1, dotsize=3,
+             colormap="cool", save_str="", mask_threshold=0.1, new_size=None, crop_size=None, batch=16, fourcc="mp4v"):
+    """plot_dgp (src/deepgraphpose/models/eval.py; step 3 of the reference demo): labels a video and renders the labelled
+    movie ``<output_dir>/<video>_labeled<save_str>.mp4`` (cv2.VideoWriter with ``fourcc`` at the source fps) in which joint j
+    is a disc of radius ``dotsize`` in ``colormap``'s colour j wherever its likelihood exceeds ``mask_threshold``.
+
+    * An existing movie is left alone (nothing is computed).
+    * No label csv ``<label_dir>/<video>_labeled<save_str>.csv`` (label_dir None = output_dir): ONE streamed pass
+      (Engine.estimate_pose_render_stream) decodes the video once, estimates the pose as ``estimate_pose`` does (same csv)
+      and draws the markers into the source frames on the device before they are written.
+    * With the csv: the labels are read with ``load_pose_from_dlc_to_dict`` and drawn by ``create_annotated_movie``.
+
+    ``proj_cfg_file`` / ``dgp_model_file`` / ``new_size`` / ``crop_size`` / ``batch`` as in estimate_pose; ``shuffle`` is
+    accepted for the reference's signature.  ``fourcc='FFV1'`` writes lossless video (used by the tests).  Every frame the
+    decoder yields is written; the reference writes ``int(duration * fps)`` frames with moviepy.  The defaults are the
+    reference's as recorded in this project (dotsize 3, 'cool', mask_threshold 0.1); they have not been checked against a
+    reference checkout.  Returns the movie's path."""
+    if not isinstance(video_file, (str, os.PathLike)):
+        raise ValueError("video_file must be a path")
+    _check_fourcc(fourcc)
+    name = os.path.basename(str(video_file)).rsplit(".", 1)[0] + "_labeled%s" % save_str
+    label_dir = output_dir if label_dir is None else label_dir
+    movie = os.path.join(str(output_dir), name + ".mp4")
+    csv = os.path.join(str(label_dir), name + ".csv")
+    if os.path.exists(movie):
+        print("labeled video already exists: %s" % movie)
+        return movie
+    dlc_cfg = _load_dlc_cfg(proj_cfg_file) if proj_cfg_file is not None else None
+    if os.path.exists(csv):
+        labels = load_pose_from_dlc_to_dict(csv)
+        marker_style(labels["x"].shape[1], dotsize, mask_threshold, colormap)
+        return create_annotated_movie(video_file, labels["x"], labels["y"], labels["likelihoods"] > mask_threshold,
+                                      dotsize=dotsize, colormap=colormap, filename=movie, fourcc=fourcc, batch=batch)
+    if dlc_cfg is None:
+        raise ValueError("no labels at %s: proj_cfg_file and dgp_model_file are needed to estimate them" % csv)
+    marker_style(int(_cfg_get(dlc_cfg, "num_joints")), dotsize, mask_threshold, colormap)
+    import cv2
+    cap = cv2.VideoCapture(str(video_file))
+    fps = cap.get(cv2.CAP_PROP_FPS)
+    cap.release()
+    source, H0, W0, _, scale_x, scale_y = _video_source(video_file, new_size)
+    sess = _setup_eval_graph(dlc_cfg, dgp_model_file, None)[0]
+    eng = sess.engine
+    vw = _video_writer(movie, fourcc, fps, H0, W0)
+    parts, chunk = [], 65536
+    try:
+        it = iter(source)
+        while True:
+            mu, peak, lik = eng.estimate_pose_render_stream(it, H0, W0, chunk, lambda fr: _write_rgb(vw, fr), dotsize,
+                                                            mask_threshold, colormap, new_size, crop_size, batch)
+            parts.append((mu, peak, lik))
+            if mu.shape[0] < chunk:
+                break
+    finally:
+        vw.release()
+        sess.close()
+    res = _readout_dict(*(torch.cat([p[i] for p in parts]) for i in range(3)), eng.stride)
+    labels = {"x": res["x"] * scale_x, "y": res["y"] * scale_y, "likelihoods": res["likelihoods"]}
+    _save_labels(labels, dlc_cfg, dgp_model_file, os.path.join(str(label_dir), name))
+    return movie
 
 
 def evaluate_dgp_frames(engine, frames, loc_ref=True, loc_ref_calc="dlc", batch=16, gamma=1.0, gauss_len=1.0):

@@ -346,6 +346,38 @@ typedef struct dgp_cyclic_source {
 } dgp_cyclic_source;
 int dgp_cyclic_reader(void* user, uint8_t* slot, int max_frames, const uint8_t** direct);
 
+/* ---- labelled video (plot_dgp / create_annotated_movie, src/deepgraphpose/models/eval.py) ----
+ * Markers drawn into uint8 (N,H,W,3) RGB frames.  For frame t and joint j with video-pixel coordinates x, y (float64) and
+ * likelihood lik: the joint is drawn iff (double)lik > mask_threshold (strictly; NaN in x, y or lik: not drawn); centre
+ * xc = min(trunc(x), W - 1), yc = min(trunc(y), H - 1) in double (truncation toward zero, negative centres kept, +inf
+ * clamps to the last row / column); the disc is every pixel (r, c) of the frame with (r - yc)^2 + (c - xc)^2 < dotsize^2 in
+ * integers, painted colors[j].  Joints are drawn in index order (where discs overlap the higher index wins); pixels outside
+ * every disc keep their bytes.  dotsize in [0, 64] (0 draws nothing). */
+typedef struct dgp_marker_style {
+  int32_t dotsize;
+  double mask_threshold;
+  double scale_x, scale_y;  /* fused pass only: soft-argmax coordinates -> video pixels (W0 / new_w, H0 / new_h, else 1) */
+  const uint8_t* colors;    /* host (nj,3) RGB, nj = the handle's num_joints */
+} dgp_marker_style;
+/* Draws the markers of x_dev, y_dev, lik_dev (float64 (N,nj) on the device) into frames_dev (N,H,W,3) in place; `scale_x`
+ * and `scale_y` are not used (the coordinates are video pixels already).  Asynchronous on `stream`; the colour table
+ * travels as a kernel argument.  The render-only entry, for labels that already exist (a DLC csv). */
+int dgp_draw_markers(dgp_handle* h, uint8_t* frames_dev, int N, int H, int W, const double* x_dev, const double* y_dev,
+                     const double* lik_dev, const dgp_marker_style* style, void* stream);
+/* writer(user, frames, n): n uint8 (H0,W0,3) RGB annotated frames, valid only during the call; return < 0 to abort.  Called
+ * from a thread owned by the call, never concurrently, with frames in video order. */
+typedef int (*dgp_frame_writer)(void* user, const uint8_t* frames, int n);
+/* dgp_estimate_pose_stream_transform that also renders the labelled video in the same pass: per batch, after the
+ * soft-argmax, the markers of x = ((double)mu[..,1] * stride + 0.5 * stride) * scale_x, y likewise with mu[..,0] and
+ * scale_y, and lik are drawn into the batch's (H0,W0) source frames on the device (stride = the handle's, as a double),
+ * the n real frames are copied into a ring of 3 pinned writer slots and handed to `writer` on a writer thread.  Read-outs
+ * as in dgp_estimate_pose_stream_transform.  A failing writer aborts the call like a failing reader (DGP_ERR_INVALID). */
+int dgp_estimate_pose_stream_render(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                    const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                    int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                    int64_t* frames_done, const dgp_marker_style* style, dgp_frame_writer writer,
+                                    void* writer_user);
+
 /* ---- training step (fit_dgp, src/deepgraphpose/models/fitdgp.py:706-713 and :817-818) ----
  * Replaces sess.run([train_op, loss], feed_dict): dgp_train_forward_backward computes the loss and the gradients of
  * total_loss (visible_only = 1: total_loss_visible, fit_dgp_labeledonly fitdgp.py:416) w.r.t. every trainable variable
