@@ -74,6 +74,8 @@ class DgpMarkerStyle(C.Structure):
 FRAME_READER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_void_p))
 # writer(user, frames, n) -> < 0 aborts
 FRAME_WRITER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int)
+# packet writer(user, data, sizes, n) -> < 0 aborts
+PACKET_WRITER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int)
 
 
 # name -> (restype, argtypes); kept in one table so the CPU test-suite can check every exported symbol.
@@ -112,6 +114,11 @@ SIGNATURES = {
     "dgp_draw_markers": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, C.POINTER(DgpMarkerStyle), _vp]),
     "dgp_estimate_pose_stream_render": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f, C.c_int64,
                                              _vp, _vp, _vp, _i64p, C.POINTER(DgpMarkerStyle), _vp, _vp]),
+    "dgp_jpeg_capacity": (C.c_int64, [_i, _i]),
+    "dgp_encode_jpeg": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, C.c_int64, _vp, _vp, _vp]),
+    "dgp_estimate_pose_stream_render_jpeg": (_i, [_vp, _vp, _vp, _i, _i, C.POINTER(DgpFrameTransform), _i, _f, _f,
+                                                  C.c_int64, _vp, _vp, _vp, _i64p, C.POINTER(DgpMarkerStyle), _i, _vp,
+                                                  _vp]),
     "dgp_motion_blur_kernel": (_i, [_i, C.c_double, C.c_double, _vp]),
     "dgp_elastic_field": (_i, [_vp, _i, _i, C.c_double, C.c_double, C.c_uint64, _vp, _vp, _vp]),
     "dgp_augment": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, C.POINTER(DgpAugmentParams), _vp, C.c_double, _vp]),

@@ -765,8 +765,9 @@ int PoseStaging::reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W,
   return DGP_OK;
 }
 
-int PoseStaging::reserve_render(dgp_handle* h) {
+int PoseStaging::reserve_render(dgp_handle* h, bool jpeg) {
   if (!d2h_stream) CU_OK(h, create(&d2h_stream, cudaStreamNonBlocking));
+  if (jpeg && !packet_stream) CU_OK(h, create(&packet_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; ++i)
     if (!ev_drawn[i]) CU_OK(h, create(&ev_drawn[i], cudaEventDisableTiming));
   return DGP_OK;
@@ -802,10 +803,21 @@ int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_
     if ((rc = draw_markers_fused(h, frames[slot].get<uint8_t>(), n, j.H0, j.W0, mu.get<float>(), lik.get<float>(),
                                  *render->args, s)))
       return rc;
-    CU_OK(h, cudaEventRecord(ev_drawn[slot].get(), s));
-    CU_OK(h, cudaStreamWaitEvent(ds, ev_drawn[slot].get(), 0));
-    CU_OK(h, cudaMemcpyAsync(render->dst, frames[slot].get(), (size_t)j.H0 * j.W0 * 3 * n, cudaMemcpyDeviceToHost, ds));
-    CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), ds));
+    if (render->quality) {
+      // the encode is the last reader of the slot; only the packets' offsets | sizes go D2H here, the writer thread copies
+      // the packets themselves once it knows their total
+      if ((rc = encode_jpeg_impl(h, frames[slot].get<uint8_t>(), n, j.H0, j.W0, render->quality, render->packets,
+                                 render->packets_bytes, render->meta, render->meta + n, s)))
+        return rc;
+      CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), s));
+      CU_OK(h, cudaStreamWaitEvent(ds, ev_consumed[slot].get(), 0));
+      CU_OK(h, cudaMemcpyAsync(render->dst, render->meta, (size_t)2 * n * sizeof(int64_t), cudaMemcpyDeviceToHost, ds));
+    } else {
+      CU_OK(h, cudaEventRecord(ev_drawn[slot].get(), s));
+      CU_OK(h, cudaStreamWaitEvent(ds, ev_drawn[slot].get(), 0));
+      CU_OK(h, cudaMemcpyAsync(render->dst, frames[slot].get(), (size_t)j.H0 * j.W0 * 3 * n, cudaMemcpyDeviceToHost, ds));
+      CU_OK(h, cudaEventRecord(ev_consumed[slot].get(), ds));
+    }
     CU_OK(h, cudaLaunchHostFunc(ds, render->handoff, render->handoff_arg));
   }
   CU_OK(h, cudaMemcpyAsync(j.mu_host + (size_t)t0 * nj * 2, mu.get(), (size_t)n * nj * 2 * 4, cudaMemcpyDeviceToHost, s));

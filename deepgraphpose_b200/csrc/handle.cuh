@@ -125,13 +125,28 @@ int marker_args(dgp_handle* h, const dgp_marker_style* st, MarkerArgs* a);
 int draw_markers_fused(dgp_handle* h, uint8_t* frames, int N, int H, int W, const float* mu, const float* lik,
                        const MarkerArgs& a, cudaStream_t s);
 
+// Motion-JPEG (jpeg_kernels.cu): bytes of the header template (SOI .. SOS) and the largest frame side.
+constexpr int kJpegHeaderBytes = 629;
+constexpr int kJpegMaxDim = 16383;
+// dgp_jpeg_capacity (-1 for an invalid size)
+int64_t jpeg_capacity(int H, int W);
+// dgp_encode_jpeg without the device switch
+int encode_jpeg_impl(dgp_handle* h, const uint8_t* frames, int N, int H, int W, int quality, uint8_t* out, int64_t capacity,
+                     int64_t* offsets, int64_t* sizes, cudaStream_t s);
+
 // The rendering half of a dgp_estimate_pose_stream_render batch: markers drawn into the batch's source frames, the n real
-// frames copied to the pinned writer slot `dst`, then handoff(handoff_arg) on the D2H stream.
+// frames copied to the pinned writer slot `dst`, then handoff(handoff_arg) on the D2H stream.  With quality > 0
+// (dgp_estimate_pose_stream_render_jpeg) the frames are encoded into `packets` instead (offsets | sizes of the n frames at
+// `meta`), and only offsets | sizes go to `dst`; the writer thread copies the packets themselves.
 struct RenderBatch {
   const MarkerArgs* args;
   uint8_t* dst;
   cudaHostFn_t handoff;
   void* handoff_arg;
+  int quality;
+  uint8_t* packets;
+  int64_t packets_bytes;
+  int64_t* meta;
 };
 
 // estimate_pose staging: source frames double-buffered between the H2D of the copy stream and the compute stream (slot =
@@ -143,6 +158,8 @@ struct PoseStaging {
   // rendering: the annotated frames leave on their own stream so that their D2H overlaps the next batch's forward
   Stream d2h_stream;
   Event ev_drawn[2];
+  // Motion-JPEG rendering: the writer thread's copies of the encoded packets
+  Stream packet_stream;
   int reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W, bool identity);
   // Batch number `it` (n frames at host_frames, output rows [t0, t0 + n)): H2D, transform, forward + soft-argmax of run_n
   // rows, D2H of n read-outs.  release(release_arg) runs on the copy stream once host_frames has been copied.  With
@@ -150,8 +167,9 @@ struct PoseStaging {
   // copy.
   int run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
                 cudaHostFn_t release, void* release_arg, const RenderBatch* render = nullptr);
-  // the D2H stream and events of run_batch's `render` step (created at the first rendering call)
-  int reserve_render(dgp_handle* h);
+  // the D2H stream and events of run_batch's `render` step (created at the first rendering call), and with `jpeg` the
+  // packet stream
+  int reserve_render(dgp_handle* h, bool jpeg);
 };
 
 }  // namespace dgp
@@ -217,6 +235,14 @@ struct dgp_handle {
   PinnedBuf ring_slot[3];
   // dgp_estimate_pose_stream_render: pinned host ring of annotated frames the writer thread drains (stream.cu)
   PinnedBuf writer_slot[3];
+  // dgp_encode_jpeg: header template + Huffman codes per (H, W, quality), and the scratch of its launches (coefficients,
+  // block bit offsets, segment bit buffers, segment sizes / offsets)
+  std::map<std::tuple<int, int, int>, DevBuf> jpeg_tables;
+  DevBuf jpeg_coef, jpeg_bitoff, jpeg_raw, jpeg_seg;
+  // dgp_estimate_pose_stream_render_jpeg, per writer slot: device packets and their offsets | sizes, and the pinned copy of
+  // the packets (grown by the writer thread to what a batch needs)
+  DevBuf jpeg_packets[3], jpeg_meta[3];
+  PinnedBuf jpeg_host[3];
 };
 
 // loss forward (+ optional loss-side backward) shared by dgp_loss_forward / dgp_loss_backward / the training step

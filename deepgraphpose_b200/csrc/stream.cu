@@ -55,7 +55,9 @@ struct WriterRing {
   struct Ready { int slot; int n; };
   std::deque<Ready> ready;
   bool done = false;  // nothing more will be handed over
-  int error = 0;      // first negative return of the writer
+  int error = 0;      // first negative return of the writer, or DGP_ERR_CUDA when a slot's packets could not be fetched
+  cudaError_t cuda = cudaSuccess;  // the failed packet copy or pinned allocation
+  bool overflow = false;           // a JPEG frame above dgp_jpeg_capacity
 };
 
 struct HandoffArg {
@@ -73,11 +75,12 @@ void CUDART_CB handoff_slot(void* p) {
   a->ring->cv.notify_all();
 }
 
-// The body of dgp_estimate_pose_stream_transform; with a writer, also that of dgp_estimate_pose_stream_render.
+// The body of dgp_estimate_pose_stream_transform; with a writer, also that of dgp_estimate_pose_stream_render, and with a
+// packet writer that of dgp_estimate_pose_stream_render_jpeg.
 int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0, const dgp_frame_transform* transform,
                 int batch, float gamma, float gauss_len, int64_t max_frames, float* mu_host, int32_t* peak_host,
                 float* lik_host, int64_t* frames_done, const dgp_marker_style* style, dgp_frame_writer writer,
-                void* writer_user) {
+                void* writer_user, int quality = 0, dgp_packet_writer packet_writer = nullptr) {
   if (!h) return DGP_ERR_INVALID;
   if (frames_done) *frames_done = 0;
   if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_estimate_pose_stream before dgp_finalize_weights");
@@ -86,7 +89,11 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
   bool identity;
   if (transform_dims(H0, W0, transform, &H, &W, &identity))
     return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: invalid frame size or transform");
-  const bool render = writer != nullptr;
+  const bool jpeg = packet_writer != nullptr;
+  const bool render = writer != nullptr || jpeg;
+  if (jpeg && (quality < 1 || quality > 100 || jpeg_capacity(H0, W0) < 0))
+    return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render_jpeg: quality %d or a %dx%d frame outside the JPEG range",
+                quality, H0, W0);
   MarkerArgs marker;
   if (render) {
     int rc = marker_args(h, style, &marker);
@@ -99,11 +106,19 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
   const size_t frame_bytes = (size_t)H0 * W0 * 3;
   for (PinnedBuf& r : h->ring_slot)
     if (r.bytes() < frame_bytes * batch) CU_OK(h, r.alloc(frame_bytes * batch));
+  // a writer slot holds a batch's frames, or with JPEG the offsets | sizes of its packets
+  const size_t slot_bytes = jpeg ? 2 * sizeof(int64_t) * batch : frame_bytes * batch;
+  const int64_t packets_bytes = jpeg ? jpeg_capacity(H0, W0) * batch : 0;
   if (render) {
-    if ((rc = h->pose.reserve_render(h))) return rc;
+    if ((rc = h->pose.reserve_render(h, jpeg))) return rc;
     for (PinnedBuf& r : h->writer_slot)
-      if (r.bytes() < frame_bytes * batch) CU_OK(h, r.alloc(frame_bytes * batch));
+      if (r.bytes() < slot_bytes) CU_OK(h, r.alloc(slot_bytes));
   }
+  if (jpeg)
+    for (int i = 0; i < kSlots; ++i) {
+      if ((rc = ensure(h, &h->jpeg_packets[i], (size_t)packets_bytes))) return rc;
+      if ((rc = ensure(h, &h->jpeg_meta[i], 2 * sizeof(int64_t) * batch))) return rc;
+    }
   const PoseJob job = {H0, W0, H, W, identity, transform, gamma, gauss_len, mu_host, peak_host, lik_host};
 
   Ring ring;
@@ -158,8 +173,29 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
   uint8_t* wslots[kSlots];
   for (int i = 0; i < kSlots; ++i) wslots[i] = h->writer_slot[i].get<uint8_t>();
   std::thread writer_thread;
+  // JPEG: the packets of a slot are copied once their total is known (offsets | sizes have arrived in the writer slot)
+  auto fetch_packets = [h](WriterRing& wr, int slot, int n, const int64_t* meta) -> const uint8_t* {
+    for (int k = 0; k < n; ++k)
+      if (meta[n + k] < 0) {
+        wr.overflow = true;
+        return nullptr;
+      }
+    const size_t total = (size_t)(meta[n - 1] + meta[2 * n - 1]);
+    PinnedBuf& host = h->jpeg_host[slot];
+    cudaError_t e = cudaSuccess;
+    if (host.bytes() < total) e = host.alloc(total + total / 4);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync(host.get(), h->jpeg_packets[slot].get(), total, cudaMemcpyDeviceToHost, h->pose.packet_stream.get());
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->pose.packet_stream.get());
+    if (e != cudaSuccess) {
+      wr.cuda = e;
+      return nullptr;
+    }
+    return host.get<uint8_t>();
+  };
   if (render) {
-    writer_thread = std::thread([&wring, &wslots, writer, writer_user]() {
+    writer_thread = std::thread([&wring, &wslots, writer, writer_user, packet_writer, &fetch_packets, h]() {
+      if (packet_writer) cudaSetDevice(h->device);  // the pinned packet buffers belong to the handle's device
       for (;;) {
         WriterRing::Ready r;
         {
@@ -174,7 +210,14 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
             continue;
           }
         }
-        const int rc = writer(writer_user, wslots[r.slot], r.n);
+        int rc;
+        if (packet_writer) {
+          const int64_t* meta = reinterpret_cast<const int64_t*>(wslots[r.slot]);
+          const uint8_t* data = fetch_packets(wring, r.slot, r.n, meta);
+          rc = data ? packet_writer(writer_user, data, meta + r.n, r.n) : DGP_ERR_CUDA;
+        } else {
+          rc = writer(writer_user, wslots[r.slot], r.n);
+        }
         {
           std::lock_guard<std::mutex> lk(wring.mu);
           if (rc < 0 && !wring.error) wring.error = rc;
@@ -220,7 +263,8 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
         wring.slot_free[ws] = false;
       }
       hand[ws].n = f.n;
-      rb = {&marker, wslots[ws], handoff_slot, &hand[ws]};
+      rb = {&marker, wslots[ws], handoff_slot, &hand[ws], jpeg ? quality : 0, h->jpeg_packets[ws].get<uint8_t>(),
+            packets_bytes, h->jpeg_meta[ws].get<int64_t>()};
     }
     // the host slot is reusable once its frames have been copied
     if ((status = h->pose.run_batch(h, job, f.src, f.n, run_n, it, t0, release_slot, &rel[f.slot], render ? &rb : nullptr)))
@@ -252,6 +296,9 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
   if (e1 != cudaSuccess || e2 != cudaSuccess)
     return fail(h, DGP_ERR_CUDA, "dgp_estimate_pose_stream: %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
   if (ring.reader_error) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream: the frame reader failed (%d)", ring.reader_error);
+  if (wring.overflow) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render_jpeg: a frame exceeded dgp_jpeg_capacity");
+  if (wring.cuda != cudaSuccess)
+    return fail(h, DGP_ERR_CUDA, "dgp_estimate_pose_stream_render_jpeg: packet copy: %s", cudaGetErrorString(wring.cuda));
   if (wring.error) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render: the frame writer failed (%d)", wring.error);
   return DGP_OK;
 }
@@ -299,6 +346,17 @@ int dgp_estimate_pose_stream_render(dgp_handle* h, dgp_frame_reader reader, void
   if (!writer) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render: no frame writer");
   return stream_impl(h, reader, user, H0, W0, transform, batch, gamma, gauss_len, max_frames, mu_host, peak_host, lik_host,
                      frames_done, style, writer, writer_user);
+}
+
+int dgp_estimate_pose_stream_render_jpeg(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                         const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                         int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                         int64_t* frames_done, const dgp_marker_style* style, int quality,
+                                         dgp_packet_writer writer, void* writer_user) {
+  if (!h) return DGP_ERR_INVALID;
+  if (!writer) return fail(h, DGP_ERR_INVALID, "dgp_estimate_pose_stream_render_jpeg: no packet writer");
+  return stream_impl(h, reader, user, H0, W0, transform, batch, gamma, gauss_len, max_frames, mu_host, peak_host, lik_host,
+                     frames_done, style, nullptr, writer_user, quality, writer);
 }
 
 }  // extern "C"

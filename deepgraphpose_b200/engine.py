@@ -87,6 +87,21 @@ def marker_style(nj, dotsize=3, mask_threshold=0.1, colors=None, scale_x=1.0, sc
     return st, table
 
 
+def check_jpeg_quality(quality):
+    """``quality`` as an int in 1..100 (Pillow's JPEG quality); ValueError otherwise."""
+    if isinstance(quality, bool) or not isinstance(quality, (int, np.integer)) or not 1 <= int(quality) <= 100:
+        raise ValueError("quality must be an integer in [1, 100], got %r" % (quality,))
+    return int(quality)
+
+
+def jpeg_capacity(H, W):
+    """Bytes one (H, W) frame's JPEG file can take at most (dgp_jpeg_capacity); ValueError outside 1..16383."""
+    cap = _lib.load().dgp_jpeg_capacity(int(H), int(W))
+    if cap < 0:
+        raise ValueError("JPEG frames must be 1..16383 pixels on each side, got %dx%d" % (H, W))
+    return int(cap)
+
+
 def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3)):
     """Frames per batch that minimise wave quantisation of the persistent conv-GEMM grid (one CTA per SM).
 
@@ -447,6 +462,28 @@ class Engine:
                                               C.byref(st), _stream(frames_dev.device)))
         return frames_dev
 
+    def encode_jpeg(self, frames_dev, quality=90):
+        """The JPEG file of every frame of ``frames_dev`` (uint8 contiguous CUDA (N,H,W,3) RGB), encoded on the device
+        (dgp_encode_jpeg): exactly the bytes of ``PIL.Image.fromarray(frame).save(buf, format="JPEG", quality=quality,
+        subsampling=2, restart_marker_rows=1)``.  Returns a list of N ``bytes``; synchronises with the current stream."""
+        q = check_jpeg_quality(quality)
+        if frames_dev.dtype != torch.uint8 or frames_dev.dim() != 4 or frames_dev.shape[-1] != 3 or not frames_dev.is_cuda:
+            raise ValueError("frames must be a uint8 CUDA tensor of shape (N,H,W,3)")
+        frames_dev = frames_dev.contiguous()
+        N, H, W, _ = frames_dev.shape
+        cap = jpeg_capacity(H, W) * N
+        out = torch.empty(max(cap, 1), dtype=torch.uint8, device=frames_dev.device)
+        meta = torch.empty((2, max(N, 1)), dtype=torch.int64, device=frames_dev.device)
+        self._check(self.lib.dgp_encode_jpeg(self.h, _ptr(frames_dev), N, H, W, q, _ptr(out), cap, _ptr(meta[0]),
+                                             _ptr(meta[1]), _stream(frames_dev.device)))
+        if N == 0:
+            return []
+        offsets, sizes = meta.cpu().numpy()
+        if (sizes < 0).any():
+            raise DgpError(-1, "dgp_encode_jpeg: a frame exceeded dgp_jpeg_capacity")
+        data = out[:int(offsets[-1] + sizes[-1])].cpu().numpy()
+        return [data[o:o + n].tobytes() for o, n in zip(offsets, sizes)]
+
     def _frame_reader(self, source, H, W, T, start):
         """(reader, user, keep, state) of a stream source (see estimate_pose_stream); state["error"] holds an exception the
         source raised."""
@@ -518,14 +555,23 @@ class Engine:
         return mu[:n], peak[:n], lik[:n]
 
     def estimate_pose_render_stream(self, source, H, W, max_frames, writer, dotsize=3, mask_threshold=0.1, colors=None,
-                                    new_size=None, crop_size=None, batch=16, gamma=1.0, gauss_len=1.0, start=0):
+                                    new_size=None, crop_size=None, batch=16, gamma=1.0, gauss_len=1.0, start=0, encoder="raw",
+                                    quality=90):
         """estimate_pose_stream that renders plot_dgp's labelled video in the same pass (dgp_estimate_pose_stream_render):
         after each batch's soft-argmax the markers are drawn on the device into the batch's source frames (coordinates
         converted to video pixels as eval.estimate_pose does, scale W / new_size[1], H / new_size[0] under ``new_size``) and
         the annotated frames are handed to ``writer(frames)`` -- a uint8 (n,H,W,3) RGB array valid only during the call --
         from a writer thread, in video order.  An exception the writer raises aborts the pass and is re-raised here; a
         negative integer it returns aborts it with DgpError, as in the C ABI.
+        ``encoder="jpeg"`` (dgp_estimate_pose_stream_render_jpeg) encodes the annotated frames on the device instead, as
+        encode_jpeg does at ``quality``, and calls ``writer(data, sizes)``: a uint8 array holding the batch's JPEG files back
+        to back in video order and an int64 array of their sizes, both valid only during the call.
         Sources and return value as in estimate_pose_stream; style arguments as in draw_markers."""
+        if encoder not in ("raw", "jpeg"):
+            raise ValueError("encoder must be 'raw' or 'jpeg', got %r" % (encoder,))
+        q = check_jpeg_quality(quality)
+        if encoder == "jpeg":
+            jpeg_capacity(H, W)
         T = int(max_frames)
         transform_dims(H, W, new_size, crop_size)
         tf = frame_transform(new_size, crop_size)
@@ -548,11 +594,24 @@ class Engine:
                 werr["error"] = ex
                 return -1
 
-        wcb = _lib.FRAME_WRITER(_write)
-        status = self.lib.dgp_estimate_pose_stream_render(self.h, reader, user, int(H), int(W),
-                                                          C.byref(tf) if tf is not None else None, int(batch), float(gamma),
-                                                          float(gauss_len), T, _ptr(mu), _ptr(peak), _ptr(lik), C.byref(done),
-                                                          C.byref(st), C.cast(wcb, C.c_void_p), None)
+        def _write_packets(user_, data, sizes, n):
+            try:
+                sz = np.ctypeslib.as_array(C.cast(sizes, C.POINTER(C.c_int64)), shape=(n,))
+                buf = np.ctypeslib.as_array(C.cast(data, C.POINTER(C.c_uint8)), shape=(int(sz.sum()),))
+                rc = writer(buf, sz)
+                return int(rc) if isinstance(rc, (int, np.integer)) and rc < 0 else 0
+            except Exception as ex:  # never unwind through the C frame
+                werr["error"] = ex
+                return -1
+
+        args = (self.h, reader, user, int(H), int(W), C.byref(tf) if tf is not None else None, int(batch), float(gamma),
+                float(gauss_len), T, _ptr(mu), _ptr(peak), _ptr(lik), C.byref(done), C.byref(st))
+        if encoder == "jpeg":
+            wcb = _lib.PACKET_WRITER(_write_packets)
+            status = self.lib.dgp_estimate_pose_stream_render_jpeg(*args, q, C.cast(wcb, C.c_void_p), None)
+        else:
+            wcb = _lib.FRAME_WRITER(_write)
+            status = self.lib.dgp_estimate_pose_stream_render(*args, C.cast(wcb, C.c_void_p), None)
         for err in (state["error"], werr["error"]):
             if err is not None:
                 raise err

@@ -11,7 +11,8 @@ import numpy as np
 import torch
 
 from . import synthetic
-from .engine import Engine, marker_colors, marker_style  # noqa: F401  (marker_colors: eval's public name)
+from .engine import Engine, check_jpeg_quality, marker_colors, marker_style  # noqa: F401  (marker_colors: eval's public name)
+from .mp4 import MJPEGWriter
 from .session import Handle, Session
 
 
@@ -323,8 +324,23 @@ def _check_fourcc(fourcc):
         raise ValueError("fourcc must be a four-character code such as 'mp4v' or 'FFV1', got %r" % (fourcc,))
 
 
+def _check_encoder(encoder, fourcc, quality):
+    """'cv2' (cv2.VideoWriter with ``fourcc``) or 'jpeg' (Motion-JPEG encoded on the device at ``quality``)."""
+    if encoder == "cv2":
+        _check_fourcc(fourcc)
+    elif encoder == "jpeg":
+        check_jpeg_quality(quality)
+    else:
+        raise ValueError("encoder must be 'cv2' or 'jpeg', got %r" % (encoder,))
+
+
+def _mjpeg_writer(filename, fps, H, W):
+    os.makedirs(os.path.dirname(str(filename)) or ".", exist_ok=True)
+    return MJPEGWriter(str(filename), fps, W, H)
+
+
 def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colormap="cool", filename="movie.mp4", fps=None,
-                           fourcc="mp4v", batch=16, engine=None):
+                           fourcc="mp4v", batch=16, engine=None, encoder="cv2", quality=90):
     """plot_dgp's renderer (src/deepgraphpose/models/eval.py): a video of ``clip`` with joint j of frame t marked by a disc
     of radius ``dotsize`` at (``df_x[t, j]``, ``df_y[t, j]``) (video pixels) where ``mask_array[t, j]`` (None: every joint),
     coloured by ``colormap`` (the name 'cool' or an (nj, 3) uint8 RGB table) -- the drawing contract of dgp_draw_markers.
@@ -332,7 +348,9 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
     of ``batch`` (``engine``: an Engine with nj joints, else one is created for the call) and written with
     ``cv2.VideoWriter(filename, fourcc, fps)``; ``fps`` None = the video's own rate (required for an array).  Every frame
     the decoder yields is written, one label row per frame.  The reference writes ``int(duration * fps)`` frames with
-    moviepy (libx264) and draws with matplotlib / skimage on the host; bitstream and anti-aliasing parity are not goals."""
+    moviepy (libx264) and draws with matplotlib / skimage on the host; bitstream and anti-aliasing parity are not goals.
+    ``encoder="jpeg"`` encodes the drawn frames on the device instead (Engine.encode_jpeg at ``quality``) and writes them
+    to ``filename`` as Motion-JPEG (deepgraphpose_b200.mp4); ``fourcc`` is then unused."""
     x = np.asarray(df_x, dtype=np.float64)
     y = np.asarray(df_y, dtype=np.float64)
     if x.ndim != 2 or y.shape != x.shape:
@@ -342,7 +360,7 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
     if mask.shape != x.shape:
         raise ValueError("mask_array must be (T, nj) like df_x")
     marker_style(nj, dotsize, 0.5, colormap)  # validates dotsize and colours before any decode or device work
-    _check_fourcc(fourcc)
+    _check_encoder(encoder, fourcc, quality)
     if isinstance(clip, (str, os.PathLike)):
         if fps is None:
             import cv2
@@ -375,21 +393,27 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
                 raise ValueError("the clip has more frames than the %d label rows" % x.shape[0])
             host = torch.from_numpy(np.ascontiguousarray(np.stack(chunk)))
             if vw is None:
-                vw = _video_writer(filename, fourcc, fps, host.shape[1], host.shape[2])
+                vw = (_mjpeg_writer(filename, fps, host.shape[1], host.shape[2]) if encoder == "jpeg"
+                      else _video_writer(filename, fourcc, fps, host.shape[1], host.shape[2]))
             dev = host.to(eng.device)
             eng.draw_markers(dev, x[t0:t0 + n], y[t0:t0 + n], mask[t0:t0 + n], dotsize, 0.5, colormap)
-            _write_rgb(vw, dev.cpu().numpy())
+            if encoder == "jpeg":
+                for packet in eng.encode_jpeg(dev, quality):
+                    vw.write(packet)
+            else:
+                _write_rgb(vw, dev.cpu().numpy())
             t0 += n
     finally:
         if vw is not None:
-            vw.release()
+            vw.close() if encoder == "jpeg" else vw.release()
         if own:
             eng.close()
     return filename
 
 
 def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_model_file=None, shuffle=1, dotsize=3,
-             colormap="cool", save_str="", mask_threshold=0.1, new_size=None, crop_size=None, batch=16, fourcc="mp4v"):
+             colormap="cool", save_str="", mask_threshold=0.1, new_size=None, crop_size=None, batch=16, fourcc="mp4v",
+             encoder="cv2", quality=90):
     """plot_dgp (src/deepgraphpose/models/eval.py; step 3 of the reference demo): labels a video and renders the labelled
     movie ``<output_dir>/<video>_labeled<save_str>.mp4`` (cv2.VideoWriter with ``fourcc`` at the source fps) in which joint j
     is a disc of radius ``dotsize`` in ``colormap``'s colour j wherever its likelihood exceeds ``mask_threshold``.
@@ -404,10 +428,12 @@ def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_
     accepted for the reference's signature.  ``fourcc='FFV1'`` writes lossless video (used by the tests).  Every frame the
     decoder yields is written; the reference writes ``int(duration * fps)`` frames with moviepy.  The defaults are the
     reference's as recorded in this project (dotsize 3, 'cool', mask_threshold 0.1); they have not been checked against a
-    reference checkout.  Returns the movie's path."""
+    reference checkout.  Returns the movie's path.
+    ``encoder="jpeg"`` writes the same path as Motion-JPEG at ``quality`` (Pillow's JPEG quality), encoded on the device
+    in both branches, so that only the encoded bytes reach the host; the csv is the same."""
     if not isinstance(video_file, (str, os.PathLike)):
         raise ValueError("video_file must be a path")
-    _check_fourcc(fourcc)
+    _check_encoder(encoder, fourcc, quality)
     name = os.path.basename(str(video_file)).rsplit(".", 1)[0] + "_labeled%s" % save_str
     label_dir = output_dir if label_dir is None else label_dir
     movie = os.path.join(str(output_dir), name + ".mp4")
@@ -420,7 +446,8 @@ def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_
         labels = load_pose_from_dlc_to_dict(csv)
         marker_style(labels["x"].shape[1], dotsize, mask_threshold, colormap)
         return create_annotated_movie(video_file, labels["x"], labels["y"], labels["likelihoods"] > mask_threshold,
-                                      dotsize=dotsize, colormap=colormap, filename=movie, fourcc=fourcc, batch=batch)
+                                      dotsize=dotsize, colormap=colormap, filename=movie, fourcc=fourcc, batch=batch,
+                                      encoder=encoder, quality=quality)
     if dlc_cfg is None:
         raise ValueError("no labels at %s: proj_cfg_file and dgp_model_file are needed to estimate them" % csv)
     marker_style(int(_cfg_get(dlc_cfg, "num_joints")), dotsize, mask_threshold, colormap)
@@ -431,18 +458,24 @@ def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_
     source, H0, W0, _, scale_x, scale_y = _video_source(video_file, new_size)
     sess = _setup_eval_graph(dlc_cfg, dgp_model_file, None)[0]
     eng = sess.engine
-    vw = _video_writer(movie, fourcc, fps, H0, W0)
+    if encoder == "jpeg":
+        vw = _mjpeg_writer(movie, fps, H0, W0)
+        write, close = vw.write_packed, vw.close
+    else:
+        vw = _video_writer(movie, fourcc, fps, H0, W0)
+        write, close = (lambda fr: _write_rgb(vw, fr)), vw.release
     parts, chunk = [], 65536
     try:
         it = iter(source)
         while True:
-            mu, peak, lik = eng.estimate_pose_render_stream(it, H0, W0, chunk, lambda fr: _write_rgb(vw, fr), dotsize,
-                                                            mask_threshold, colormap, new_size, crop_size, batch)
+            mu, peak, lik = eng.estimate_pose_render_stream(it, H0, W0, chunk, write, dotsize, mask_threshold, colormap,
+                                                            new_size, crop_size, batch,
+                                                            encoder="raw" if encoder == "cv2" else "jpeg", quality=quality)
             parts.append((mu, peak, lik))
             if mu.shape[0] < chunk:
                 break
     finally:
-        vw.release()
+        close()
         sess.close()
     res = _readout_dict(*(torch.cat([p[i] for p in parts]) for i in range(3)), eng.stride)
     labels = {"x": res["x"] * scale_x, "y": res["y"] * scale_y, "likelihoods": res["likelihoods"]}

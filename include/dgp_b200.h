@@ -378,6 +378,35 @@ int dgp_estimate_pose_stream_render(dgp_handle* h, dgp_frame_reader reader, void
                                     int64_t* frames_done, const dgp_marker_style* style, dgp_frame_writer writer,
                                     void* writer_user);
 
+/* ---- Motion-JPEG of the labelled video ----
+ * Each uint8 (H,W,3) RGB frame becomes exactly the bytes of Pillow's (libjpeg-turbo's)
+ *   Image.fromarray(frame).save(buf, format="JPEG", quality=quality, subsampling=2, restart_marker_rows=1)
+ * for 1 <= H, W <= 16383 and quality 1..100: baseline JPEG, JFIF 1.01 APP0, the Annex K quantisation tables scaled by
+ * libjpeg's quality rule, 4:2:0 (Y 2x2, Cb / Cr 1x1), the Annex K Huffman tables, one restart interval per MCU row (RST0..7
+ * between rows).  The contract, down to the fixed-point colour conversion and the islow DCT, is in DESIGN.md §4.5. */
+/* Bytes one frame's file can take at most (the header, 64 x (16 + 11) bits per 8x8 block doubled for 0xFF stuffing, the
+ * markers); -1 for a size outside 1..16383. */
+int64_t dgp_jpeg_capacity(int H, int W);
+/* Encodes N frames of frames_dev (device (N,H,W,3)) into out_dev (device, `capacity` >= N * dgp_jpeg_capacity(H, W) bytes):
+ * the files are packed in frame order, frame i at out_dev + offsets_dev[i] with sizes_dev[i] bytes (device int64 (N)).  A
+ * frame's bytes do not depend on N or on its position.  A frame that would exceed its bound (never, for valid input) gets
+ * size -1 and is not written.  Asynchronous on `stream`; scratch and the (H, W, quality) header template are kept on the
+ * handle, so calls on one handle are ordered on one stream. */
+int dgp_encode_jpeg(dgp_handle* h, const uint8_t* frames_dev, int N, int H, int W, int quality, uint8_t* out_dev,
+                    int64_t capacity, int64_t* offsets_dev, int64_t* sizes_dev, void* stream);
+/* writer(user, data, sizes, n): the JPEG files of n frames, packed back to back in video order at `data` (frame i has
+ * sizes[i] bytes), valid only during the call; return < 0 to abort.  Called from a thread owned by the call, never
+ * concurrently. */
+typedef int (*dgp_packet_writer)(void* user, const uint8_t* data, const int64_t* sizes, int n);
+/* dgp_estimate_pose_stream_render whose annotated frames are encoded on the device (dgp_encode_jpeg at `quality`) right
+ * after the markers are drawn: only the encoded bytes cross to the host, into a ring of 3 pinned writer slots that a writer
+ * thread hands to `writer`.  Read-outs, markers and failure handling as in dgp_estimate_pose_stream_render. */
+int dgp_estimate_pose_stream_render_jpeg(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
+                                         const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
+                                         int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
+                                         int64_t* frames_done, const dgp_marker_style* style, int quality,
+                                         dgp_packet_writer writer, void* writer_user);
+
 /* ---- training step (fit_dgp, src/deepgraphpose/models/fitdgp.py:706-713 and :817-818) ----
  * Replaces sess.run([train_op, loss], feed_dict): dgp_train_forward_backward computes the loss and the gradients of
  * total_loss (visible_only = 1: total_loss_visible, fit_dgp_labeledonly fitdgp.py:416) w.r.t. every trainable variable
