@@ -88,6 +88,9 @@ SIGNATURES = {
     "dgp_finalize_weights": (_i, [_vp]),
     "dgp_net_depth": (_i, [_vp, C.POINTER(_i)]),
     "dgp_output_dims": (_i, [_i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
+    "dgp_output_dims_os": (_i, [_i, _i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
+    "dgp_set_output_stride": (_i, [_vp, _i]),
+    "dgp_get_output_stride": (_i, [_vp, C.POINTER(_i)]),
     "dgp_forward": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "dgp_extract_features": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "dgp_prediction_layers": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),

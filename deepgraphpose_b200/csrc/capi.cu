@@ -747,7 +747,7 @@ int ensure(dgp_handle* h, DevBuf* b, size_t bytes) {
 int PoseStaging::reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W, bool identity) {
   const int nj = h->cfg.num_joints;
   int hf, wf, ho, wo;
-  dgp_output_dims(H, W, &hf, &wf, &ho, &wo);
+  dgp_output_dims_os(H, W, h->output_stride, &hf, &wf, &ho, &wo);
   const size_t frame_bytes = (size_t)H0 * W0 * 3;
   int rc;
   if ((rc = ensure(h, &frames[0], frame_bytes * batch))) return rc;
@@ -777,7 +777,7 @@ int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_
                            cudaHostFn_t release, void* release_arg, const RenderBatch* render) {
   const int nj = h->cfg.num_joints;
   int hf, wf, ho, wo;
-  dgp_output_dims(j.H, j.W, &hf, &wf, &ho, &wo);
+  dgp_output_dims_os(j.H, j.W, h->output_stride, &hf, &wf, &ho, &wo);
   cudaStream_t s = h->stream.get(), cs = copy_stream.get();
   const int slot = it & 1;
   // H2D of this batch on the copy stream, as soon as the batch that last used this slot has been consumed
@@ -919,11 +919,12 @@ int dgp_finalize_weights(dgp_handle* h) {
   h->net_scope = scope;
   int rc = build_conv1_layer(h);
   if (rc) return rc;
-  // slim resnet_v1_<depth> + stack_blocks_dense(output_stride=16): see oracle/resnet_v1.py::unit_plan
+  // slim resnet_v1_<depth> + stack_blocks_dense(output_stride): see oracle/resnet_v1.py::unit_plan.  The root block has
+  // stride 4; once the units reach output_stride / 4, every later unit runs at stride 1 and its rate takes the stride over.
   static const struct { const char* name; int base, stride; } blocks[4] = {
       {"block1", 64, 2}, {"block2", 128, 2}, {"block3", 256, 2}, {"block4", 512, 1}};
   int cin = 64, current_stride = 1, rate = 1;
-  const int target = 4;
+  const int target = h->output_stride / 4;
   for (int bi = 0; bi < 4; ++bi) {
     const auto& b = blocks[bi];
     for (int u = 0; u < units[bi]; ++u) {
@@ -959,10 +960,31 @@ int dgp_net_depth(const dgp_handle* h, int* depth) {
   return DGP_OK;
 }
 
+int dgp_set_output_stride(dgp_handle* h, int output_stride) {
+  if (!h) return DGP_ERR_INVALID;
+  if (output_stride != 8 && output_stride != 16)
+    return fail(h, DGP_ERR_UNSUPPORTED, "dgp_set_output_stride: output_stride must be 8 or 16, got %d", output_stride);
+  if (h->finalized) return fail(h, DGP_ERR_STATE, "dgp_set_output_stride after dgp_finalize_weights");
+  h->output_stride = output_stride;
+  return DGP_OK;
+}
+
+int dgp_get_output_stride(const dgp_handle* h, int* output_stride) {
+  if (!h || !output_stride) return DGP_ERR_INVALID;
+  *output_stride = h->output_stride;
+  return DGP_OK;
+}
+
 int dgp_output_dims(int H, int W, int* h_feat, int* w_feat, int* h_out, int* w_out) {
-  if (H < 1 || W < 1) return DGP_ERR_INVALID;
+  return dgp_output_dims_os(H, W, 16, h_feat, w_feat, h_out, w_out);
+}
+
+int dgp_output_dims_os(int H, int W, int output_stride, int* h_feat, int* w_feat, int* h_out, int* w_out) {
+  if (H < 1 || W < 1 || (output_stride != 8 && output_stride != 16)) return DGP_ERR_INVALID;
+  // every stride-2 layer (conv1, pool1 and the last unit of each block before output_stride is reached) is SAME: ceil(v / 2)
+  const int halvings = output_stride == 16 ? 4 : 3;
   int a = H, b = W;
-  for (int i = 0; i < 4; ++i) { a = (a + 1) / 2; b = (b + 1) / 2; }
+  for (int i = 0; i < halvings; ++i) { a = (a + 1) / 2; b = (b + 1) / 2; }
   if (h_feat) *h_feat = a;
   if (w_feat) *w_feat = b;
   if (h_out) *h_out = 2 * a;

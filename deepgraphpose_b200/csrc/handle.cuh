@@ -186,6 +186,7 @@ struct dgp_handle {
   std::map<std::string, HostVar> host_vars;
   bool finalized = false;
   int depth = 0;             // 50, 101 or 152: slim resnet_v1_<depth>, read from the variable names at finalize
+  int output_stride = 16;    // 8 or 16: slim's output_stride (dgp_set_output_stride, before finalize)
   std::string net_scope;     // "resnet_v1_<depth>": prefix of every backbone variable and end point
   std::vector<ConvLayer> layers;
   int conv1_layer = -1, head_layer = -1;

@@ -16,11 +16,24 @@ STRIDE = 8.0                             # PTF/default_config.py:18
 LOCREF_STDEV = 7.2801                    # PTF/default_config.py:29
 
 
-def output_dims(H, W):
-    """(h_feat, w_feat), (h_out, w_out) -- closed form of Dataset._compute_pred_dims (dataset.py:348-371)."""
+OUTPUT_STRIDES = (8, 16)                 # slim resnet_v1 output_stride values of the B200 path (pose_net.py:31-34)
+
+
+def check_output_stride(output_stride):
+    """``output_stride`` as an int in OUTPUT_STRIDES; ValueError otherwise."""
+    if isinstance(output_stride, bool) or not isinstance(output_stride, (int, np.integer, float)) \
+            or output_stride not in OUTPUT_STRIDES:
+        raise ValueError("output_stride must be 8 or 16, got %r" % (output_stride,))
+    return int(output_stride)
+
+
+def output_dims(H, W, output_stride=16):
+    """(h_feat, w_feat), (h_out, w_out) -- closed form of Dataset._compute_pred_dims (dataset.py:348-371) for a backbone at
+    ``output_stride`` 8 or 16."""
     lib = _lib.load()
     a, b, c, d = C.c_int(), C.c_int(), C.c_int(), C.c_int()
-    check(lib.dgp_output_dims(int(H), int(W), C.byref(a), C.byref(b), C.byref(c), C.byref(d)))
+    check(lib.dgp_output_dims_os(int(H), int(W), check_output_stride(output_stride), C.byref(a), C.byref(b), C.byref(c),
+                                 C.byref(d)))
     return (a.value, b.value), (c.value, d.value)
 
 
@@ -102,13 +115,14 @@ def jpeg_capacity(H, W):
     return int(cap)
 
 
-def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3)):
+def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3), output_stride=16):
     """Frames per batch that minimise wave quantisation of the persistent conv-GEMM grid (one CTA per SM).
 
     Every GEMM layer runs ceil(B*pixels/tile_rows) * n_blocks tiles on `num_sms` CTAs; a batch size for which the
     dominant layers' tile counts are (just under) a multiple of the SM count avoids a nearly empty last wave.  Layers are
     weighted by their roofline bound (max of bf16 tensor time and HBM time), tile shapes follow csrc/capi.cu.  ``units``: the
-    bottleneck units per block of the backbone (ResNet-50 by default; synthetic.BLOCK_UNITS for the others)."""
+    bottleneck units per block of the backbone (ResNet-50 by default; synthetic.BLOCK_UNITS for the others).  At
+    ``output_stride`` 8 block 2 keeps its resolution (stride as executed: (2, 1, 1, 1))."""
     c2 = lambda v: -(-v // 2)
     layers = []  # (pixels per frame, tile rows, n_blocks, weight)
     hh, ww = c2(H), c2(W)
@@ -120,7 +134,8 @@ def suggest_batch(H, W, lo=24, hi=48, num_sms=148, units=(3, 4, 6, 3)):
     add(hh * ww, 256, 64, 32 + 128)
     hh, ww = c2(hh), c2(ww)
     cin = 64
-    for base, n_units, bstride in zip((64, 128, 256, 512), units, (2, 2, 1, 1)):
+    strides = (2, 2, 1, 1) if check_output_stride(output_stride) == 16 else (2, 1, 1, 1)
+    for base, n_units, bstride in zip((64, 128, 256, 512), units, strides):
         for u in range(n_units):
             s_ = bstride if u == n_units - 1 else 1
             depth = 4 * base
@@ -165,8 +180,14 @@ def _stream(device):
 
 
 class Engine:
-    def __init__(self, num_joints, location_refinement=True, device=None, stride=STRIDE, locref_stdev=LOCREF_STDEV,
-                 mean_pixel=MEAN_PIXEL, precision="fp16"):
+    def __init__(self, num_joints, location_refinement=True, device=None, stride=None, locref_stdev=LOCREF_STDEV,
+                 mean_pixel=MEAN_PIXEL, precision="fp16", output_stride=16):
+        """``output_stride``: slim's output_stride of the backbone, 8 or 16 (pose_cfg.yaml ``output_stride``).  At 8 the
+        scoremaps have twice the resolution on each axis.  ``stride``: input pixels per scoremap pixel (pose_cfg.yaml
+        ``stride``); None = output_stride / 2, the value DLC's configs pair with it (8.0 at 16, 4.0 at 8)."""
+        output_stride = check_output_stride(output_stride)
+        if stride is None:
+            stride = output_stride / 2.0
         if not torch.cuda.is_available():
             raise DgpError(-2, "no CUDA device: deepgraphpose_b200 has no CPU fallback")
         self.lib = _lib.load()
@@ -193,6 +214,8 @@ class Engine:
         h = C.c_void_p()
         check(self.lib.dgp_create(C.byref(cfg), C.byref(h)))
         self.h = h
+        self._check(self.lib.dgp_set_output_stride(self.h, output_stride))
+        self.output_stride = output_stride
         self.weights_loaded = False
         self.net_type = None  # "resnet_50" / "resnet_101" / "resnet_152": the backbone the loaded weights name
 
@@ -226,6 +249,10 @@ class Engine:
         self._frozen = {k: np.array(v, dtype=np.float32) for k, v in variables.items()
                         if k.endswith("/moving_mean") or k.endswith("/moving_variance")}
 
+    def output_dims(self, H, W):
+        """(h_feat, w_feat), (h_out, w_out) of an H x W frame through this engine's backbone (its output_stride)."""
+        return output_dims(H, W, self.output_stride)
+
     # ------------------------------------------------------------------ forward
     def forward(self, frames, want_locref=None):
         """frames: uint8 cuda tensor (B,H,W,3). Returns (logits (B,2h,2w,nj) f32, locref (B,2h,2w,2nj) f32 | None)."""
@@ -233,7 +260,7 @@ class Engine:
             raise ValueError("frames must be a uint8 CUDA tensor of shape (B,H,W,3)")
         frames = frames.contiguous()
         B, H, W, _ = frames.shape
-        _, (ho, wo) = output_dims(H, W)
+        _, (ho, wo) = self.output_dims(H, W)
         if want_locref is None:
             want_locref = self.location_refinement
         logits = torch.empty((B, ho, wo, self.nj), dtype=torch.float32, device=frames.device)
@@ -247,7 +274,7 @@ class Engine:
             raise ValueError("frames must be a uint8 CUDA tensor of shape (B,H,W,3)")
         frames = frames.contiguous()
         B, H, W, _ = frames.shape
-        (hf, wf), _ = output_dims(H, W)
+        (hf, wf), _ = self.output_dims(H, W)
         net = torch.empty((B, hf, wf, 2048), dtype=torch.float32, device=frames.device)
         self._check(self.lib.dgp_extract_features(self.h, _ptr(frames), B, H, W, _ptr(net), _stream(frames.device)))
         return net
@@ -660,7 +687,7 @@ class Engine:
         self.train_enable()
         frames = frames.contiguous()
         B, H, W, _ = frames.shape
-        _, (ho, wo) = output_dims(H, W)
+        _, (ho, wo) = self.output_dims(H, W)
         if want_locref is None:
             want_locref = self.location_refinement
         logits = torch.empty((B, ho, wo, self.nj), dtype=torch.float32, device=frames.device)
@@ -714,7 +741,7 @@ class Engine:
         """Views of the head outputs (logits, locref) the last training step at this input shape produced."""
         a, b = C.c_void_p(), C.c_void_p()
         self._check(self.lib.dgp_train_outputs(self.h, int(nt), int(H), int(W), C.byref(a), C.byref(b)))
-        _, (ho, wo) = output_dims(H, W)
+        _, (ho, wo) = self.output_dims(H, W)
         logits = _device_view(a.value, (nt, ho, wo, self.nj), "<f4", self.device)
         locref = _device_view(b.value, (nt, ho, wo, 2 * self.nj), "<f4", self.device) if b.value else None
         return logits, locref

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from . import synthetic
-from .engine import Engine, check_jpeg_quality, marker_colors, marker_style  # noqa: F401  (marker_colors: eval's public name)
+from .engine import OUTPUT_STRIDES, STRIDE, Engine, check_jpeg_quality, marker_colors, marker_style  # noqa: F401  (marker_colors: eval's public name)
 from .mp4 import MJPEGWriter
 from .session import Handle, Session
 
@@ -56,6 +56,22 @@ def check_net_type(net_type, variables):
     return found
 
 
+def check_geometry(cfg):
+    """(output_stride, stride) of a dlc_cfg / pose_cfg (pose_cfg.yaml keys ``output_stride``, default 16, ``stride``,
+    default 8.0, and ``deconvolutionstride``, default 2; pose_net.py:31-34).  ValueError for an output_stride other than 8 or
+    16, a deconvolutionstride other than 2, or output_stride 8 with a stride other than 4.0: DLC cannot have trained such a
+    model (its targets and predictions disagree in shape), and reading it out would put every joint at twice its distance."""
+    output_stride = _cfg_get(cfg, "output_stride", 16)
+    if isinstance(output_stride, bool) or output_stride not in OUTPUT_STRIDES:
+        raise ValueError("the B200 path implements output_stride 8 or 16 (pose_net.py:31-34), got %r" % (output_stride,))
+    if _cfg_get(cfg, "deconvolutionstride", 2) != 2:
+        raise ValueError("the B200 path implements deconvolutionstride=2 (pose_net.py:31-34)")
+    stride = float(_cfg_get(cfg, "stride", STRIDE))
+    if output_stride == 8 and stride != 4.0:
+        raise ValueError("output_stride 8 makes scoremaps of stride 4.0, but the config's stride is %r" % (stride,))
+    return int(output_stride), stride
+
+
 def setup_dgp_eval_graph(dlc_cfg, dgp_model_file, loc_ref=False, gauss_len=1, gamma=1, device=None):
     """eval.py:147-214.  Returns (sess, mu_n, softmax_tensor, scmap, locref, inputs).  ``dlc_cfg.net_type`` (resnet_50,
     resnet_101 or resnet_152) must match the backbone the weights name; without it the weights decide."""
@@ -63,14 +79,14 @@ def setup_dgp_eval_graph(dlc_cfg, dgp_model_file, loc_ref=False, gauss_len=1, ga
 
 
 def _setup_eval_graph(dlc_cfg, dgp_model_file, net_type, loc_ref=False, gauss_len=1, gamma=1, device=None):
+    output_stride, stride = check_geometry(dlc_cfg)
     nj = int(_cfg_get(dlc_cfg, "num_joints"))
     variables = load_variables(dgp_model_file, nj, bool(loc_ref), net_type or "resnet_50")
     check_net_type(net_type, variables)
-    eng = Engine(nj, location_refinement=bool(loc_ref), device=device,
-                 stride=float(_cfg_get(dlc_cfg, "stride", 8.0)),
+    eng = Engine(nj, location_refinement=bool(loc_ref), device=device, stride=stride,
                  locref_stdev=float(_cfg_get(dlc_cfg, "locref_stdev", 7.2801)),
                  mean_pixel=tuple(_cfg_get(dlc_cfg, "mean_pixel", (123.68, 116.779, 103.939))),
-                 precision=_cfg_get(dlc_cfg, "precision", "fp16"))
+                 precision=_cfg_get(dlc_cfg, "precision", "fp16"), output_stride=output_stride)
     eng.load_weights(variables)
     handles = {
         "inputs": Handle("Placeholder:0", "inputs"),

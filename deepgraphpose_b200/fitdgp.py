@@ -186,11 +186,13 @@ class _DgpLossFunction(torch.autograd.Function):
 
 
 def _loss_engine(dev, nj, cfg):
-    """A weight-less handle that runs the loss kernels, one per (device, joints, stride, locref_stdev)."""
-    key = (str(dev), int(nj), float(_get(cfg, "stride", 8.0)), float(_get(cfg, "locref_stdev", 7.2801)))
+    """A weight-less handle that runs the loss kernels, one per (device, joints, stride, locref_stdev, output_stride)."""
+    from .eval import check_geometry
+    output_stride, stride = check_geometry(cfg)
+    key = (str(dev), int(nj), stride, float(_get(cfg, "locref_stdev", 7.2801)), output_stride)
     eng = _LOSS_ENGINES.get(key)
     if eng is None:
-        eng = _LOSS_ENGINES[key] = Engine(nj, device=dev, stride=key[2], locref_stdev=key[3])
+        eng = _LOSS_ENGINES[key] = Engine(nj, device=dev, stride=key[2], locref_stdev=key[3], output_stride=output_stride)
     return eng
 
 
@@ -218,10 +220,9 @@ def train_forward_backward(engine, frames, feed, cfg, edges, ws, ws_max, n_frame
     """Forward + loss + full backward of one fit_dgp batch (fitdgp.py:817-818 without the apply step): fills the
     engine's gradient buffer.  frames: uint8 CUDA tensor (nt,H,W,3).  Returns the loss dict (or the device tensor of the 6
     loss values when sync=False)."""
-    from .engine import output_dims
     dev = frames.device
     nt, Hin, Win, _ = frames.shape
-    _, (H, W) = output_dims(Hin, Win)
+    _, (H, W) = engine.output_dims(Hin, Win)
     engine.train_enable()
     c, b, keep = _loss_args(dev, feed, cfg, edges, ws, ws_max, n_frames_total, n_visible_frames_total, nt, H, W, engine.nj,
                             with_locref=engine.location_refinement, engine=engine)
@@ -245,7 +246,8 @@ def dgp_loss(data_batcher, dgp_cfg, variables=None, device=None):
     ``{tf_var_name: ndarray}`` dict, an ``.npz``, a TensorFlow checkpoint prefix, or ``'synthetic[:seed]'`` spelled out) or,
     when that is None, from ``dgp_cfg.init_weights`` -- the snapshot the reference would restore.  There is no default: a
     drop-in call never trains from random weights silently."""
-    from .eval import load_variables
+    from .eval import check_geometry, load_variables
+    output_stride, stride = check_geometry(dgp_cfg)
     S0 = np.asarray(data_batcher.S0)
     nj = int(data_batcher.nj)
     gm2, gm3 = int(_get(dgp_cfg, "gm2", 1)), int(_get(dgp_cfg, "gm3", 3))
@@ -259,13 +261,12 @@ def dgp_loss(data_batcher, dgp_cfg, variables=None, device=None):
         if variables is None:
             raise ValueError("dgp_loss needs the network variables: pass variables=... or set dgp_cfg.init_weights to the "
                              "snapshot fit_dgp would restore (fitdgp.py:592, 720)")
-    stride = float(_get(dgp_cfg, "stride", 8.0))
     ws, ws_max = spatial_clique_params([d.labels for d in data_batcher.datasets], S0, stride,
                                        float(_get(dgp_cfg, "ws", 1000.0)), float(_get(dgp_cfg, "ws_max", 1.2)))
     eng = Engine(nj, location_refinement=True, device=device, stride=stride,
                  locref_stdev=float(_get(dgp_cfg, "locref_stdev", 7.2801)),
                  mean_pixel=tuple(_get(dgp_cfg, "mean_pixel", (123.68, 116.779, 103.939))),
-                 precision=_get(dgp_cfg, "precision", "fp16"))
+                 precision=_get(dgp_cfg, "precision", "fp16"), output_stride=output_stride)
     eng.load_weights(load_variables(variables, nj, True, _get(dgp_cfg, "net_type", "resnet_50")))
     graph = SimpleNamespace(engine=eng, cfg=dgp_cfg, edges=skeleton_edges(S0) if S0.shape[0] else [], ws=ws, ws_max=ws_max,
                             n_frames_total=float(data_batcher.n_frames_total),

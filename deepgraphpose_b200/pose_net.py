@@ -13,8 +13,8 @@ import numpy as np
 import torch
 
 from . import synthetic
-from .engine import Engine, LOCREF_STDEV, MEAN_PIXEL, STRIDE, _ptr, _stream
-from .eval import check_net_type
+from .engine import Engine, LOCREF_STDEV, MEAN_PIXEL, _ptr, _stream
+from .eval import check_geometry, check_net_type
 
 
 def _get(cfg, key, default=None):
@@ -54,19 +54,19 @@ def prediction_layer(cfg, input, name, num_outputs, engine=None):
 
 class PoseNet:
     def __init__(self, cfg, variables=None, device=None):
-        """pose_net.py:28-34 (defaults output_stride=16, deconvolutionstride=2 are the only supported values)."""
+        """pose_net.py:28-34: output_stride 8 or 16 (the default), deconvolutionstride 2; at output_stride 8 the cfg's
+        stride must be 4.0 (eval.check_geometry)."""
         self.cfg = cfg
-        if _get(cfg, "output_stride", 16) != 16 or _get(cfg, "deconvolutionstride", 2) != 2:
-            raise ValueError("the B200 path implements output_stride=16, deconvolutionstride=2 (pose_net.py:31-34)")
+        output_stride, stride = check_geometry(cfg)
         self.net_type = _get(cfg, "net_type", "resnet_50")
         synthetic.net_scope(self.net_type)   # resnet_50, resnet_101 or resnet_152 (pose_net.py:14-16)
         if _get(cfg, "intermediate_supervision", False):
             raise ValueError("intermediate_supervision is not on the B200 path (DGP never enables it)")
         self.num_joints = int(_get(cfg, "num_joints"))
         self.location_refinement = bool(_get(cfg, "location_refinement", True))
-        self.engine = Engine(self.num_joints, self.location_refinement, device,
-                             float(_get(cfg, "stride", STRIDE)), float(_get(cfg, "locref_stdev", LOCREF_STDEV)),
-                             tuple(_get(cfg, "mean_pixel", MEAN_PIXEL)), _get(cfg, "precision", "fp16"))
+        self.engine = Engine(self.num_joints, self.location_refinement, device, stride,
+                             float(_get(cfg, "locref_stdev", LOCREF_STDEV)), tuple(_get(cfg, "mean_pixel", MEAN_PIXEL)),
+                             _get(cfg, "precision", "fp16"), output_stride)
         if variables is not None:
             self.restore(variables)
 

@@ -73,8 +73,18 @@ int dgp_finalize_weights(dgp_handle* h);
 /* Depth of the backbone built by dgp_finalize_weights: 50, 101 or 152. */
 int dgp_net_depth(const dgp_handle* h, int* depth);
 
-/* Closed form of Dataset._compute_pred_dims (src/deepgraphpose/dataset.py:348-371). */
+/* slim's output_stride of the backbone (pose_cfg.yaml `output_stride`, pose_net.py:31-34): 8 or 16 (the default), set
+ * before dgp_finalize_weights.  At 8, block 2 runs at stride 1, block 3 at rate 2 and block 4 at rate 4 (slim
+ * stack_blocks_dense), so features and scoremaps have twice the resolution on each axis; pose_cfg's `stride` is then 4.0.
+ * The weights are the same variables at either stride.  Other values are DGP_ERR_UNSUPPORTED; a call after
+ * dgp_finalize_weights is DGP_ERR_STATE. */
+int dgp_set_output_stride(dgp_handle* h, int output_stride);
+int dgp_get_output_stride(const dgp_handle* h, int* output_stride);
+
+/* Closed form of Dataset._compute_pred_dims (src/deepgraphpose/dataset.py:348-371) at output_stride 16. */
 int dgp_output_dims(int H, int W, int* h_feat, int* w_feat, int* h_out, int* w_out);
+/* The same at output_stride 8 or 16: h_feat = ceil(H / output_stride) by repeated SAME halving, h_out = 2 * h_feat. */
+int dgp_output_dims_os(int H, int W, int output_stride, int* h_feat, int* w_feat, int* h_out, int* w_out);
 
 /* Replaces sess.run([scmap(, locref)], {inputs: frames}) (eval.py:328, 746): PoseNet.extract_features
  * (pose_net.py:36-54: mean subtraction + slim resnet_v1_<depth> OS16, frozen BN) and the 3x3 stride-2 deconv heads

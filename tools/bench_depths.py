@@ -26,15 +26,16 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 import bench  # noqa: E402
 
 
-def conv_flops_per_frame(h, w, nj, units, locref=False):
+def conv_flops_per_frame(h, w, nj, units, locref=False, output_stride=16):
     """bench.conv_flops_per_frame with the units per block of the backbone: algorithmic forward FLOPs (2*MACs) of the convs
-    and the deconv heads at output stride 16."""
+    and the deconv heads at output stride 16, or 8 (block 2 keeps its resolution; atrous convs cost what dense ones do)."""
     c2 = lambda v: -(-v // 2)
     hh, ww = c2(h), c2(w)
     total = 2 * hh * ww * 147 * 64
     hh, ww = c2(hh), c2(ww)
     cin = 64
-    for base, n_units, bstride in zip((64, 128, 256, 512), units, (2, 2, 1, 1)):  # stride as executed at output_stride 16
+    strides = (2, 2, 1, 1) if output_stride == 16 else (2, 1, 1, 1)   # stride of each block as executed
+    for base, n_units, bstride in zip((64, 128, 256, 512), units, strides):
         for u in range(n_units):
             s = bstride if u == n_units - 1 else 1
             depth = 4 * base

@@ -52,9 +52,10 @@ def cpu_train_step_seconds(nt, H, W, NJ):
 
 
 def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=True, precision="fp16", wt=1.0,
-            net_type="resnet_50"):
+            net_type="resnet_50", output_stride=16):
     """One data-parallel training benchmark on the already-initialised process group; returns the JSON dict (rank 0) or None.
-    ``net_type`` picks the backbone of the synthetic weights (the FLOP figures of the line are ResNet-50's)."""
+    ``net_type`` picks the backbone of the synthetic weights (the FLOP figures of the line are ResNet-50's at output stride
+    16); ``output_stride`` 8 trains on stride-4 scoremaps of twice the resolution."""
     import argparse as _a
     args = _a.Namespace(steps=steps, warmup=warmup, nt=nt, height=height, width=width)
     import torch.distributed as dist
@@ -63,7 +64,8 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     H, W, NJ, nt = args.height, args.width, bench.NJ, args.nt
-    _, (hs, ws_) = output_dims(H, W)
+    _, (hs, ws_) = output_dims(H, W, output_stride)
+    stride = output_stride / 2.0
     vis = [0, 3, 6][: max(1, nt // 3)]
     # feed_dict contract of fit_dgp; the locref target / mask maps are generated on the device by the coord2map feeder
     # kernel (no 6 MB feed per step)
@@ -73,14 +75,15 @@ def measure(rank, local_rank, world, steps, warmup, nt, height, width, profile=T
     for l, (a, b) in enumerate(edges):
         S0[l, a], S0[l, b] = 1.0, -1.0
     cfg = dict(gm2=1, gm3=3, wt=float(wt), wt_max=0.0, wn_visible=5.0, wn_hidden=3.0, gamma=1.0, gauss_len=1.0, lengthscale=1.0,
-               locref_loss_weight=0.05, stride=8.0)
-    ws, ws_max = fitdgp.spatial_clique_params([labels], S0, 8.0, 1000.0, 1.2)
-    eng = Engine(NJ, location_refinement=True, device=local_rank, precision=precision)
+               locref_loss_weight=0.05, stride=stride, output_stride=output_stride)
+    ws, ws_max = fitdgp.spatial_clique_params([labels], S0, stride, 1000.0, 1.2)
+    eng = Engine(NJ, location_refinement=True, device=local_rank, precision=precision, output_stride=output_stride)
     eng.load_weights(synthetic.make_weights(NJ, seed=0, net_type=net_type))
     frames_host = bench.make_frame_pool(nt, seed=1234 + rank) if (H, W) == (bench.H, bench.W) else \
         synthetic.make_video(nt, H, W, NJ, seed=1234 + rank)[0]
     frames = torch.from_numpy(frames_host).to(dev)
-    flops_fwd, _ = bench.conv_flops_per_frame(H, W, NJ, locref=True)
+    import bench_depths
+    flops_fwd, _ = bench_depths.conv_flops_per_frame(H, W, NJ, synthetic.BLOCK_UNITS["resnet_50"], True, output_stride)
     flow_pinned = None
     if wt > 0:
         # temporal clique (fitdgp.py:1079-1124): vector_field_tf = optical-flow magnitude per consecutive frame pair
