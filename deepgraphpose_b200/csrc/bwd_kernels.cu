@@ -54,11 +54,14 @@ __global__ void __launch_bounds__(256) relu_bn_bwd_kernel(uint4* __restrict__ g,
     }
     float dyv[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      dyv[j] = av[j] > 0.0f ? gv[j] : 0.0f;
-      S[j] += dyv[j];
-    }
-    g[idx] = pack8v(dyv, fp16);
+    for (int j = 0; j < 8; ++j) dyv[j] = av[j] > 0.0f ? gv[j] : 0.0f;
+    const uint4 o = pack8v(dyv, fp16);
+    g[idx] = o;
+    // the sums are those of dy as stored (what the wgrad GEMM consumes, so that dgamma's <W, dW_raw> - mean * dbeta cancels
+    // exactly): with the scatter, g + d is rounded on the store
+    unpack8(o, dyv, fp16);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) S[j] += dyv[j];
   }
   __shared__ float sm[256][9];
 #pragma unroll

@@ -451,6 +451,27 @@ int make_wgrad_params(dgp_handle* h, const char* scope, int R, int S, int Cin, i
   return DGP_OK;
 }
 
+// conv1's weight gradient in the space-to-depth form of build_conv1_layer: dy (B*H1*W1, 64) against the im2col view of s2d
+// (B, Hs, Ws, 16) in which one 64-channel pixel is a window of 4 horizontally adjacent s2d pixels and the 4 window rows are
+// the taps, exactly as the forward's conv1 map reads it.
+int make_conv1_wgrad_params(dgp_handle* h, const void* dy, const void* s2d, int B, int H1, int W1, int Hs, int Ws,
+                            WgradParams* wp) {
+  memset(wp, 0, sizeof(*wp));
+  tmap_set_fp16(h->fp16);
+  wp->fp16 = h->fp16;
+  const int M = B * H1 * W1;
+  wp->Cout = 64; wp->Kw = 256; wp->num_pix_blocks = ceil_div(M, 64);
+  wp->x_mode = 1; wp->P = H1; wp->Q = W1; wp->conv_stride = 1; wp->lower_h = 0; wp->lower_w = 0; wp->S = 1; wp->dil = 1;
+  wp->cblocks = 1;
+  const char* e = make_tmap_2d(&wp->tmap_dy, dy, (uint64_t)M, 64, 128, 64);
+  if (e) return fail(h, DGP_ERR_CUDA, "conv1 wgrad (dy map): %s", e);
+  e = make_tmap_im2col(&wp->tmap_x, s2d, 64, (uint64_t)W1, (uint64_t)Hs, (uint64_t)B, 32, (uint64_t)Ws * 32,
+                       (uint64_t)Hs * Ws * 32, 0, 0, 0, -3, 1, (uint64_t)B * Hs * Ws * 32, 64);
+  if (e) return fail(h, DGP_ERR_CUDA, "conv1 wgrad (x map): %s", e);
+  wgrad_plan(wp, h->num_sms);
+  return DGP_OK;
+}
+
 int keep_activation(dgp_handle* h, const Step& st, cudaStream_t s);
 
 int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out) {

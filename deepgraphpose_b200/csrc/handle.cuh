@@ -276,6 +276,9 @@ int make_gemm_step(dgp_handle* h, const ConvLayer& L, const void* x, int N, int 
                    Step* st, int* Ho, int* Wo);
 int make_wgrad_params(dgp_handle* h, const char* scope, int R, int S, int Cin, int Cout, int stride, int dil,
                       const void* x, int N, int H, int W, int pad_mode, const void* dy, WgradParams* wp);
+// conv1's wgrad params: dy (B*H1*W1, 64) 16-bit against the space-to-depth input s2d (B, Hs, Ws, 16) of launch_prep_s2d
+int make_conv1_wgrad_params(dgp_handle* h, const void* dy, const void* s2d, int B, int H1, int W1, int Hs, int Ws,
+                            WgradParams* wp);
 int alloc_buf(dgp_handle* h, std::vector<DevBuf>* bufs, size_t bytes, void** out);
 int build_plan(dgp_handle* h, int B, int H, int W, bool train, Plan** out);
 int run_forward_plan(dgp_handle* h, Plan* pl, const uint8_t* frames_dev, float* logits_dev, float* locref_dev,

@@ -443,18 +443,7 @@ int build_backward(dgp_handle* h, Plan* pl) {
     bw->steps.back().wr = g_c1;
     add_mask(h, bw.get(), g_c1, c1, B * H1 * W1, 64, &L, nullptr, site, rows);
     WgradParams wp;
-    memset(&wp, 0, sizeof(wp));
-    tmap_set_fp16(h->fp16);
-    wp.fp16 = h->fp16;
-    const int M = B * H1 * W1;
-    wp.Cout = 64; wp.Kw = 256; wp.num_pix_blocks = ceil_div(M, 64);
-    wp.x_mode = 1; wp.P = H1; wp.Q = W1; wp.conv_stride = 1; wp.lower_h = 0; wp.lower_w = 0; wp.S = 1; wp.dil = 1; wp.cblocks = 1;
-    const char* e = make_tmap_2d(&wp.tmap_dy, g_c1, (uint64_t)M, 64, 128, 64);
-    if (e) return fail(h, DGP_ERR_CUDA, "conv1 wgrad (dy map): %s", e);
-    e = make_tmap_im2col(&wp.tmap_x, pl->s2d, 64, (uint64_t)W1, (uint64_t)pl->Hs, (uint64_t)B, 32, (uint64_t)pl->Ws * 32,
-                         (uint64_t)pl->Hs * pl->Ws * 32, 0, 0, 0, -3, 1, (uint64_t)B * pl->Hs * pl->Ws * 32, 64);
-    if (e) return fail(h, DGP_ERR_CUDA, "conv1 wgrad (x map): %s", e);
-    wgrad_plan(&wp, h->num_sms);
+    if ((rc = make_conv1_wgrad_params(h, g_c1, pl->s2d, B, H1, W1, pl->Hs, pl->Ws, &wp))) return rc;
     if ((rc = add_wgrad_params(h, bw.get(), wp, g_c1, L.scale, h->conv1_mask.get<float>(), ts->grads.get<float>() + L.w_off,
                                &ws_need, &L)))
       return rc;
