@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 LIB = os.path.join(HERE, "libdgp_b200.so")
-SOURCES = ["capi.cu", "conv_gemm_sm100.cu", "wgrad_gemm_sm100.cu", "softargmax.cu", "aux_kernels.cu", "loss_kernels.cu", "param_kernels.cu", "bwd_kernels.cu", "train.cu", "feeder_kernels.cu", "boundary.cu", "stream.cu", "flow_kernels.cu", "resize_kernels.cu", "augment_kernels.cu", "render_kernels.cu", "jpeg_kernels.cu"]
+SOURCES = ["capi.cu", "conv_gemm_sm100.cu", "wgrad_gemm_sm100.cu", "softargmax.cu", "aux_kernels.cu", "loss_kernels.cu", "param_kernels.cu", "bwd_kernels.cu", "train.cu", "feeder_kernels.cu", "boundary.cu", "variables.cu", "stream.cu", "flow_kernels.cu", "resize_kernels.cu", "augment_kernels.cu", "render_kernels.cu", "jpeg_kernels.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-Xcompiler", "-Wno-unused-function",

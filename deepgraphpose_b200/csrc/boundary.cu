@@ -75,19 +75,16 @@ int dgp_deconv2d(dgp_handle* h, const float* x_dev, int N, int H, int W, int Cin
   if (Cin % 64) return fail(h, DGP_ERR_UNSUPPORTED, "dgp_deconv2d: input channels must be a multiple of 64");
   CU_OK(h, cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  // the same packing as the network's own heads (capi.cu build_head_layer): GEMM column (kh*3+kw)*Cout + co
+  // the same packing as the network's own heads, with this one head as all of the GEMM's channels
   ConvLayer L;
   L.scope = "dgp_deconv2d"; L.R = 1; L.S = 1; L.Cin = Cin; L.Cout = 9 * Cout; L.relu = false;
   L.K = Cin;
   L.block_n = pick_block_n(9 * Cout);
   L.Npad = ceil_div(9 * Cout, L.block_n) * L.block_n;
-  std::vector<W16> wm((size_t)L.Npad * Cin, cvt16(h, 0.0f));
-  for (int t = 0; t < 9; ++t)
-    for (int co = 0; co < Cout; ++co) {
-      const float* src = &w_host[((size_t)t * Cout + co) * Cin];
-      W16* d = &wm[(size_t)(t * Cout + co) * Cin];
-      for (int c = 0; c < Cin; ++c) d[c] = cvt16(h, src[c]);
-    }
+  std::vector<float> wf((size_t)L.Npad * Cin, 0.0f);
+  pack({L.scope, 4, {3, 3, Cout, Cin}, VAR_HEAD, 0, wf.size(), Cout, 0}, w_host, wf.data());
+  std::vector<W16> wm(wf.size());
+  for (size_t i = 0; i < wf.size(); ++i) wm[i] = cvt16(h, wf[i]);
   const size_t npix = (size_t)N * H * W;
   DevBuf x16, w16, contrib, bias;
   CU_OK(h, x16.alloc(npix * Cin * 2 + 1024));

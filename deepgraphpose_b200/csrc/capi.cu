@@ -1,4 +1,4 @@
-// libdgp_b200.so -- handle, weight conversion, per-shape execution plans and the C ABI of include/dgp_b200.h.
+// libdgp_b200.so -- handle, weight loading, per-shape execution plans and the C ABI of include/dgp_b200.h.
 #include "../../include/dgp_b200.h"
 
 #include <cuda.h>
@@ -100,43 +100,28 @@ int refresh_operands(dgp_handle* h, cudaStream_t s) {
 
 // Frozen batch norm (slim batch_norm, is_training=False): gamma / beta are trainable and live in the parameter arena,
 // the moving statistics are constants; the fp32 scale/shift applied in the GEMM epilogue are derived on the device
-// (refresh_bn_kernel), never folded into the 16-bit weights.
+// (refresh_bn_kernel), never folded into the 16-bit weights.  A missing gamma is slim's default scale, 1.
 int append_bn(dgp_handle* h, const std::string& scope, int C, int* ch_off) {
-  const HostVar* g = find_var(h, scope + "/BatchNorm/gamma");
-  const HostVar* b = find_var(h, scope + "/BatchNorm/beta");
-  const HostVar* m = find_var(h, scope + "/BatchNorm/moving_mean");
-  const HostVar* v = find_var(h, scope + "/BatchNorm/moving_variance");
-  if (!b || !m || !v) return fail(h, DGP_ERR_STATE, "missing BatchNorm variables for %s", scope.c_str());
-  *ch_off = (int)h->host_gamma.size();
-  for (int c = 0; c < C; ++c) {
-    h->host_gamma.push_back(g ? g->data[c] : 1.0f);
-    h->host_beta.push_back(b->data[c]);
-    h->host_mean.push_back(m->data[c]);
-    h->host_var.push_back(v->data[c]);
-  }
+  const std::string bn = scope + "/BatchNorm/";
+  if (!find_var(h, bn + "beta") || !find_var(h, bn + "moving_mean") || !find_var(h, bn + "moving_variance"))
+    return fail(h, DGP_ERR_STATE, "missing BatchNorm variables for %s", scope.c_str());
+  if (!find_var(h, bn + "gamma")) h->host_vars[bn + "gamma"] = HostVar{std::vector<float>(C, 1.0f), {C}};
+  *ch_off = (int)h->n_ch;
+  h->n_ch += C;
   return DGP_OK;
 }
 
 int build_conv_layer(dgp_handle* h, const std::string& scope, int R, int S, int Cin, int Cout, int stride, int dil,
                      bool relu, int* index) {
-  const HostVar* w = find_var(h, scope + "/weights");
-  if (!w) return fail(h, DGP_ERR_STATE, "missing variable %s/weights", scope.c_str());
-  if (w->shape.size() != 4 || w->shape[0] != R || w->shape[1] != S || w->shape[2] != Cin || w->shape[3] != Cout)
-    return fail(h, DGP_ERR_INVALID, "%s/weights has the wrong shape (want [%d,%d,%d,%d])", scope.c_str(), R, S, Cin, Cout);
+  if (!find_var(h, scope + "/weights")) return fail(h, DGP_ERR_STATE, "missing variable %s/weights", scope.c_str());
   if (Cin % 64 != 0 || Cout % 16 != 0) return fail(h, DGP_ERR_UNSUPPORTED, "%s: channels not tileable", scope.c_str());
   ConvLayer L;
   L.scope = scope; L.R = R; L.S = S; L.Cin = Cin; L.Cout = Cout; L.stride = stride; L.dil = dil; L.relu = relu;
   L.K = R * S * Cin;
   L.block_n = Cout >= 256 ? 256 : Cout;
   L.Npad = Cout;
-  L.w_off = h->host_master.size();
-  h->host_master.resize(L.w_off + (size_t)Cout * L.K);
-  float* wm = h->host_master.data() + L.w_off;
-  for (int t = 0; t < R * S; ++t)
-    for (int c = 0; c < Cin; ++c) {
-      const float* src = &w->data[((size_t)t * Cin + c) * Cout];
-      for (int o = 0; o < Cout; ++o) wm[(size_t)o * L.K + (size_t)t * Cin + c] = src[o];
-    }
+  L.w_off = h->n_w;
+  h->n_w += (size_t)Cout * L.K;
   int rc = append_bn(h, scope, Cout, &L.ch_off);
   if (rc) return rc;
   *index = (int)h->layers.size();
@@ -148,30 +133,12 @@ int build_conv_layer(dgp_handle* h, const std::string& scope, int R, int S, int 
 // one TMA "pixel" is a window of 4 horizontally adjacent s2d pixels (64 channels), the 4 window rows are the taps.
 int build_conv1_layer(dgp_handle* h) {
   const std::string scope = h->net_scope + "/conv1";
-  const HostVar* w = find_var(h, scope + "/weights");
-  if (!w) return fail(h, DGP_ERR_STATE, "missing variable %s/weights", scope.c_str());
-  if (w->shape.size() != 4 || w->shape[0] != 7 || w->shape[1] != 7 || w->shape[2] != 3 || w->shape[3] != 64)
-    return fail(h, DGP_ERR_INVALID, "%s/weights must be [7,7,3,64]", scope.c_str());
+  if (!find_var(h, scope + "/weights")) return fail(h, DGP_ERR_STATE, "missing variable %s/weights", scope.c_str());
   ConvLayer L;
   L.scope = scope; L.R = 4; L.S = 1; L.Cin = 64; L.Cout = 64; L.stride = 1; L.dil = 1; L.relu = true;
   L.K = 256; L.block_n = 64; L.Npad = 64;
-  L.w_off = h->host_master.size();
-  h->host_master.resize(L.w_off + (size_t)64 * 256, 0.0f);
-  float* wm = h->host_master.data() + L.w_off;
-  h->host_conv1_mask.assign((size_t)64 * 256, 0.0f);
-  for (int a = 0; a < 4; ++a)
-    for (int b = 0; b < 4; ++b)
-      for (int u = 0; u < 2; ++u)
-        for (int v = 0; v < 2; ++v) {
-          const int kh = 2 * a + u, kw = 2 * b + v;
-          if (kh >= 7 || kw >= 7) continue;
-          for (int c = 0; c < 3; ++c)
-            for (int o = 0; o < 64; ++o) {
-              const size_t d = (size_t)o * 256 + a * 64 + b * 16 + (u * 2 + v) * 3 + c;
-              wm[d] = w->data[(((size_t)kh * 7 + kw) * 3 + c) * 64 + o];
-              h->host_conv1_mask[d] = 1.0f;
-            }
-        }
+  L.w_off = h->n_w;
+  h->n_w += (size_t)64 * 256;
   int rc = append_bn(h, scope, 64, &L.ch_off);
   if (rc) return rc;
   h->conv1_layer = (int)h->layers.size();
@@ -183,67 +150,61 @@ int build_conv1_layer(dgp_handle* h) {
 int build_head_layer(dgp_handle* h) {
   const int nj = h->cfg.num_joints;
   const int ctot = h->cfg.location_refinement ? 3 * nj : nj;
-  const HostVar* wp = find_var(h, "pose/part_pred/block4/weights");
-  const HostVar* bp = find_var(h, "pose/part_pred/block4/biases");
-  if (!wp || !bp) return fail(h, DGP_ERR_STATE, "missing pose/part_pred/block4 variables");
-  if (wp->shape.size() != 4 || wp->shape[0] != 3 || wp->shape[1] != 3 || wp->shape[2] != nj || wp->shape[3] != 2048)
-    return fail(h, DGP_ERR_INVALID, "pose/part_pred/block4/weights must be [3,3,%d,2048]", nj);
-  const HostVar* wl = nullptr;
-  const HostVar* bl = nullptr;
-  if (h->cfg.location_refinement) {
-    wl = find_var(h, "pose/locref_pred/block4/weights");
-    bl = find_var(h, "pose/locref_pred/block4/biases");
-    if (!wl || !bl) return fail(h, DGP_ERR_STATE, "missing pose/locref_pred/block4 variables");
-    if (wl->shape.size() != 4 || wl->shape[2] != 2 * nj || wl->shape[3] != 2048)
-      return fail(h, DGP_ERR_INVALID, "pose/locref_pred/block4/weights must be [3,3,%d,2048]", 2 * nj);
-  }
+  if (!find_var(h, "pose/part_pred/block4/weights") || !find_var(h, "pose/part_pred/block4/biases"))
+    return fail(h, DGP_ERR_STATE, "missing pose/part_pred/block4 variables");
+  if (h->cfg.location_refinement &&
+      (!find_var(h, "pose/locref_pred/block4/weights") || !find_var(h, "pose/locref_pred/block4/biases")))
+    return fail(h, DGP_ERR_STATE, "missing pose/locref_pred/block4 variables");
   ConvLayer L;
   L.scope = "pose/heads"; L.R = 1; L.S = 1; L.Cin = 2048; L.Cout = 9 * ctot; L.relu = false;
   L.K = 2048;
   L.block_n = pick_block_n(9 * ctot);
   L.Npad = ceil_div(9 * ctot, L.block_n) * L.block_n;
-  L.w_off = h->host_master.size();
-  h->host_master.resize(L.w_off + (size_t)L.Npad * 2048, 0.0f);
-  float* wm = h->host_master.data() + L.w_off;
-  for (int t = 0; t < 9; ++t)
-    for (int co = 0; co < ctot; ++co) {
-      const HostVar* src = co < nj ? wp : wl;
-      const int cc = co < nj ? co : co - nj;
-      const int cn = co < nj ? nj : 2 * nj;
-      const float* s = &src->data[((size_t)t * cn + cc) * 2048];
-      float* d = &wm[(size_t)(t * ctot + co) * 2048];
-      for (int c = 0; c < 2048; ++c) d[c] = s[c];
-    }
-  h->host_bias.assign((size_t)ceil_div(ctot, 8) * 8, 0.0f);
-  for (int co = 0; co < ctot; ++co) h->host_bias[co] = co < nj ? bp->data[co] : bl->data[co - nj];
+  L.w_off = h->n_w;
+  h->n_w += (size_t)L.Npad * 2048;
+  h->n_bias = (size_t)ceil_div(ctot, 8) * 8;
   h->ctot = ctot;
   h->head_layer = (int)h->layers.size();
   h->layers.push_back(L);
   return DGP_OK;
 }
 
-// Uploads the parameter arena [weights | gamma | beta | head bias] (fp32 master copy) and derives the tensor-core
-// operands on the device.
+// Checks every loaded variable of `vars` against its TF shape and packs it into its span of `base`.
+int pack_loaded(dgp_handle* h, const std::vector<ArenaVar>& vars, float* base) {
+  for (const ArenaVar& v : vars) {
+    const HostVar* x = find_var(h, v.name);  // present: the layer walk checked every name
+    bool same = x && (int)x->shape.size() == v.ndim;
+    for (int i = 0; same && i < v.ndim; ++i) same = x->shape[i] == v.shape[i];
+    if (!same) return fail(h, DGP_ERR_INVALID, "%s has the wrong shape (want %s)", v.name.c_str(), shape_str(v).c_str());
+    pack(v, x->data.data(), base + v.off);
+  }
+  return DGP_OK;
+}
+
+// Packs the loaded variables into the parameter arena [weights | gamma | beta | head bias] (fp32 master copy) and the
+// frozen moving statistics, uploads both and derives the tensor-core operands on the device.
 int upload_arena(dgp_handle* h) {
-  h->n_w = h->host_master.size();
-  h->n_ch = h->host_gamma.size();
-  h->n_bias = h->host_bias.size();
   h->n_params = h->n_w + 2 * h->n_ch + h->n_bias;
   if (h->n_w % 8 || h->n_ch % 4) return fail(h, DGP_ERR_STATE, "parameter arena is not vector aligned");
+  std::vector<ArenaVar> frozen;
+  build_variable_table(h, &frozen);
+  std::vector<float> arena(h->n_params, 0.0f), stats(2 * h->n_ch);  // stats: [moving_mean | moving_variance]
+  int rc;
+  if ((rc = pack_loaded(h, h->vars, arena.data())) || (rc = pack_loaded(h, frozen, stats.data()))) return rc;
+  const ArenaVar& conv1 = h->vars[h->var_index[h->net_scope + "/conv1/weights"]];
+  std::vector<float> ones(tf_elems(conv1), 1.0f), mask(conv1.len, 0.0f);
+  pack(conv1, ones.data(), mask.data());
   CU_OK(h, h->master.alloc(h->n_params * sizeof(float)));
   CU_OK(h, h->w16.alloc(h->n_w * sizeof(W16)));
   CU_OK(h, h->bn_mean.alloc(h->n_ch * sizeof(float)));
   CU_OK(h, h->bn_var.alloc(h->n_ch * sizeof(float)));
   CU_OK(h, h->bn_ss.alloc(2 * h->n_ch * sizeof(float)));
+  CU_OK(h, h->conv1_mask.alloc(mask.size() * sizeof(float)));
   float* master = h->master.get<float>();
-  CU_OK(h, cudaMemcpy(master, h->host_master.data(), h->n_w * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(master + h->n_w, h->host_gamma.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(master + h->n_w + h->n_ch, h->host_beta.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(master + h->n_w + 2 * h->n_ch, h->host_bias.data(), h->n_bias * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->bn_mean.get(), h->host_mean.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, cudaMemcpy(h->bn_var.get(), h->host_var.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
-  CU_OK(h, h->conv1_mask.alloc(h->host_conv1_mask.size() * 4));
-  CU_OK(h, cudaMemcpy(h->conv1_mask.get(), h->host_conv1_mask.data(), h->host_conv1_mask.size() * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(master, arena.data(), h->n_params * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(h->bn_mean.get(), stats.data(), h->n_ch * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(h->bn_var.get(), stats.data() + h->n_ch, h->n_ch * 4, cudaMemcpyHostToDevice));
+  CU_OK(h, cudaMemcpy(h->conv1_mask.get(), mask.data(), mask.size() * 4, cudaMemcpyHostToDevice));
   float* bn_ss = h->bn_ss.get<float>();
   for (ConvLayer& L : h->layers) {
     L.w = h->w16.get<W16>() + L.w_off;
@@ -253,10 +214,8 @@ int upload_arena(dgp_handle* h) {
     }
   }
   h->head_bias = master + h->n_w + 2 * h->n_ch;
-  int rc = refresh_operands(h, nullptr);
-  if (rc) return rc;
+  if ((rc = refresh_operands(h, nullptr))) return rc;
   CU_OK(h, cudaDeviceSynchronize());
-  std::vector<float>().swap(h->host_master);
   return DGP_OK;
 }
 
@@ -1316,11 +1275,10 @@ int dgp_conv2d(dgp_handle* h, const void* x_dev, int N, int H, int W, int Cin, c
   L.block_n = block_n > 0 ? block_n : pick_block_n(Cout);
   L.Npad = ceil_div(Cout, L.block_n) * L.block_n;
   if (L.Npad != Cout) return fail(h, DGP_ERR_INVALID, "dgp_conv2d: block_n must divide Cout");
-  std::vector<__nv_bfloat16> wm((size_t)L.Npad * L.K, cvt16(h, 0.0f));
-  for (int t = 0; t < R * S; ++t)
-    for (int c = 0; c < Cin; ++c)
-      for (int o = 0; o < Cout; ++o)
-        wm[(size_t)o * L.K + (size_t)t * Cin + c] = cvt16(h, w_host[((size_t)t * Cin + c) * Cout + o]);
+  std::vector<float> wf((size_t)L.Npad * L.K, 0.0f);
+  pack({L.scope, 4, {R, S, Cin, Cout}, VAR_CONV, 0, wf.size()}, w_host, wf.data());
+  std::vector<W16> wm(wf.size());
+  for (size_t i = 0; i < wf.size(); ++i) wm[i] = cvt16(h, wf[i]);
   DevBuf w, scale, shift;
   CU_OK(h, w.alloc(wm.size() * sizeof(__nv_bfloat16)));
   CU_OK(h, cudaMemcpy(w.get(), wm.data(), wm.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));

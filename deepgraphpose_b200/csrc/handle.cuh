@@ -33,6 +33,22 @@ struct HostVar {
   std::vector<int64_t> shape;
 };
 
+// How a trainable variable's TF layout maps onto its span of the parameter arena (variables.cu):
+//   VAR_VECTOR     gamma, beta, biases: the same order
+//   VAR_CONV       HWIO [R,S,Cin,Cout] <-> GEMM rows [Cout][R*S*Cin]
+//   VAR_CONV1_S2D  [7,7,3,64] <-> the [64][256] space-to-depth matrix of conv1
+//   VAR_HEAD       [3,3,cn,Cin] <-> rows t*ctot + c0 + cc (tap t, cc < cn) of the deconv heads' [Npad][Cin] GEMM matrix
+enum VarLayout { VAR_VECTOR, VAR_CONV, VAR_CONV1_S2D, VAR_HEAD };
+
+struct ArenaVar {
+  std::string name;                  // TF name
+  int ndim = 1;
+  int64_t shape[4] = {0, 0, 0, 0};   // TF shape
+  VarLayout layout = VAR_VECTOR;
+  size_t off = 0, len = 0;           // arena span [off, off + len); pack writes only the variable's own elements of it
+  int ctot = 0, c0 = 0;              // VAR_HEAD (cn = shape[2], Cin = shape[3])
+};
+
 struct ConvLayer {
   std::string scope;
   int R = 1, S = 1, Cin = 0, Cout = 0, stride = 1, dil = 1;
@@ -201,7 +217,8 @@ struct dgp_handle {
   DevBuf bn_ss;        // [scale n_ch | shift n_ch]
   DevBuf conv1_mask;   // [64][256] 1 = real 7x7x3 tap of the space-to-depth conv1 matrix
   size_t n_w = 0, n_ch = 0, n_bias = 0, n_params = 0;
-  std::vector<float> host_master, host_gamma, host_beta, host_mean, host_var, host_bias, host_conv1_mask;
+  std::vector<ArenaVar> vars;              // the trainable variables in layer order (variables.cu)
+  std::map<std::string, int> var_index;    // TF name -> index into vars
   std::map<std::tuple<int, int, int>, std::unique_ptr<Plan>> plans, train_plans;  // inference key (-B,..) = unchunked debug plan
   uint64_t plan_clock = 0;
   bool debug_keep = false;
@@ -285,6 +302,21 @@ int run_forward_plan(dgp_handle* h, Plan* pl, const uint8_t* frames_dev, float* 
                      cudaStream_t s, int first_step = 0, int last_step = -1);
 int ensure(dgp_handle* h, DevBuf* b, size_t bytes);
 int refresh_operands(dgp_handle* h, cudaStream_t s);
+
+// variables.cu
+size_t tf_elems(const ArenaVar& v);
+std::string shape_str(const ArenaVar& v);  // "[7,7,3,64]"
+// TF layout <-> the variable's span (span = arena + v.off)
+void pack(const ArenaVar& v, const float* tf, float* span);
+void unpack(const ArenaVar& v, const float* span, float* tf);
+// Fills h->vars / h->var_index from the finalized layers: arena [weights n_w | gamma n_ch | beta n_ch | head bias n_bias].
+// *frozen gets the moving statistics, with spans in [moving_mean n_ch | moving_variance n_ch].
+void build_variable_table(dgp_handle* h, std::vector<ArenaVar>* frozen);
+// train.cu: the arena dgp_get_variable / dgp_set_variable address with `what` (0 value, 1 gradient, 2 momentum) and the
+// factor that turns a stored element into the variable's value (gradients are stored multiplied by arena_scale).
+float* variable_arena(dgp_handle* h, int what, float* unscale);
+// train.cu: dgp_set_variable changed the weights: every dgp_train_forward token is stale, the dgrad operands too.
+void weights_changed(dgp_handle* h);
 // Size of a transformed frame (DGP_ERR_INVALID for an invalid transform); *identity: the transform leaves frames unchanged.
 int transform_dims(int H0, int W0, const dgp_frame_transform* t, int* H, int* W, bool* identity);
 // dgp_resize_crop without the device switch (resize_kernels.cu)

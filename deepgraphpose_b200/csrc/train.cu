@@ -481,38 +481,6 @@ int build_backward(dgp_handle* h, Plan* pl) {
   return DGP_OK;
 }
 
-// host-side TF-layout view of one variable of the arena
-struct VarRef {
-  int kind = -1;  // 0 conv weights HWIO, 1 conv1 weights, 2 gamma, 3 beta, 4 head weights, 5 head bias
-  const ConvLayer* L = nullptr;
-  int head_part = 0;  // 0 = part_pred, 1 = locref_pred
-};
-
-bool find_variable(dgp_handle* h, const std::string& name, VarRef* r) {
-  const std::string pp = "pose/part_pred/block4/", pl = "pose/locref_pred/block4/";
-  for (int part = 0; part < 2; ++part) {
-    const std::string& pre = part ? pl : pp;
-    if (name.compare(0, pre.size(), pre) == 0) {
-      if (part == 1 && !h->cfg.location_refinement) return false;
-      r->head_part = part;
-      r->L = &h->layers[h->head_layer];
-      const std::string leaf = name.substr(pre.size());
-      if (leaf == "weights") { r->kind = 4; return true; }
-      if (leaf == "biases") { r->kind = 5; return true; }
-      return false;
-    }
-  }
-  for (const ConvLayer& L : h->layers) {
-    if (name.compare(0, L.scope.size(), L.scope) != 0 || name.size() <= L.scope.size() || name[L.scope.size()] != '/') continue;
-    const std::string leaf = name.substr(L.scope.size() + 1);
-    r->L = &L;
-    if (leaf == "weights") { r->kind = (&L == &h->layers[h->conv1_layer]) ? 1 : 0; return true; }
-    if (leaf == "BatchNorm/gamma") { r->kind = 2; return true; }
-    if (leaf == "BatchNorm/beta") { r->kind = 3; return true; }
-  }
-  return false;
-}
-
 // Stores the arena write mode the backward kernels read (GradMode) on `s`, when it differs from the stored one.
 int set_grad_mode(dgp_handle* h, int accumulate, float out_scale, cudaStream_t s) {
   TrainState* ts = h->train.get();
@@ -641,6 +609,17 @@ int run_backward(dgp_handle* h, Backward* bw, cudaStream_t s) {
 }
 
 }  // namespace
+
+float* variable_arena(dgp_handle* h, int what, float* unscale) {
+  *unscale = what == 1 ? 1.0f / h->train->arena_scale : 1.0f;
+  return (what == 0 ? h->master : (what == 1 ? h->train->grads : h->train->accum)).get<float>();
+}
+
+void weights_changed(dgp_handle* h) {
+  drop_train_tokens(h);
+  if (h->train) h->train->wd_fresh = false;
+}
+
 }  // namespace dgp
 
 extern "C" {
@@ -857,134 +836,6 @@ int dgp_train_outputs(dgp_handle* h, int nt, int H, int W, float** logits_dev, f
   if (it == h->train_plans.end()) return fail(h, DGP_ERR_STATE, "dgp_train_outputs: no training step has run at this shape");
   if (logits_dev) *logits_dev = it->second->logits;
   if (locref_dev) *locref_dev = it->second->locref;
-  return DGP_OK;
-}
-
-int dgp_get_variable(dgp_handle* h, const char* tf_var_name, int what, float* host_out, size_t max_elems, int64_t* shape4,
-                     int* ndim) {
-  if (!h || !tf_var_name) return DGP_ERR_INVALID;
-  if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_get_variable before dgp_finalize_weights");
-  if (what < 0 || what > 2) return fail(h, DGP_ERR_INVALID, "dgp_get_variable: what must be 0 (value), 1 (gradient) or 2 (momentum)");
-  if (what > 0 && !h->train) return fail(h, DGP_ERR_STATE, "dgp_get_variable: gradients need dgp_train_enable");
-  VarRef r;
-  if (!find_variable(h, tf_var_name, &r)) return fail(h, DGP_ERR_INVALID, "unknown variable %s", tf_var_name);
-  const DevBuf& buf = what == 0 ? h->master : (what == 1 ? h->train->grads : h->train->accum);
-  const float* arena = buf.get<float>();
-  const ConvLayer& L = *r.L;
-  const int nj = h->cfg.num_joints;
-  int64_t shp[4] = {0, 0, 0, 0};
-  int nd = 1;
-  switch (r.kind) {
-    case 0: shp[0] = L.R; shp[1] = L.S; shp[2] = L.Cin; shp[3] = L.Cout; nd = 4; break;
-    case 1: shp[0] = 7; shp[1] = 7; shp[2] = 3; shp[3] = 64; nd = 4; break;
-    case 2: case 3: shp[0] = L.Cout; nd = 1; break;
-    case 4: shp[0] = 3; shp[1] = 3; shp[2] = r.head_part ? 2 * nj : nj; shp[3] = 2048; nd = 4; break;
-    case 5: shp[0] = r.head_part ? 2 * nj : nj; nd = 1; break;
-  }
-  size_t n = 1;
-  for (int i = 0; i < nd; ++i) n *= (size_t)shp[i];
-  if (shape4) for (int i = 0; i < 4; ++i) shape4[i] = shp[i];
-  if (ndim) *ndim = nd;
-  if (!host_out) return DGP_OK;
-  if (n > max_elems) return fail(h, DGP_ERR_INVALID, "buffer too small for %s", tf_var_name);
-  struct Unscale {  // gradients are stored multiplied by arena_scale; hand back the true gradient
-    float* p; size_t n; float f;
-    ~Unscale() { if (f != 1.0f) for (size_t i = 0; i < n; ++i) p[i] *= f; }
-  } unscale{host_out, n, what == 1 ? 1.0f / h->train->arena_scale : 1.0f};
-  CU_OK(h, cudaSetDevice(h->device));
-  CU_OK(h, cudaDeviceSynchronize());
-  if (r.kind == 2 || r.kind == 3) {
-    const size_t off = h->n_w + (r.kind == 3 ? h->n_ch : 0) + (size_t)L.ch_off;
-    CU_OK(h, cudaMemcpy(host_out, arena + off, n * 4, cudaMemcpyDeviceToHost));
-    return DGP_OK;
-  }
-  if (r.kind == 5) {
-    const size_t off = h->n_w + 2 * h->n_ch + (r.head_part ? nj : 0);
-    CU_OK(h, cudaMemcpy(host_out, arena + off, n * 4, cudaMemcpyDeviceToHost));
-    return DGP_OK;
-  }
-  std::vector<float> m((size_t)L.Npad * L.K);
-  CU_OK(h, cudaMemcpy(m.data(), arena + L.w_off, m.size() * 4, cudaMemcpyDeviceToHost));
-  if (r.kind == 0) {
-    const int T = L.R * L.S;
-    for (int t = 0; t < T; ++t)
-      for (int c = 0; c < L.Cin; ++c)
-        for (int o = 0; o < L.Cout; ++o) host_out[((size_t)t * L.Cin + c) * L.Cout + o] = m[(size_t)o * L.K + (size_t)t * L.Cin + c];
-  } else if (r.kind == 1) {
-    for (int kh = 0; kh < 7; ++kh)
-      for (int kw = 0; kw < 7; ++kw)
-        for (int c = 0; c < 3; ++c)
-          for (int o = 0; o < 64; ++o)
-            host_out[(((size_t)kh * 7 + kw) * 3 + c) * 64 + o] =
-                m[(size_t)o * 256 + (kh >> 1) * 64 + (kw >> 1) * 16 + ((kh & 1) * 2 + (kw & 1)) * 3 + c];
-  } else {
-    const int ctot = h->ctot, cn = r.head_part ? 2 * nj : nj, c0 = r.head_part ? nj : 0;
-    for (int t = 0; t < 9; ++t)
-      for (int cc = 0; cc < cn; ++cc)
-        memcpy(&host_out[((size_t)t * cn + cc) * 2048], &m[(size_t)(t * ctot + c0 + cc) * 2048], 2048 * sizeof(float));
-  }
-  return DGP_OK;
-}
-
-int dgp_set_variable(dgp_handle* h, const char* tf_var_name, int what, const float* host_in, size_t n_elems) {
-  if (!h || !tf_var_name || !host_in) return DGP_ERR_INVALID;
-  if (!h->finalized) return fail(h, DGP_ERR_STATE, "dgp_set_variable before dgp_finalize_weights");
-  if (what != 0 && what != 2) return fail(h, DGP_ERR_INVALID, "dgp_set_variable: what must be 0 (value) or 2 (momentum)");
-  if (what == 2 && !h->train) return fail(h, DGP_ERR_STATE, "dgp_set_variable: momentum needs dgp_train_enable");
-  VarRef r;
-  if (!find_variable(h, tf_var_name, &r)) return fail(h, DGP_ERR_INVALID, "unknown variable %s", tf_var_name);
-  float* arena = (what == 0 ? h->master : h->train->accum).get<float>();
-  const ConvLayer& L = *r.L;
-  const int nj = h->cfg.num_joints;
-  CU_OK(h, cudaSetDevice(h->device));
-  CU_OK(h, cudaDeviceSynchronize());
-  size_t want = 0;
-  if (r.kind == 2 || r.kind == 3) {
-    want = (size_t)L.Cout;
-    if (n_elems != want) return fail(h, DGP_ERR_INVALID, "%s: expected %zu elements", tf_var_name, want);
-    const size_t off = h->n_w + (r.kind == 3 ? h->n_ch : 0) + (size_t)L.ch_off;
-    CU_OK(h, cudaMemcpy(arena + off, host_in, want * 4, cudaMemcpyHostToDevice));
-  } else if (r.kind == 5) {
-    want = (size_t)(r.head_part ? 2 * nj : nj);
-    if (n_elems != want) return fail(h, DGP_ERR_INVALID, "%s: expected %zu elements", tf_var_name, want);
-    const size_t off = h->n_w + 2 * h->n_ch + (r.head_part ? nj : 0);
-    CU_OK(h, cudaMemcpy(arena + off, host_in, want * 4, cudaMemcpyHostToDevice));
-  } else {
-    std::vector<float> m((size_t)L.Npad * L.K);
-    CU_OK(h, cudaMemcpy(m.data(), arena + L.w_off, m.size() * 4, cudaMemcpyDeviceToHost));
-    if (r.kind == 0) {
-      const int T = L.R * L.S;
-      want = (size_t)T * L.Cin * L.Cout;
-      if (n_elems != want) return fail(h, DGP_ERR_INVALID, "%s: expected %zu elements", tf_var_name, want);
-      for (int t = 0; t < T; ++t)
-        for (int c = 0; c < L.Cin; ++c)
-          for (int o = 0; o < L.Cout; ++o) m[(size_t)o * L.K + (size_t)t * L.Cin + c] = host_in[((size_t)t * L.Cin + c) * L.Cout + o];
-    } else if (r.kind == 1) {
-      want = (size_t)7 * 7 * 3 * 64;
-      if (n_elems != want) return fail(h, DGP_ERR_INVALID, "%s: expected %zu elements", tf_var_name, want);
-      for (int kh = 0; kh < 7; ++kh)
-        for (int kw = 0; kw < 7; ++kw)
-          for (int c = 0; c < 3; ++c)
-            for (int o = 0; o < 64; ++o)
-              m[(size_t)o * 256 + (kh >> 1) * 64 + (kw >> 1) * 16 + ((kh & 1) * 2 + (kw & 1)) * 3 + c] =
-                  host_in[(((size_t)kh * 7 + kw) * 3 + c) * 64 + o];
-    } else {
-      const int ctot = h->ctot, cn = r.head_part ? 2 * nj : nj, c0 = r.head_part ? nj : 0;
-      want = (size_t)9 * cn * 2048;
-      if (n_elems != want) return fail(h, DGP_ERR_INVALID, "%s: expected %zu elements", tf_var_name, want);
-      for (int t = 0; t < 9; ++t)
-        for (int cc = 0; cc < cn; ++cc)
-          memcpy(&m[(size_t)(t * ctot + c0 + cc) * 2048], &host_in[((size_t)t * cn + cc) * 2048], 2048 * sizeof(float));
-    }
-    CU_OK(h, cudaMemcpy(arena + L.w_off, m.data(), m.size() * 4, cudaMemcpyHostToDevice));
-  }
-  if (what == 0) {  // the tensor-core operands are derived from the master copy
-    drop_train_tokens(h);
-    int rc = refresh_operands(h, nullptr);
-    if (rc) return rc;
-    if (h->train) h->train->wd_fresh = false;
-    CU_OK(h, cudaDeviceSynchronize());
-  }
   return DGP_OK;
 }
 
