@@ -67,7 +67,8 @@ class DgpAugmentParams(C.Structure):
 
 class DgpMarkerStyle(C.Structure):
     _fields_ = [("dotsize", C.c_int32), ("mask_threshold", C.c_double), ("scale_x", C.c_double), ("scale_y", C.c_double),
-                ("colors", C.c_void_p)]
+                ("colors", C.c_void_p), ("edges", C.c_void_p), ("n_edges", C.c_int32), ("skeleton_color", C.c_uint8 * 3),
+                ("trailpoints", C.c_int32), ("history", C.c_int32)]
 
 
 # reader(user, slot, max_frames, &direct) -> frames delivered (0 = end of video, < 0 = error)

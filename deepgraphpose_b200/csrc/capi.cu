@@ -745,12 +745,13 @@ int PoseStaging::reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W,
   return DGP_OK;
 }
 
-int PoseStaging::reserve_render(dgp_handle* h, bool jpeg) {
+int PoseStaging::reserve_render(dgp_handle* h, bool jpeg, int batch, int trailpoints) {
   if (!d2h_stream) CU_OK(h, create(&d2h_stream, cudaStreamNonBlocking));
   if (jpeg && !packet_stream) CU_OK(h, create(&packet_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; ++i)
     if (!ev_drawn[i]) CU_OK(h, create(&ev_drawn[i], cudaEventDisableTiming));
-  return DGP_OK;
+  marker_rows = (trailpoints > 1 ? trailpoints - 1 : 0) + batch;
+  return ensure(h, &marker_table, (size_t)2 * 3 * marker_rows * h->cfg.num_joints * sizeof(double));
 }
 
 int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
@@ -780,9 +781,22 @@ int PoseStaging::run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_
   if (render) {
     // the next H2D into this slot waits for ev_consumed, so it must follow the copy of the annotated frames, not the forward
     cudaStream_t ds = d2h_stream.get();
-    if ((rc = draw_markers_fused(h, frames[slot].get<uint8_t>(), n, j.H0, j.W0, mu.get<float>(), lik.get<float>(),
-                                 *render->args, s)))
+    const MarkerArgs& ma = *render->args;
+    // the batch's rows go after the carried ones; the last `carry` rows of the sequence are copied to the front of the other
+    // half for the next batch (two halves, because for a batch shorter than the trail the rows would overlap in one)
+    const int trail = ma.trailpoints > 1 ? ma.trailpoints - 1 : 0;
+    const int history = (int)std::min<int64_t>(trail, t0), carry = std::min(trail, history + n);
+    const size_t plane = (size_t)marker_rows * nj;
+    double* xs = marker_table.get<double>() + (size_t)(it & 1) * 3 * plane + (size_t)trail * nj;
+    if ((rc = marker_table_fused(h, mu.get<float>(), lik.get<float>(), n, ma, xs, xs + plane, xs + 2 * plane, s))) return rc;
+    if ((rc = draw_markers_impl(h, frames[slot].get<uint8_t>(), n, j.H0, j.W0, xs, xs + plane, xs + 2 * plane, history, ma,
+                                s)))
       return rc;
+    if (carry > 0) {
+      double* next = marker_table.get<double>() + (size_t)((it + 1) & 1) * 3 * plane + (size_t)(trail - carry) * nj;
+      CU_OK(h, cudaMemcpy2DAsync(next, plane * sizeof(double), xs + (ptrdiff_t)(n - carry) * nj, plane * sizeof(double),
+                                 (size_t)carry * nj * sizeof(double), 3, cudaMemcpyDeviceToDevice, s));
+    }
     if (render->quality) {
       // the encode is the last reader of the slot; only the packets' offsets | sizes go D2H here, the writer thread copies
       // the packets themselves once it knows their total

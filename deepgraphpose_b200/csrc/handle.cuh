@@ -127,19 +127,28 @@ struct PoseJob {
   float* lik_host;
 };
 
-// Kernel argument of the marker drawing (render_kernels.cu): the style of dgp_marker_style with its colour table by value,
-// so a launch needs no allocation.
+// Kernel argument of the marker drawing (render_kernels.cu): the style of dgp_marker_style with its colour and edge tables
+// by value, so a launch needs no allocation.
 constexpr int kMaxDotsize = 64;
+constexpr int kMaxEdges = 256;
+constexpr int kMaxTrailpoints = 64;
 struct MarkerArgs {
-  int nj, dotsize;
+  int nj, dotsize, n_edges, trailpoints;
   double mask_threshold, scale_x, scale_y, stride, half_stride;
   uint8_t colors[3 * 256];
+  uint8_t edges[2 * kMaxEdges];
+  uint8_t skeleton_color[3];
 };
-// Validates `st` and fills `a` for the handle's joints and stride.
-int marker_args(dgp_handle* h, const dgp_marker_style* st, MarkerArgs* a);
-// Markers of N frames from the soft-argmax read-outs mu (N,nj,2) / lik (N,nj) of an estimate_pose batch.
-int draw_markers_fused(dgp_handle* h, uint8_t* frames, int N, int H, int W, const float* mu, const float* lik,
-                       const MarkerArgs& a, cudaStream_t s);
+// Validates `st` for (H, W) frames and fills `a` for the handle's joints and stride.
+int marker_args(dgp_handle* h, const dgp_marker_style* st, int H, int W, MarkerArgs* a);
+// Paints N frames from the float64 tables xs / ys / liks (rows of nj; row t is frame t, rows -history .. -1 the frames
+// before it).
+int draw_markers_impl(dgp_handle* h, uint8_t* frames, int N, int H, int W, const double* xs, const double* ys,
+                      const double* liks, int history, const MarkerArgs& a, cudaStream_t s);
+// The fused pass's table rows of an estimate_pose batch: x, y, lik of the soft-argmax read-outs mu (n,nj,2) / lik (n,nj) in
+// video pixels, as eval.estimate_pose forms them on the host.
+int marker_table_fused(dgp_handle* h, const float* mu, const float* lik, int n, const MarkerArgs& a, double* xs, double* ys,
+                       double* liks, cudaStream_t s);
 
 // Motion-JPEG (jpeg_kernels.cu): bytes of the header template (SOI .. SOS) and the largest frame side.
 constexpr int kJpegHeaderBytes = 629;
@@ -176,6 +185,11 @@ struct PoseStaging {
   Event ev_drawn[2];
   // Motion-JPEG rendering: the writer thread's copies of the encoded packets
   Stream packet_stream;
+  // rendering: the float64 marker table, two halves used by alternate batches, each three planes (x | y | lik) of
+  // marker_rows = K - 1 + batch rows of nj.  Rows [0, K-1) of a half hold the last frames before the batch (carried from
+  // the other half), rows [K-1, K-1+n) the batch's own.
+  DevBuf marker_table;
+  int marker_rows = 0;
   int reserve(dgp_handle* h, int batch, int H0, int W0, int H, int W, bool identity);
   // Batch number `it` (n frames at host_frames, output rows [t0, t0 + n)): H2D, transform, forward + soft-argmax of run_n
   // rows, D2H of n read-outs.  release(release_arg) runs on the copy stream once host_frames has been copied.  With
@@ -183,9 +197,9 @@ struct PoseStaging {
   // copy.
   int run_batch(dgp_handle* h, const PoseJob& j, const uint8_t* host_frames, int n, int run_n, int it, int64_t t0,
                 cudaHostFn_t release, void* release_arg, const RenderBatch* render = nullptr);
-  // the D2H stream and events of run_batch's `render` step (created at the first rendering call), and with `jpeg` the
-  // packet stream
-  int reserve_render(dgp_handle* h, bool jpeg);
+  // the D2H stream and events of run_batch's `render` step (created at the first rendering call), with `jpeg` the packet
+  // stream, and the marker table for `batch` frames and `trailpoints`
+  int reserve_render(dgp_handle* h, bool jpeg, int batch, int trailpoints);
 };
 
 }  // namespace dgp

@@ -96,7 +96,7 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
                 quality, H0, W0);
   MarkerArgs marker;
   if (render) {
-    int rc = marker_args(h, style, &marker);
+    int rc = marker_args(h, style, H0, W0, &marker);
     if (rc) return rc;
   }
   if (max_frames == 0) return DGP_OK;
@@ -110,7 +110,7 @@ int stream_impl(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int 
   const size_t slot_bytes = jpeg ? 2 * sizeof(int64_t) * batch : frame_bytes * batch;
   const int64_t packets_bytes = jpeg ? jpeg_capacity(H0, W0) * batch : 0;
   if (render) {
-    if ((rc = h->pose.reserve_render(h, jpeg))) return rc;
+    if ((rc = h->pose.reserve_render(h, jpeg, batch, marker.trailpoints))) return rc;
     for (PinnedBuf& r : h->writer_slot)
       if (r.bytes() < slot_bytes) CU_OK(h, r.alloc(slot_bytes));
   }

@@ -67,6 +67,8 @@ def transform_dims(H0, W0, new_size=None, crop_size=None):
 
 
 MAX_DOTSIZE = 64  # kMaxDotsize of csrc/handle.cuh
+MAX_EDGES = 256  # kMaxEdges
+MAX_TRAILPOINTS = 64  # kMaxTrailpoints
 
 
 def marker_colors(nj, colormap="cool"):
@@ -83,12 +85,38 @@ def marker_colors(nj, colormap="cool"):
     return np.stack([idx, 255 - idx, np.full(nj, 255)], axis=1).astype(np.uint8)
 
 
-def marker_style(nj, dotsize=3, mask_threshold=0.1, colors=None, scale_x=1.0, scale_y=1.0):
-    """(dgp_marker_style, colour table) of a drawing call; the table must stay alive while the style is in use.  ``colors``:
-    None (the 'cool' table), a colormap name, or an (nj, 3) table of values in [0, 255].  ValueError for a dotsize outside
-    [0, 64] or a table of another shape."""
-    if isinstance(dotsize, bool) or not isinstance(dotsize, (int, np.integer)) or not 0 <= int(dotsize) <= MAX_DOTSIZE:
-        raise ValueError("dotsize must be an integer in [0, %d], got %r" % (MAX_DOTSIZE, dotsize))
+def _check_int(name, value, lo, hi):
+    if isinstance(value, bool) or not isinstance(value, (int, np.integer)) or not lo <= int(value) <= hi:
+        raise ValueError("%s must be an integer in [%d, %d], got %r" % (name, lo, hi, value))
+    return int(value)
+
+
+def skeleton_edges(nj, edges):
+    """``edges`` (pairs of joint indices, or None) as a contiguous int32 (n, 2) table; ValueError for more than 256 pairs,
+    a shape other than (n, 2) or an index outside [0, nj)."""
+    if edges is None:
+        return np.zeros((0, 2), np.int32)
+    arr = np.asarray(edges)
+    if arr.size == 0:
+        return np.zeros((0, 2), np.int32)
+    if arr.ndim != 2 or arr.shape[1] != 2 or not np.issubdtype(arr.dtype, np.integer):
+        raise ValueError("edges must be (n, 2) pairs of joint indices, got %s %s" % (arr.dtype, arr.shape))
+    if arr.shape[0] > MAX_EDGES:
+        raise ValueError("at most %d skeleton edges, got %d" % (MAX_EDGES, arr.shape[0]))
+    if arr.min() < 0 or arr.max() >= int(nj):
+        raise ValueError("skeleton edge joints must lie in [0, %d), got %s" % (nj, arr.tolist()))
+    return np.ascontiguousarray(arr, dtype=np.int32)
+
+
+def marker_style(nj, dotsize=3, mask_threshold=0.1, colors=None, scale_x=1.0, scale_y=1.0, edges=None,
+                 skeleton_color=(0, 0, 0), trailpoints=0, history=0):
+    """(dgp_marker_style, tables) of a drawing call; the tables must stay alive while the style is in use.  ``colors``:
+    None (the 'cool' table), a colormap name, or an (nj, 3) table of values in [0, 255].  ``edges``: joint index pairs
+    joined by a line in ``skeleton_color`` (an RGB triple); ``trailpoints`` K >= 2 also paints each joint's discs of the
+    K - 1 previous frames; ``history``: rows before the first frame in the coordinate tables (dgp_draw_markers), at most
+    K - 1.  ValueError for a dotsize outside [0, 64], a table of another shape, a bad edge, K outside [0, 64] or a bad
+    history."""
+    _check_int("dotsize", dotsize, 0, MAX_DOTSIZE)
     if colors is None or isinstance(colors, str):
         table = marker_colors(nj, "cool" if colors is None else colors)
     else:
@@ -96,8 +124,16 @@ def marker_style(nj, dotsize=3, mask_threshold=0.1, colors=None, scale_x=1.0, sc
         if arr.shape != (int(nj), 3) or not (np.issubdtype(arr.dtype, np.integer) and arr.min() >= 0 and arr.max() <= 255):
             raise ValueError("colors must be an (%d, 3) table of RGB values in [0, 255], got %s %s" % (nj, arr.dtype, arr.shape))
         table = np.ascontiguousarray(arr, dtype=np.uint8)
-    st = _lib.DgpMarkerStyle(int(dotsize), float(mask_threshold), float(scale_x), float(scale_y), table.ctypes.data)
-    return st, table
+    edge_table = skeleton_edges(nj, edges)
+    sk = np.asarray(skeleton_color)
+    if sk.shape != (3,) or not (np.issubdtype(sk.dtype, np.integer) and sk.min() >= 0 and sk.max() <= 255):
+        raise ValueError("skeleton_color must be an RGB triple of integers in [0, 255], got %r" % (skeleton_color,))
+    K = _check_int("trailpoints", trailpoints, 0, MAX_TRAILPOINTS)
+    hist = _check_int("history", history, 0, max(K - 1, 0))
+    st = _lib.DgpMarkerStyle(int(dotsize), float(mask_threshold), float(scale_x), float(scale_y), table.ctypes.data,
+                             edge_table.ctypes.data if len(edge_table) else None, len(edge_table),
+                             (C.c_uint8 * 3)(*(int(v) for v in sk)), K, hist)
+    return st, (table, edge_table)
 
 
 def check_jpeg_quality(quality):
@@ -466,24 +502,29 @@ class Engine:
                                                               float(gauss_len), _ptr(mu), _ptr(peak), _ptr(lik)))
         return mu, peak, lik
 
-    def draw_markers(self, frames_dev, x, y, lik, dotsize=3, mask_threshold=0.1, colors=None):
+    def draw_markers(self, frames_dev, x, y, lik, dotsize=3, mask_threshold=0.1, colors=None, edges=None,
+                     skeleton_color=(0, 0, 0), trailpoints=0, history=0):
         """plot_dgp's markers drawn into ``frames_dev`` (uint8 contiguous CUDA (N,H,W,3) RGB, modified in place;
         dgp_draw_markers): joint j of frame t where ``lik[t, j] > mask_threshold``, a disc of radius ``dotsize`` at the
-        video-pixel coordinates ``x[t, j]``, ``y[t, j]`` in ``colors[j]`` (see ``marker_style``).  ``x``, ``y``, ``lik``:
-        (N, nj) float64 CUDA tensors, or host arrays (uploaded).  Asynchronous on the current stream."""
+        video-pixel coordinates ``x[t, j]``, ``y[t, j]`` in ``colors[j]`` (see ``marker_style``); with ``edges`` a line
+        in ``skeleton_color`` per edge under the discs, with ``trailpoints`` K >= 2 the discs of the K - 1 previous frames
+        under both (the contract is in include/dgp_b200.h).  ``x``, ``y``, ``lik``: (history + N, nj) float64 CUDA
+        tensors, or host arrays (uploaded), whose first ``history`` rows are the frames before ``frames_dev[0]``.
+        Asynchronous on the current stream."""
         if frames_dev.dtype != torch.uint8 or frames_dev.dim() != 4 or frames_dev.shape[-1] != 3 or not frames_dev.is_cuda:
             raise ValueError("frames must be a uint8 CUDA tensor of shape (N,H,W,3)")
         if not frames_dev.is_contiguous():
             raise ValueError("frames must be contiguous: markers are drawn in place")
         N, H, W, _ = frames_dev.shape
-        st, table = marker_style(self.nj, dotsize, mask_threshold, colors)
+        st, table = marker_style(self.nj, dotsize, mask_threshold, colors, edges=edges, skeleton_color=skeleton_color,
+                                 trailpoints=trailpoints, history=history)
         cols = []
         for v in (x, y, lik):
             if not isinstance(v, torch.Tensor):
                 v = torch.from_numpy(np.ascontiguousarray(np.asarray(v, dtype=np.float64)))
             v = v.to(device=frames_dev.device, dtype=torch.float64).contiguous()
-            if tuple(v.shape) != (N, self.nj):
-                raise ValueError("x, y and lik must be (%d, %d)" % (N, self.nj))
+            if tuple(v.shape) != (int(history) + N, self.nj):
+                raise ValueError("x, y and lik must be (%d, %d)" % (int(history) + N, self.nj))
             cols.append(v)
         self._check(self.lib.dgp_draw_markers(self.h, _ptr(frames_dev), N, H, W, _ptr(cols[0]), _ptr(cols[1]), _ptr(cols[2]),
                                               C.byref(st), _stream(frames_dev.device)))
@@ -583,7 +624,7 @@ class Engine:
 
     def estimate_pose_render_stream(self, source, H, W, max_frames, writer, dotsize=3, mask_threshold=0.1, colors=None,
                                     new_size=None, crop_size=None, batch=16, gamma=1.0, gauss_len=1.0, start=0, encoder="raw",
-                                    quality=90):
+                                    quality=90, edges=None, skeleton_color=(0, 0, 0), trailpoints=0):
         """estimate_pose_stream that renders plot_dgp's labelled video in the same pass (dgp_estimate_pose_stream_render):
         after each batch's soft-argmax the markers are drawn on the device into the batch's source frames (coordinates
         converted to video pixels as eval.estimate_pose does, scale W / new_size[1], H / new_size[0] under ``new_size``) and
@@ -593,7 +634,8 @@ class Engine:
         ``encoder="jpeg"`` (dgp_estimate_pose_stream_render_jpeg) encodes the annotated frames on the device instead, as
         encode_jpeg does at ``quality``, and calls ``writer(data, sizes)``: a uint8 array holding the batch's JPEG files back
         to back in video order and an int64 array of their sizes, both valid only during the call.
-        Sources and return value as in estimate_pose_stream; style arguments as in draw_markers."""
+        Sources and return value as in estimate_pose_stream; style arguments as in draw_markers.  Trails reach back to the
+        first frame of the call across batches, so the frames do not depend on ``batch``."""
         if encoder not in ("raw", "jpeg"):
             raise ValueError("encoder must be 'raw' or 'jpeg', got %r" % (encoder,))
         q = check_jpeg_quality(quality)
@@ -603,7 +645,7 @@ class Engine:
         transform_dims(H, W, new_size, crop_size)
         tf = frame_transform(new_size, crop_size)
         sx, sy = (1.0, 1.0) if new_size is None else (W / new_size[1], H / new_size[0])
-        st, table = marker_style(self.nj, dotsize, mask_threshold, colors, sx, sy)
+        st, table = marker_style(self.nj, dotsize, mask_threshold, colors, sx, sy, edges, skeleton_color, trailpoints)
         if not callable(writer):
             raise ValueError("writer must be callable")
         mu = torch.empty((T, self.nj, 2), dtype=torch.float32).pin_memory()

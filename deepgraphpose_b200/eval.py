@@ -287,7 +287,34 @@ def _load_dlc_cfg(proj_cfg_file):
     import yaml
     with open(proj_cfg_file, "r") as stream:
         proj = yaml.safe_load(stream)
-    return {"num_joints": len(proj["bodyparts"]), "all_joints_names": list(proj["bodyparts"]), "stride": 8.0}
+    return {"num_joints": len(proj["bodyparts"]), "all_joints_names": list(proj["bodyparts"]), "stride": 8.0,
+            "skeleton": proj.get("skeleton") or []}
+
+
+def skeleton_from_cfg(dlc_cfg):
+    """The (n, 2) joint index pairs of a dlc_cfg's ``skeleton``: pairs of bodypart names (a DLC project's config.yaml,
+    mapped through ``all_joints_names``, its ``bodyparts``) or of joint indices.  ValueError for no skeleton, an unknown
+    name or a malformed pair."""
+    skel = _cfg_get(dlc_cfg, "skeleton") if dlc_cfg is not None else None
+    if not skel:
+        raise ValueError("draw_skeleton needs a 'skeleton' in the project config (pairs of bodypart names)")
+    names = list(_cfg_get(dlc_cfg, "all_joints_names") or [])
+    edges = []
+    for pair in skel:
+        if isinstance(pair, (str, bytes)) or len(pair) != 2:
+            raise ValueError("skeleton entries must be pairs, got %r" % (pair,))
+        e = []
+        for v in pair:
+            if isinstance(v, str):
+                if v not in names:
+                    raise ValueError("skeleton bodypart %r is not one of the bodyparts %s" % (v, names))
+                e.append(names.index(v))
+            elif isinstance(v, (int, np.integer)) and not isinstance(v, bool):
+                e.append(int(v))
+            else:
+                raise ValueError("skeleton entries must be bodypart names or joint indices, got %r" % (pair,))
+        edges.append(e)
+    return np.asarray(edges, dtype=np.int64).reshape(-1, 2)
 
 
 def _save_labels(labels, dlc_cfg, dgp_model_file, save_file):
@@ -356,7 +383,8 @@ def _mjpeg_writer(filename, fps, H, W):
 
 
 def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colormap="cool", filename="movie.mp4", fps=None,
-                           fourcc="mp4v", batch=16, engine=None, encoder="cv2", quality=90):
+                           fourcc="mp4v", batch=16, engine=None, encoder="cv2", quality=90, skeleton=None,
+                           skeleton_color=(0, 0, 0), trailpoints=0):
     """plot_dgp's renderer (src/deepgraphpose/models/eval.py): a video of ``clip`` with joint j of frame t marked by a disc
     of radius ``dotsize`` at (``df_x[t, j]``, ``df_y[t, j]``) (video pixels) where ``mask_array[t, j]`` (None: every joint),
     coloured by ``colormap`` (the name 'cool' or an (nj, 3) uint8 RGB table) -- the drawing contract of dgp_draw_markers.
@@ -366,7 +394,9 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
     the decoder yields is written, one label row per frame.  The reference writes ``int(duration * fps)`` frames with
     moviepy (libx264) and draws with matplotlib / skimage on the host; bitstream and anti-aliasing parity are not goals.
     ``encoder="jpeg"`` encodes the drawn frames on the device instead (Engine.encode_jpeg at ``quality``) and writes them
-    to ``filename`` as Motion-JPEG (deepgraphpose_b200.mp4); ``fourcc`` is then unused."""
+    to ``filename`` as Motion-JPEG (deepgraphpose_b200.mp4); ``fourcc`` is then unused.
+    ``skeleton`` (joint index pairs) joins the joints of each pair by a line in ``skeleton_color`` (RGB) where both are
+    marked; ``trailpoints`` K >= 2 also marks each joint in the K - 1 previous frames, counted from the first label row."""
     x = np.asarray(df_x, dtype=np.float64)
     y = np.asarray(df_y, dtype=np.float64)
     if x.ndim != 2 or y.shape != x.shape:
@@ -375,7 +405,9 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
     mask = np.ones(x.shape, np.float64) if mask_array is None else np.asarray(mask_array, dtype=bool).astype(np.float64)
     if mask.shape != x.shape:
         raise ValueError("mask_array must be (T, nj) like df_x")
-    marker_style(nj, dotsize, 0.5, colormap)  # validates dotsize and colours before any decode or device work
+    # validates the style before any decode or device work
+    marker_style(nj, dotsize, 0.5, colormap, edges=skeleton, skeleton_color=skeleton_color, trailpoints=trailpoints)
+    trail = max(int(trailpoints) - 1, 0)
     _check_encoder(encoder, fourcc, quality)
     if isinstance(clip, (str, os.PathLike)):
         if fps is None:
@@ -412,7 +444,9 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
                 vw = (_mjpeg_writer(filename, fps, host.shape[1], host.shape[2]) if encoder == "jpeg"
                       else _video_writer(filename, fourcc, fps, host.shape[1], host.shape[2]))
             dev = host.to(eng.device)
-            eng.draw_markers(dev, x[t0:t0 + n], y[t0:t0 + n], mask[t0:t0 + n], dotsize, 0.5, colormap)
+            hist = min(trail, t0)   # the previous batches' last rows, for the trails
+            eng.draw_markers(dev, x[t0 - hist:t0 + n], y[t0 - hist:t0 + n], mask[t0 - hist:t0 + n], dotsize, 0.5, colormap,
+                             skeleton, skeleton_color, trailpoints, hist)
             if encoder == "jpeg":
                 for packet in eng.encode_jpeg(dev, quality):
                     vw.write(packet)
@@ -429,7 +463,7 @@ def create_annotated_movie(clip, df_x, df_y, mask_array=None, dotsize=3, colorma
 
 def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_model_file=None, shuffle=1, dotsize=3,
              colormap="cool", save_str="", mask_threshold=0.1, new_size=None, crop_size=None, batch=16, fourcc="mp4v",
-             encoder="cv2", quality=90):
+             encoder="cv2", quality=90, draw_skeleton=False, skeleton_color=(0, 0, 0), trailpoints=0):
     """plot_dgp (src/deepgraphpose/models/eval.py; step 3 of the reference demo): labels a video and renders the labelled
     movie ``<output_dir>/<video>_labeled<save_str>.mp4`` (cv2.VideoWriter with ``fourcc`` at the source fps) in which joint j
     is a disc of radius ``dotsize`` in ``colormap``'s colour j wherever its likelihood exceeds ``mask_threshold``.
@@ -446,7 +480,10 @@ def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_
     reference's as recorded in this project (dotsize 3, 'cool', mask_threshold 0.1); they have not been checked against a
     reference checkout.  Returns the movie's path.
     ``encoder="jpeg"`` writes the same path as Motion-JPEG at ``quality`` (Pillow's JPEG quality), encoded on the device
-    in both branches, so that only the encoded bytes reach the host; the csv is the same."""
+    in both branches, so that only the encoded bytes reach the host; the csv is the same.
+    ``draw_skeleton`` joins the joints of each ``skeleton`` edge of the project config (pairs of bodypart names, or of
+    joint indices in a dict-like dlc_cfg) by a line in ``skeleton_color`` (RGB); ``trailpoints`` K >= 2 also marks each
+    joint in the K - 1 previous frames.  Both branches draw the same frames."""
     if not isinstance(video_file, (str, os.PathLike)):
         raise ValueError("video_file must be a path")
     _check_encoder(encoder, fourcc, quality)
@@ -458,20 +495,22 @@ def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_
         print("labeled video already exists: %s" % movie)
         return movie
     dlc_cfg = _load_dlc_cfg(proj_cfg_file) if proj_cfg_file is not None else None
+    skeleton = skeleton_from_cfg(dlc_cfg) if draw_skeleton else None
+    overlay = {"skeleton_color": skeleton_color, "trailpoints": trailpoints}
     if os.path.exists(csv):
         labels = load_pose_from_dlc_to_dict(csv)
-        marker_style(labels["x"].shape[1], dotsize, mask_threshold, colormap)
+        marker_style(labels["x"].shape[1], dotsize, mask_threshold, colormap, edges=skeleton, **overlay)
         return create_annotated_movie(video_file, labels["x"], labels["y"], labels["likelihoods"] > mask_threshold,
                                       dotsize=dotsize, colormap=colormap, filename=movie, fourcc=fourcc, batch=batch,
-                                      encoder=encoder, quality=quality)
+                                      encoder=encoder, quality=quality, skeleton=skeleton, **overlay)
     if dlc_cfg is None:
         raise ValueError("no labels at %s: proj_cfg_file and dgp_model_file are needed to estimate them" % csv)
-    marker_style(int(_cfg_get(dlc_cfg, "num_joints")), dotsize, mask_threshold, colormap)
+    marker_style(int(_cfg_get(dlc_cfg, "num_joints")), dotsize, mask_threshold, colormap, edges=skeleton, **overlay)
     import cv2
     cap = cv2.VideoCapture(str(video_file))
     fps = cap.get(cv2.CAP_PROP_FPS)
     cap.release()
-    source, H0, W0, _, scale_x, scale_y = _video_source(video_file, new_size)
+    source, H0, W0, count, scale_x, scale_y = _video_source(video_file, new_size)
     sess = _setup_eval_graph(dlc_cfg, dgp_model_file, None)[0]
     eng = sess.engine
     if encoder == "jpeg":
@@ -480,13 +519,16 @@ def plot_dgp(video_file, output_dir="", label_dir=None, proj_cfg_file=None, dgp_
     else:
         vw = _video_writer(movie, fourcc, fps, H0, W0)
         write, close = (lambda fr: _write_rgb(vw, fr)), vw.release
-    parts, chunk = [], 65536
+    # one call covers the whole video unless the container under-reports its frame count by more than the margin; trails
+    # restart at a call boundary
+    parts, chunk = [], max(65536, (count or 0) + 4096)
     try:
         it = iter(source)
         while True:
             mu, peak, lik = eng.estimate_pose_render_stream(it, H0, W0, chunk, write, dotsize, mask_threshold, colormap,
                                                             new_size, crop_size, batch,
-                                                            encoder="raw" if encoder == "cv2" else "jpeg", quality=quality)
+                                                            encoder="raw" if encoder == "cv2" else "jpeg", quality=quality,
+                                                            edges=skeleton, **overlay)
             parts.append((mu, peak, lik))
             if mu.shape[0] < chunk:
                 break

@@ -362,16 +362,33 @@ int dgp_cyclic_reader(void* user, uint8_t* slot, int max_frames, const uint8_t**
  * xc = min(trunc(x), W - 1), yc = min(trunc(y), H - 1) in double (truncation toward zero, negative centres kept, +inf
  * clamps to the last row / column); the disc is every pixel (r, c) of the frame with (r - yc)^2 + (c - xc)^2 < dotsize^2 in
  * integers, painted colors[j].  Joints are drawn in index order (where discs overlap the higher index wins); pixels outside
- * every disc keep their bytes.  dotsize in [0, 64] (0 draws nothing). */
+ * every disc keep their bytes.  dotsize in [0, 64] (0 draws nothing).
+ * Skeleton and trails (zero-initialised fields draw neither).  Frame t is painted in this order:
+ *  1. trails, when trailpoints = K >= 2: for k = K-1 down to 1, and within each k for j = 0..nj-1, the disc of joint j of
+ *     frame t-k by the rule above (dotsize, colors[j], the mask of frame t-k's own lik); frames t-k < 0 are skipped.  Frame
+ *     indices count from the first frame of the call (in dgp_draw_markers, from its first history row).  K in [0, 64].
+ *  2. skeleton: for each edge (a, b) in the order given, a line in skeleton_color, drawn iff both joints of frame t pass the
+ *     mask, their x and y are finite and both centres (xc, yc above) are >= -2^20.  With dr = yc_b - yc_a, dc = xc_b - xc_a,
+ *     n = max(|dr|, |dc|), the line is the pixels k = 0..n with r = yc_a + floor((2 k dr + n) / 2n),
+ *     c = xc_a + floor((2 k dc + n) / 2n) (integer floor division; n = 0 is one pixel), those inside the frame written.  At
+ *     most 256 edges, joints in [0, nj); frames with an edge are at most 2^30 pixels high and wide.
+ *  3. the discs of frame t, as without an overlay, so that they stay on top.
+ * With no edges and K <= 1 the bytes are those of the markers alone. */
 typedef struct dgp_marker_style {
   int32_t dotsize;
   double mask_threshold;
   double scale_x, scale_y;  /* fused pass only: soft-argmax coordinates -> video pixels (W0 / new_w, H0 / new_h, else 1) */
   const uint8_t* colors;    /* host (nj,3) RGB, nj = the handle's num_joints */
+  const int32_t* edges;     /* host (n_edges,2) joint index pairs of the skeleton */
+  int32_t n_edges;
+  uint8_t skeleton_color[3];
+  int32_t trailpoints;      /* K: frames of a joint's trail, the current one included (0 or 1: no trail) */
+  int32_t history;          /* dgp_draw_markers only: rows before frames_dev[0] in x_dev / y_dev / lik_dev, <= K - 1 */
 } dgp_marker_style;
-/* Draws the markers of x_dev, y_dev, lik_dev (float64 (N,nj) on the device) into frames_dev (N,H,W,3) in place; `scale_x`
- * and `scale_y` are not used (the coordinates are video pixels already).  Asynchronous on `stream`; the colour table
- * travels as a kernel argument.  The render-only entry, for labels that already exist (a DLC csv). */
+/* Draws the markers of x_dev, y_dev, lik_dev (float64 (history + N, nj) on the device; row history + t is frame t of
+ * frames_dev, the first `history` rows are the frames before it) into frames_dev (N,H,W,3) in place; `scale_x` and
+ * `scale_y` are not used (the coordinates are video pixels already).  Asynchronous on `stream`; the colour and edge tables
+ * travel as kernel arguments.  The render-only entry, for labels that already exist (a DLC csv). */
 int dgp_draw_markers(dgp_handle* h, uint8_t* frames_dev, int N, int H, int W, const double* x_dev, const double* y_dev,
                      const double* lik_dev, const dgp_marker_style* style, void* stream);
 /* writer(user, frames, n): n uint8 (H0,W0,3) RGB annotated frames, valid only during the call; return < 0 to abort.  Called
@@ -380,8 +397,9 @@ typedef int (*dgp_frame_writer)(void* user, const uint8_t* frames, int n);
 /* dgp_estimate_pose_stream_transform that also renders the labelled video in the same pass: per batch, after the
  * soft-argmax, the markers of x = ((double)mu[..,1] * stride + 0.5 * stride) * scale_x, y likewise with mu[..,0] and
  * scale_y, and lik are drawn into the batch's (H0,W0) source frames on the device (stride = the handle's, as a double),
- * the n real frames are copied into a ring of 3 pinned writer slots and handed to `writer` on a writer thread.  Read-outs
- * as in dgp_estimate_pose_stream_transform.  A failing writer aborts the call like a failing reader (DGP_ERR_INVALID). */
+ * the n real frames are copied into a ring of 3 pinned writer slots and handed to `writer` on a writer thread.  Trails
+ * reach back across batches to the first frame of the call, so the frames do not depend on `batch`.  Read-outs as in
+ * dgp_estimate_pose_stream_transform.  A failing writer aborts the call like a failing reader (DGP_ERR_INVALID). */
 int dgp_estimate_pose_stream_render(dgp_handle* h, dgp_frame_reader reader, void* user, int H0, int W0,
                                     const dgp_frame_transform* transform, int batch, float gamma, float gauss_len,
                                     int64_t max_frames, float* mu_host, int32_t* peak_host, float* lik_host,
